@@ -14,6 +14,7 @@ prediction + dynamics, expand, backup}, action sampling, environment step and hi
   learner    learner samples/s (get_batch gather + K-step unroll forward + loss + gradients + allreduce + ADAM)
 
 `--impl reference` times the reference's CPU path instead (the oracle port: Julia is not available in this image).
+`--dump-outputs DIR` writes every GameHistory of the last timed wave as DIR/<name>.npy, so that two builds can be compared output for output.
 """
 import argparse
 import json
@@ -23,6 +24,7 @@ import sys
 import threading
 import time
 
+sys.dont_write_bytecode = True                                            # the tree may be read-only: no __pycache__ beside the sources
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
@@ -55,7 +57,14 @@ def parse():
     ap.add_argument("--connect-games", type=int, default=1776)
     ap.add_argument("--connect-sims", type=int, default=200)
     ap.add_argument("--no-parity-check", action="store_true", help="skip the comparison of the last timed wave with the oracle")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write every GameHistory of the last timed wave (rank 0), in game-id order, and its simulation "
+                                                          "and move counts as DIR/<name>.npy (float32 / float64)")
+    a = ap.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if a.dump_outputs and a.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of --impl b200")
+    return a
 
 
 def workload_name(a):
@@ -132,6 +141,25 @@ def cpu_self_play_rate(ocfg, blob, games, threads, first_game=10 ** 6):
     h = O.self_play(ocfg, blob, first_game, games, 1.0, threads)
     dt = time.perf_counter() - t0
     return h["sims"] / dt, h["sims"], dt
+
+
+def dump_outputs(out_dir, ctx, n_games, sims, moves, max_bytes=64 * 10 ** 6):
+    """What a caller of the timed self_play wave receives: its simulation and move counts and the GameHistory of each of its games
+    (what save_game stores, read back with history_export), sorted by game id.  Integer arrays are written as float64 (exact).  When
+    the histories exceed `max_bytes`, a fixed seeded sample of the games is written (game_id.npy says which)."""
+    info = ctx.replay_info()
+    h = ctx.history_export(key0=info["first_key"] + info["n_games"] - n_games, n=n_games)
+    h = {k: v if v.dtype == np.float32 else v.astype(np.float64) for k, v in h.items()}
+    order = np.argsort(h["game_id"], kind="stable")
+    per_game = sum(v[0].nbytes for v in h.values())
+    budget = max_bytes - 4096                                             # .npy headers
+    if n_games * per_game > budget:
+        order = order[np.sort(np.random.default_rng(0).choice(n_games, budget // per_game, replace=False))]
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in h.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v[order])
+    np.save(os.path.join(out_dir, "simulations.npy"), np.array([sims], np.float64))
+    np.save(os.path.join(out_dir, "moves.npy"), np.array([moves], np.float64))
 
 
 def profiled_traffic(kernel_tag):
@@ -281,6 +309,8 @@ def run_b200(a):
         ctx.kernel_time_reset(False)
         clocks = sampler.stop()
         stats = ctx.search_stats()
+        if a.dump_outputs and rank == 0:
+            dump_outputs(a.dump_outputs, ctx, G, s, m)
         # ---- parity of what was just timed: every GameHistory of the last timed wave against the oracle (outside the timed region) ----
         def compare_with_oracle(c_, last_first_game):
             """Every GameHistory of the wave that started at `last_first_game` against the Float32 oracle."""
