@@ -656,7 +656,7 @@ int mz_create(const mz_config *cfg, int device, mz_ctx **out) {
             mz_sp_args &A = c->spa;
             A.image = c->d_w_sp; A.bias = c->d_bias_sp; A.rounds = c->d_rounds_sp;
             for (int n = 0; n < 3; n++) { A.first[n] = S.first[n]; A.n_rounds[n] = S.n_rounds[n]; A.set_first[n] = S.set_first[n]; A.n_sets[n] = S.n_sets[n]; }
-            A.total_rounds = S.total_rounds; A.total_sets = S.total_sets; A.warea_bytes = S.warea_bytes; A.bias_floats = S.bias_floats; A.pbc_smem = S.pbc_smem;
+            A.total_rounds = S.total_rounds; A.total_sets = S.total_sets; A.warea_bytes = S.warea_bytes; A.bias_floats = S.bias_floats; A.pbc_smem = S.pbc_smem; A.tail = S.tail;
             // the learner's backward rounds on the same machinery
             mzh::build_lr_plan(P, S, c->lrp);
             c->smem_bytes_lr = mz_lr_smem_bytes(S.warea_bytes, S.bias_floats, S.total_rounds, c->lrp.btotal_rounds, P.hidden_pad);
@@ -960,7 +960,7 @@ int mz_run_mcts(mz_ctx *c, int n, const float *stacked_obs, const uint32_t *lega
             launch_scope ls(c, 0); mz_k_search_rn<MZ_MODE_API><<<(m + nt - 1) / nt, MZ_RN_THREADS, c->smem_bytes_rn, c->stream>>>(P, c->rn.R, t);
         } else if (c->cfg.nn_mode == MZ_NN_SPLIT_MMA) {
             mz_search_sp_args t{}; t.base = a; t.sp = c->spa;
-            launch_scope ls(c, 0); mz_k_search_sp<MZ_MODE_API><<<(m + MZ_ROWS - 1) / MZ_ROWS, MZ_SP_THREADS, c->smem_bytes_sp, c->stream>>>(P, t);
+            launch_scope ls(c, 0); mz_k_search_sp<MZ_MODE_API><<<(m + MZ_ROWS - 1) / MZ_ROWS, MZ_SP_SEARCH_THREADS, c->smem_bytes_sp, c->stream>>>(P, t);
         } else if (c->cfg.nn_mode == MZ_NN_BF16_TC) {
             mz_search_tc_args t{}; t.base = a; t.w_image = c->d_w_tc; t.bias = c->d_bias_tc;
             launch_scope ls(c, 0); mz_k_search_tc<MZ_MODE_API><<<(m + MZ_ROWS - 1) / MZ_ROWS, MZ_THREADS, c->smem_bytes_tc, c->stream>>>(P, t);
@@ -1087,7 +1087,7 @@ static int run_wave_body(mz_ctx *c, uint64_t first_game, int64_t n_games, float 
     // the end, in slot order (= game id order).  MUZERO_B200_PERSIST=0 keeps one launch per move.
     if (overlap && !use_lat && arena_player == 0 && c->cfg.net_type == MZ_NET_FEEDFORWARD && c->cfg.nn_mode == MZ_NN_SPLIT_MMA && c->persist_ok) {
         mz_search_sp_args t{}; t.base = a; t.base.persist = 1; t.sp = c->spa;
-        { launch_scope ls(c, 0); mz_k_search_sp<MZ_MODE_SLOTS><<<(G + MZ_ROWS - 1) / MZ_ROWS, MZ_SP_THREADS, c->smem_bytes_sp, c->stream>>>(P, t); }
+        { launch_scope ls(c, 0); mz_k_search_sp<MZ_MODE_SLOTS><<<(G + MZ_ROWS - 1) / MZ_ROWS, MZ_SP_SEARCH_THREADS, c->smem_bytes_sp, c->stream>>>(P, t); }
         MZ_TRY(launch_save_refill(c, P, G, tally, c->d_wave + 8));
         MZ_CUDA(c, cudaGetLastError());
         MZ_CUDA(c, cudaMemcpyAsync(c->h_stats, c->d_stats, 64 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, c->stream));
@@ -1114,7 +1114,7 @@ static int run_wave_body(mz_ctx *c, uint64_t first_game, int64_t n_games, float 
             launch_scope ls(c, 0); mz_k_search_rn<MZ_MODE_SLOTS><<<(G + nt - 1) / nt, MZ_RN_THREADS, c->smem_bytes_rn, c->stream>>>(P, c->rn.R, t);
         } else if (c->cfg.nn_mode == MZ_NN_SPLIT_MMA) {
             mz_search_sp_args t{}; t.base = a; t.sp = c->spa;
-            launch_scope ls(c, 0); mz_k_search_sp<MZ_MODE_SLOTS><<<(G + MZ_ROWS - 1) / MZ_ROWS, MZ_SP_THREADS, c->smem_bytes_sp, c->stream>>>(P, t);
+            launch_scope ls(c, 0); mz_k_search_sp<MZ_MODE_SLOTS><<<(G + MZ_ROWS - 1) / MZ_ROWS, MZ_SP_SEARCH_THREADS, c->smem_bytes_sp, c->stream>>>(P, t);
         } else if (c->cfg.nn_mode == MZ_NN_BF16_TC) {
             mz_search_tc_args t{}; t.base = a; t.w_image = c->d_w_tc; t.bias = c->d_bias_tc;
             launch_scope ls(c, 0); mz_k_search_tc<MZ_MODE_SLOTS><<<(G + MZ_ROWS - 1) / MZ_ROWS, MZ_THREADS, c->smem_bytes_tc, c->stream>>>(P, t);

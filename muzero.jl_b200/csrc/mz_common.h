@@ -210,13 +210,14 @@ struct mz_sp_plan {
     int32_t set_first[3], n_sets[3];                // per network: its weight sets (the representation has one, loaded once, over the dynamics area)
     int32_t total_rounds, total_sets;
     int32_t image_bytes, warea_bytes, bias_floats, divisor, ok, pbc_smem;
-    int32_t out_off[4];                             // float offsets of value / logits / reward / hidden outputs in the output area
+    int32_t tail;                                   // trailing rounds of the dynamics network without a reward job (the state head alone)
+    int32_t out_off[4];                            // float offsets of value / logits / reward / hidden outputs in the output area
     int32_t w_off[MZ_MAX_LAYERS], w_bytes[MZ_MAX_LAYERS];   // image: hi block at w_off, lo block at w_off + w_bytes
     mz_sp_round round[MZ_SP_MAX_ROUNDS];
 };
 
 #define MZ_SP_RDESC_BYTES 128                       // sizeof(mz_sp_rdesc), the device form of a round (mz_sp.cuh)
-#define MZ_SP_CTRL_BYTES 1024                       // mbarriers, TMEM slot, per-set use counters
+#define MZ_SP_CTRL_BYTES 1024                       // mbarriers, TMEM slot, active-tree flags
 // dynamic shared memory of a kernel on this path (the carve-up is mz_sp_carve in mz_sp.cuh)
 // pbc_smem: the kernel keeps a compact copy of ucb_score's Float64 table (rows N = 0..S+1, entries n = 0..N) in shared memory
 MZ_HD size_t mz_sp_smem_bytes(int warea_bytes, int bias_floats, int total_rounds, int hidden_pad, int S, int pbc_smem) {

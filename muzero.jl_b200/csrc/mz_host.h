@@ -376,6 +376,11 @@ inline void build_sp_plan(const mz_params &P, size_t smem_limit, mz_sp_plan &S) 
     sp_build_net(P, S, 1, S.out_off[0], S.out_off[1]);
     sp_build_net(P, S, 2, S.out_off[3], S.out_off[2]);
     if (!S.ok) return;
+    // the dynamics rounds after the reward is final: with the heads side by side, the state head's last n_h1 - n_h2 layers.  Nothing
+    // but the next simulation's staging reads their output, so mz_k_search_sp runs them beside the tree phases.  Heads one after the
+    // other end with the reward head: no tail.
+    const mz_net &D = P.nets[2];
+    S.tail = D.n_h1 > 0 && D.n_h2 > 0 && D.n_h2 <= 2 && D.n_h2 <= D.n_h1 ? D.n_h1 - D.n_h2 : 0;
     // smallest divisor d (sets per network = ceil(rounds / d)) whose weight area fits; d = 1 keeps every weight resident
     for (int d = 1; d <= MZ_SP_MAX_ROUNDS; d++) {
         const int np = (S.n_rounds[1] + d - 1) / d, nd = (S.n_rounds[2] + d - 1) / d;

@@ -2,6 +2,8 @@
 // near-Float32 accuracy (nn_mode = MZ_NN_SPLIT_MMA, mz_sp.cuh: bf16 hi / lo split of both operands, fp32 accumulation in TMEM).  Tree
 // phases, move epilogue and data layout are the ones of mz_k_search; group 0 (threads 0..127) runs prediction(parent), group 1 the
 // representation (at the root) and dynamics(parent, a), concurrently (SURVEY Q5), each with its own weight sets and TMEM columns.
+// The dynamics rounds after the reward is final (the state head alone) and the hidden-state write run on a tail team of warps beside
+// expand, backup and the next selection (DESIGN.md 2.1c).
 #pragma once
 #include "mz_kernels.cuh"
 #include "mz_sp.cuh"
@@ -52,8 +54,30 @@ __device__ __forceinline__ void mz_sp_drain(const mz_sp_ctx &C, const mz_sp_args
 }
 __device__ __forceinline__ uint32_t mz_sp_group_tile(const mz_sp_plan_s &sp, int grp, int tile) { return sp.tiles + (uint32_t)((grp * MZ_SP_TILES_PER_GROUP + tile) * 2 * MZ_SP_TILE_BYTES); }
 
+// the tail team, once per simulation: the tail rounds (mz_sp_run_tail), then the new hidden state of every active tree -> tree.hidden[sim]
+// (8 threads per tree, as the tree phases; two trees per thread), then the "tail done" arrival that the workers wait for before staging
+__device__ __forceinline__ uint32_t mz_sp_tail(const mz_params &P, const mz_search_args &a, const float *outH, const uint8_t *active, const mz_sp_ctx C, int first, int count,
+                                            uint32_t tmem_d, uint32_t mbar, uint32_t q, uint32_t pass, uint32_t bias, int ttid, int sim, uint32_t mbar_tail) {
+#ifdef MZ_PHASE_TIMERS
+    const long long t0_ = clock64();
+#endif
+    q = mz_sp_run_tail(C, first, count, tmem_d, mbar, q, pass, bias, ttid);
+    mz_named_sync(MZ_SP_BAR_TAIL, MZ_SP_TAIL_THREADS);                  // all four quadrants of the last round's outputs are in outH
+    for (int rr = ttid / MZ_LANES; rr < MZ_ROWS; rr += MZ_SP_TAIL_THREADS / MZ_LANES) {
+        if (!active[rr]) continue;
+        float *nh = mz_tree_at(P, a.tree_pool, (int64_t)blockIdx.x * MZ_ROWS + rr).hidden + (size_t)sim * P.hidden_pad;
+        for (int k = ttid & (MZ_LANES - 1); k < P.hidden; k += MZ_LANES) nh[k] = outH[k * MZ_SP_OS + rr];
+    }
+    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(mbar_tail) : "memory");
+#ifdef MZ_PHASE_TIMERS
+    // profiling build: the dynamics issuer's lane 0 times the tail from the end of its chain rounds' issue to "tail done"
+    if (a.stats && ttid == 32) { atomicAdd(&a.stats[59], (unsigned long long)(clock64() - t0_)); atomicAdd(&a.stats[60], 1ull); }
+#endif
+    return q;
+}
+
 template <int MODE>
-__global__ void __launch_bounds__(MZ_SP_THREADS) mz_k_search_sp(const __grid_constant__ mz_params P, const __grid_constant__ mz_search_sp_args sa) {
+__global__ void __launch_bounds__(MZ_SP_SEARCH_THREADS) mz_k_search_sp(const __grid_constant__ mz_params P, const __grid_constant__ mz_search_sp_args sa) {
     extern __shared__ __align__(1024) unsigned char mz_smem_sp[];
     const mz_search_args &a = sa.base;
     const mz_sp_args &A = sa.sp;
@@ -64,17 +88,19 @@ __global__ void __launch_bounds__(MZ_SP_THREADS) mz_k_search_sp(const __grid_con
     const uint32_t segmask = 0xffu << ((tid & 31) & ~7);
     const int64_t g = (int64_t)blockIdx.x * MZ_ROWS + r;
     MZ_KSTAMP_DECL;
-    const uint32_t tmem_base = mz_sp_setup(sp, A, MZ_SP_THREADS);
+    const uint32_t tmem_base = mz_sp_setup(sp, A, MZ_SP_SEARCH_THREADS);
     MZ_KSTAMP(0);
     mz_sp_ctx C; C.prog = mz_smem_u32(sp.prog); C.image = A.image; C.bars = mz_smem_u32(sp.bars);
     const double *pbc = a.pbc0;
     if (A.pbc_smem) {                                                   // compact copy of ucb_score's table: row N holds n = 0..N
-        for (int N = tid; N < P.S + 2; N += MZ_SP_THREADS) for (int n = 0; n <= N; n++) sp.pbc[(N * (N + 1)) / 2 + n] = a.pbc0[N * (P.S + 2) + n];
+        for (int N = tid; N < P.S + 2; N += MZ_SP_SEARCH_THREADS) for (int n = 0; n <= N; n++) sp.pbc[(N * (N + 1)) / 2 + n] = a.pbc0[N * (P.S + 2) + n];
         pbc = sp.pbc;
     }
-    const bool worker = tid < MZ_THREADS;                               // warps 0..7: tree phases + epilogues; warp 8 / 9: issuer of group 0 / 1
-    const int grp = worker ? tid >> 7 : (tid - MZ_THREADS) >> 5, gtid = tid & (MZ_GROUP - 1);
-    const bool issuer0 = !worker && (tid & 31) == 0;                    // lane 0 of an issuer warp: one-off TMA work
+    // warps 0..7: tree phases + epilogues; warp 8 / 9: issuer of group 0 / 1; warps 8..11: the tail team (TMEM lane quadrants 0..3), which
+    // runs the last `tail` dynamics rounds and the hidden-state write beside the tree phases (warps 10, 11 do nothing else)
+    const bool worker = tid < MZ_THREADS, issuer = !worker && tid < MZ_THREADS + 64;
+    const int grp = worker ? tid >> 7 : (tid < MZ_THREADS + 32 ? 0 : 1), gtid = tid & (MZ_GROUP - 1);
+    const bool issuer0 = issuer && (tid & 31) == 0;                     // lane 0 of an issuer warp: one-off TMA work
     if (issuer0) {
         if (grp == 0) mz_sp_prime(C, A, 1);
         else mz_sp_fill_many(C, A.first[0], A.n_rounds[0]);
@@ -120,7 +146,8 @@ __global__ void __launch_bounds__(MZ_SP_THREADS) mz_k_search_sp(const __grid_con
     for (int j = 0; j < P.A; j++) if ((legal >> (P.order[j] - 1)) & 1u) posmask |= 1u << j;
 
     // ---- stage the stacked observations (hi / lo operand tiles of group 1) ----
-    for (int i = tid; i < MZ_ROWS * P.stack_size; i += MZ_SP_THREADS) {
+    if (worker && ln == 0) sp.active[r] = active;                       // for the tail team's hidden-state write
+    for (int i = tid; i < MZ_ROWS * P.stack_size; i += MZ_SP_SEARCH_THREADS) {
         float v = 0.0f; int rr, k;
         if (MODE == MZ_MODE_API) {
             rr = i / P.stack_size; k = i % P.stack_size;
@@ -142,11 +169,11 @@ __global__ void __launch_bounds__(MZ_SP_THREADS) mz_k_search_sp(const __grid_con
     //      group 0 runs prediction(h0) -> (v0, p0) ----
     if (grp == 1) {
         if (worker) q = mz_sp_run(C, A.first[0], A.n_rounds[0], tmem_d, mbar_mma, q, grp, gtid, nullptr);
-        else { q = mz_sp_run_issuer(C, A.first[0], A.n_rounds[0], tmem_d, mbar_mma, q, 0u, grp, nullptr, 0u, ply); if (issuer0) mz_sp_prime(C, A, 2); }
+        else if (issuer) { q = mz_sp_run_issuer(C, A.first[0], A.n_rounds[0], tmem_d, mbar_mma, q, 0u, grp, nullptr, 0u, ply); if (issuer0) mz_sp_prime(C, A, 2); }
     }
     __syncthreads();
     MZ_KSTAMP(2);
-    for (int i = tid; i < MZ_ROWS * P.hidden; i += MZ_SP_THREADS) { const int k = i / MZ_ROWS, rr = i % MZ_ROWS; mz_sp_stage(in_pred, k, rr, sp.outH[k * MZ_SP_OS + rr]); }
+    for (int i = tid; i < MZ_ROWS * P.hidden; i += MZ_SP_SEARCH_THREADS) { const int k = i / MZ_ROWS, rr = i % MZ_ROWS; mz_sp_stage(in_pred, k, rr, sp.outH[k * MZ_SP_OS + rr]); }
     mz_fence_proxy_async();
     __syncthreads();
     if (grp == 0) {
@@ -173,18 +200,28 @@ __global__ void __launch_bounds__(MZ_SP_THREADS) mz_k_search_sp(const __grid_con
     }
 
     MZ_KSTAMP(4);
+    // ---- simulations: the worker warps and the others (issuers, tail team) run separate loops that meet at named barriers ----
+    if (worker) {
     // byte offsets of this lane's staging positions (k = ln + 8 i, tree r) inside an operand tile: the same in every simulation
     uint32_t soff[8];
 #pragma unroll
     for (int i = 0; i < 8; i++) soff[i] = mz_sp_tile_offset(ln + MZ_LANES * i, r & (MZ_ROWS - 1));
-    // ---- simulations ----
     for (int sim = 1; sim <= P.S; sim++) {
         mz_leaf leaf; leaf.node = 0; leaf.parent = 0; leaf.action = 1; leaf.depth = 0; leaf.prior = 0.0f; leaf.parent_x = 0;
         MZ_TIMER(0);
         if (active) {
             leaf = mz_tree_select_lanes(P, tree, pbc, a.sqrtN, legal, posmask, mm, game, move, (uint32_t)sim, ln, segmask, path, A.pbc_smem != 0);
             depth_sum += (unsigned long long)leaf.depth;
-            MZ_TIMER(1);
+        }
+        MZ_TIMER(1);
+        // The tail of the previous simulation (its last dynamics rounds and its hidden-state write) must be done before staging: staging
+        // reads tree.hidden[pe], where pe may be the node that simulation expanded, and overwrites group 1's input tile, which the tail's
+        // rounds may still read.  The next pass's MMAs (TMEM, operand tiles) start after the barrier behind staging, so after this wait
+        // too.  The tail team arrives after tcgen05.wait::ld + tcgen05.fence::before_thread_sync of its last round.  The first
+        // simulation of a move follows CTA-wide barriers that the team joins when its last tail is done.
+        if (A.tail && sim > 1) mz_sp_wait_mma(mz_smem_u32(sp.mbar_tail), (uint32_t)(ply * P.S + sim - 2));
+        MZ_TIMER(6);
+        if (active) {
             const int pe = mz_nx_exp(leaf.parent_x), dbl = mz_nx_dbl(leaf.parent_x);
             const float *h = tree.hidden + (size_t)pe * P.hidden_pad;
             const float sc = mz_bits2f((uint32_t)(127 + dbl) << 23);
@@ -208,20 +245,19 @@ __global__ void __launch_bounds__(MZ_SP_THREADS) mz_k_search_sp(const __grid_con
         }
         mz_fence_proxy_async();
         MZ_TIMER(2);
-        __syncthreads();
+        mz_named_sync(MZ_SP_BAR_SIM, MZ_THREADS + 64);                 // workers + issuers
         MZ_TIMER(3);
-        {
-            const int net = grp == 0 ? 1 : 2;
-            if (worker) q = mz_sp_run(C, A.first[net], A.n_rounds[net], tmem_d, mbar_mma, q, grp, gtid, tk);
-            else q = mz_sp_run_issuer(C, A.first[net], A.n_rounds[net], tmem_d, mbar_mma, q, pass, grp, nullptr, 0u, grp == 1 ? ply : 0u);
-            pass++;
-        }
+        q = mz_sp_run(C, A.first[grp + 1], grp == 0 ? A.n_rounds[1] : A.n_rounds[2] - A.tail, tmem_d, mbar_mma, q, grp, gtid, tk);
+        if (grp == 1 && A.tail) { mz_sp_bar_arrive(1); q += (uint32_t)A.tail; }     // the issuer syncs on it before the tail's first round
+        pass++;
         MZ_TIMER(4);
-        __syncthreads();
+        mz_named_sync(MZ_SP_BAR_WORK, MZ_THREADS);                     // both networks' outputs but the tail's are in place
         MZ_TIMER(5);
         if (active) {
-            float *nh = tree.hidden + (size_t)sim * P.hidden_pad;
-            for (int k = ln; k < P.hidden; k += MZ_LANES) nh[k] = sp.outH[k * MZ_SP_OS + r];
+            if (!A.tail) {
+                float *nh = tree.hidden + (size_t)sim * P.hidden_pad;
+                for (int k = ln; k < P.hidden; k += MZ_LANES) nh[k] = sp.outH[k * MZ_SP_OS + r];
+            }
             MZ_TIMER(6);
             float rw = sp.outR[r], vl = sp.outV[r];
             if (tanh_r || tanh_v) {                                // both tanh side by side: even lanes the value, odd lanes the reward
@@ -239,7 +275,8 @@ __global__ void __launch_bounds__(MZ_SP_THREADS) mz_k_search_sp(const __grid_con
     MZ_KSTAMP(5);
     MZ_TIMER_FLUSH(a.stats);
 #ifdef MZ_PHASE_TIMERS
-    if (a.stats && tk) { int o_ = tid == 0 ? 16 : 24; for (int i_ = 0; i_ < 6; i_++) atomicAdd(&a.stats[o_ + i_], (unsigned long long)rt[i_]); atomicAdd(&a.stats[o_ + 6], (unsigned long long)q); }
+    // rounds timed: the tail's rounds run on the tail team
+    if (a.stats && tk) { int o_ = tid == 0 ? 16 : 24; for (int i_ = 0; i_ < 6; i_++) atomicAdd(&a.stats[o_ + i_], (unsigned long long)rt[i_]); atomicAdd(&a.stats[o_ + 6], (unsigned long long)(q - (tid == 0 ? 0u : (uint32_t)A.tail * pass))); }
 #endif
     // ---- results (lane 0 of each tree), identical to mz_k_search ----
     if (active && ln == 0) {
@@ -262,6 +299,21 @@ __global__ void __launch_bounds__(MZ_SP_THREADS) mz_k_search_sp(const __grid_con
             }
             a.root_value[g] = rv;
         } else mz_slot_epilogue(P, a.slots, g, vc, sum_visits, legal, rv, a.temperature, game, move);
+    }
+    } else {
+    for (int sim = 1; sim <= P.S; sim++) {
+        if (issuer) {
+            mz_named_sync(MZ_SP_BAR_SIM, MZ_THREADS + 64);
+            q = mz_sp_run_issuer(C, A.first[grp + 1], grp == 0 ? A.n_rounds[1] : A.n_rounds[2] - A.tail, tmem_d, mbar_mma, q, pass, grp, nullptr, 0u, grp == 1 ? ply : 0u);
+            pass++;
+        }
+        if (A.tail) {               // the tail team: warp 8 is done with prediction, warp 9 goes on issuing, warps 10, 11 only run tails
+            const uint32_t qt = mz_sp_tail(P, a, sp.outH, sp.active, C, A.first[2] + A.n_rounds[2] - A.tail, A.tail, tmem_base + 128u, mz_smem_u32(sp.mbar_mma[1]),
+                                           issuer && grp == 1 ? q : (uint32_t)((ply + 1) * A.n_rounds[0] + (ply * P.S + sim - 1) * A.n_rounds[2] + A.n_rounds[2] - A.tail),
+                                           pass - 1u, ply, gtid, sim, mz_smem_u32(sp.mbar_tail));
+            if (issuer && grp == 1) q = qt;
+        }
+    }
     }
     if (!persist) break;
     __syncthreads();                                                    // the epilogues' slot updates are visible to the CTA: the next ply starts from them

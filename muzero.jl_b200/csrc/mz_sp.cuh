@@ -24,6 +24,7 @@
 #define MZ_SP_IDESC32 (MZ_TC_IDESC | (1u << 16))                                          // M = 64, N = 32, B operand MN-major (cute::UMMA::InstrDescriptor::b_major_)
 #define MZ_SP_IDESC64 ((MZ_TC_IDESC & ~(0x3fu << 17)) | ((64u >> 3) << 17) | (1u << 16))    // M = 64, N = 64
 #define MZ_SP_TMEM_COLS 256            // two groups x two jobs x (32 + 32) fp32 columns
+#define MZ_SP_TAIL_THREADS 128         // mz_k_search_sp's tail team: warps 8..11, one per TMEM lane quadrant
 
 struct __align__(16) mz_sp_rdesc {                  // device form of mz_sp_round: everything a round needs, shared addresses resolved
     unsigned long long a_hi[2], a_lo[2], b_hi[2];   // words  0..11: UMMA descriptors at k-step 0
@@ -82,6 +83,7 @@ struct mz_sp_plan_s {                               // carve-up of the dynamic s
     unsigned char *tiles_ptr;
     uint64_t *bars;                                 // [MZ_SP_MAX_SETS] weight-set barriers
     uint64_t *mbar_mma[2]; uint32_t *tmem_slot;
+    uint64_t *mbar_tail; uint8_t *active;           // mz_k_search_sp: "tail done" barrier, per-tree active flags of the current move
     float *bias, *outV, *outL, *outR, *outH; double *pbc; uint16_t *path; mz_sp_rdesc *prog;
 };
 __device__ __forceinline__ mz_sp_plan_s mz_sp_carve(unsigned char *raw, int warea_bytes, int bias_floats, int total_rounds, int hidden_pad, int S, int pbc_smem) {
@@ -91,6 +93,7 @@ __device__ __forceinline__ mz_sp_plan_s mz_sp_carve(unsigned char *raw, int ware
     p.w_base = mz_smem_u32(c); c += warea_bytes;
     p.tiles = mz_smem_u32(c); p.tiles_ptr = c; c += 2 * MZ_SP_TILES_PER_GROUP * 2 * MZ_SP_TILE_BYTES;
     p.bars = (uint64_t *)c; p.mbar_mma[0] = (uint64_t *)(c + 8 * MZ_SP_MAX_SETS); p.mbar_mma[1] = p.mbar_mma[0] + 1; p.tmem_slot = (uint32_t *)(c + 8 * MZ_SP_MAX_SETS + 16);
+    p.mbar_tail = (uint64_t *)(c + 8 * MZ_SP_MAX_SETS + 24); p.active = c + 8 * MZ_SP_MAX_SETS + 32;
     c += MZ_SP_CTRL_BYTES;
     p.bias = (float *)c; c += ((size_t)bias_floats * 4 + 127) & ~(size_t)127;
     p.outV = (float *)c; p.outL = p.outV + 4 * MZ_SP_OS; p.outR = p.outV + 20 * MZ_SP_OS; p.outH = p.outV + 24 * MZ_SP_OS; c += (size_t)(24 + hidden_pad) * MZ_SP_OS * 4;
@@ -105,6 +108,7 @@ struct mz_sp_args {                                 // what a kernel on this pat
     const unsigned char *image; const float *bias; const mz_sp_round *rounds;
     int32_t first[3], n_rounds[3], set_first[3], n_sets[3];
     int32_t total_rounds, total_sets, warea_bytes, bias_floats, pbc_smem;
+    int32_t tail;                                   // mz_sp_plan::tail: trailing dynamics rounds that mz_k_search_sp runs off the simulation chain
 };
 
 // one-time set-up by all threads: barriers, TMEM, zeroed tiles, biases, the round table.  Ends with a CTA barrier.
@@ -112,7 +116,7 @@ __device__ __forceinline__ uint32_t mz_sp_setup(const mz_sp_plan_s &sp, const mz
     const int tid = threadIdx.x;
     if (tid == 0) {
         for (int i = 0; i < A.total_sets; i++) mz_mbar_init(&sp.bars[i], 1);
-        mz_mbar_init(sp.mbar_mma[0], 1); mz_mbar_init(sp.mbar_mma[1], 1);
+        mz_mbar_init(sp.mbar_mma[0], 1); mz_mbar_init(sp.mbar_mma[1], 1); mz_mbar_init(sp.mbar_tail, MZ_SP_TAIL_THREADS);
         mz_fence_mbar_init();
     }
     __syncwarp();
@@ -217,6 +221,12 @@ __device__ __forceinline__ void mz_sp_epilogue(const uint32_t (&v)[16], const ui
 // The epilogue warps never wait for each other, and everything that is not on the chain MMA -> epilogue -> MMA (descriptor loads, weight
 // waits, refills) sits on the issuer warp, which has a whole epilogue of slack per round.
 #define MZ_SP_THREADS (MZ_THREADS + 64)             // 8 worker warps (tree phases + epilogues) + one issuer warp per group
+#define MZ_SP_SEARCH_THREADS (MZ_THREADS + MZ_SP_TAIL_THREADS)   // mz_k_search_sp: + warps 10, 11, which with the two issuers form the tail team
+// named barriers: 1, 2 = group 0 / 1 (epilogue warps + issuer); in mz_k_search_sp 3 = workers + issuers before a network pass, 4 = the
+// workers after it, 5 = the tail team between its rounds, 6 = the gate of a tail's first round
+enum { MZ_SP_BAR_SIM = 3, MZ_SP_BAR_WORK = 4, MZ_SP_BAR_TAIL = 5, MZ_SP_BAR_GATE = 6 };
+__device__ __forceinline__ void mz_named_sync(int id, int n) { asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(n) : "memory"); }
+__device__ __forceinline__ void mz_named_arrive(int id, int n) { asm volatile("bar.arrive %0, %1;" ::"r"(id), "r"(n) : "memory"); }
 __device__ __forceinline__ void mz_sp_bar_arrive(int grp) { asm volatile("bar.arrive %0, %1;" ::"r"(grp + 1), "n"(MZ_GROUP + 32) : "memory"); }
 __device__ __forceinline__ void mz_sp_bar_sync(int grp) { asm volatile("bar.sync %0, %1;" ::"r"(grp + 1), "n"(MZ_GROUP + 32) : "memory"); }
 __device__ __forceinline__ void mz_sp_wait_mma(uint32_t mbar, uint32_t q) {
@@ -236,6 +246,21 @@ __device__ __forceinline__ void mz_sp_store_commit() { asm volatile("cp.async.bu
 __device__ __forceinline__ void mz_sp_store_wait_read() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
 __device__ __forceinline__ void mz_sp_store_wait_all() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
 
+// one thread: the MMAs of a round (descriptor words 0..11 in d0..d2, k-steps in e1.z)
+__device__ __forceinline__ void mz_sp_issue_mmas(uint4 d0, uint4 d1, uint4 d2, uint4 e1, int njobs, uint32_t tmem_d) {
+#pragma unroll 1
+    for (int j = 0; j < njobs; j++) {
+        const uint64_t ah = j ? mz_u64(d0.z, d0.w) : mz_u64(d0.x, d0.y), al = j ? mz_u64(d1.z, d1.w) : mz_u64(d1.x, d1.y), bh = j ? mz_u64(d2.z, d2.w) : mz_u64(d2.x, d2.y);
+        const uint32_t d = tmem_d + 64u * (uint32_t)j;
+        const int ks = (int)(short)(j ? (e1.z >> 16) : (e1.z & 0xffffu));
+#pragma unroll 1
+        for (int k = 0; k < ks; k++) {           // A: +32 B per K = 16 step inside the 128-byte swizzle row; B: 16 k rows = 1024 B
+            const uint64_t ka = (uint64_t)(2 * k), kb = (uint64_t)(64 * k);
+            mz_sp_mma(d, ah + ka, bh + kb, MZ_SP_IDESC64, k > 0 ? 1u : 0u);          // W_hi [X_hi | X_lo] -> columns 0..31 | 32..63
+            mz_sp_mma(d, al + ka, bh + kb, MZ_SP_IDESC32, 1u);                       // W_lo X_hi          -> columns 0..31
+        }
+    }
+}
 // save / fslot: learner only -- the hi tile of every job's input goes to save + fslot[2 * round + job] * 4 KB (fslot: shared address of an int16 table)
 // bias: extra fills every weight set of this network has seen (a persistent self-play kernel primes the representation / dynamics sets anew at every ply)
 __device__ __noinline__ uint32_t mz_sp_run_issuer(const mz_sp_ctx C, int first, int count, uint32_t tmem_d, uint32_t mbar, uint32_t q, uint32_t pass, int grp,
@@ -249,18 +274,7 @@ __device__ __noinline__ uint32_t mz_sp_run_issuer(const mz_sp_ctx C, int first, 
         if (r > 0) mz_sp_bar_sync(grp);                                 // the previous round's outputs are in the operand tiles, its accumulators have been read
         mz_tc_fence_after();
         if (mz_elect_one()) {
-#pragma unroll 1
-            for (int j = 0; j < njobs; j++) {
-                const uint64_t ah = j ? mz_u64(d0.z, d0.w) : mz_u64(d0.x, d0.y), al = j ? mz_u64(d1.z, d1.w) : mz_u64(d1.x, d1.y), bh = j ? mz_u64(d2.z, d2.w) : mz_u64(d2.x, d2.y);
-                const uint32_t d = tmem_d + 64u * (uint32_t)j;
-                const int ks = (int)(short)(j ? (e1.z >> 16) : (e1.z & 0xffffu));
-#pragma unroll 1
-                for (int k = 0; k < ks; k++) {           // A: +32 B per K = 16 step inside the 128-byte swizzle row; B: 16 k rows = 1024 B
-                    const uint64_t ka = (uint64_t)(2 * k), kb = (uint64_t)(64 * k);
-                    mz_sp_mma(d, ah + ka, bh + kb, MZ_SP_IDESC64, k > 0 ? 1u : 0u);          // W_hi [X_hi | X_lo] -> columns 0..31 | 32..63
-                    mz_sp_mma(d, al + ka, bh + kb, MZ_SP_IDESC32, 1u);                       // W_lo X_hi          -> columns 0..31
-                }
-            }
+            mz_sp_issue_mmas(d0, d1, d2, e1, njobs, tmem_d);
             // learner: the commit releases this round's epilogue, which may overwrite tiles the previous round's stores still read
             if (save) mz_sp_store_wait_read();
             asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(mbar) : "memory");
@@ -304,6 +318,60 @@ __device__ __noinline__ uint32_t mz_sp_run(const mz_sp_ctx C, int first, int cou
         MZ_RT(4);
         if (r + 1 < count) mz_sp_bar_arrive(grp);
         MZ_RT(5);
+    }
+    return q;
+}
+
+// ---- the TAIL of a dynamics pass in mz_k_search_sp: its trailing rounds [first, first + count), which feed no reward job ----------------
+// Run by the tail team (warps 8..11 = TMEM lane quadrants 0..3, ttid = thread index in the team) beside the tree phases of the worker
+// warps.  Warp 9, the dynamics issuer, issues every round and runs quadrant 1 of its epilogue; warps 8, 10, 11 run quadrants 0, 2, 3.
+// Round `first`: the issuer syncs on group 1's barrier (the worker warps arrive after their last round), issues, and opens the gate
+// for the other three -- before it they could not tell round `first`'s phase of the MMA barrier from an earlier one with the same
+// parity.  Later rounds: the team arrives on the tail barrier after its epilogue and the issuer syncs on it, as in mz_sp_run_issuer /
+// mz_sp_run.  q = group 1's rounds before round `first`.  Issue and epilogue are separate calls: one function with both would need
+// more registers than either.
+__device__ __noinline__ void mz_sp_tail_issue(const mz_sp_ctx C, uint32_t R, uint32_t tmem_d, uint32_t mbar, uint32_t q, uint32_t pass, uint32_t bias, bool first) {
+    const uint4 d0 = mz_lds_u4(R), d1 = mz_lds_u4(R + 16), d2 = mz_lds_u4(R + 32), e1 = mz_lds_u4(R + 64), e2 = mz_lds_u4(R + 80);
+    const uint32_t fo = mz_lds_u4(R + 96).y;
+    const int njobs = (int)(short)(e2.z & 0xffffu), set = (int)(short)(e2.w & 0xffffu), next = (int)(short)(e2.w >> 16);
+    if (mz_elect_one()) mz_sp_wait_weights(C, set, pass * (fo & 0xffffu) + (fo >> 16) + bias);
+    if (first) mz_sp_bar_sync(1); else mz_named_sync(MZ_SP_BAR_TAIL, MZ_SP_TAIL_THREADS);
+    mz_tc_fence_after();
+    if (mz_elect_one()) {
+        mz_sp_issue_mmas(d0, d1, d2, e1, njobs, tmem_d);
+        asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(mbar) : "memory");
+    }
+    __syncwarp();
+    if (first) mz_named_arrive(MZ_SP_BAR_GATE, MZ_SP_TAIL_THREADS);
+    if (mz_elect_one()) {
+        mz_sp_wait_mma(mbar, q);
+        if (next >= 0) mz_sp_fill(C, C.prog + (uint32_t)next * MZ_SP_RDESC_BYTES);      // the round's weights are free: hand the set to its next user
+    }
+    __syncwarp();
+}
+// one quadrant of a tail round's epilogue (as a round of mz_sp_run).  A tail round has one job, the state head's layer: the reward head
+// has ended before the tail begins.  Reading one job's accumulators keeps this call 32 registers lighter than mz_sp_run, and the
+// kernel has no registers to spare around it.
+__device__ __noinline__ void mz_sp_tail_epilogue(uint32_t R, uint32_t lane_base, uint32_t mbar, uint32_t q, int w, int t) {
+    const uint4 e0 = mz_lds_u4(R + 48), e1 = mz_lds_u4(R + 64), e2 = mz_lds_u4(R + 80);
+    mz_sp_wait_mma(mbar, q);
+    mz_tc_fence_after();
+    __syncwarp();
+    uint32_t v0[16], u0[16];
+    mz_tc_ld16x256(lane_base, v0); mz_tc_ld16x256(lane_base + 32u, u0);
+    mz_tc_wait_ld();
+    mz_sp_epilogue(v0, u0, (int)(short)(e1.w & 0xffffu), (int)(short)(e2.x & 0xffffu), (int)(short)(e2.y & 0xffffu), e1.x, e0.x, e0.z, w, t);
+    mz_fence_proxy_async();
+    mz_tc_fence_before();
+}
+__device__ __forceinline__ uint32_t mz_sp_run_tail(const mz_sp_ctx C, int first, int count, uint32_t tmem_d, uint32_t mbar, uint32_t q, uint32_t pass, uint32_t bias, int ttid) {
+    const int w = ttid >> 5;
+    uint32_t R = C.prog + (uint32_t)first * MZ_SP_RDESC_BYTES;
+    for (int r = 0; r < count; r++, R += MZ_SP_RDESC_BYTES, q++) {
+        if (w == 1) mz_sp_tail_issue(C, R, tmem_d, mbar, q, pass, bias, r == 0);
+        else if (r == 0) mz_named_sync(MZ_SP_BAR_GATE, MZ_SP_TAIL_THREADS);
+        mz_sp_tail_epilogue(R, tmem_d + ((uint32_t)(32 * w) << 16), mbar, q, w, ttid & 31);
+        if (w != 1 && r + 1 < count) mz_named_arrive(MZ_SP_BAR_TAIL, MZ_SP_TAIL_THREADS);
     }
     return q;
 }

@@ -19,7 +19,10 @@ for mode, label in ((capi.NN_FP32_EXACT, "fp32_exact"), (capi.NN_BF16_TC, "bf16_
         if n == 0:
             print(label, who, "no timers in this build"); continue
         tot = pc[g, :8].sum()
-        print("%s %s: %.0f cycles/round; " % (label, who, tot / rounds) + ", ".join("%s %.0f" % (names[i], pc[g, i] / rounds) for i in range(8) if names[i] != "-"))
+        nm = list(names)
+        if mode == capi.NN_SPLIT_MMA:      # with a dynamics tail the hidden state is written by the tail team; the workers wait for it before staging
+            nm[5] = "tail-done wait + hidden write"
+        print("%s %s: %.0f cycles/round; " % (label, who, tot / rounds) + ", ".join("%s %.0f" % (nm[i], pc[g, i] / rounds) for i in range(8) if nm[i] != "-"))
     for o, who in ((12, 'issuing thread, group 0'), (20, 'epilogue thread, group 1')):
         q = raw[o + 6]
         if q > 0:
@@ -27,6 +30,8 @@ for mode, label in ((capi.NN_FP32_EXACT, "fp32_exact"), (capi.NN_BF16_TC, "bf16_
             if mode == capi.NN_SPLIT_MMA:      # epilogue threads only (the issuer is a warp of its own): wait for the MMAs, read, compute + store, fences, arrive
                 lab = ['mbarrier wait', 'tcgen05.ld', 'epilogue', 'fences', 'bar.arrive', '-']
             print('%s TC round (%s): %.0f cycles; ' % (label, who, raw[o:o + 6].sum() / q) + ', '.join('%s %.0f' % (lab[i], raw[o + i] / q) for i in range(6)))
+    if raw[56] > 0:   # split-precision kernel with a dynamics tail: the issuer of group 1 times each tail (its rounds + the hidden-state write)
+        print('%s dynamics tail (off the chain; issuer warp, end of its chain rounds -> tail done): %.0f cycles' % (label, raw[55] / raw[56]))
     if raw[53] > 0:   # kernel-level stamps of thread 0 (split-precision kernel)
         ks = ['set-up', 'stage observations', 'representation', 'root prediction', 'root expansion + noise', 'simulation loop', 'move epilogue + teardown']
         print('%s whole kernel (thread 0, mean cycles per launch): ' % label + ', '.join('%s %.0f' % (ks[i], raw[46 + i] / raw[53]) for i in range(7)) + '; slowest CTA of any launch %.0f vs mean %.0f' % (raw[54], raw[46:53].sum() / raw[53]))
