@@ -68,7 +68,6 @@ struct mz_ctx {
     cudaStream_t stream2 = nullptr; cudaEvent_t ev_search[2] = {nullptr, nullptr};   // save / refill of move k beside the search of move k + 1 (run_wave)
     std::string err;
     size_t smem_bytes = 0; int sm_count = 0;
-    int exact_gt = 128;   // threads per network group of the exact search kernel: 128 (4x4 register tiles) or 256 (2x4 tiles, twice the warps; measured no faster: the layer is bound by shared-memory wavefronts, DESIGN.md section 4)
     float *d_w = nullptr, *d_m = nullptr, *d_v = nullptr, *d_grad = nullptr;
     unsigned char *d_w_tc = nullptr; float *d_bias_tc = nullptr; size_t smem_bytes_tc = 0;   // tensor-core weight image
     // data-parallel learner over peer memory (mz_k_dp_adam): gradient exchange buffers (double-buffered) and arrival flags of every rank
@@ -499,6 +498,36 @@ int launch_update(mz_ctx *c, int64_t t, int grad_mode) {
     return MZ_OK;
 }
 
+// the fields of a search launch that do not depend on where its roots come from
+static mz_search_args search_args(const mz_ctx *c, int n, int exploration) {
+    mz_search_args a{}; a.wglob = c->d_w; a.pbc0 = c->d_pbc0; a.sqrtN = c->d_sqrtN; a.tree_pool = c->d_trees; a.n = n; a.max_dim = c->M.max_dim;
+    a.max_layer_floats = c->M.max_layer_floats; a.exploration = exploration;
+    return a;
+}
+// One search over the roots of `a` (MODE_API: the caller's a.n roots; MODE_SLOTS: the a.n game slots) in ONE launch of kernel family 0
+// (run_wave_body relabels the last one of an idle iteration).  lat > 0: the low-latency kernel (mz_kernels_lat.cuh) on roots [0, lat),
+// one 2-CTA cluster each; otherwise the batched kernel of the context's networks.
+template <int MODE>
+static void launch_search(mz_ctx *c, const mz_params &P, const mz_search_args &a, int lat) {
+    const unsigned ctas = (unsigned)((a.n + MZ_ROWS - 1) / MZ_ROWS);
+    launch_scope ls(c, 0);
+    if (lat > 0) {
+        mz_lat_args t{}; t.base = a; t.image = c->d_w_lat; t.w_floats = c->lat_w_floats; t.pbc_smem = c->lat_pbc_smem;
+        mz_k_search_lat<MODE><<<2 * lat, MZ_LAT_THREADS, c->smem_bytes_lat, c->stream>>>(P, t);
+    } else if (c->cfg.net_type == MZ_NET_RESNET) {
+        mz_search_rn_args t{}; t.base = a; t.image = c->d_rn_image; t.steps = c->d_rn_steps;
+        const int nt = c->rn.R.ntrees;
+        mz_k_search_rn<MODE><<<(a.n + nt - 1) / nt, MZ_RN_THREADS, c->smem_bytes_rn, c->stream>>>(P, c->rn.R, t);
+    } else if (c->cfg.nn_mode == MZ_NN_SPLIT_MMA) {
+        mz_search_sp_args t{}; t.base = a; t.sp = c->spa;
+        mz_k_search_sp<MODE><<<ctas, MZ_SP_SEARCH_THREADS, c->smem_bytes_sp, c->stream>>>(P, t);
+    } else if (c->cfg.nn_mode == MZ_NN_BF16_TC) {
+        mz_search_tc_args t{}; t.base = a; t.w_image = c->d_w_tc; t.bias = c->d_bias_tc;
+        mz_k_search_tc<MODE><<<ctas, MZ_THREADS, c->smem_bytes_tc, c->stream>>>(P, t);
+    } else if (c->cfg.use_batch_norm) mz_k_search<MODE, true><<<ctas, MZ_THREADS, c->smem_bytes, c->stream>>>(P, a);
+    else mz_k_search<MODE><<<ctas, MZ_THREADS, c->smem_bytes, c->stream>>>(P, a);
+}
+
 }  // namespace
 
 extern "C" {
@@ -566,16 +595,12 @@ int mz_create(const mz_config *cfg, int device, mz_ctx **out) {
     if (c->smem_bytes > (size_t)prop.sharedMemPerBlockOptin) { int r = fail(nullptr, MZ_E_UNSUPPORTED, "network needs %zu B of shared memory per CTA, device allows %zu", c->smem_bytes, (size_t)prop.sharedMemPerBlockOptin); mz_destroy(c); return r; }
     MZ_CREATE(allow_max_smem(mz_k_search<MZ_MODE_API>, prop));
     MZ_CREATE(allow_max_smem(mz_k_search<MZ_MODE_SLOTS>, prop));
-    MZ_CREATE(allow_max_smem(mz_k_search<MZ_MODE_API, 256>, prop));
-    MZ_CREATE(allow_max_smem(mz_k_search<MZ_MODE_SLOTS, 256>, prop));
-    if (const char *eg = getenv("MZ_EXACT_GROUP")) c->exact_gt = atoi(eg) == 256 ? 256 : 128;   // measurement switch
     MZ_CREATE(allow_max_smem(mz_k_nn_forward<false>, prop));
     MZ_CREATE(allow_max_smem(mz_k_reanalyse<false>, prop));
     MZ_CREATE(allow_max_smem(mz_k_learn_forward<false>, prop));
     if (!resnet && cfg->use_batch_norm) {   // the same kernels instantiated with the BatchNorm epilogue
-        MZ_CREATE(allow_max_smem(mz_k_search<MZ_MODE_API, MZ_GROUP, true>, prop)); MZ_CREATE(allow_max_smem(mz_k_search<MZ_MODE_SLOTS, MZ_GROUP, true>, prop));
+        MZ_CREATE(allow_max_smem(mz_k_search<MZ_MODE_API, true>, prop)); MZ_CREATE(allow_max_smem(mz_k_search<MZ_MODE_SLOTS, true>, prop));
         MZ_CREATE(allow_max_smem(mz_k_nn_forward<true>, prop)); MZ_CREATE(allow_max_smem(mz_k_reanalyse<true>, prop)); MZ_CREATE(allow_max_smem(mz_k_learn_forward<true>, prop));
-        c->exact_gt = 128;
     }
     if (!resnet) {   // the low-latency search kernel for few roots: does a network pair fit one SM's shared memory in fp32?
         int nf[3] = {0, 0, 0}; bool narrow = true;
@@ -903,7 +928,7 @@ int mz_run_mcts(mz_ctx *c, int n, const float *stacked_obs, const uint32_t *lega
     const mz_params &P = c->M.P;
     for (int i = 0; i < n; i++) {
         if (legal_mask[i] == 0 || (legal_mask[i] >> P.A) != 0) return fail(c, MZ_E_ARG, "legal actions of root %d must be a non-empty subset of the action space (SelfPlay.jl:243-244)", i);
-        if (to_play[i] < 1 || to_play[i] > P.P) return fail(c, MZ_E_ARG, "to_play of root %d out of range", i);
+        if (to_play[i] < 1 || to_play[i] > P.P) return fail(c, MZ_E_ARG, "to_play of root %d out of range", i);   // the search itself does not read it
     }
     if (c->lat_ok && n > 0 && n <= c->lat_max_roots && c->cfg.nn_mode != MZ_NN_BF16_TC) {
         // few roots: one tree per cluster in exact fp32 (mz_kernels_lat.cuh); every input in ONE pinned block and one copy each way -- at
@@ -911,7 +936,7 @@ int mz_run_mcts(mz_ctx *c, int n, const float *stacked_obs, const uint32_t *lega
         // flight here: a wave ends with every slot idle or resets the slots.
         MZ_TRY(ensure_lat_image(c));
         auto al = [](size_t x) { return (x + 15) & ~(size_t)15; };
-        const size_t o_st = 0, o_legal = al(o_st + (size_t)n * P.stack_size * 4), o_tp = al(o_legal + (size_t)n * 4), o_gid = al(o_tp + (size_t)n * 4), o_mv = al(o_gid + (size_t)n * 8),
+        const size_t o_st = 0, o_legal = al(o_st + (size_t)n * P.stack_size * 4), o_gid = al(o_legal + (size_t)n * 4), o_mv = al(o_gid + (size_t)n * 8),
                      o_vc = al(o_mv + (size_t)n * 4), o_rv = al(o_vc + (size_t)n * P.A * 4), o_pri = al(o_rv + (size_t)n * 4), total = al(o_pri + (size_t)n * P.A * 4);
         if (total > c->lat_stage_cap) {
             if (c->h_lat_stage) cudaFreeHost(c->h_lat_stage);
@@ -922,16 +947,13 @@ int mz_run_mcts(mz_ctx *c, int n, const float *stacked_obs, const uint32_t *lega
             c->lat_stage_cap = want;
         }
         unsigned char *h = c->h_lat_stage, *d = c->d_lat_stage;
-        memcpy(h + o_st, stacked_obs, (size_t)n * P.stack_size * 4); memcpy(h + o_legal, legal_mask, (size_t)n * 4); memcpy(h + o_tp, to_play, (size_t)n * 4);
+        memcpy(h + o_st, stacked_obs, (size_t)n * P.stack_size * 4); memcpy(h + o_legal, legal_mask, (size_t)n * 4);
         memcpy(h + o_gid, game_id, (size_t)n * 8); memcpy(h + o_mv, move_idx, (size_t)n * 4);
         MZ_CUDA(c, cudaMemcpyAsync(d, h, o_vc, cudaMemcpyHostToDevice, c->stream));
-        mz_lat_args t{};
-        mz_search_args &a = t.base; a.wglob = c->d_w; a.pbc0 = c->d_pbc0; a.sqrtN = c->d_sqrtN; a.tree_pool = c->d_trees; a.n = n; a.max_dim = c->M.max_dim;
-        a.max_layer_floats = c->M.max_layer_floats; a.exploration = exploration; a.stacked = (const float *)(d + o_st); a.legal = (const uint32_t *)(d + o_legal);
-        a.to_play = (const int32_t *)(d + o_tp); a.game_id = (const uint64_t *)(d + o_gid); a.move_idx = (const int32_t *)(d + o_mv);
-        a.visit_counts = (int32_t *)(d + o_vc); a.root_value = (float *)(d + o_rv); a.root_priors = (float *)(d + o_pri); a.stats = nullptr;
-        t.image = c->d_w_lat; t.w_floats = c->lat_w_floats; t.pbc_smem = c->lat_pbc_smem;
-        { launch_scope ls(c, 0); mz_k_search_lat<MZ_MODE_API><<<2 * n, MZ_LAT_THREADS, c->smem_bytes_lat, c->stream>>>(P, t); }
+        mz_search_args a = search_args(c, n, exploration);
+        a.stacked = (const float *)(d + o_st); a.legal = (const uint32_t *)(d + o_legal); a.game_id = (const uint64_t *)(d + o_gid); a.move_idx = (const int32_t *)(d + o_mv);
+        a.visit_counts = (int32_t *)(d + o_vc); a.root_value = (float *)(d + o_rv); a.root_priors = (float *)(d + o_pri);
+        launch_search<MZ_MODE_API>(c, P, a, n);
         MZ_CUDA(c, cudaGetLastError());
         MZ_CUDA(c, cudaMemcpyAsync(h + o_vc, d + o_vc, total - o_vc, cudaMemcpyDeviceToHost, c->stream));
         MZ_CUDA(c, cudaStreamSynchronize(c->stream));
@@ -945,28 +967,15 @@ int mz_run_mcts(mz_ctx *c, int n, const float *stacked_obs, const uint32_t *lega
     MZ_TRY(ensure_images(c));
     for (int off = 0; off < n; off += cap) {
         int m = n - off < cap ? n - off : cap;
-        float *d_st, *d_rv, *d_pri; uint32_t *d_legal; int32_t *d_tp, *d_mv, *d_vc; uint64_t *d_gid;
+        float *d_st, *d_rv, *d_pri; uint32_t *d_legal; int32_t *d_mv, *d_vc; uint64_t *d_gid;
         MZ_TRY(h2d(c, c->scratch[0], stacked_obs + (size_t)off * P.stack_size, (size_t)m * P.stack_size, &d_st));
-        MZ_TRY(h2d(c, c->scratch[1], legal_mask + off, (size_t)m, &d_legal)); MZ_TRY(h2d(c, c->scratch[2], to_play + off, (size_t)m, &d_tp));
+        MZ_TRY(h2d(c, c->scratch[1], legal_mask + off, (size_t)m, &d_legal));
         MZ_TRY(h2d(c, c->scratch[3], game_id + off, (size_t)m, &d_gid)); MZ_TRY(h2d(c, c->scratch[4], move_idx + off, (size_t)m, &d_mv));
         MZ_TRY(h2d<int32_t>(c, c->scratch[5], nullptr, (size_t)m * P.A, &d_vc)); MZ_TRY(h2d<float>(c, c->scratch[6], nullptr, (size_t)m, &d_rv));
         MZ_TRY(h2d<float>(c, c->scratch[7], nullptr, (size_t)m * P.A, &d_pri));
-        mz_search_args a{}; a.wglob = c->d_w; a.pbc0 = c->d_pbc0; a.sqrtN = c->d_sqrtN; a.tree_pool = c->d_trees; a.n = m; a.max_dim = c->M.max_dim;
-        a.max_layer_floats = c->M.max_layer_floats; a.exploration = exploration; a.stacked = d_st; a.legal = d_legal; a.to_play = d_tp; a.game_id = d_gid;
-        a.move_idx = d_mv; a.visit_counts = d_vc; a.root_value = d_rv; a.root_priors = d_pri; a.stats = nullptr;
-        if (c->cfg.net_type == MZ_NET_RESNET) {
-            mz_search_rn_args t{}; t.base = a; t.image = c->d_rn_image; t.steps = c->d_rn_steps;
-            const int nt = c->rn.R.ntrees;
-            launch_scope ls(c, 0); mz_k_search_rn<MZ_MODE_API><<<(m + nt - 1) / nt, MZ_RN_THREADS, c->smem_bytes_rn, c->stream>>>(P, c->rn.R, t);
-        } else if (c->cfg.nn_mode == MZ_NN_SPLIT_MMA) {
-            mz_search_sp_args t{}; t.base = a; t.sp = c->spa;
-            launch_scope ls(c, 0); mz_k_search_sp<MZ_MODE_API><<<(m + MZ_ROWS - 1) / MZ_ROWS, MZ_SP_SEARCH_THREADS, c->smem_bytes_sp, c->stream>>>(P, t);
-        } else if (c->cfg.nn_mode == MZ_NN_BF16_TC) {
-            mz_search_tc_args t{}; t.base = a; t.w_image = c->d_w_tc; t.bias = c->d_bias_tc;
-            launch_scope ls(c, 0); mz_k_search_tc<MZ_MODE_API><<<(m + MZ_ROWS - 1) / MZ_ROWS, MZ_THREADS, c->smem_bytes_tc, c->stream>>>(P, t);
-        } else if (c->cfg.use_batch_norm) { launch_scope ls(c, 0); mz_k_search<MZ_MODE_API, MZ_GROUP, true><<<(m + MZ_ROWS - 1) / MZ_ROWS, MZ_THREADS, c->smem_bytes, c->stream>>>(P, a); }
-        else if (c->exact_gt == 256) { launch_scope ls(c, 0); mz_k_search<MZ_MODE_API, 256><<<(m + MZ_ROWS - 1) / MZ_ROWS, 512, c->smem_bytes, c->stream>>>(P, a); }
-        else { launch_scope ls(c, 0); mz_k_search<MZ_MODE_API><<<(m + MZ_ROWS - 1) / MZ_ROWS, MZ_THREADS, c->smem_bytes, c->stream>>>(P, a); }
+        mz_search_args a = search_args(c, m, exploration);
+        a.stacked = d_st; a.legal = d_legal; a.game_id = d_gid; a.move_idx = d_mv; a.visit_counts = d_vc; a.root_value = d_rv; a.root_priors = d_pri;
+        launch_search<MZ_MODE_API>(c, P, a, 0);
         MZ_CUDA(c, cudaGetLastError());
         MZ_TRY(d2h(c, visit_counts + (size_t)off * P.A, d_vc, (size_t)m * P.A)); MZ_TRY(d2h(c, root_value + off, d_rv, (size_t)m));
         if (root_priors) MZ_TRY(d2h(c, root_priors + (size_t)off * P.A, d_pri, (size_t)m * P.A));
@@ -1057,13 +1066,13 @@ static int run_wave_body(mz_ctx *c, uint64_t first_game, int64_t n_games, float 
     MZ_CUDA(c, cudaMemcpyAsync(c->ring.counters + 3, c->h_counters + 3, 3 * sizeof(int64_t), cudaMemcpyHostToDevice, c->stream));
     MZ_CUDA(c, cudaMemsetAsync(c->d_stats, 0, 64 * sizeof(unsigned long long), c->stream));
     MZ_TRY(ensure_images(c));
-    mz_search_args a{}; a.wglob = c->d_w; a.pbc0 = c->d_pbc0; a.sqrtN = c->d_sqrtN; a.tree_pool = c->d_trees; a.n = G; a.max_dim = c->M.max_dim;
-    a.max_layer_floats = c->M.max_layer_floats; a.exploration = 1 /* play_game hard-codes exploration=true, SelfPlay.jl:359 */;
+    mz_search_args a = search_args(c, G, 1 /* play_game hard-codes exploration=true, SelfPlay.jl:359 */);
     a.slots = c->slots; a.temperature = temperature; a.stats = c->d_stats;
     // A wave starts with every slot idle and games are handed out in slot order, so a call for n_games <= num_slots games only ever uses the
     // slots [0, n_games): few games go to the low-latency kernel whatever the context's size (the bf16 mode keeps its own arithmetic)
     const int G_lat = (int64_t)G < n_games ? G : (int)n_games;
     const bool use_lat = allow_lat && c->lat_ok && G_lat >= 1 && G_lat <= c->lat_max_slots && c->cfg.nn_mode != MZ_NN_BF16_TC;
+    if (use_lat) MZ_TRY(ensure_lat_image(c));
     int64_t total_moves = 0; int last_snap = 0;
     // The host runs one iteration behind the device: iteration k (opponent plies, search, save/refill, counter snapshot) is queued before
     // the snapshot of iteration k - 1 is read, so the GPU never waits for a launch.  When that snapshot says no game is active any more,
@@ -1086,8 +1095,8 @@ static int run_wave_body(mz_ctx *c, uint64_t first_game, int64_t n_games, float 
     // pays launch gaps: here a CTA starts its next move when its own trees are done.  All finished games are saved by one save / refill at
     // the end, in slot order (= game id order).  MUZERO_B200_PERSIST=0 keeps one launch per move.
     if (overlap && !use_lat && arena_player == 0 && c->cfg.net_type == MZ_NET_FEEDFORWARD && c->cfg.nn_mode == MZ_NN_SPLIT_MMA && c->persist_ok) {
-        mz_search_sp_args t{}; t.base = a; t.base.persist = 1; t.sp = c->spa;
-        { launch_scope ls(c, 0); mz_k_search_sp<MZ_MODE_SLOTS><<<(G + MZ_ROWS - 1) / MZ_ROWS, MZ_SP_SEARCH_THREADS, c->smem_bytes_sp, c->stream>>>(P, t); }
+        mz_search_args ap = a; ap.persist = 1;
+        launch_search<MZ_MODE_SLOTS>(c, P, ap, 0);
         MZ_TRY(launch_save_refill(c, P, G, tally, c->d_wave + 8));
         MZ_CUDA(c, cudaGetLastError());
         MZ_CUDA(c, cudaMemcpyAsync(c->h_stats, c->d_stats, 64 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, c->stream));
@@ -1104,23 +1113,7 @@ static int run_wave_body(mz_ctx *c, uint64_t first_game, int64_t n_games, float 
         if (k > n_games * (int64_t)(P.max_moves + 2) + 8) return fail(c, MZ_E_STATE, "self-play did not terminate");
         P.fin_tag = (int32_t)(k & 1);
         if (arena_player != 0) { launch_scope ls(c, 6); mz_k_opponent_move<<<(G + 127) / 128, 128, 0, c->stream>>>(P, c->slots, G); }
-        if (use_lat) {   // few games (play_game one game at a time): one tree per cluster (mz_kernels_lat.cuh), exact fp32
-            MZ_TRY(ensure_lat_image(c));
-            mz_lat_args t{}; t.base = a; t.image = c->d_w_lat; t.w_floats = c->lat_w_floats; t.pbc_smem = c->lat_pbc_smem;
-            launch_scope ls(c, 0); mz_k_search_lat<MZ_MODE_SLOTS><<<2 * G_lat, MZ_LAT_THREADS, c->smem_bytes_lat, c->stream>>>(P, t);
-        } else if (c->cfg.net_type == MZ_NET_RESNET) {
-            mz_search_rn_args t{}; t.base = a; t.image = c->d_rn_image; t.steps = c->d_rn_steps;
-            const int nt = c->rn.R.ntrees;
-            launch_scope ls(c, 0); mz_k_search_rn<MZ_MODE_SLOTS><<<(G + nt - 1) / nt, MZ_RN_THREADS, c->smem_bytes_rn, c->stream>>>(P, c->rn.R, t);
-        } else if (c->cfg.nn_mode == MZ_NN_SPLIT_MMA) {
-            mz_search_sp_args t{}; t.base = a; t.sp = c->spa;
-            launch_scope ls(c, 0); mz_k_search_sp<MZ_MODE_SLOTS><<<(G + MZ_ROWS - 1) / MZ_ROWS, MZ_SP_SEARCH_THREADS, c->smem_bytes_sp, c->stream>>>(P, t);
-        } else if (c->cfg.nn_mode == MZ_NN_BF16_TC) {
-            mz_search_tc_args t{}; t.base = a; t.w_image = c->d_w_tc; t.bias = c->d_bias_tc;
-            launch_scope ls(c, 0); mz_k_search_tc<MZ_MODE_SLOTS><<<(G + MZ_ROWS - 1) / MZ_ROWS, MZ_THREADS, c->smem_bytes_tc, c->stream>>>(P, t);
-        } else if (c->cfg.use_batch_norm) { launch_scope ls(c, 0); mz_k_search<MZ_MODE_SLOTS, MZ_GROUP, true><<<(G + MZ_ROWS - 1) / MZ_ROWS, MZ_THREADS, c->smem_bytes, c->stream>>>(P, a); }
-        else if (c->exact_gt == 256) { launch_scope ls(c, 0); mz_k_search<MZ_MODE_SLOTS, 256><<<(G + MZ_ROWS - 1) / MZ_ROWS, 512, c->smem_bytes, c->stream>>>(P, a); }
-        else { launch_scope ls(c, 0); mz_k_search<MZ_MODE_SLOTS><<<(G + MZ_ROWS - 1) / MZ_ROWS, MZ_THREADS, c->smem_bytes, c->stream>>>(P, a); }
+        launch_search<MZ_MODE_SLOTS>(c, P, a, use_lat ? G_lat : 0);   // few games (play_game one game at a time): one tree per cluster, exact fp32
         const size_t search_entry = c->timed.size();                       // (timing builds) index just past this iteration's search launch
         if (overlap) { MZ_CUDA(c, cudaEventRecord(c->ev_search[k & 1], c->stream)); MZ_CUDA(c, cudaStreamWaitEvent(sB, c->ev_search[k & 1], 0)); }
         MZ_TRY(launch_save_refill(c, P, G, tally, c->d_wave + 8 * ((k + 1) & 1), sB));

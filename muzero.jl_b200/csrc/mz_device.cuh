@@ -46,8 +46,7 @@ __device__ __forceinline__ void mz_mbar_wait(uint64_t *bar, uint32_t parity) {
 }
 __device__ __forceinline__ void mz_fence_proxy_async() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 // named barrier over one 128-thread group (ids 1 and 2; 0 is __syncthreads)
-template <int GT = MZ_GROUP>
-__device__ __forceinline__ void mz_group_sync(int grp) { asm volatile("bar.sync %0, %1;" ::"r"(grp + 1), "n"(GT) : "memory"); }
+__device__ __forceinline__ void mz_group_sync(int grp) { asm volatile("bar.sync %0, %1;" ::"r"(grp + 1), "n"(MZ_GROUP) : "memory"); }
 
 __device__ __forceinline__ float4 mz_lds128(uint32_t addr) {
     float4 v;
@@ -152,90 +151,41 @@ __device__ __noinline__ void mz_dense_tile_save(int in, int out_pad, int act, ui
     mz_dense_tile_body<true>(in, out_pad, act, w_smem, src_smem, dst_smem, gtid, gsave);
 }
 
-// The same layer for a 256-thread group (8 warps): 2 rows x 4 outputs per thread, so every layer is a single pass of
-// 16 row groups x 16 output groups.  Twice the warps of the 4x4 tile for the same work: the instruction stream of a warp
-// is 40 % shorter, which is what matters for a chain of latency-bound layers (mz_k_search<MODE, 256>).  Per output the
-// accumulation is still k = 0..in-1 in order with fmaf, i.e. bit-identical to mz_dense_tile.
-__device__ __noinline__ void mz_dense_tile_g256(int in, int out_pad, int act, uint32_t w_smem, uint32_t src_smem, uint32_t dst_smem, int gtid) {
-    const int lane = gtid & 31, warp = gtid >> 5;
-    const int rg = lane & 15;                                  // rows 2*rg, 2*rg + 1
-    const int opq = out_pad >> 2;
-    const uint32_t wstride = (uint32_t)out_pad * 4u;
-    for (int g = (warp << 1) | (lane >> 4); g < opq; g += 16) {
-        unsigned long long acc2[2][2];
-        acc2[0][0] = acc2[0][1] = acc2[1][0] = acc2[1][1] = 0ull;
-        uint32_t wa = w_smem + (uint32_t)g * 16u;
-        uint32_t xa = src_smem + (uint32_t)rg * 8u;
-MZ_UNROLL_K
-        for (int k = 0; k < in; k++) {
-            const float4 wv = mz_lds128(wa);
-            float x0, x1;
-            asm("ld.shared.v2.f32 {%0, %1}, [%2];" : "=f"(x0), "=f"(x1) : "r"(xa));
-            unsigned long long w01, w23, xx0, xx1;
-            asm("mov.b64 %0, {%1, %2};" : "=l"(w01) : "f"(wv.x), "f"(wv.y));
-            asm("mov.b64 %0, {%1, %2};" : "=l"(w23) : "f"(wv.z), "f"(wv.w));
-            asm("mov.b64 %0, {%1, %1};" : "=l"(xx0) : "f"(x0));
-            asm("mov.b64 %0, {%1, %1};" : "=l"(xx1) : "f"(x1));
-            asm("fma.rn.f32x2 %0, %1, %2, %0;" : "+l"(acc2[0][0]) : "l"(w01), "l"(xx0));
-            asm("fma.rn.f32x2 %0, %1, %2, %0;" : "+l"(acc2[0][1]) : "l"(w23), "l"(xx0));
-            asm("fma.rn.f32x2 %0, %1, %2, %0;" : "+l"(acc2[1][0]) : "l"(w01), "l"(xx1));
-            asm("fma.rn.f32x2 %0, %1, %2, %0;" : "+l"(acc2[1][1]) : "l"(w23), "l"(xx1));
-            wa += wstride; xa += MZ_ROWS * 4;
-        }
-        float acc[2][4];
-#pragma unroll
-        for (int i = 0; i < 2; i++) {
-            asm("mov.b64 {%0, %1}, %2;" : "=f"(acc[i][0]), "=f"(acc[i][1]) : "l"(acc2[i][0]));
-            asm("mov.b64 {%0, %1}, %2;" : "=f"(acc[i][2]), "=f"(acc[i][3]) : "l"(acc2[i][1]));
-        }
-        const float4 bv = mz_lds128(w_smem + (uint32_t)in * wstride + (uint32_t)g * 16u);
-        const float bj[4] = {bv.x, bv.y, bv.z, bv.w};
-#pragma unroll
-        for (int j = 0; j < 4; j++) {
-            float r0 = acc[0][j] + bj[j], r1 = acc[1][j] + bj[j];
-            if (act == MZ_ACT_RELU) { r0 = fmaxf(r0, 0.0f); r1 = fmaxf(r1, 0.0f); }
-            else if (act == MZ_ACT_TANH) { r0 = mz_tanhf_ni(r0); r1 = mz_tanhf_ni(r1); }
-            asm volatile("st.shared.v2.f32 [%0], {%1, %2};" ::"r"(dst_smem + (uint32_t)((4 * g + j) * MZ_ROWS * 4) + (uint32_t)rg * 8u), "f"(r0), "f"(r1) : "memory");
-        }
-    }
-}
-
 // One layer for one group: prefetch `next` (or nothing when next < 0) into the other buffer, wait for this layer's
 // weights, compute, group barrier.  Preconditions: this layer's copy was issued earlier; a barrier separates the last
 // reads of the other buffer (layer q-1) and of `dst`'s previous contents from this call.
 // BN: the kernel was instantiated for use_batch_norm networks.  A template parameter, not a run-time test: with the test (or the BatchNorm
 // epilogue inside mz_dense_tile) the ordinary networks' search kernel ran 9 - 20 % slower (88 - 98 M instead of 107 M simulations/s).
-template <int GT = MZ_GROUP, bool BN = false>
+template <bool BN = false>
 __device__ __forceinline__ void mz_nn_layer(mz_nn_pipe &s, const mz_params &P, int layer, int next, const float *src, float *dst) {
     if (s.gtid == 0 && next >= 0) mz_nn_issue(s, P, next, (s.q + 1) & 1u);
     mz_mbar_wait(&s.mbar[s.q & 1u], (s.q >> 1) & 1u);
     const mz_layer &L = P.layers[layer];
-    if (BN && L.bn) mz_dense_tile_bn(L.in, L.out_pad, L.act, mz_smem_u32(s.wbuf[s.q & 1u]), mz_smem_u32(src), mz_smem_u32(dst), s.gtid);   // (both group sizes: 4 warps do the layer)
-    else if (GT == 256) mz_dense_tile_g256(L.in, L.out_pad, L.act, mz_smem_u32(s.wbuf[s.q & 1u]), mz_smem_u32(src), mz_smem_u32(dst), s.gtid);
+    if (BN && L.bn) mz_dense_tile_bn(L.in, L.out_pad, L.act, mz_smem_u32(s.wbuf[s.q & 1u]), mz_smem_u32(src), mz_smem_u32(dst), s.gtid);
     else mz_dense_tile(L.in, L.out_pad, L.act, mz_smem_u32(s.wbuf[s.q & 1u]), mz_smem_u32(src), mz_smem_u32(dst), s.gtid);
-    mz_group_sync<GT>(s.grp);
+    mz_group_sync(s.grp);
     s.q++;
 }
-template <int GT = MZ_GROUP, bool BN = false>
+template <bool BN = false>
 __device__ __forceinline__ void mz_nn_chain(mz_nn_pipe &s, const mz_params &P, int first, int n, int after, const float *src,
                                             float *dst, float *t0, float *t1) {
     const float *cur = src;
     for (int i = 0; i < n; i++) {
         float *d = (i == n - 1) ? dst : ((i & 1) ? t1 : t0);
-        mz_nn_layer<GT, BN>(s, P, first + i, (i == n - 1) ? after : first + i + 1, cur, d);
+        mz_nn_layer<BN>(s, P, first + i, (i == n - 1) ? after : first + i + 1, cur, d);
         cur = d;
     }
 }
 // trunk -> bufT, head 1 -> h1dst, head 2 -> h2dst (Split, src/Learning.jl:60-68); `after` = layer prefetched last
-template <int GT = MZ_GROUP, bool BN = false>
+template <bool BN = false>
 __device__ __noinline__ void mz_nn_net(mz_nn_pipe &s, const mz_params &P, int net, int after, const float *src, float *bufT,
                                        float *h1dst, float *h2dst, float *t0, float *t1) {
     const mz_net &N = P.nets[net];
     int f = N.first;
-    if (N.n_h1 == 0) { mz_nn_chain<GT, BN>(s, P, f, N.n_trunk, after, src, h1dst, t0, t1); return; }
-    mz_nn_chain<GT, BN>(s, P, f, N.n_trunk, f + N.n_trunk, src, bufT, t0, t1);
-    mz_nn_chain<GT, BN>(s, P, f + N.n_trunk, N.n_h1, f + N.n_trunk + N.n_h1, bufT, h1dst, t0, t1);
-    mz_nn_chain<GT, BN>(s, P, f + N.n_trunk + N.n_h1, N.n_h2, after, bufT, h2dst, t0, t1);
+    if (N.n_h1 == 0) { mz_nn_chain<BN>(s, P, f, N.n_trunk, after, src, h1dst, t0, t1); return; }
+    mz_nn_chain<BN>(s, P, f, N.n_trunk, f + N.n_trunk, src, bufT, t0, t1);
+    mz_nn_chain<BN>(s, P, f + N.n_trunk, N.n_h1, f + N.n_trunk + N.n_h1, bufT, h1dst, t0, t1);
+    mz_nn_chain<BN>(s, P, f + N.n_trunk + N.n_h1, N.n_h2, after, bufT, h2dst, t0, t1);
 }
 
 // shared-memory carve-up used by every NN-running kernel
@@ -274,16 +224,14 @@ __device__ __forceinline__ mz_smem_plan mz_smem_carve(unsigned char *base, int m
     return p;
 }
 // both pipes are initialised by thread 0 of the CTA; every thread builds the descriptor of its own group
-template <int GT = MZ_GROUP>
 __device__ __forceinline__ void mz_pipe_init(mz_nn_pipe &s, const mz_smem_plan &sp, const float *wglob) {
-    s.grp = threadIdx.x / GT; s.gtid = threadIdx.x & (GT - 1);
+    s.grp = threadIdx.x / MZ_GROUP; s.gtid = threadIdx.x & (MZ_GROUP - 1);
     s.wbuf[0] = sp.wbuf[s.grp][0]; s.wbuf[1] = sp.wbuf[s.grp][1]; s.mbar = sp.mbar[s.grp]; s.wglob = wglob; s.q = 0;
     if (threadIdx.x == 0) {
         mz_mbar_init(&sp.mbar[0][0], 1); mz_mbar_init(&sp.mbar[0][1], 1); mz_mbar_init(&sp.mbar[1][0], 1); mz_mbar_init(&sp.mbar[1][1], 1);
         mz_fence_mbar_init();
     }
 }
-template <int NT = MZ_THREADS>
 __device__ __forceinline__ void mz_zero_activations(const mz_smem_plan &sp, int max_dim) {
-    for (int i = threadIdx.x; i < 8 * max_dim * MZ_ROWS; i += NT) sp.in0[i] = 0.0f;
+    for (int i = threadIdx.x; i < 8 * max_dim * MZ_ROWS; i += MZ_THREADS) sp.in0[i] = 0.0f;
 }

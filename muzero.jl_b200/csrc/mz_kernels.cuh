@@ -58,7 +58,7 @@ struct mz_search_args {
     int32_t persist;             // MODE_SLOTS, mz_k_search_sp: 1 = the kernel plays every game of its CTA to the end (one launch per wave: a CTA starts its next
                                  // move when ITS trees are done instead of waiting for the slowest CTA of the grid)
     // MODE_API inputs / outputs
-    const float *stacked; const uint32_t *legal; const int32_t *to_play; const uint64_t *game_id; const int32_t *move_idx;
+    const float *stacked; const uint32_t *legal; const uint64_t *game_id; const int32_t *move_idx;
     int32_t *visit_counts; float *root_value; float *root_priors;
     // MODE_SLOTS
     mz_slots slots; float temperature;
@@ -191,7 +191,7 @@ __device__ __forceinline__ void mz_tree_backup_lanes(const mz_params &P, const m
 }
 
 // play_game's loop body after run_mcts (src/SelfPlay.jl:344-346, 360-379) for one game slot: temperature rule, select_action, environment
-// step, store_search_stats! (Q12), history append, termination.  Shared by every search kernel (lane 0 of the tree).
+// step, store_search_stats! (Q12), history append, termination.  Lane 0 of the tree, from mz_root_finish.
 __device__ __forceinline__ void mz_slot_epilogue(const mz_params &P, const mz_slots &s, int64_t g, const int32_t *vc, int sum_visits, uint32_t legal, float rv,
                                                  float temperature, uint32_t game, uint32_t move) {
     int T = s.T[g];
@@ -213,8 +213,73 @@ __device__ __forceinline__ void mz_slot_epilogue(const mz_params &P, const mz_sl
     if (done || T > P.max_moves) s.status[g] = MZ_SLOT_FINISHED + P.fin_tag;                    // loop condition :343
 }
 
-// GT = threads per network group: 128 (4x4 register tiles) or 256 (2x4 tiles, twice the warps for the same work; the tree
-// phases still use 8 lanes x 32 trees = the first 256 threads).
+// ---- run_mcts for one root (SelfPlay.jl:230-285), the part every search kernel shares: the root's state, its stacked observation, the
+// root node and its expansion, the results.  The kernels differ in how they run the networks and in which threads own a tree. ----
+struct mz_root { bool active; uint32_t legal, game, move, posmask; };
+// root g: MODE_API from the caller's arrays, MODE_SLOTS from the slot's board (SelfPlay.jl:351,359); in competitive play a slot is searched
+// only on MuZero's plies.  valid = false (no root g for this thread: g >= a.n, or not a tree lane) gives an inactive root with no legal action.
+template <int MODE>
+__device__ __forceinline__ mz_root mz_root_begin(const mz_params &P, const mz_search_args &a, int64_t g, bool valid) {
+    mz_root R; R.active = false; R.legal = 0; R.game = 0; R.move = 0; R.posmask = 0;
+    if (MODE == MZ_MODE_API) {
+        if (valid) { R.legal = a.legal[g]; R.game = (uint32_t)a.game_id[g]; R.move = (uint32_t)a.move_idx[g]; }
+        R.active = R.legal != 0;   // run_mcts asserts !isempty(legal_actions) (SelfPlay.jl:243)
+    } else if (valid) {
+        R.active = a.slots.status[g] == MZ_SLOT_ACTIVE && (P.arena_player == 0 || a.slots.player[g] == P.arena_player);
+        if (R.active) {
+            mz_board b; b.p1 = a.slots.p1[g]; b.p2 = a.slots.p2[g]; b.player = a.slots.player[g];
+            R.legal = mz_env_legal_b(P, b); R.game = (uint32_t)a.slots.game_id[g]; R.move = (uint32_t)a.slots.T[g] + 1u;
+        }
+        if (R.legal == 0) R.active = false;   // never reached in play
+    }
+    for (int j = 0; j < P.A; j++) if ((R.legal >> (P.order[j] - 1)) & 1u) R.posmask |= 1u << j;   // legal actions as a mask over Dict positions
+    return R;
+}
+// entry k of root gg's stacked observations (get_stacked_observations, SelfPlay.jl:128-149); 0 past the launch's roots and for a slot
+// that has no ply to search
+template <int MODE>
+__device__ __forceinline__ float mz_root_obs(const mz_params &P, const mz_search_args &a, int64_t gg, int k) {
+    if (gg >= a.n) return 0.0f;
+    if (MODE == MZ_MODE_API) return a.stacked[gg * P.stack_size + k];
+    if (a.slots.status[gg] != MZ_SLOT_ACTIVE) return 0.0f;
+    return mz_stacked_value(P, a.slots.h_p1 + gg * P.Tmax, a.slots.h_p2 + gg * P.Tmax, a.slots.h_action + gg * P.Tmax, a.slots.T[gg] + 1, k);
+}
+// the 8 lanes of an active tree, after the root prediction: Node(prior=0) (:232), its expansion (:245; logits[a * ls] = logit of action
+// a + 1), then the exploration noise (:247-249; eps = 0 is the identity)
+__device__ __forceinline__ void mz_root_init(const mz_params &P, const mz_tree &t, const mz_root &R, int exploration, const float *logits, int ls, int ln,
+                                             uint32_t segmask) {
+    if (ln == 0) { mz_f4 root; root.x = mz_bits2f(mz_nx_pack(0, -1, 0)); root.y = 0.0f; root.z = 0.0f; root.w = 0.0f; t.A[0] = root; }
+    __syncwarp(segmask);
+    mz_tree_expand_lanes(P, t, 0, 0, R.legal, logits, 0.0f, 0.0f, ln, segmask, ls);
+    if (ln == 0 && exploration && P.exploration_eps != 0.0f) mz_tree_add_noise(P, t, R.legal, R.game, R.move);
+    __syncwarp(segmask);
+}
+// results of root g, lane 0 of an active tree: the launch's statistics (stats[0] sum of leaf depths, [1] simulations, [2] sum of legal
+// actions, [3] roots), then visit counts, root value and priors to the caller (MODE_API) or the move of the game (MODE_SLOTS)
+template <int MODE>
+__device__ __forceinline__ void mz_root_finish(const mz_params &P, const mz_search_args &a, int64_t g, const mz_tree &t, const mz_root &R,
+                                               unsigned long long depth_sum) {
+    int32_t vc[MZ_MAX_A]; int sum_visits = 0, nlegal = 0;
+    for (int i = 0; i < P.A; i++) {
+        vc[i] = ((R.legal >> i) & 1u) ? (int32_t)mz_nx_visit(mz_f2bits(t.A[1 + i].x)) : 0;
+        sum_visits += vc[i]; nlegal += (int)((R.legal >> i) & 1u);
+    }
+    const mz_f4 root = t.A[0];
+    const int rvc = mz_nx_visit(mz_f2bits(root.x));
+    const float rv = rvc == 0 ? 0.0f : root.y / (float)rvc;                                 // node_value(root)
+    if (a.stats) {
+        atomicAdd(&a.stats[0], depth_sum); atomicAdd(&a.stats[1], (unsigned long long)P.S);
+        atomicAdd(&a.stats[2], (unsigned long long)nlegal); atomicAdd(&a.stats[3], 1ull);
+    }
+    if (MODE == MZ_MODE_API) {
+        for (int i = 0; i < P.A; i++) {
+            a.visit_counts[g * P.A + i] = vc[i];
+            if (a.root_priors) a.root_priors[g * P.A + i] = ((R.legal >> i) & 1u) ? t.A[1 + i].z : 0.0f;
+        }
+        a.root_value[g] = rv;
+    } else mz_slot_epilogue(P, a.slots, g, vc, sum_visits, R.legal, rv, a.temperature, R.game, R.move);
+}
+
 // Self-play launches run one iteration ahead of the host (run_wave, mz_api.cu): a CTA none of whose slots has a ply to search -- every
 // CTA of the iteration queued past the end of a wave -- returns at its first instruction, before any barrier, TMA or TMEM state exists.
 template <int MODE>
@@ -226,70 +291,43 @@ __device__ __forceinline__ bool mz_cta_idle(const mz_params &P, const mz_search_
     return __syncthreads_or(any) == 0;
 }
 
-template <int MODE, int GT = MZ_GROUP, bool BN = false>
-__global__ void __launch_bounds__(2 * GT) mz_k_search(const __grid_constant__ mz_params P, const mz_search_args a) {
+template <int MODE, bool BN = false>
+__global__ void __launch_bounds__(MZ_THREADS) mz_k_search(const __grid_constant__ mz_params P, const mz_search_args a) {
     extern __shared__ __align__(128) unsigned char mz_smem[];
     if (mz_cta_idle<MODE>(P, a, MZ_ROWS)) return;
     const mz_smem_plan sp = mz_smem_carve(mz_smem, a.max_dim, a.max_layer_floats, P.hidden_pad, P.S);
-    constexpr int NT = 2 * GT;
     const int tid = threadIdx.x;
     const int r = tid >> 3, ln = tid & (MZ_LANES - 1);              // tree (row) of this thread and its lane within the tree
     const uint32_t segmask = 0xffu << ((tid & 31) & ~7);
     const int64_t g = (int64_t)blockIdx.x * MZ_ROWS + r;
     mz_nn_pipe pipe;
-    mz_pipe_init<GT>(pipe, sp, a.wglob);
-    mz_zero_activations<NT>(sp, a.max_dim);
+    mz_pipe_init(pipe, sp, a.wglob);
+    mz_zero_activations(sp, a.max_dim);
     uint16_t *path = sp.path + (size_t)r * (P.S + 2);
 
     // ---- per-tree state, replicated in the 8 lanes of the tree ----
-    bool active = false; uint32_t legal = 0, game = 0, move = 0; int to_play = 1;
     mz_tree tree; tree.A = nullptr; tree.hidden = nullptr;
-    if (r < MZ_ROWS && g < a.n) {
-        tree = mz_tree_at(P, a.tree_pool, g);
-        if (MODE == MZ_MODE_API) {
-            active = true; legal = a.legal[g]; to_play = a.to_play[g]; game = (uint32_t)a.game_id[g]; move = (uint32_t)a.move_idx[g];
-        } else {
-            active = a.slots.status[g] == MZ_SLOT_ACTIVE && (P.arena_player == 0 || a.slots.player[g] == P.arena_player);   // competitive play: MuZero's plies only
-            if (active) {
-                mz_board b; b.p1 = a.slots.p1[g]; b.p2 = a.slots.p2[g]; b.player = a.slots.player[g];
-                legal = mz_env_legal_b(P, b); to_play = b.player;                       // SelfPlay.jl:351,359
-                game = (uint32_t)a.slots.game_id[g]; move = (uint32_t)a.slots.T[g] + 1u;
-            }
-        }
-        if (legal == 0) active = false;   // run_mcts asserts !isempty(legal_actions) (SelfPlay.jl:243); never reached in play
-    }
-    uint32_t posmask = 0;                 // legal actions as a mask over Dict positions
-    for (int j = 0; j < P.A; j++) if ((legal >> (P.order[j] - 1)) & 1u) posmask |= 1u << j;
+    if (g < a.n) tree = mz_tree_at(P, a.tree_pool, g);
+    const mz_root root = mz_root_begin<MODE>(P, a, g, g < a.n);
+    const bool active = root.active;
     __syncthreads();   // mbarrier init + zeroed buffers visible
     const int pred_first = P.nets[1].first, dyn_first = P.nets[2].first;
     if (tid == 0) mz_nn_issue(pipe, P, P.nets[0].first, 0);            // group 0: representation, then prediction
-    if (tid == GT) mz_nn_issue(pipe, P, dyn_first, 0);           // group 1: dynamics (first used in simulation 1)
+    if (tid == MZ_GROUP) mz_nn_issue(pipe, P, dyn_first, 0);     // group 1: dynamics (first used in simulation 1)
 
     // ---- stage the stacked observations, k-major (get_stacked_observations, SelfPlay.jl:128-149) ----
-    if (MODE == MZ_MODE_API) {
-        for (int i = tid; i < MZ_ROWS * P.stack_size; i += NT) {
-            int rr = i / P.stack_size, k = i % P.stack_size;
-            int64_t gg = (int64_t)blockIdx.x * MZ_ROWS + rr;
-            sp.in0[k * MZ_ROWS + rr] = gg < a.n ? a.stacked[gg * P.stack_size + k] : 0.0f;
-        }
-    } else {
-        for (int i = tid; i < MZ_ROWS * P.stack_size; i += NT) {
-            int k = i / MZ_ROWS, rr = i % MZ_ROWS;
-            int64_t gg = (int64_t)blockIdx.x * MZ_ROWS + rr;
-            float v = 0.0f;
-            if (gg < a.n && a.slots.status[gg] == MZ_SLOT_ACTIVE) {
-                int T = a.slots.T[gg];
-                v = mz_stacked_value(P, a.slots.h_p1 + gg * P.Tmax, a.slots.h_p2 + gg * P.Tmax, a.slots.h_action + gg * P.Tmax, T + 1, k);
-            }
-            sp.in0[k * MZ_ROWS + rr] = v;
-        }
+    for (int i = tid; i < MZ_ROWS * P.stack_size; i += MZ_THREADS) {
+        int rr, k;
+        if (MODE == MZ_MODE_API) { rr = i / P.stack_size; k = i % P.stack_size; }   // the caller's rows are contiguous
+        else { k = i / MZ_ROWS; rr = i % MZ_ROWS; }
+        sp.in0[k * MZ_ROWS + rr] = mz_root_obs<MODE>(P, a, (int64_t)blockIdx.x * MZ_ROWS + rr, k);
     }
     __syncthreads();
 
     // ---- root: representation -> h0; prediction(h0) -> (v0, p0)  (SelfPlay.jl:233-245), group 0 only ----
     if (pipe.grp == 0) {
-        mz_nn_net<GT, BN>(pipe, P, 0, pred_first, sp.in0, sp.bufT[0], sp.outH, nullptr, sp.t0[0], sp.t1[0]);
-        mz_nn_net<GT, BN>(pipe, P, 1, pred_first, sp.outH, sp.bufT[0], sp.outV, sp.outL, sp.t0[0], sp.t1[0]);   // prefetches simulation 1's first layer
+        mz_nn_net<BN>(pipe, P, 0, pred_first, sp.in0, sp.bufT[0], sp.outH, nullptr, sp.t0[0], sp.t1[0]);
+        mz_nn_net<BN>(pipe, P, 1, pred_first, sp.outH, sp.bufT[0], sp.outV, sp.outL, sp.t0[0], sp.t1[0]);   // prefetches simulation 1's first layer
     }
     __syncthreads();
 
@@ -298,14 +336,7 @@ __global__ void __launch_bounds__(2 * GT) mz_k_search(const __grid_constant__ mz
     MZ_TIMER_DECL;
     if (active) {
         for (int k = ln; k < P.hidden; k += MZ_LANES) tree.hidden[k] = sp.outH[k * MZ_ROWS + r];
-        if (ln == 0) {
-            mz_f4 root; root.x = mz_bits2f(mz_nx_pack(0, -1, 0)); root.y = 0.0f; root.z = 0.0f; root.w = 0.0f;   // Node(prior=0), :232
-            tree.A[0] = root;
-        }
-        __syncwarp(segmask);
-        mz_tree_expand_lanes(P, tree, 0, 0, legal, sp.outL + r, 0.0f, 0.0f, ln, segmask);        // :245
-        if (ln == 0 && a.exploration && P.exploration_eps != 0.0f) mz_tree_add_noise(P, tree, legal, game, move);   // :247-249 (eps = 0 is the identity)
-        __syncwarp(segmask);
+        mz_root_init(P, tree, root, a.exploration, sp.outL + r, MZ_ROWS, ln, segmask);
     }
 
     // ---- simulations (SelfPlay.jl:254-283) ----
@@ -313,7 +344,7 @@ __global__ void __launch_bounds__(2 * GT) mz_k_search(const __grid_constant__ mz
         mz_leaf leaf; leaf.node = 0; leaf.parent = 0; leaf.action = 1; leaf.depth = 0; leaf.prior = 0.0f; leaf.parent_x = 0;
         MZ_TIMER(0);
         if (active) {
-            leaf = mz_tree_select_lanes(P, tree, a.pbc0, a.sqrtN, legal, posmask, mm, game, move, (uint32_t)sim, ln, segmask, path);
+            leaf = mz_tree_select_lanes(P, tree, a.pbc0, a.sqrtN, root.legal, root.posmask, mm, root.game, root.move, (uint32_t)sim, ln, segmask, path);
             depth_sum += (unsigned long long)leaf.depth;
             MZ_TIMER(1);
             const int pe = mz_nx_exp(leaf.parent_x), dbl = mz_nx_dbl(leaf.parent_x);
@@ -332,8 +363,8 @@ __global__ void __launch_bounds__(2 * GT) mz_k_search(const __grid_constant__ mz
         MZ_TIMER(2);
         __syncthreads();
         MZ_TIMER(3);
-        if (pipe.grp == 0) mz_nn_net<GT, BN>(pipe, P, 1, sim < P.S ? pred_first : -1, sp.in1, sp.bufT[0], sp.outV, sp.outL, sp.t0[0], sp.t1[0]);
-        else               mz_nn_net<GT, BN>(pipe, P, 2, sim < P.S ? dyn_first : -1, sp.in0, sp.bufT[1], sp.outH, sp.outR, sp.t0[1], sp.t1[1]);
+        if (pipe.grp == 0) mz_nn_net<BN>(pipe, P, 1, sim < P.S ? pred_first : -1, sp.in1, sp.bufT[0], sp.outV, sp.outL, sp.t0[0], sp.t1[0]);
+        else               mz_nn_net<BN>(pipe, P, 2, sim < P.S ? dyn_first : -1, sp.in0, sp.bufT[1], sp.outH, sp.outR, sp.t0[1], sp.t1[1]);
         MZ_TIMER(4);
         __syncthreads();
         MZ_TIMER(5);
@@ -341,7 +372,7 @@ __global__ void __launch_bounds__(2 * GT) mz_k_search(const __grid_constant__ mz
             float *nh = tree.hidden + (size_t)sim * P.hidden_pad;
             for (int k = ln; k < P.hidden; k += MZ_LANES) nh[k] = sp.outH[k * MZ_ROWS + r];
             MZ_TIMER(6);
-            mz_tree_expand_lanes(P, tree, leaf.node, sim, legal, sp.outL + r, sp.outR[r], leaf.prior, ln, segmask);   // :280 (root's legal set, Q7)
+            mz_tree_expand_lanes(P, tree, leaf.node, sim, root.legal, sp.outL + r, sp.outR[r], leaf.prior, ln, segmask);   // :280 (root's legal set, Q7)
             MZ_TIMER(7);
             mz_tree_backup_lanes(P, tree, path, leaf.depth, sp.outV[r], mm, ln, segmask);                  // :281
         }
@@ -351,30 +382,7 @@ __global__ void __launch_bounds__(2 * GT) mz_k_search(const __grid_constant__ mz
     }
 
     MZ_TIMER_FLUSH(a.stats);
-    // ---- results (lane 0 of each tree) ----
-    if (active && ln == 0) {
-        int32_t vc[MZ_MAX_A]; int sum_visits = 0, nlegal = 0;
-        for (int i = 0; i < P.A; i++) {
-            vc[i] = ((legal >> i) & 1u) ? (int32_t)mz_nx_visit(mz_f2bits(tree.A[1 + i].x)) : 0;
-            sum_visits += vc[i]; nlegal += (int)((legal >> i) & 1u);
-        }
-        mz_f4 root = tree.A[0];
-        int rvc = mz_nx_visit(mz_f2bits(root.x));
-        float rv = rvc == 0 ? 0.0f : root.y / (float)rvc;                                   // node_value(root)
-        if (a.stats) {
-            atomicAdd(&a.stats[0], depth_sum); atomicAdd(&a.stats[1], (unsigned long long)P.S);
-            atomicAdd(&a.stats[2], (unsigned long long)nlegal); atomicAdd(&a.stats[3], 1ull);
-        }
-        if (MODE == MZ_MODE_API) {
-            for (int i = 0; i < P.A; i++) {
-                a.visit_counts[g * P.A + i] = vc[i];
-                if (a.root_priors) a.root_priors[g * P.A + i] = ((legal >> i) & 1u) ? tree.A[1 + i].z : 0.0f;
-            }
-            a.root_value[g] = rv;
-        } else {
-            mz_slot_epilogue(P, a.slots, g, vc, sum_visits, legal, rv, a.temperature, game, move);
-        }
-    }
+    if (active && ln == 0) mz_root_finish<MODE>(P, a, g, tree, root, depth_sum);
 }
 
 // Initial priorities of one stored game (save_game, ReplayBuffer.jl:136-145): |root_value - compute_target_value|^alpha per
@@ -595,7 +603,7 @@ __global__ void __launch_bounds__(MZ_THREADS) mz_k_nn_forward(const __grid_const
     }
     __syncthreads();
     float *h1 = a.net == 1 ? sp.outV : sp.outH, *h2 = a.net == 1 ? sp.outL : sp.outR;
-    if (pipe.grp == 0) mz_nn_net<MZ_GROUP, BN>(pipe, P, a.net, -1, sp.in0, sp.bufT[0], h1, h2, sp.t0[0], sp.t1[0]);
+    if (pipe.grp == 0) mz_nn_net<BN>(pipe, P, a.net, -1, sp.in0, sp.bufT[0], h1, h2, sp.t0[0], sp.t1[0]);
     __syncthreads();
     const int64_t g = (int64_t)blockIdx.x * MZ_ROWS + tid;
     if (tid < MZ_ROWS && g < a.B) {
@@ -640,8 +648,8 @@ __global__ void __launch_bounds__(MZ_THREADS) mz_k_reanalyse(const __grid_consta
     }
     __syncthreads();
     if (pipe.grp == 0) {
-        mz_nn_net<MZ_GROUP, BN>(pipe, P, 0, P.nets[1].first, sp.in0, sp.bufT[0], sp.outH, nullptr, sp.t0[0], sp.t1[0]);
-        mz_nn_net<MZ_GROUP, BN>(pipe, P, 1, -1, sp.outH, sp.bufT[0], sp.outV, sp.outL, sp.t0[0], sp.t1[0]);
+        mz_nn_net<BN>(pipe, P, 0, P.nets[1].first, sp.in0, sp.bufT[0], sp.outH, nullptr, sp.t0[0], sp.t1[0]);
+        mz_nn_net<BN>(pipe, P, 1, -1, sp.outH, sp.bufT[0], sp.outV, sp.outL, sp.t0[0], sp.t1[0]);
     }
     __syncthreads();
     const int64_t item = (int64_t)blockIdx.x * MZ_ROWS + tid;

@@ -206,30 +206,18 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(MZ_LAT_THREADS) mz_k
     const int ln = tid & (MZ_LANES - 1);
     const uint32_t segmask = 0xffu;
     const bool lanes = rank == 0 && tid < MZ_LANES;                     // the 8 lanes that own the tree
-    bool active = false; uint32_t legal = 0, game = 0, move = 0;
+    const mz_root root = mz_root_begin<MODE>(P, a, g, rank == 0);
     mz_tree tree; tree.A = (mz_f4 *)sp.tree; tree.hidden = (float *)(sp.tree + P.hidden_off_bytes);
     const double *pbc = a.pbc0;
     if (rank == 0) {
-        if (MODE == MZ_MODE_API) { active = true; legal = a.legal[g]; game = (uint32_t)a.game_id[g]; move = (uint32_t)a.move_idx[g]; }
-        else {
-            mz_board b; b.p1 = a.slots.p1[g]; b.p2 = a.slots.p2[g]; b.player = a.slots.player[g];
-            active = true; legal = mz_env_legal_b(P, b); game = (uint32_t)a.slots.game_id[g]; move = (uint32_t)a.slots.T[g] + 1u;
-        }
-        if (legal == 0) active = false;
         if (la.pbc_smem) {                                              // compact copy of ucb_score's table: row N holds n = 0..N
             for (int N = tid; N < P.S + 2; N += MZ_LAT_THREADS) for (int n = 0; n <= N; n++) sp.pbc[(N * (N + 1)) / 2 + n] = a.pbc0[N * (P.S + 2) + n];
             pbc = sp.pbc;
         }
         // stacked observations (get_stacked_observations, SelfPlay.jl:128-149)
-        for (int k = tid; k < P.stack_size; k += MZ_LAT_THREADS) {
-            float v;
-            if (MODE == MZ_MODE_API) v = a.stacked[g * P.stack_size + k];
-            else v = mz_stacked_value(P, a.slots.h_p1 + g * P.Tmax, a.slots.h_p2 + g * P.Tmax, a.slots.h_action + g * P.Tmax, a.slots.T[g] + 1, k);
-            sp.xin[k] = v;
-        }
+        for (int k = tid; k < P.stack_size; k += MZ_LAT_THREADS) sp.xin[k] = mz_root_obs<MODE>(P, a, g, k);
     }
-    uint32_t posmask = 0;
-    for (int j = 0; j < P.A; j++) if ((legal >> (P.order[j] - 1)) & 1u) posmask |= 1u << j;
+    const bool active = root.active;
     __syncthreads();
     mz_mbar_wait(sp.mbar, 0);
     cluster.sync();                                                     // both CTAs are resident: distributed shared memory may be written
@@ -250,7 +238,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(MZ_LAT_THREADS) mz_k
     for (int it = rank == 0 ? -1 : 1; it <= P.S; it++) {
         MZ_LT(7);
         if (lanes && active && it >= 1) {
-            leaf = mz_tree_select_lanes(P, tree, pbc, a.sqrtN, legal, posmask, mm, game, move, (uint32_t)it, ln, segmask, sp.path, la.pbc_smem != 0);
+            leaf = mz_tree_select_lanes(P, tree, pbc, a.sqrtN, root.legal, root.posmask, mm, root.game, root.move, (uint32_t)it, ln, segmask, sp.path, la.pbc_smem != 0);
             depth_sum += (unsigned long long)leaf.depth;
             MZ_LT(0);
             const int pe = mz_nx_exp(leaf.parent_x), dbl = mz_nx_dbl(leaf.parent_x);
@@ -280,12 +268,15 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(MZ_LAT_THREADS) mz_k
         if (lanes && active && it >= 0) {
             float *nh = tree.hidden + (size_t)it * P.hidden_pad;
             for (int k = ln; k < P.hidden; k += MZ_LANES) nh[k] = sp.outH[k];
-            if (it == 0 && ln == 0) { mz_f4 root; root.x = mz_bits2f(mz_nx_pack(0, -1, 0)); root.y = 0.0f; root.z = 0.0f; root.w = 0.0f; tree.A[0] = root; }   // Node(prior=0), :232
+            // the root's expansion shares the simulations' call site instead of calling mz_root_init: with a second inlined expansion this
+            // kernel compiled (sm_100a, -Xptxas -v, cuobjdump -sass) to 6680 instead of 6008 SASS instructions and 241 instead of 239 registers
+            // in MODE_API, 8000 instead of 7320 instructions in MODE_SLOTS
+            if (it == 0 && ln == 0) { mz_f4 node; node.x = mz_bits2f(mz_nx_pack(0, -1, 0)); node.y = 0.0f; node.z = 0.0f; node.w = 0.0f; tree.A[0] = node; }   // Node(prior=0), :232
             __syncwarp(segmask);
-            mz_tree_expand_lanes(P, tree, it == 0 ? 0 : leaf.node, it, legal, sp.outL, it == 0 ? 0.0f : sp.outR[0], it == 0 ? 0.0f : leaf.prior, ln, segmask, 1);   // :245, :280 (Q7)
+            mz_tree_expand_lanes(P, tree, it == 0 ? 0 : leaf.node, it, root.legal, sp.outL, it == 0 ? 0.0f : sp.outR[0], it == 0 ? 0.0f : leaf.prior, ln, segmask, 1);   // :245, :280 (Q7)
             MZ_LT(5);
             if (it == 0) {
-                if (ln == 0 && a.exploration && P.exploration_eps != 0.0f) mz_lat_add_noise(P, tree.A, tree.hidden, legal, game, move);   // :247-249
+                if (ln == 0 && a.exploration && P.exploration_eps != 0.0f) mz_lat_add_noise(P, tree.A, tree.hidden, root.legal, root.game, root.move);   // :247-249
                 __syncwarp(segmask);
             } else mz_tree_backup_lanes(P, tree, sp.path, leaf.depth, sp.outV[0], mm, ln, segmask);                         // :281
         }
@@ -296,26 +287,5 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(MZ_LAT_THREADS) mz_k
     if (tid == 0 && g == 0) printf("lat timers (cycles / simulation): select %lld stage %lld sync1 %lld pred %lld sync2(wait dyn) %lld expand %lld backup %lld loop %lld\n",
                                    lt[0] / P.S, lt[1] / P.S, lt[2] / P.S, lt[3] / P.S, lt[4] / P.S, lt[5] / P.S, lt[6] / P.S, lt[7] / P.S);
 #endif
-    // ---- results (lane 0), identical to mz_k_search ----
-    if (lanes && active && ln == 0) {
-        int32_t vc[MZ_MAX_A]; int sum_visits = 0, nlegal = 0;
-        for (int i = 0; i < P.A; i++) {
-            vc[i] = ((legal >> i) & 1u) ? (int32_t)mz_nx_visit(mz_f2bits(tree.A[1 + i].x)) : 0;
-            sum_visits += vc[i]; nlegal += (int)((legal >> i) & 1u);
-        }
-        const mz_f4 root = tree.A[0];
-        const int rvc = mz_nx_visit(mz_f2bits(root.x));
-        const float rv = rvc == 0 ? 0.0f : root.y / (float)rvc;
-        if (a.stats) {
-            atomicAdd(&a.stats[0], depth_sum); atomicAdd(&a.stats[1], (unsigned long long)P.S);
-            atomicAdd(&a.stats[2], (unsigned long long)nlegal); atomicAdd(&a.stats[3], 1ull);
-        }
-        if (MODE == MZ_MODE_API) {
-            for (int i = 0; i < P.A; i++) {
-                a.visit_counts[g * P.A + i] = vc[i];
-                if (a.root_priors) a.root_priors[g * P.A + i] = ((legal >> i) & 1u) ? tree.A[1 + i].z : 0.0f;
-            }
-            a.root_value[g] = rv;
-        } else mz_slot_epilogue(P, a.slots, g, vc, sum_visits, legal, rv, a.temperature, game, move);
-    }
+    if (lanes && active && ln == 0) mz_root_finish<MODE>(P, a, g, tree, root, depth_sum);
 }

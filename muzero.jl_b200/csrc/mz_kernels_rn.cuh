@@ -507,41 +507,23 @@ __global__ void __launch_bounds__(MZ_RN_THREADS) mz_k_search_rn(const __grid_con
     const uint32_t segmask = 0xffu << ((tid & 31) & ~7);
 
     // ---- per-tree state: 64 trees x 8 lanes, replicated in the lanes of each tree ----
-    bool active[MZ_RN_NPASS]; uint32_t legal[MZ_RN_NPASS], game[MZ_RN_NPASS], move[MZ_RN_NPASS], posmask[MZ_RN_NPASS]; mz_tree tree[MZ_RN_NPASS]; mz_minmax mm[MZ_RN_NPASS]; int ts[MZ_RN_NPASS]; int64_t gidx[MZ_RN_NPASS];
+    mz_root root[MZ_RN_NPASS]; mz_tree tree[MZ_RN_NPASS]; mz_minmax mm[MZ_RN_NPASS]; int ts[MZ_RN_NPASS]; int64_t gidx[MZ_RN_NPASS];
 #pragma unroll
     for (int p = 0; p < MZ_RN_NPASS; p++) {
         ts[p] = 64 * p + (tid >> 3); gidx[p] = (int64_t)blockIdx.x * R.ntrees + ts[p];
-        active[p] = false; legal[p] = 0; game[p] = 0; move[p] = 0; tree[p].A = nullptr; tree[p].hidden = nullptr;
+        root[p] = mz_root{}; tree[p].A = nullptr; tree[p].hidden = nullptr;
         if (ts[p] < R.ntrees && gidx[p] < a.n) {
-            const int64_t g = gidx[p];
-            tree[p] = mz_tree_at(P, a.tree_pool, g);
-            if (MODE == MZ_MODE_API) { active[p] = true; legal[p] = a.legal[g]; game[p] = (uint32_t)a.game_id[g]; move[p] = (uint32_t)a.move_idx[g]; }
-            else {
-                active[p] = a.slots.status[g] == MZ_SLOT_ACTIVE && (P.arena_player == 0 || a.slots.player[g] == P.arena_player);   // competitive play: MuZero's plies only
-                if (active[p]) {
-                    mz_board b; b.p1 = a.slots.p1[g]; b.p2 = a.slots.p2[g]; b.player = a.slots.player[g];
-                    legal[p] = mz_env_legal_b(P, b); game[p] = (uint32_t)a.slots.game_id[g]; move[p] = (uint32_t)a.slots.T[g] + 1u;
-                }
-            }
-            if (legal[p] == 0) active[p] = false;
-            if (ln == 0) { sp.active[ts[p]] = active[p] ? 1 : 0; sp.tree_base[ts[p]] = (unsigned long long)(uintptr_t)tree[p].A; }
+            tree[p] = mz_tree_at(P, a.tree_pool, gidx[p]);
+            root[p] = mz_root_begin<MODE>(P, a, gidx[p], true);
+            if (ln == 0) { sp.active[ts[p]] = root[p].active ? 1 : 0; sp.tree_base[ts[p]] = (unsigned long long)(uintptr_t)tree[p].A; }
         }
-        posmask[p] = 0;
-        for (int j = 0; j < P.A; j++) if ((legal[p] >> (P.order[j] - 1)) & 1u) posmask[p] |= 1u << j;
         mm[p].mn = INFINITY; mm[p].mx = -INFINITY;
     }
     __syncthreads();
     mz_rn_bind_rows(X, R);
 
     // ---- root: representation (im2col of the stacked observation) -> h0 in the pool; prediction(h0) ----
-    if (MODE == MZ_MODE_API) {
-        mz_rn_im2col(X, P, R, [&](int t, int pl, int cell) { return a.stacked[((int64_t)blockIdx.x * R.ntrees + t) * P.stack_size + cell + P.cells * pl]; });
-    } else {
-        mz_rn_im2col(X, P, R, [&](int t, int pl, int cell) {
-            const int64_t gg = (int64_t)blockIdx.x * R.ntrees + t;
-            return mz_stacked_value(P, a.slots.h_p1 + gg * P.Tmax, a.slots.h_p2 + gg * P.Tmax, a.slots.h_action + gg * P.Tmax, a.slots.T[gg] + 1, cell + P.cells * pl);
-        });
-    }
+    mz_rn_im2col(X, P, R, [&](int t, int pl, int cell) { return mz_root_obs<MODE>(P, a, (int64_t)blockIdx.x * R.ntrees + t, cell + P.cells * pl); });
     // ---- phases: 0 = representation (root), 1 = prediction(h0), then per simulation 2 = prediction(parent), 3 = dynamics.
     //      One loop so that the step executor is inlined exactly once. ----
     const float *outV = sp.out, *outL = sp.out + 4 * MZ_RN_OUT_ROWS, *outR = sp.out + 20 * MZ_RN_OUT_ROWS;
@@ -562,9 +544,9 @@ __global__ void __launch_bounds__(MZ_RN_THREADS) mz_k_search_rn(const __grid_con
 #pragma unroll
             for (int p = 0; p < MZ_RN_NPASS; p++) {
                 leaf[p].node = 0; leaf[p].parent = 0; leaf[p].action = 1; leaf[p].depth = 0; leaf[p].prior = 0.0f; leaf[p].parent_x = 0;
-                if (active[p]) {
+                if (root[p].active) {
                     uint16_t *path = sp.path + (size_t)ts[p] * (P.S + 2);
-                    leaf[p] = mz_tree_select_lanes(P, tree[p], a.pbc0, a.sqrtN, legal[p], posmask[p], mm[p], game[p], move[p], (uint32_t)sim, ln, segmask, path);
+                    leaf[p] = mz_tree_select_lanes(P, tree[p], a.pbc0, a.sqrtN, root[p].legal, root[p].posmask, mm[p], root[p].game, root[p].move, (uint32_t)sim, ln, segmask, path);
                     depth_sum += (unsigned long long)leaf[p].depth;
                     if (ln == 0) {
                         sp.pe[ts[p]] = mz_nx_exp(leaf[p].parent_x); sp.dbl[ts[p]] = mz_nx_dbl(leaf[p].parent_x);
@@ -589,20 +571,14 @@ __global__ void __launch_bounds__(MZ_RN_THREADS) mz_k_search_rn(const __grid_con
         if (phase == 1) {
 #pragma unroll
             for (int p = 0; p < MZ_RN_NPASS; p++) {
-                if (active[p]) {
-                    if (ln == 0) { mz_f4 root; root.x = mz_bits2f(mz_nx_pack(0, -1, 0)); root.y = 0.0f; root.z = 0.0f; root.w = 0.0f; tree[p].A[0] = root; }
-                    __syncwarp(segmask);
-                    mz_tree_expand_lanes(P, tree[p], 0, 0, legal[p], outL + ts[p], 0.0f, 0.0f, ln, segmask, MZ_RN_OUT_ROWS);
-                    if (ln == 0 && a.exploration && P.exploration_eps != 0.0f) mz_tree_add_noise(P, tree[p], legal[p], game[p], move[p]);
-                    __syncwarp(segmask);
-                }
+                if (root[p].active) mz_root_init(P, tree[p], root[p], a.exploration, outL + ts[p], MZ_RN_OUT_ROWS, ln, segmask);
             }
         } else if (phase == 3) {
 #pragma unroll
             for (int p = 0; p < MZ_RN_NPASS; p++) {
-                if (active[p]) {
+                if (root[p].active) {
                     const uint16_t *path = sp.path + (size_t)ts[p] * (P.S + 2);
-                    mz_tree_expand_lanes(P, tree[p], leaf[p].node, sim, legal[p], outL + ts[p], outR[ts[p]], leaf[p].prior, ln, segmask, MZ_RN_OUT_ROWS);
+                    mz_tree_expand_lanes(P, tree[p], leaf[p].node, sim, root[p].legal, outL + ts[p], outR[ts[p]], leaf[p].prior, ln, segmask, MZ_RN_OUT_ROWS);
                     mz_tree_backup_lanes(P, tree[p], path, leaf[p].depth, outV[ts[p]], mm[p], ln, segmask);
                 }
             }
@@ -614,49 +590,12 @@ __global__ void __launch_bounds__(MZ_RN_THREADS) mz_k_search_rn(const __grid_con
     if (a.stats && (tid == 0 || tid == 128)) { for (int i = 0; i < 6; i++) atomicAdd(&a.stats[41 + 7 * (tid >> 7) + i], (unsigned long long)X.st_t[i]); atomicAdd(&a.stats[47 + 7 * (tid >> 7)], (unsigned long long)X.wq); }
 #endif
 
-    // ---- results (lane 0 of each tree), as in mz_k_search ----
+    // ---- results (lane 0 of each tree): the trees' leaf depths are summed over the passes, so only the first pass adds them ----
 #pragma unroll
     for (int p = 0; p < MZ_RN_NPASS; p++) {
-        if (!(active[p] && ln == 0)) continue;
-        const int64_t g = gidx[p];
-        int32_t vc[MZ_MAX_A]; int sum_visits = 0, nlegal = 0;
-        for (int i = 0; i < P.A; i++) {
-            vc[i] = ((legal[p] >> i) & 1u) ? (int32_t)mz_nx_visit(mz_f2bits(tree[p].A[1 + i].x)) : 0;
-            sum_visits += vc[i]; nlegal += (int)((legal[p] >> i) & 1u);
-        }
-        mz_f4 root = tree[p].A[0];
-        int rvc = mz_nx_visit(mz_f2bits(root.x));
-        float rv = rvc == 0 ? 0.0f : root.y / (float)rvc;
-        if (a.stats) {
-            atomicAdd(&a.stats[0], depth_sum); atomicAdd(&a.stats[1], (unsigned long long)P.S);
-            atomicAdd(&a.stats[2], (unsigned long long)nlegal); atomicAdd(&a.stats[3], 1ull);
-            depth_sum = 0;
-        }
-        if (MODE == MZ_MODE_API) {
-            for (int i = 0; i < P.A; i++) {
-                a.visit_counts[g * P.A + i] = vc[i];
-                if (a.root_priors) a.root_priors[g * P.A + i] = ((legal[p] >> i) & 1u) ? tree[p].A[1 + i].z : 0.0f;
-            }
-            a.root_value[g] = rv;
-        } else {
-            int T = a.slots.T[g];
-            int action = mz_select_action_counts(P, vc, legal[p], mz_play_temperature(P, T, a.temperature), game[p], move[p]);
-            mz_board b; b.p1 = a.slots.p1[g]; b.p2 = a.slots.p2[g]; b.player = a.slots.player[g];
-            int pl = b.player;
-            mz_env_step_b(P, b, action);
-            float reward = (float)mz_env_reward_b(P, b, pl);
-            bool done = mz_env_terminated_b(P, b);
-            float *cv = a.slots.h_cv + ((size_t)g * P.Tmax + T) * P.A;
-            for (int i = 0; i < P.A; i++) cv[i] = ((legal[p] >> i) & 1u) ? (float)((double)vc[i] / (double)sum_visits) : 0.0f;
-            a.slots.h_rv[(size_t)g * P.Tmax + T] = rv;
-            a.slots.h_action[(size_t)g * P.Tmax + T] = action;
-            a.slots.h_reward[(size_t)g * P.Tmax + T] = reward;
-            a.slots.h_to_play[(size_t)g * P.Tmax + T] = (uint8_t)pl;
-            T += 1;
-            a.slots.p1[g] = b.p1; a.slots.p2[g] = b.p2; a.slots.player[g] = b.player; a.slots.T[g] = T;
-            if (T < P.Tmax) { a.slots.h_p1[(size_t)g * P.Tmax + T] = b.p1; a.slots.h_p2[(size_t)g * P.Tmax + T] = b.p2; }
-            if (done || T > P.max_moves) a.slots.status[g] = MZ_SLOT_FINISHED + P.fin_tag;
-        }
+        if (!(root[p].active && ln == 0)) continue;
+        mz_root_finish<MODE>(P, a, gidx[p], tree[p], root[p], depth_sum);
+        depth_sum = 0;
     }
     mz_rn_teardown(X);
 }

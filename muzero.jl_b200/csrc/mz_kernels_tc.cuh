@@ -65,40 +65,17 @@ __global__ void __launch_bounds__(MZ_THREADS) mz_k_search_tc(const __grid_consta
     uint16_t *path = sp.path + (size_t)r * (P.S + 2);
 
     // ---- per-tree state, replicated in the 8 lanes of the tree ----
-    bool active = false; uint32_t legal = 0, game = 0, move = 0; int to_play = 1;
     mz_tree tree; tree.A = nullptr; tree.hidden = nullptr;
-    if (g < a.n) {
-        tree = mz_tree_at(P, a.tree_pool, g);
-        if (MODE == MZ_MODE_API) {
-            active = true; legal = a.legal[g]; to_play = a.to_play[g]; game = (uint32_t)a.game_id[g]; move = (uint32_t)a.move_idx[g];
-        } else {
-            active = a.slots.status[g] == MZ_SLOT_ACTIVE && (P.arena_player == 0 || a.slots.player[g] == P.arena_player);   // competitive play: MuZero's plies only
-            if (active) {
-                mz_board b; b.p1 = a.slots.p1[g]; b.p2 = a.slots.p2[g]; b.player = a.slots.player[g];
-                legal = mz_env_legal_b(P, b); to_play = b.player;
-                game = (uint32_t)a.slots.game_id[g]; move = (uint32_t)a.slots.T[g] + 1u;
-            }
-        }
-        if (legal == 0) active = false;
-    }
-    (void)to_play;
-    uint32_t posmask = 0;
-    for (int j = 0; j < P.A; j++) if ((legal >> (P.order[j] - 1)) & 1u) posmask |= 1u << j;
+    if (g < a.n) tree = mz_tree_at(P, a.tree_pool, g);
+    const mz_root root = mz_root_begin<MODE>(P, a, g, g < a.n);
+    const bool active = root.active;
 
     // ---- stage the stacked observations as a bf16 B tile (values are 0/1 and raw action indices: exact in bf16) ----
     for (int i = tid; i < MZ_ROWS * P.stack_size; i += MZ_THREADS) {
-        float v = 0.0f; int rr, k;
-        if (MODE == MZ_MODE_API) {
-            rr = i / P.stack_size; k = i % P.stack_size;
-            int64_t gg = (int64_t)blockIdx.x * MZ_ROWS + rr;
-            if (gg < a.n) v = a.stacked[gg * P.stack_size + k];
-        } else {
-            k = i / MZ_ROWS; rr = i % MZ_ROWS;
-            int64_t gg = (int64_t)blockIdx.x * MZ_ROWS + rr;
-            if (gg < a.n && a.slots.status[gg] == MZ_SLOT_ACTIVE)
-                v = mz_stacked_value(P, a.slots.h_p1 + gg * P.Tmax, a.slots.h_p2 + gg * P.Tmax, a.slots.h_action + gg * P.Tmax, a.slots.T[gg] + 1, k);
-        }
-        mz_tc_store_bf16(sp.inS, rr, k, v);
+        int rr, k;
+        if (MODE == MZ_MODE_API) { rr = i / P.stack_size; k = i % P.stack_size; }
+        else { k = i / MZ_ROWS; rr = i % MZ_ROWS; }
+        mz_tc_store_bf16(sp.inS, rr, k, mz_root_obs<MODE>(P, a, (int64_t)blockIdx.x * MZ_ROWS + rr, k));
     }
     mz_fence_proxy_async();
     mz_mbar_wait(sp.mbar_w, 0);          // weights + biases have landed
@@ -119,14 +96,7 @@ __global__ void __launch_bounds__(MZ_THREADS) mz_k_search_tc(const __grid_consta
     MZ_TIMER_DECL;
     if (active) {
         for (int k = ln; k < P.hidden; k += MZ_LANES) tree.hidden[k] = sp.outH[k * MZ_ROWS + r];
-        if (ln == 0) {
-            mz_f4 root; root.x = mz_bits2f(mz_nx_pack(0, -1, 0)); root.y = 0.0f; root.z = 0.0f; root.w = 0.0f;
-            tree.A[0] = root;
-        }
-        __syncwarp(segmask);
-        mz_tree_expand_lanes(P, tree, 0, 0, legal, sp.outL + r, 0.0f, 0.0f, ln, segmask);
-        if (ln == 0 && a.exploration && P.exploration_eps != 0.0f) mz_tree_add_noise(P, tree, legal, game, move);
-        __syncwarp(segmask);
+        mz_root_init(P, tree, root, a.exploration, sp.outL + r, MZ_ROWS, ln, segmask);
     }
 
     // ---- simulations ----
@@ -134,7 +104,7 @@ __global__ void __launch_bounds__(MZ_THREADS) mz_k_search_tc(const __grid_consta
         mz_leaf leaf; leaf.node = 0; leaf.parent = 0; leaf.action = 1; leaf.depth = 0; leaf.prior = 0.0f; leaf.parent_x = 0;
         MZ_TIMER(0);
         if (active) {
-            leaf = mz_tree_select_lanes(P, tree, a.pbc0, a.sqrtN, legal, posmask, mm, game, move, (uint32_t)sim, ln, segmask, path);
+            leaf = mz_tree_select_lanes(P, tree, a.pbc0, a.sqrtN, root.legal, root.posmask, mm, root.game, root.move, (uint32_t)sim, ln, segmask, path);
             depth_sum += (unsigned long long)leaf.depth;
             MZ_TIMER(1);
             const int pe = mz_nx_exp(leaf.parent_x), dbl = mz_nx_dbl(leaf.parent_x);
@@ -163,7 +133,7 @@ __global__ void __launch_bounds__(MZ_THREADS) mz_k_search_tc(const __grid_consta
             float *nh = tree.hidden + (size_t)sim * P.hidden_pad;
             for (int k = ln; k < P.hidden; k += MZ_LANES) nh[k] = sp.outH[k * MZ_ROWS + r];
             MZ_TIMER(6);
-            mz_tree_expand_lanes(P, tree, leaf.node, sim, legal, sp.outL + r, sp.outR[r], leaf.prior, ln, segmask);
+            mz_tree_expand_lanes(P, tree, leaf.node, sim, root.legal, sp.outL + r, sp.outR[r], leaf.prior, ln, segmask);
             MZ_TIMER(7);
             mz_tree_backup_lanes(P, tree, path, leaf.depth, sp.outV[r], mm, ln, segmask);
         }
@@ -174,30 +144,7 @@ __global__ void __launch_bounds__(MZ_THREADS) mz_k_search_tc(const __grid_consta
 #ifdef MZ_PHASE_TIMERS
     if (a.stats && tk) { int o_ = tid == 0 ? 16 : 24; for (int i_ = 0; i_ < 6; i_++) atomicAdd(&a.stats[o_ + i_], (unsigned long long)rt[i_]); atomicAdd(&a.stats[o_ + 6], (unsigned long long)q); }
 #endif
-    // ---- results (lane 0 of each tree), identical to mz_k_search ----
-    if (active && ln == 0) {
-        int32_t vc[MZ_MAX_A]; int sum_visits = 0, nlegal = 0;
-        for (int i = 0; i < P.A; i++) {
-            vc[i] = ((legal >> i) & 1u) ? (int32_t)mz_nx_visit(mz_f2bits(tree.A[1 + i].x)) : 0;
-            sum_visits += vc[i]; nlegal += (int)((legal >> i) & 1u);
-        }
-        mz_f4 root = tree.A[0];
-        int rvc = mz_nx_visit(mz_f2bits(root.x));
-        float rv = rvc == 0 ? 0.0f : root.y / (float)rvc;
-        if (a.stats) {
-            atomicAdd(&a.stats[0], depth_sum); atomicAdd(&a.stats[1], (unsigned long long)P.S);
-            atomicAdd(&a.stats[2], (unsigned long long)nlegal); atomicAdd(&a.stats[3], 1ull);
-        }
-        if (MODE == MZ_MODE_API) {
-            for (int i = 0; i < P.A; i++) {
-                a.visit_counts[g * P.A + i] = vc[i];
-                if (a.root_priors) a.root_priors[g * P.A + i] = ((legal >> i) & 1u) ? tree.A[1 + i].z : 0.0f;
-            }
-            a.root_value[g] = rv;
-        } else {
-            mz_slot_epilogue(P, a.slots, g, vc, sum_visits, legal, rv, a.temperature, game, move);
-        }
-    }
+    if (active && ln == 0) mz_root_finish<MODE>(P, a, g, tree, root, depth_sum);
     // ---- teardown: every tcgen05 operation has completed (all layers were waited on) ----
     mz_tc_fence_before();
     __syncthreads();

@@ -109,8 +109,8 @@ __global__ void __launch_bounds__(MZ_THREADS) mz_k_learn_forward(const __grid_co
     __syncthreads();
     // representation (:347) then row 0 = prediction(h0) (:351) on group 0; in1 keeps the current hidden state
     if (pipe.grp == 0) {
-        mz_nn_net<MZ_GROUP, BN>(pipe, P, 0, pred_first, sp.in0, sp.bufT[0], sp.in1, nullptr, sp.t0[0], sp.t1[0]);
-        mz_nn_net<MZ_GROUP, BN>(pipe, P, 1, P.K > 0 ? pred_first : -1, sp.in1, sp.bufT[0], sp.outV, sp.outL, sp.t0[0], sp.t1[0]);
+        mz_nn_net<BN>(pipe, P, 0, pred_first, sp.in0, sp.bufT[0], sp.in1, nullptr, sp.t0[0], sp.t1[0]);
+        mz_nn_net<BN>(pipe, P, 1, P.K > 0 ? pred_first : -1, sp.in1, sp.bufT[0], sp.outV, sp.outL, sp.t0[0], sp.t1[0]);
     }
     __syncthreads();
     for (int i = 0; i <= P.K; i++) {
@@ -133,8 +133,8 @@ __global__ void __launch_bounds__(MZ_THREADS) mz_k_learn_forward(const __grid_co
         }
         __syncthreads();
         const bool more = i + 1 < P.K;
-        if (pipe.grp == 0) mz_nn_net<MZ_GROUP, BN>(pipe, P, 1, more ? pred_first : -1, sp.in1, sp.bufT[0], sp.outV, sp.outL, sp.t0[0], sp.t1[0]);   // :356
-        else               mz_nn_net<MZ_GROUP, BN>(pipe, P, 2, more ? dyn_first : -1, sp.in0, sp.bufT[1], sp.outH, sp.outR, sp.t0[1], sp.t1[1]);     // :362
+        if (pipe.grp == 0) mz_nn_net<BN>(pipe, P, 1, more ? pred_first : -1, sp.in1, sp.bufT[0], sp.outV, sp.outL, sp.t0[0], sp.t1[0]);   // :356
+        else               mz_nn_net<BN>(pipe, P, 2, more ? dyn_first : -1, sp.in0, sp.bufT[1], sp.outH, sp.outR, sp.t0[1], sp.t1[1]);     // :362
         __syncthreads();
         for (int k = tid; k < P.hidden * MZ_ROWS; k += MZ_THREADS) sp.in1[k] = sp.outH[k];          // h_{i+1}
         __syncthreads();
