@@ -185,6 +185,16 @@ int mz_replay_clear(mz_ctx *ctx);
  * counter); from then on get_batch / mz_learn_step bootstrap those games' value targets from the reanalysed values. */
 int mz_reanalyse(mz_ctx *ctx, int64_t key0, int n);
 int mz_reanalysed_export(mz_ctx *ctx, int64_t key0, int n, float *values /* [n][Tmax] */, int32_t *is_set /* [n]: 0 = nothing */);
+/* MuZero Reanalyze: for every stored position t < T of games key0 .. key0+n-1, run_mcts (src/SelfPlay.jl:230-285) again with the
+ * CURRENT networks on the context's network path, from the root self-play searched there: stacked observation
+ * get_stacked_observations(history, t+1), the legal actions of the stored board, the stored game id, move index t + 1, and every
+ * Philox draw (Dirichlet noise when exploration != 0, tie-breaks) keyed by (game id, t + 1).  child_visits[t] receives the visit
+ * distribution (store_search_stats!, src/SelfPlay.jl:115-122) and reanalysed_predicted_root_values[t] node_value(root) (0 for t >= T);
+ * the games' values are marked as set, so get_batch bootstraps from them.  Nothing else changes -- in particular root_values and the
+ * PER priorities stay as stored.  The results depend neither on num_slots nor on the other games of the call.  Every network path is
+ * supported.  *simulations (may be NULL) = simulations run.  MZ_E_ARG for n < 0 or keys outside the buffer, MZ_E_STATE while
+ * self-play is in progress. */
+int mz_reanalyse_search(mz_ctx *ctx, int64_t key0, int n, int exploration, int64_t *simulations);
 /* checkpoint / resume of the replay state (the reference never persists its buffer, main.jl:21 TODO): the three save_game counters
  * (num_played_games, num_played_steps, total_samples; ReplayBuffer.jl:147-152) and, per stored game, what mz_history_import does not carry:
  * history.priorities / game_priority as updated by update_priorities! and reanalysed_predicted_root_values.  Resume = mz_replay_clear,

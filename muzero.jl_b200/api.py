@@ -386,6 +386,13 @@ def reanalyse(engine: Engine, key0=None, n=None):
     engine.ctx.reanalyse(key0, n)
 
 
+def reanalyse_search(engine: Engine, key0=None, n=None, exploration=False):
+    """MuZero Reanalyze: run_mcts again at every stored position of games key0 .. key0+n-1 (default: the whole buffer) with the
+    current networks, from the root self-play searched there.  Refreshes the policy target (child_visits) and the value target
+    (reanalysed_predicted_root_values); PER priorities stay as stored.  Returns the number of simulations run."""
+    return engine.ctx.reanalyse_search(key0, n, exploration)
+
+
 def learning(engine: Engine, steps: int, grad_mode=capi.GRAD_REFERENCE_L2, log_every=0):
     """learning! (Learning.jl:306-438): `steps` iterations of get_batch -> unroll -> loss -> gradients -> ADAM(Cos schedule).
     Returns the three losses (representation, prediction, dynamics) of the last step."""

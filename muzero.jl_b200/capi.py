@@ -109,6 +109,7 @@ def lib():
         "mz_replay_clear": ([ctx], C.c_int),
         "mz_reanalyse": ([ctx, C.c_int64, C.c_int], C.c_int),
         "mz_reanalysed_export": ([ctx, C.c_int64, C.c_int, f32p, i32p], C.c_int),
+        "mz_reanalyse_search": ([ctx, C.c_int64, C.c_int, C.c_int, i64p], C.c_int),
         "mz_replay_counters": ([ctx, i64p], C.c_int),
         "mz_replay_set_counters": ([ctx, C.c_int64, C.c_int64, C.c_int64], C.c_int),
         "mz_replay_set_priorities": ([ctx, C.c_int64, C.c_int, u32p, u32p], C.c_int),
@@ -429,6 +430,16 @@ class Context:
         n = info["n_games"] - (key0 - info["first_key"]) if n is None else n
         self._ck(self.L.mz_reanalyse(self._h, key0, n))
 
+    def reanalyse_search(self, key0=None, n=None, exploration=False):
+        """MuZero Reanalyze for games key0 .. key0+n-1 (default: the whole buffer): the search again at every stored position with the
+        current networks; refreshes child_visits and the reanalysed root values.  Returns the number of simulations run."""
+        info = self.replay_info()
+        key0 = info["first_key"] if key0 is None else key0
+        n = info["n_games"] - (key0 - info["first_key"]) if n is None else n
+        sims = C.c_int64()
+        self._ck(self.L.mz_reanalyse_search(self._h, key0, n, int(exploration), C.byref(sims)))
+        return sims.value
+
     def reanalysed_export(self, key0=None, n=None):
         info = self.replay_info()
         key0 = info["first_key"] if key0 is None else key0
@@ -487,8 +498,7 @@ class Context:
             ck.update({"hist_" + k: a for k, a in self.history_export().items()})
             if self.cfg.per:                                 # priorities as update_priorities! left them
                 ck["per_q_pos"], ck["per_q_game"] = self.replay_priorities()
-            if self.cfg.net_type == NET_FEEDFORWARD:
-                ck["reanalysed_values"], ck["reanalysed_set"] = self.reanalysed_export()
+            ck["reanalysed_values"], ck["reanalysed_set"] = self.reanalysed_export()   # every network path: reanalyse_search
         return ck
 
     def restore(self, ck):

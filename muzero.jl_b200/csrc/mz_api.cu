@@ -504,17 +504,22 @@ static mz_search_args search_args(const mz_ctx *c, int n, int exploration) {
     a.max_layer_floats = c->M.max_layer_floats; a.exploration = exploration;
     return a;
 }
-// One search over the roots of `a` (MODE_API: the caller's a.n roots; MODE_SLOTS: the a.n game slots) in ONE launch of kernel family 0
-// (run_wave_body relabels the last one of an idle iteration).  lat > 0: the low-latency kernel (mz_kernels_lat.cuh) on roots [0, lat),
-// one 2-CTA cluster each; otherwise the batched kernel of the context's networks.
+// One search over the roots of `a` (MODE_API: the caller's a.n roots; MODE_SLOTS: the a.n game slots; MODE_REPLAY: a.n stored positions)
+// in ONE launch of kernel family 0 (run_wave_body relabels the last one of an idle iteration).  lat > 0: the low-latency kernel
+// (mz_kernels_lat.cuh) on roots [0, lat), one 2-CTA cluster each; otherwise the batched kernel of the context's networks.  MODE_REPLAY
+// always takes the batched kernel: the latency kernel has no instantiation for it.
 template <int MODE>
 static void launch_search(mz_ctx *c, const mz_params &P, const mz_search_args &a, int lat) {
     const unsigned ctas = (unsigned)((a.n + MZ_ROWS - 1) / MZ_ROWS);
     launch_scope ls(c, 0);
-    if (lat > 0) {
-        mz_lat_args t{}; t.base = a; t.image = c->d_w_lat; t.w_floats = c->lat_w_floats; t.pbc_smem = c->lat_pbc_smem;
-        mz_k_search_lat<MODE><<<2 * lat, MZ_LAT_THREADS, c->smem_bytes_lat, c->stream>>>(P, t);
-    } else if (c->cfg.net_type == MZ_NET_RESNET) {
+    if constexpr (MODE != MZ_MODE_REPLAY) {
+        if (lat > 0) {
+            mz_lat_args t{}; t.base = a; t.image = c->d_w_lat; t.w_floats = c->lat_w_floats; t.pbc_smem = c->lat_pbc_smem;
+            mz_k_search_lat<MODE><<<2 * lat, MZ_LAT_THREADS, c->smem_bytes_lat, c->stream>>>(P, t);
+            return;
+        }
+    }
+    if (c->cfg.net_type == MZ_NET_RESNET) {
         mz_search_rn_args t{}; t.base = a; t.image = c->d_rn_image; t.steps = c->d_rn_steps;
         const int nt = c->rn.R.ntrees;
         mz_k_search_rn<MODE><<<(a.n + nt - 1) / nt, MZ_RN_THREADS, c->smem_bytes_rn, c->stream>>>(P, c->rn.R, t);
@@ -576,6 +581,7 @@ int mz_create(const mz_config *cfg, int device, mz_ctx **out) {
         c->smem_bytes_rn = mz_rn_smem_bytes(c->rn.R.slot_bytes, c->M.P.S, c->rn.R.ntrees, c->rn.R.n_steps - c->rn.R.smem_first);
         if (c->smem_bytes_rn + 1024 > (size_t)prop.sharedMemPerBlockOptin) { int r = fail(nullptr, MZ_E_UNSUPPORTED, "the ResNet search kernel needs %zu B of shared memory per CTA, device allows %zu", c->smem_bytes_rn, (size_t)prop.sharedMemPerBlockOptin); mz_destroy(c); return r; }
         MZ_CREATE(allow_max_smem(mz_k_search_rn<MZ_MODE_API>, prop)); MZ_CREATE(allow_max_smem(mz_k_search_rn<MZ_MODE_SLOTS>, prop)); MZ_CREATE(allow_max_smem(mz_k_rn_forward, prop));
+        MZ_CREATE(allow_max_smem(mz_k_search_rn<MZ_MODE_REPLAY>, prop));
         MZ_CREATE(cudaMalloc((void **)&c->d_rn_image, (size_t)c->rn.image_bytes + 4096));
         MZ_CREATE(dmalloc(&c->d_rn_steps, c->rn.steps.size() + 1));
         MZ_CREATE(cudaMemcpy(c->d_rn_steps, c->rn.steps.data(), c->rn.steps.size() * sizeof(mz_rn_step), cudaMemcpyHostToDevice));
@@ -595,11 +601,13 @@ int mz_create(const mz_config *cfg, int device, mz_ctx **out) {
     if (c->smem_bytes > (size_t)prop.sharedMemPerBlockOptin) { int r = fail(nullptr, MZ_E_UNSUPPORTED, "network needs %zu B of shared memory per CTA, device allows %zu", c->smem_bytes, (size_t)prop.sharedMemPerBlockOptin); mz_destroy(c); return r; }
     MZ_CREATE(allow_max_smem(mz_k_search<MZ_MODE_API>, prop));
     MZ_CREATE(allow_max_smem(mz_k_search<MZ_MODE_SLOTS>, prop));
+    MZ_CREATE(allow_max_smem(mz_k_search<MZ_MODE_REPLAY>, prop));
     MZ_CREATE(allow_max_smem(mz_k_nn_forward<false>, prop));
     MZ_CREATE(allow_max_smem(mz_k_reanalyse<false>, prop));
     MZ_CREATE(allow_max_smem(mz_k_learn_forward<false>, prop));
     if (!resnet && cfg->use_batch_norm) {   // the same kernels instantiated with the BatchNorm epilogue
         MZ_CREATE(allow_max_smem(mz_k_search<MZ_MODE_API, true>, prop)); MZ_CREATE(allow_max_smem(mz_k_search<MZ_MODE_SLOTS, true>, prop));
+        MZ_CREATE(allow_max_smem(mz_k_search<MZ_MODE_REPLAY, true>, prop));
         MZ_CREATE(allow_max_smem(mz_k_nn_forward<true>, prop)); MZ_CREATE(allow_max_smem(mz_k_reanalyse<true>, prop)); MZ_CREATE(allow_max_smem(mz_k_learn_forward<true>, prop));
     }
     if (!resnet) {   // the low-latency search kernel for few roots: does a network pair fit one SM's shared memory in fp32?
@@ -654,6 +662,7 @@ int mz_create(const mz_config *cfg, int device, mz_ctx **out) {
         if (c->smem_bytes_tc <= (size_t)prop.sharedMemPerBlockOptin) {
             MZ_CREATE(allow_max_smem(mz_k_search_tc<MZ_MODE_API>, prop));
             MZ_CREATE(allow_max_smem(mz_k_search_tc<MZ_MODE_SLOTS>, prop));
+            MZ_CREATE(allow_max_smem(mz_k_search_tc<MZ_MODE_REPLAY>, prop));
             MZ_CREATE(allow_max_smem(mz_k_nn_forward_tc, prop));
             MZ_CREATE(cudaMalloc((void **)&c->d_w_tc, (size_t)P.tc_net_off[3] + 8192));
             MZ_CREATE(cudaMemset(c->d_w_tc, 0, (size_t)P.tc_net_off[3] + 8192));
@@ -671,6 +680,7 @@ int mz_create(const mz_config *cfg, int device, mz_ctx **out) {
             c->smem_bytes_sp = mz_sp_smem_bytes(S.warea_bytes, S.bias_floats, S.total_rounds, P.hidden_pad, P.S, S.pbc_smem);
             MZ_CREATE(allow_max_smem(mz_k_search_sp<MZ_MODE_API>, prop));
             MZ_CREATE(allow_max_smem(mz_k_search_sp<MZ_MODE_SLOTS>, prop));
+            MZ_CREATE(allow_max_smem(mz_k_search_sp<MZ_MODE_REPLAY>, prop));
             MZ_CREATE(allow_max_smem(mz_k_nn_forward_sp, prop));
             MZ_CREATE(allow_max_smem(mz_k_learn_forward_sp, prop));
             MZ_CREATE(cudaMalloc((void **)&c->d_w_sp, (size_t)S.image_bytes + 256));
@@ -1293,6 +1303,46 @@ int mz_reanalyse(mz_ctx *c, int64_t key0, int n) {
       if (c->cfg.use_batch_norm) mz_k_reanalyse<true><<<(unsigned)((total + MZ_ROWS - 1) / MZ_ROWS), MZ_THREADS, c->smem_bytes, c->stream>>>(P, a);
       else mz_k_reanalyse<false><<<(unsigned)((total + MZ_ROWS - 1) / MZ_ROWS), MZ_THREADS, c->smem_bytes, c->stream>>>(P, a); }
     MZ_CUDA(c, cudaGetLastError());
+    return MZ_OK;
+}
+// MuZero Reanalyze: run_mcts again at every stored position of games key0 .. key0+n-1, with the current networks and the root self-play
+// searched there.  The dense root list (ring entry pos * Tmax + t for t < T) is built on the host from the games' lengths: one small copy
+// each way, and the search launches then hold only real positions (Connect Four games fill far fewer than Tmax).  It is ordered by move
+// t, then by key: the trees of a CTA search in lock step, so a CTA takes as long as its deepest tree, and late positions (fewer legal
+// actions) search deeper -- the reason self-play keeps a wave at one ply (mz_k_save_refill's wave_sync).  The list is cut into launches
+// of at most num_slots roots, the capacity of the tree pool; every root's result depends only on its own position and keys.
+int mz_reanalyse_search(mz_ctx *c, int64_t key0, int n, int exploration, int64_t *simulations) {
+    MZ_CHECK_CTX(c);
+    if (simulations) *simulations = 0;
+    if (n < 0) return fail(c, MZ_E_ARG, "n < 0");
+    if (n == 0) return MZ_OK;
+    MZ_TRY(read_counters(c));
+    if (c->h_counters[5] != 0) return fail(c, MZ_E_STATE, "self-play in progress");
+    int64_t played = c->h_counters[0], have = played < c->ring.capacity ? played : c->ring.capacity, first = played - have + 1;
+    if (key0 < first || key0 + n - 1 > played) return fail(c, MZ_E_ARG, "keys %lld..%lld not in the buffer (holds %lld..%lld)", (long long)key0, (long long)(key0 + n - 1), (long long)first, (long long)played);
+    const mz_params &P = c->M.P;
+    const int64_t cap = c->ring.capacity, Tm = P.Tmax, pos0 = (key0 - 1) % cap, n1 = n < cap - pos0 ? n : cap - pos0;   // the range wraps after n1 games
+    std::vector<int32_t> T((size_t)n);
+    MZ_CUDA(c, cudaMemcpyAsync(T.data(), c->ring.T + pos0, (size_t)n1 * sizeof(int32_t), cudaMemcpyDeviceToHost, c->stream));
+    if (n1 < n) MZ_CUDA(c, cudaMemcpyAsync(T.data() + n1, c->ring.T, (size_t)(n - n1) * sizeof(int32_t), cudaMemcpyDeviceToHost, c->stream));
+    MZ_CUDA(c, cudaStreamSynchronize(c->stream));
+    std::vector<int64_t> roots;
+    for (int t = 0; t < Tm; t++)
+        for (int j = 0; j < n; j++) if (t < T[(size_t)j]) roots.push_back(((key0 + j - 1) % cap) * Tm + t);
+    MZ_TRY(ensure_images(c));
+    int64_t *d_roots;
+    MZ_TRY(h2d(c, c->scratch[0], roots.data(), roots.size(), &d_roots));
+    { launch_scope ls(c, 5); mz_k_reanalyse_mark<<<(unsigned)(((int64_t)n * Tm + 127) / 128), 128, 0, c->stream>>>(P, c->ring, key0, n); }
+    MZ_CUDA(c, cudaGetLastError());
+    const int64_t total = (int64_t)roots.size(), chunk = c->cfg.num_slots;
+    for (int64_t off = 0; off < total; off += chunk) {
+        mz_search_args a = search_args(c, (int)(total - off < chunk ? total - off : chunk), exploration);
+        a.ring = c->ring; a.replay = d_roots + off;   // a.stats stays NULL: mz_search_stats describes self-play
+        launch_search<MZ_MODE_REPLAY>(c, P, a, 0);
+        MZ_CUDA(c, cudaGetLastError());
+    }
+    MZ_CUDA(c, cudaStreamSynchronize(c->stream));
+    if (simulations) *simulations = total * P.S;
     return MZ_OK;
 }
 int mz_reanalysed_export(mz_ctx *c, int64_t key0, int n, float *values, int32_t *flags) {

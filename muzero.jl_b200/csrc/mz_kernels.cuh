@@ -8,12 +8,14 @@
 //                       MODE_SLOTS: roots come from the device-resident game slots; after the search the same
 //                                   kernel samples the action, steps the environment and appends to the game
 //                                   history (play_game's loop body, src/SelfPlay.jl:343-380).
+//                       MODE_REPLAY: roots are stored positions of the replay ring (MuZero Reanalyze); the results
+//                                   replace the position's policy target and reanalysed root value.
 //   mz_k_save_refill    save_game (src/ReplayBuffer.jl:133-161) for finished slots, in slot order, into the
 //                       device replay ring + assignment of the next game ids to free slots.
 #pragma once
 #include "mz_device.cuh"
 
-enum { MZ_MODE_API = 0, MZ_MODE_SLOTS = 1 };
+enum { MZ_MODE_API = 0, MZ_MODE_SLOTS = 1, MZ_MODE_REPLAY = 2 };
 
 // Optional phase timers (make EXTRA=-DMZ_PHASE_TIMERS): threads 0 (tree lane 0 / prediction group) and 128 (dynamics
 // group) of every CTA accumulate clock64() deltas of the simulation loop into stats[4 + 6*g + phase]:
@@ -63,6 +65,9 @@ struct mz_search_args {
     // MODE_SLOTS
     mz_slots slots; float temperature;
     unsigned long long *stats;   // [0] sum depth, [1] simulations, [2] sum legal, [3] roots
+    // MODE_REPLAY: root i is position t of the game at ring position pos, replay[i] = pos * Tmax + t (the index of its [R][Tmax] entries).
+    // Last, so that the fields the other modes read keep their offsets.
+    mz_ring ring; const int64_t *replay;
 };
 
 // ---- lane-parallel tree operations: MZ_LANES (8) lanes of a warp cooperate on one tree.  They are the GPU-only
@@ -190,6 +195,12 @@ __device__ __forceinline__ void mz_tree_backup_lanes(const mz_params &P, const m
     __syncwarp(segmask);
 }
 
+// store_search_stats! (src/SelfPlay.jl:115-122, Q12): the root's visit distribution over the legal actions, the policy target of the
+// position.  Self-play (mz_slot_epilogue) and reanalysis (mz_root_finish<MODE_REPLAY>) both write it through here.
+__device__ __forceinline__ void mz_store_search_stats(const mz_params &P, float *cv, const int32_t *vc, uint32_t legal, int sum_visits) {
+    for (int i = 0; i < P.A; i++) cv[i] = ((legal >> i) & 1u) ? (float)((double)vc[i] / (double)sum_visits) : 0.0f;
+}
+
 // play_game's loop body after run_mcts (src/SelfPlay.jl:344-346, 360-379) for one game slot: temperature rule, select_action, environment
 // step, store_search_stats! (Q12), history append, termination.  Lane 0 of the tree, from mz_root_finish.
 __device__ __forceinline__ void mz_slot_epilogue(const mz_params &P, const mz_slots &s, int64_t g, const int32_t *vc, int sum_visits, uint32_t legal, float rv,
@@ -201,8 +212,7 @@ __device__ __forceinline__ void mz_slot_epilogue(const mz_params &P, const mz_sl
     mz_env_step_b(P, b, action);                                                    // :366
     const float reward = (float)mz_env_reward_b(P, b, p);                           // :367
     const bool done = mz_env_terminated_b(P, b);                                    // :368
-    float *cv = s.h_cv + ((size_t)g * P.Tmax + T) * P.A;                            // store_search_stats! :115-122 (Q12)
-    for (int i = 0; i < P.A; i++) cv[i] = ((legal >> i) & 1u) ? (float)((double)vc[i] / (double)sum_visits) : 0.0f;
+    mz_store_search_stats(P, s.h_cv + ((size_t)g * P.Tmax + T) * P.A, vc, legal, sum_visits);
     s.h_rv[(size_t)g * P.Tmax + T] = rv;
     s.h_action[(size_t)g * P.Tmax + T] = action;                                    // :377-379
     s.h_reward[(size_t)g * P.Tmax + T] = reward;
@@ -217,14 +227,23 @@ __device__ __forceinline__ void mz_slot_epilogue(const mz_params &P, const mz_sl
 // root node and its expansion, the results.  The kernels differ in how they run the networks and in which threads own a tree. ----
 struct mz_root { bool active; uint32_t legal, game, move, posmask; };
 // root g: MODE_API from the caller's arrays, MODE_SLOTS from the slot's board (SelfPlay.jl:351,359); in competitive play a slot is searched
-// only on MuZero's plies.  valid = false (no root g for this thread: g >= a.n, or not a tree lane) gives an inactive root with no legal action.
+// only on MuZero's plies.  MODE_REPLAY: stored position t of a ring game, with the root self-play searched there (board before move t,
+// its side to move, game id, move index t + 1).  valid = false (no root g for this thread: g >= a.n, or not a tree lane) gives an inactive
+// root with no legal action.
 template <int MODE>
 __device__ __forceinline__ mz_root mz_root_begin(const mz_params &P, const mz_search_args &a, int64_t g, bool valid) {
     mz_root R; R.active = false; R.legal = 0; R.game = 0; R.move = 0; R.posmask = 0;
     if (MODE == MZ_MODE_API) {
         if (valid) { R.legal = a.legal[g]; R.game = (uint32_t)a.game_id[g]; R.move = (uint32_t)a.move_idx[g]; }
         R.active = R.legal != 0;   // run_mcts asserts !isempty(legal_actions) (SelfPlay.jl:243)
-    } else if (valid) {
+    } else if (MODE == MZ_MODE_REPLAY) {
+        if (valid) {
+            const int64_t e = a.replay[g], pos = e / P.Tmax;
+            mz_board b; b.p1 = a.ring.h_p1[e]; b.p2 = a.ring.h_p2[e]; b.player = a.ring.h_to_play[e];
+            R.legal = mz_env_legal_b(P, b); R.game = (uint32_t)a.ring.game_id[pos]; R.move = (uint32_t)(e - pos * P.Tmax) + 1u;
+        }
+        R.active = R.legal != 0;   // a stored position precedes a move: it has a legal action
+    } else if (valid) {            // MODE_SLOTS
         R.active = a.slots.status[g] == MZ_SLOT_ACTIVE && (P.arena_player == 0 || a.slots.player[g] == P.arena_player);
         if (R.active) {
             mz_board b; b.p1 = a.slots.p1[g]; b.p2 = a.slots.p2[g]; b.player = a.slots.player[g];
@@ -236,11 +255,15 @@ __device__ __forceinline__ mz_root mz_root_begin(const mz_params &P, const mz_se
     return R;
 }
 // entry k of root gg's stacked observations (get_stacked_observations, SelfPlay.jl:128-149); 0 past the launch's roots and for a slot
-// that has no ply to search
+// that has no ply to search.  MODE_REPLAY reads the stored history as mz_k_reanalyse and get_batch do: index t + 1 of the game.
 template <int MODE>
 __device__ __forceinline__ float mz_root_obs(const mz_params &P, const mz_search_args &a, int64_t gg, int k) {
     if (gg >= a.n) return 0.0f;
     if (MODE == MZ_MODE_API) return a.stacked[gg * P.stack_size + k];
+    if (MODE == MZ_MODE_REPLAY) {
+        const int64_t e = a.replay[gg], pos = e / P.Tmax, row = pos * P.Tmax;
+        return mz_stacked_value(P, a.ring.h_p1 + row, a.ring.h_p2 + row, a.ring.h_action + row, (int)(e - row) + 1, k);
+    }
     if (a.slots.status[gg] != MZ_SLOT_ACTIVE) return 0.0f;
     return mz_stacked_value(P, a.slots.h_p1 + gg * P.Tmax, a.slots.h_p2 + gg * P.Tmax, a.slots.h_action + gg * P.Tmax, a.slots.T[gg] + 1, k);
 }
@@ -255,7 +278,8 @@ __device__ __forceinline__ void mz_root_init(const mz_params &P, const mz_tree &
     __syncwarp(segmask);
 }
 // results of root g, lane 0 of an active tree: the launch's statistics (stats[0] sum of leaf depths, [1] simulations, [2] sum of legal
-// actions, [3] roots), then visit counts, root value and priors to the caller (MODE_API) or the move of the game (MODE_SLOTS)
+// actions, [3] roots), then visit counts, root value and priors to the caller (MODE_API), the move of the game (MODE_SLOTS), or the
+// stored position's policy target and reanalysed root value (MODE_REPLAY)
 template <int MODE>
 __device__ __forceinline__ void mz_root_finish(const mz_params &P, const mz_search_args &a, int64_t g, const mz_tree &t, const mz_root &R,
                                                unsigned long long depth_sum) {
@@ -277,11 +301,16 @@ __device__ __forceinline__ void mz_root_finish(const mz_params &P, const mz_sear
             if (a.root_priors) a.root_priors[g * P.A + i] = ((R.legal >> i) & 1u) ? t.A[1 + i].z : 0.0f;
         }
         a.root_value[g] = rv;
+    } else if (MODE == MZ_MODE_REPLAY) {
+        const int64_t e = a.replay[g];
+        mz_store_search_stats(P, a.ring.h_cv + e * P.A, vc, R.legal, sum_visits);
+        a.ring.h_rrv[e] = rv;
     } else mz_slot_epilogue(P, a.slots, g, vc, sum_visits, R.legal, rv, a.temperature, R.game, R.move);
 }
 
 // Self-play launches run one iteration ahead of the host (run_wave, mz_api.cu): a CTA none of whose slots has a ply to search -- every
 // CTA of the iteration queued past the end of a wave -- returns at its first instruction, before any barrier, TMA or TMEM state exists.
+// MODE_API and MODE_REPLAY launches cover exactly their roots (the replay root list is dense): no CTA is idle.
 template <int MODE>
 __device__ __forceinline__ bool mz_cta_idle(const mz_params &P, const mz_search_args &a, int rows_per_cta) {
     if (MODE != MZ_MODE_SLOTS) return false;
@@ -319,7 +348,7 @@ __global__ void __launch_bounds__(MZ_THREADS) mz_k_search(const __grid_constant_
     for (int i = tid; i < MZ_ROWS * P.stack_size; i += MZ_THREADS) {
         int rr, k;
         if (MODE == MZ_MODE_API) { rr = i / P.stack_size; k = i % P.stack_size; }   // the caller's rows are contiguous
-        else { k = i / MZ_ROWS; rr = i % MZ_ROWS; }
+        else { k = i / MZ_ROWS; rr = i % MZ_ROWS; }                                  // slots, replay positions: every entry is computed
         sp.in0[k * MZ_ROWS + rr] = mz_root_obs<MODE>(P, a, (int64_t)blockIdx.x * MZ_ROWS + rr, k);
     }
     __syncthreads();
@@ -658,6 +687,16 @@ __global__ void __launch_bounds__(MZ_THREADS) mz_k_reanalyse(const __grid_consta
         a.ring.h_rrv[pos * P.Tmax + t] = t < a.ring.T[pos] ? sp.outV[tid] : 0.0f;
         if (t == 0) a.ring.reanalysed[pos] = 1;
     }
+}
+
+// mz_reanalyse_search: the entries the search does not write -- reanalysed values of positions t >= T are 0, as mz_k_reanalyse leaves
+// them -- and the "is set" flag of every game of the range.  One thread per (game, position).
+__global__ void mz_k_reanalyse_mark(const __grid_constant__ mz_params P, mz_ring r, int64_t key0, int n) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= (int64_t)n * P.Tmax) return;
+    const int64_t pos = (key0 + i / P.Tmax - 1) % r.capacity; const int t = (int)(i % P.Tmax);
+    if (t >= r.T[pos]) r.h_rrv[pos * P.Tmax + t] = 0.0f;
+    if (t == 0) r.reanalysed[pos] = 1;
 }
 
 // ---- batched environment verbs (games/tictactoe/game.jl) --------------------------------------------

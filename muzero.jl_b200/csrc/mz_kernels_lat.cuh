@@ -164,6 +164,7 @@ struct mz_lat_args { mz_search_args base; const float *image; int32_t w_floats, 
 
 template <int MODE>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(MZ_LAT_THREADS) mz_k_search_lat(const __grid_constant__ mz_params P, const __grid_constant__ mz_lat_args la) {
+    static_assert(MODE != MZ_MODE_REPLAY, "stored positions are reanalysed in bulk by the batched kernels");
     extern __shared__ __align__(128) unsigned char mz_smem_lat[];
     namespace cg = cooperative_groups;
     const mz_search_args &a = la.base;

@@ -134,8 +134,8 @@ __global__ void __launch_bounds__(MZ_SP_SEARCH_THREADS) mz_k_search_sp(const __g
     if (worker && ln == 0) sp.active[r] = active;                       // for the tail team's hidden-state write
     for (int i = tid; i < MZ_ROWS * P.stack_size; i += MZ_SP_SEARCH_THREADS) {
         int rr, k;
-        if (MODE == MZ_MODE_API) { rr = i / P.stack_size; k = i % P.stack_size; }
-        else { k = i / MZ_ROWS; rr = i % MZ_ROWS; }
+        if (MODE == MZ_MODE_API) { rr = i / P.stack_size; k = i % P.stack_size; }   // the caller's rows are contiguous
+        else { k = i / MZ_ROWS; rr = i % MZ_ROWS; }                                  // slots, replay positions: every entry is computed
         mz_sp_stage(in_dyn, k, rr, mz_root_obs<MODE>(P, a, (int64_t)blockIdx.x * MZ_ROWS + rr, k));
     }
     mz_fence_proxy_async();

@@ -73,8 +73,8 @@ __global__ void __launch_bounds__(MZ_THREADS) mz_k_search_tc(const __grid_consta
     // ---- stage the stacked observations as a bf16 B tile (values are 0/1 and raw action indices: exact in bf16) ----
     for (int i = tid; i < MZ_ROWS * P.stack_size; i += MZ_THREADS) {
         int rr, k;
-        if (MODE == MZ_MODE_API) { rr = i / P.stack_size; k = i % P.stack_size; }
-        else { k = i / MZ_ROWS; rr = i % MZ_ROWS; }
+        if (MODE == MZ_MODE_API) { rr = i / P.stack_size; k = i % P.stack_size; }   // the caller's rows are contiguous
+        else { k = i / MZ_ROWS; rr = i % MZ_ROWS; }                                  // slots, replay positions: every entry is computed
         mz_tc_store_bf16(sp.inS, rr, k, mz_root_obs<MODE>(P, a, (int64_t)blockIdx.x * MZ_ROWS + rr, k));
     }
     mz_fence_proxy_async();

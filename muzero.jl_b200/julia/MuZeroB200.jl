@@ -255,6 +255,14 @@ end
 "Fill `reanalysed_predicted_root_values` (Constructors.jl:13) of games `key0 .. key0+n-1` from the current networks; `get_batch` then bootstraps from them (ReplayBuffer.jl:8)."
 reanalyse!(e::Engine, key0::Integer, n::Integer) = check(e, ccall((:mz_reanalyse, LIB), Cint, (Ptr{Cvoid}, Int64, Cint), e.ctx, key0, n))
 
+"""MuZero Reanalyze: `run_mcts` again at every stored position of games `key0 .. key0+n-1` with the current networks (root, game id and
+move index as self-play had them); refreshes `child_visits` and `reanalysed_predicted_root_values`.  Returns the simulations run."""
+function reanalyse_search!(e::Engine, key0::Integer, n::Integer; exploration::Bool=false)
+    sims = Ref{Int64}(0)
+    check(e, ccall((:mz_reanalyse_search, LIB), Cint, (Ptr{Cvoid}, Int64, Cint, Cint, Ptr{Int64}), e.ctx, key0, n, exploration ? 1 : 0, sims))
+    return sims[]
+end
+
 "`steps` iterations of get_batch -> unroll -> loss -> gradients -> ADAM(Cos schedule); returns the last three losses."
 function learning!(e::Engine, steps::Integer; grad_mode::Integer=0)
     losses = zeros(Float32, 3)
