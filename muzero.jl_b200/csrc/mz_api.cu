@@ -5,6 +5,7 @@
 #include <nccl.h>
 #include <cstdarg>
 #include <cstdio>
+#include <memory>
 #include <string>
 #include <vector>
 #include "mz_host.h"
@@ -68,27 +69,28 @@ struct mz_ctx {
     cudaStream_t stream2 = nullptr; cudaEvent_t ev_search[2] = {nullptr, nullptr};   // save / refill of move k beside the search of move k + 1 (run_wave)
     std::string err;
     size_t smem_bytes = 0; int sm_count = 0;
-    float *d_w = nullptr, *d_m = nullptr, *d_v = nullptr, *d_grad = nullptr;
+    // the learner's parameter store: fp32 parameters, ADAM moments and gradient, store_floats each; packed: in the padded device layout of the
+    // FeedForwardHP kernels (mzh::pack_weights), else (ResNet) in blob order.  d_mask (use_batch_norm, ResNet): 1 = Flux parameter, 0 = BatchNorm
+    // running statistic; net_bounds: where each network starts in the store, and its end
+    float *d_w = nullptr, *d_m = nullptr, *d_v = nullptr, *d_grad = nullptr; int store_floats = 0; bool packed = true;
+    unsigned char *d_mask = nullptr; int net_bounds[4] = {0, 0, 0, 0};
     unsigned char *d_w_tc = nullptr; float *d_bias_tc = nullptr; size_t smem_bytes_tc = 0;   // tensor-core weight image
     // data-parallel learner over peer memory (mz_k_dp_adam): gradient exchange buffers (double-buffered) and arrival flags of every rank
     float *d_xgrad = nullptr; uint32_t *d_xflags = nullptr; float *peer_grad[MZ_DP_MAX_RANKS] = {}; uint32_t *peer_flags[MZ_DP_MAX_RANKS] = {};
     bool p2p = false; uint32_t dp_step = 0;
-    // ResNet learner (reference_l2): fp32 parameters in blob order, ADAM moments, gradient, trainable mask, unroll scratch; the bf16 image is
-    // rebuilt from the parameters (rn_dirty) before the next kernel that reads it
-    float *d_rn_theta = nullptr, *d_rn_m = nullptr, *d_rn_v = nullptr, *d_rn_grad = nullptr, *d_rn_h = nullptr, *d_rn_nh = nullptr, *d_rn_sa = nullptr, *d_rn_o1 = nullptr, *d_rn_o2 = nullptr, *d_rn_r = nullptr;
-    unsigned char *d_rn_mask = nullptr, *d_rn_pool = nullptr; int rn_learn_cap = 0; bool rn_dirty = false;
-    // MZ_GRAD_BPTT on the tensor cores (mz_learner_tc.cuh): backward rounds, saved activation / gradient tiles, per-chunk partial gradients
-    mz_lr_plan lrp{}; mz_lr_bround *d_brounds = nullptr; unsigned char *d_xsave = nullptr, *d_dzsave = nullptr; float *d_gpart_tc = nullptr;
-    int lr_tiles_cap = 0, lr_chunks_cap = 0; size_t smem_bytes_lr = 0;
+    // the learner's scratch: the ResNet unroll (h, h', state-action input, value, policy, reward, node pool); MZ_GRAD_BPTT on the SIMT kernel
+    // (activations, per-tile partial gradients) and on the tensor cores (saved activation / gradient tiles, per-chunk partial gradients)
+    dev_buf rn_buf[7], bptt_act, bptt_gpart, lr_xsave, lr_dzsave, lr_gpart;
+    // MZ_GRAD_BPTT on the tensor cores (mz_learner_tc.cuh): backward rounds
+    mz_lr_plan lrp{}; mz_lr_bround *d_brounds = nullptr; size_t smem_bytes_lr = 0;
     // mz_k_search_lat (one tree per 2-CTA cluster, networks and tree resident in shared memory): calls with at most lat_max_roots roots
-    unsigned char *d_fc_mask = nullptr; int fc_net_bounds[4] = {0, 0, 0, 0};   // use_batch_norm: 1 = Flux parameter, 0 = BatchNorm statistics (padded device blob); network boundaries
     float *d_w_lat = nullptr; uint64_t lat_version = 0; int lat_image_floats = 0;
     unsigned char *h_lat_stage = nullptr, *d_lat_stage = nullptr; size_t lat_stage_cap = 0;   // one pinned / device block for all inputs and outputs of a small run_mcts call
     bool lat_ok = false; int lat_w_floats = 0, lat_pbc_smem = 0, lat_max_roots = 0, lat_max_slots = 0; size_t smem_bytes_lat = 0;
     bool persist_ok = true;     // MUZERO_B200_PERSIST=0: one search launch per move also for single-wave self-play on the split-precision path
     bool slots_dirty = false;   // a wave is in progress or ended with an error: the slots are reset before the next one
     int refill_wave_sync = 1;   // 1: mz_k_save_refill starts new games only when every slot is free (default; MUZERO_B200_REFILL=immediate refills at once)
-    uint64_t w_version = 1, img_version = 0;   // device weights vs the tensor-core image built from them (ensure_images)
+    uint64_t w_version = 1, img_version = 0;   // device weights vs the tensor-core or ResNet image built from them (ensure_images)
     mz_sp_plan spp{}; mz_sp_args spa{}; unsigned char *d_w_sp = nullptr; float *d_bias_sp = nullptr; mz_sp_round *d_rounds_sp = nullptr; size_t smem_bytes_sp = 0;   // split-precision tensor-core path
     double *d_pbc0 = nullptr, *d_sqrtN = nullptr;
     void *d_trees = nullptr;
@@ -101,14 +103,14 @@ struct mz_ctx {
     int64_t *h_counters = nullptr; double *h_lossout = nullptr; unsigned long long *h_stats = nullptr;   // pinned
     int64_t *h_wave = nullptr, *d_wave = nullptr; cudaEvent_t ev_wave[2] = {nullptr, nullptr};   // pinned: two snapshots of the counters, self-play runs one iteration ahead of the host
     dev_buf scratch[12];
-    int64_t adam_t = 0; double bp1 = 0.9, bp2 = 0.999;
+    int64_t adam_t = 1; double bp1 = 0.9, bp2 = 0.999;   // Flux.ADAM: the next update's step number and beta powers (adam_seek)
     ncclComm_t comm = nullptr; int rank = 0, nranks = 1;
     // net_type = MZ_NET_RESNET
-    mzh::rn_model rn; unsigned char *d_rn_image = nullptr; mz_rn_step *d_rn_steps = nullptr; size_t smem_bytes_rn = 0; std::vector<float> rn_blob;
+    mzh::rn_model rn; unsigned char *d_rn_image = nullptr; mz_rn_step *d_rn_steps = nullptr; size_t smem_bytes_rn = 0;
     // grad_mode = MZ_GRAD_BPTT
     mzh::bptt_program bptt; mz_bstage *d_bstages[2] = {nullptr, nullptr}; size_t smem_bytes_bptt = 0;
     float *d_w_fold = nullptr;   // use_batch_norm + MZ_GRAD_BPTT: the weights with every BatchNorm folded into its Dense layer
-    float *d_act = nullptr, *d_gpart = nullptr; int bptt_tiles_cap = 0; int bptt_dims[4] = {0, 0, 0, 0};   // mz_bptt_args: dim_wide, dim_narrow, wfloats[2]
+    int bptt_dims[4] = {0, 0, 0, 0};   // mz_bptt_args: dim_wide, dim_narrow, wfloats[2]
     int64_t launches = 0; bool timing = false; std::vector<timed_launch> timed; double fam_ms[8] = {0}; int64_t fam_n[8] = {0};
     double last_mean_legal = 0, last_mean_depth = 0;
 };
@@ -196,33 +198,29 @@ int alloc_batch(mz_ctx *c, int B) {
     return MZ_OK;
 }
 
-int upload_weights(mz_ctx *c, const std::vector<float> &src) {
-    if (c->cfg.net_type == MZ_NET_RESNET) {   // blob -> bf16 B-operand images + folded BatchNorm parameters, one block per program step
-        c->rn_blob = src;
-        std::vector<unsigned char> image;
-        mzh::rn_pack(c->rn, src.data(), image);
-        MZ_CUDA(c, cudaMemcpyAsync(c->d_rn_image, image.data(), (size_t)c->rn.image_bytes, cudaMemcpyHostToDevice, c->stream));
-        if (c->d_rn_theta) MZ_CUDA(c, cudaMemcpyAsync(c->d_rn_theta, src.data(), src.size() * sizeof(float), cudaMemcpyHostToDevice, c->stream));
-        MZ_CUDA(c, cudaStreamSynchronize(c->stream));
-        c->rn_dirty = false;
-        return MZ_OK;
-    }
-    std::vector<float> dev((size_t)c->M.P.total_floats);
-    mzh::pack_weights(c->M.P, src.data(), dev.data());
-    MZ_CUDA(c, cudaMemcpyAsync(c->d_w, dev.data(), dev.size() * sizeof(float), cudaMemcpyHostToDevice, c->stream));
-    c->w_version++;                                      // the tensor-core images are rebuilt on the device before their next use (ensure_images)
+// one array of the parameter store (d_w, d_m, d_v, d_grad) to / from the caller's blob order (n_params floats)
+int store_to_host(mz_ctx *c, const float *d, float *blob) {
+    std::vector<float> dev(c->packed ? (size_t)c->store_floats : 0);
+    MZ_CUDA(c, cudaMemcpyAsync(c->packed ? dev.data() : blob, d, (size_t)c->store_floats * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
+    MZ_CUDA(c, cudaStreamSynchronize(c->stream));
+    if (c->packed) mzh::unpack_weights(c->M.P, dev.data(), blob);
+    return MZ_OK;
+}
+int store_from_host(mz_ctx *c, float *d, const float *blob) {
+    std::vector<float> dev(c->packed ? (size_t)c->store_floats : 0);
+    if (c->packed) mzh::pack_weights(c->M.P, blob, dev.data());
+    MZ_CUDA(c, cudaMemcpyAsync(d, c->packed ? dev.data() : blob, (size_t)c->store_floats * sizeof(float), cudaMemcpyHostToDevice, c->stream));
     MZ_CUDA(c, cudaStreamSynchronize(c->stream));
     return MZ_OK;
 }
-int rn_sync_image(mz_ctx *c);
+int upload_weights(mz_ctx *c, const std::vector<float> &src) {
+    const int r = store_from_host(c, c->d_w, src.data());
+    c->w_version++;                                      // the images are rebuilt before their next use (ensure_images)
+    return r;
+}
 int download_weights(mz_ctx *c, std::vector<float> &src) {
-    if (c->cfg.net_type == MZ_NET_RESNET) { const int r_ = rn_sync_image(c); if (r_ != MZ_OK) return r_; src = c->rn_blob; return MZ_OK; }   // the blob is mirrored on the host
-    std::vector<float> dev((size_t)c->M.P.total_floats);
-    MZ_CUDA(c, cudaMemcpyAsync(dev.data(), c->d_w, dev.size() * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
-    MZ_CUDA(c, cudaStreamSynchronize(c->stream));
     src.resize((size_t)c->M.P.n_params);
-    mzh::unpack_weights(c->M.P, dev.data(), src.data());
-    return MZ_OK;
+    return store_to_host(c, c->d_w, src.data());
 }
 
 int read_counters(mz_ctx *c) {
@@ -255,30 +253,54 @@ template <typename T> int d2h(mz_ctx *c, T *host, const T *dev, size_t n) {
     return MZ_OK;
 }
 #define MZ_TRY(x) do { int r_ = (x); if (r_ != MZ_OK) return r_; } while (0)
+// h2d's allocation for scratch that a kernel may read before it writes it: zeroed whenever it grows
+template <typename T> int alloc_zeroed(mz_ctx *c, dev_buf &b, size_t n, T **out) {
+    const size_t cap = b.cap;
+    MZ_TRY(h2d<T>(c, b, nullptr, n, out));
+    if (b.cap != cap) MZ_CUDA(c, cudaMemsetAsync(b.p, 0, b.cap, c->stream));
+    return MZ_OK;
+}
+
+// Flux.ADAM's state after `steps_done` updates: the next update is step adam_t = steps_done + 1 with the beta powers beta^adam_t, by repeated
+// product as the running state builds them
+void adam_seek(mz_ctx *c, int64_t steps_done) {
+    c->adam_t = steps_done + 1; c->bp1 = 0.9; c->bp2 = 0.999;
+    for (int64_t i = 0; i < steps_done; i++) { c->bp1 *= 0.9; c->bp2 *= 0.999; }
+}
+
+// which kernels a learner step of `grad_mode` runs on in this context: 0 = fp32 SIMT (mz_k_learn_forward / mz_k_learn_bptt), 1 = the unroll forward
+// on the tensor cores (mz_k_learn_forward_sp), 2 = forward and backward on the tensor cores (mz_k_learn_bptt_tc + mz_k_learn_dw), 3 = ResNet: unroll
+// through the bf16 inference kernel (mz_k_rn_forward), -1 = not available (ResNet with MZ_GRAD_BPTT).  MUZERO_B200_BPTT_SIMT (set to anything) keeps
+// MZ_GRAD_BPTT on the SIMT kernel.
+int learner_path(const mz_ctx *c, int grad_mode) {
+    if (c->cfg.net_type == MZ_NET_RESNET) return grad_mode == MZ_GRAD_REFERENCE_L2 ? 3 : -1;
+    if (c->cfg.nn_mode != MZ_NN_SPLIT_MMA) return 0;
+    if (grad_mode == MZ_GRAD_BPTT) return (c->lrp.ok && !getenv("MUZERO_B200_BPTT_SIMT")) ? 2 : 0;
+    return 1;
+}
 
 // where this step's local gradient goes: d_grad, or -- data-parallel over peer memory -- the half of the exchange buffer the next
 // update reads (the other half may still be read by a peer that is one step behind)
 float *grad_out(mz_ctx *c) { return c->p2p ? c->d_xgrad + (size_t)((c->dp_step + 1u) & 1u) * (size_t)c->M.P.total_floats : c->d_grad; }
 
-// ResNet: after a learner update the device parameters are ahead of the bf16 image: fetch them, fold BatchNorm and re-pack on the host
-// (rn_pack), upload the image.  (A device-side packer would save the round trip; the ResNet learner is a functional path, not a tuned one.)
+// ResNet: fetch the parameters, fold BatchNorm and pack the bf16 B-operand images on the host (rn_pack, one block per program step), upload
+// the image.  (A device-side packer would save the round trip; the ResNet learner is a functional path, not a tuned one.)
 int rn_sync_image(mz_ctx *c) {
-    if (!c->rn_dirty) return MZ_OK;
-    MZ_CUDA(c, cudaMemcpyAsync(c->rn_blob.data(), c->d_rn_theta, c->rn_blob.size() * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
-    MZ_CUDA(c, cudaStreamSynchronize(c->stream));
+    std::unique_ptr<float[]> blob(new float[(size_t)c->store_floats]);   // not zero-filled: the copy overwrites all of it
+    MZ_TRY(store_to_host(c, c->d_w, blob.get()));
     std::vector<unsigned char> image;
-    mzh::rn_pack(c->rn, c->rn_blob.data(), image);
+    mzh::rn_pack(c->rn, blob.get(), image);
     MZ_CUDA(c, cudaMemcpyAsync(c->d_rn_image, image.data(), (size_t)c->rn.image_bytes, cudaMemcpyHostToDevice, c->stream));
     MZ_CUDA(c, cudaStreamSynchronize(c->stream));
-    c->rn_dirty = false;
+    c->img_version = c->w_version;
     return MZ_OK;
 }
 
-// The tensor-core paths read bf16 images of the weights; whenever d_w has changed (set_weights, an ADAM step) the image of the context's
-// nn_mode is rebuilt on the device before the next kernel that reads it.
+// The tensor-core and ResNet paths read bf16 images of the weights; whenever d_w has changed (set_weights, an ADAM step) the image of the
+// context's networks is rebuilt before the next kernel that reads it (FeedForwardHP: on the device).
 int ensure_images(mz_ctx *c) {
+    if (c->img_version == c->w_version) return MZ_OK;
     if (c->cfg.net_type == MZ_NET_RESNET) return rn_sync_image(c);
-    if (c->img_version == c->w_version || c->cfg.net_type != MZ_NET_FEEDFORWARD) return MZ_OK;
     const mz_params &P = c->M.P;
     mz_pack_args a{}; a.w = c->d_w;
     if (c->cfg.nn_mode == MZ_NN_SPLIT_MMA && c->d_w_sp) {
@@ -310,103 +332,91 @@ int ensure_lat_image(mz_ctx *c) {
 // ---- ResNet learner (grad_mode = MZ_GRAD_REFERENCE_L2: the reference's actual update, Q20) ---------------------------------------------
 // The K-step unroll (Learning.jl:347-370) as a sequence of the batched network kernel mz_k_rn_forward on device buffers (bf16 inference
 // arithmetic, BatchNorm with its stored statistics: the reference computes the predictions outside the pullback, i.e. in test mode), then
-// the generic loss kernels; the update is ADAM on 2 * theta over Flux.params (mz_k_grad_l2_masked), after which the bf16 image is rebuilt.
-int rn_forward_dev(mz_ctx *c, int net, int B, const float *d_in, float *d_o1, float *d_o2) {
-    mz_search_rn_args t{}; t.image = c->d_rn_image; t.steps = c->d_rn_steps; t.net = net; t.B = B; t.in = d_in; t.out1 = d_o1; t.out2 = d_o2; t.scratch_pool = c->d_rn_pool;
+// the loss tail; the update is ADAM on 2 * theta over Flux.params (launch_update), after which the bf16 image is rebuilt (ensure_images).
+int rn_forward_dev(mz_ctx *c, int net, int B, const float *d_in, float *d_o1, float *d_o2, unsigned char *pool) {
+    mz_search_rn_args t{}; t.image = c->d_rn_image; t.steps = c->d_rn_steps; t.net = net; t.B = B; t.in = d_in; t.out1 = d_o1; t.out2 = d_o2; t.scratch_pool = pool;
     const int nt = c->rn.R.ntrees;
     launch_scope ls(c, 3); mz_k_rn_forward<<<(B + nt - 1) / nt, MZ_RN_THREADS, c->smem_bytes_rn, c->stream>>>(c->M.P, c->rn.R, t);
     return MZ_OK;
 }
-int rn_learn_forward(mz_ctx *c, int B, int grad_mode) {
+int rn_learn_forward(mz_ctx *c, int B) {
     const mz_params &P = c->M.P;
-    if (grad_mode != MZ_GRAD_REFERENCE_L2) return fail(c, MZ_E_UNSUPPORTED, "the ResNet learner implements MZ_GRAD_REFERENCE_L2 (the reference's update); the backward pass through the convolution towers is not built");
     MZ_TRY(ensure_images(c));
-    if (B > c->rn_learn_cap) {
-        void **ptrs[] = {(void **)&c->d_rn_h, (void **)&c->d_rn_nh, (void **)&c->d_rn_sa, (void **)&c->d_rn_o1, (void **)&c->d_rn_o2, (void **)&c->d_rn_r, (void **)&c->d_rn_pool};
-        for (void **q : ptrs) { if (*q) cudaFree(*q); *q = nullptr; }
-        c->rn_learn_cap = 0;
-        MZ_CUDA(c, dmalloc(&c->d_rn_h, (size_t)B * P.hidden)); MZ_CUDA(c, dmalloc(&c->d_rn_nh, (size_t)B * P.hidden)); MZ_CUDA(c, dmalloc(&c->d_rn_sa, (size_t)B * P.sa_size));
-        MZ_CUDA(c, dmalloc(&c->d_rn_o1, (size_t)B)); MZ_CUDA(c, dmalloc(&c->d_rn_o2, (size_t)B * P.A)); MZ_CUDA(c, dmalloc(&c->d_rn_r, (size_t)B));
-        MZ_CUDA(c, cudaMalloc((void **)&c->d_rn_pool, (size_t)B * c->rn.R.node_bytes + 256));
-        c->rn_learn_cap = B;
-    }
+    float *h, *nh, *sa, *o1, *o2, *r; unsigned char *pool;
+    MZ_TRY(h2d<float>(c, c->rn_buf[0], nullptr, (size_t)B * P.hidden, &h)); MZ_TRY(h2d<float>(c, c->rn_buf[1], nullptr, (size_t)B * P.hidden, &nh));
+    MZ_TRY(h2d<float>(c, c->rn_buf[2], nullptr, (size_t)B * P.sa_size, &sa)); MZ_TRY(h2d<float>(c, c->rn_buf[3], nullptr, (size_t)B, &o1));
+    MZ_TRY(h2d<float>(c, c->rn_buf[4], nullptr, (size_t)B * P.A, &o2)); MZ_TRY(h2d<float>(c, c->rn_buf[5], nullptr, (size_t)B, &r));
+    MZ_TRY(h2d<unsigned char>(c, c->rn_buf[6], nullptr, (size_t)B * c->rn.R.node_bytes + 256, &pool));
     const int K1 = P.K + 1, tb = (B + 127) / 128;
-    float *h = c->d_rn_h, *nh = c->d_rn_nh;
-    MZ_TRY(rn_forward_dev(c, 0, B, c->batch.obs, h, nullptr));                                            // :347
-    MZ_TRY(rn_forward_dev(c, 1, B, h, c->d_rn_o1, c->d_rn_o2));                                           // :351 (= row 1's prediction, Q19)
-    { launch_scope ls(c, 3); mz_k_rn_scatter<<<tb, 128, 0, c->stream>>>(B, P.A, K1, 0, P.K > 0 ? 1 : -1, c->d_rn_o1, c->d_rn_o2, nullptr, 1, c->d_pv, c->d_pp, c->d_pr); }
+    MZ_TRY(rn_forward_dev(c, 0, B, c->batch.obs, h, nullptr, pool));                                      // :347
+    MZ_TRY(rn_forward_dev(c, 1, B, h, o1, o2, pool));                                                      // :351 (= row 1's prediction, Q19)
+    { launch_scope ls(c, 3); mz_k_rn_scatter<<<tb, 128, 0, c->stream>>>(B, P.A, K1, 0, P.K > 0 ? 1 : -1, o1, o2, nullptr, 1, c->d_pv, c->d_pp, c->d_pr); }
     for (int i = 1; i <= P.K; i++) {                                                                       // :355-370
         if (i > 1) {
-            MZ_TRY(rn_forward_dev(c, 1, B, h, c->d_rn_o1, c->d_rn_o2));
-            launch_scope ls(c, 3); mz_k_rn_scatter<<<tb, 128, 0, c->stream>>>(B, P.A, K1, i, -1, c->d_rn_o1, c->d_rn_o2, nullptr, 0, c->d_pv, c->d_pp, c->d_pr);
+            MZ_TRY(rn_forward_dev(c, 1, B, h, o1, o2, pool));
+            launch_scope ls(c, 3); mz_k_rn_scatter<<<tb, 128, 0, c->stream>>>(B, P.A, K1, i, -1, o1, o2, nullptr, 0, c->d_pv, c->d_pp, c->d_pr);
         }
-        { launch_scope ls(c, 3); mz_k_rn_make_sa<<<(B * P.sa_size + 255) / 256, 256, 0, c->stream>>>(B, P.hidden, P.cells, P.A, K1, i - 1, h, c->batch.actions, c->d_rn_sa); }
-        MZ_TRY(rn_forward_dev(c, 2, B, c->d_rn_sa, nh, c->d_rn_r));
-        { launch_scope ls(c, 3); mz_k_rn_scatter<<<tb, 128, 0, c->stream>>>(B, P.A, K1, i, -1, nullptr, nullptr, c->d_rn_r, 0, c->d_pv, c->d_pp, c->d_pr); }
+        { launch_scope ls(c, 3); mz_k_rn_make_sa<<<(B * P.sa_size + 255) / 256, 256, 0, c->stream>>>(B, P.hidden, P.cells, P.A, K1, i - 1, h, c->batch.actions, sa); }
+        MZ_TRY(rn_forward_dev(c, 2, B, sa, nh, r, pool));
+        { launch_scope ls(c, 3); mz_k_rn_scatter<<<tb, 128, 0, c->stream>>>(B, P.A, K1, i, -1, nullptr, nullptr, r, 0, c->d_pv, c->d_pp, c->d_pr); }
         float *t = h; h = nh; nh = t;
     }
-    const int ry = K1 < MZ_LOSS_RY ? K1 : MZ_LOSS_RY;
-    { launch_scope ls(c, 3); mz_k_loss_rows<<<(B + 31) / 32, dim3(32, (unsigned)ry), 0, c->stream>>>(P, B, c->batch, c->d_pv, c->d_pr, c->d_pp, c->d_rowv, c->d_rowr, c->d_rowp, c->d_rowinvg); }
-    { launch_scope ls(c, 3); mz_k_loss_reduce<<<4, 1024, 0, c->stream>>>(P, B, c->d_rowv, c->d_rowr, c->d_rowp, c->d_rowinvg, c->d_rn_theta, c->d_lossout, 4); }
-    { launch_scope ls(c, 3); mz_k_rn_sqnorm<<<3, 1024, 0, c->stream>>>(c->rn.base[0], c->rn.base[1], c->rn.base[2], c->M.P.n_params, c->d_rn_theta, c->d_rn_mask, c->d_lossout); }
-    MZ_CUDA(c, cudaGetLastError());
     return MZ_OK;
+}
+
+// the loss (Learning.jl:261-288) from the unroll's predictions: per-sample partial sums, then the data terms and each network's sum(theta^2).
+// Without a mask, the 7-CTA reduce sums theta^2 layer by layer over the padded store (the FeedForwardHP losses' summation order); with one,
+// the data terms and then the masked sums over net_bounds (Flux.params leave out the BatchNorm statistics)
+void launch_loss(mz_ctx *c, int B) {
+    const mz_params &P = c->M.P;
+    { launch_scope ls(c, 3); const int ry = P.K + 1 < MZ_LOSS_RY ? P.K + 1 : MZ_LOSS_RY;
+      mz_k_loss_rows<<<(B + 31) / 32, dim3(32, (unsigned)ry), 0, c->stream>>>(P, B, c->batch, c->d_pv, c->d_pr, c->d_pp, c->d_rowv, c->d_rowr, c->d_rowp, c->d_rowinvg); }
+    if (c->d_mask) {
+        { launch_scope ls(c, 3); mz_k_loss_reduce<<<4, 1024, 0, c->stream>>>(P, B, c->d_rowv, c->d_rowr, c->d_rowp, c->d_rowinvg, c->d_w, c->d_lossout, 4); }
+        { launch_scope ls(c, 3); mz_k_sqnorm_masked<<<3, 1024, 0, c->stream>>>(c->net_bounds[0], c->net_bounds[1], c->net_bounds[2], c->net_bounds[3], c->d_w, c->d_mask, c->d_lossout); }
+    } else { launch_scope ls(c, 3); mz_k_loss_reduce<<<7, 1024, 0, c->stream>>>(P, B, c->d_rowv, c->d_rowr, c->d_rowp, c->d_rowinvg, c->d_w, c->d_lossout); }
 }
 
 int launch_learn_forward(mz_ctx *c, int B, int grad_mode = MZ_GRAD_REFERENCE_L2) {
     const mz_params &P = c->M.P;
-    if (c->cfg.net_type == MZ_NET_RESNET) return rn_learn_forward(c, B, grad_mode);
+    const int path = learner_path(c, grad_mode);
+    if (path == -1) return fail(c, MZ_E_UNSUPPORTED, "the ResNet learner implements MZ_GRAD_REFERENCE_L2 (the reference's update); the backward pass through the convolution towers is not built");
+    if (path != 3 && grad_mode != MZ_GRAD_REFERENCE_L2 && grad_mode != MZ_GRAD_BPTT) return fail(c, MZ_E_ARG, "unknown grad_mode %d", grad_mode);
     mz_learn_args a{}; a.wglob = c->d_w; a.B = B; a.max_dim = c->M.max_dim; a.max_layer_floats = c->M.max_layer_floats; a.batch = c->batch;
     a.pred_values = c->d_pv; a.pred_rewards = c->d_pr; a.pred_policies = c->d_pp;
     const int tiles = (B + MZ_ROWS - 1) / MZ_ROWS;
-    if (grad_mode == MZ_GRAD_BPTT && c->cfg.nn_mode == MZ_NN_SPLIT_MMA && c->lrp.ok && !getenv("MUZERO_B200_BPTT_SIMT")) {
+    if (path == 3) MZ_TRY(rn_learn_forward(c, B));
+    else if (path == 2) {
         // forward + backward on the tensor cores (mz_learner_tc.cuh): kernel 1 = unroll forward + dX chain with saved tiles, kernel 2 = dW / db
         MZ_TRY(ensure_images(c));
         const mz_lr_plan &L = c->lrp;
         const int chunks = tiles < 16 ? tiles : 16;
-        if (tiles > c->lr_tiles_cap) {
-            if (c->d_xsave) cudaFree(c->d_xsave);
-            if (c->d_dzsave) cudaFree(c->d_dzsave);
-            c->d_xsave = c->d_dzsave = nullptr; c->lr_tiles_cap = 0;
-            const size_t bytes = (size_t)tiles * L.slots_per_cta * MZ_SP_TILE_BYTES;
-            MZ_CUDA(c, cudaMalloc((void **)&c->d_xsave, bytes)); MZ_CUDA(c, cudaMalloc((void **)&c->d_dzsave, bytes));
-            MZ_CUDA(c, cudaMemsetAsync(c->d_xsave, 0, bytes, c->stream)); MZ_CUDA(c, cudaMemsetAsync(c->d_dzsave, 0, bytes, c->stream));
-            c->lr_tiles_cap = tiles;
-        }
-        if (chunks > c->lr_chunks_cap) {
-            if (c->d_gpart_tc) cudaFree(c->d_gpart_tc);
-            c->d_gpart_tc = nullptr; c->lr_chunks_cap = 0;
-            MZ_CUDA(c, dmalloc(&c->d_gpart_tc, (size_t)chunks * P.total_floats));
-            MZ_CUDA(c, cudaMemsetAsync(c->d_gpart_tc, 0, (size_t)chunks * P.total_floats * sizeof(float), c->stream));
-            c->lr_chunks_cap = chunks;
-        }
+        const size_t bytes = (size_t)tiles * L.slots_per_cta * MZ_SP_TILE_BYTES;
+        unsigned char *xsave, *dzsave; float *gpart;
+        MZ_TRY(alloc_zeroed(c, c->lr_xsave, bytes, &xsave)); MZ_TRY(alloc_zeroed(c, c->lr_dzsave, bytes, &dzsave));
+        MZ_TRY(alloc_zeroed(c, c->lr_gpart, (size_t)chunks * P.total_floats, &gpart));
         mz_lr_args t{}; t.sp = c->spa; t.sp.pbc_smem = 0; t.brounds = c->d_brounds;
         for (int n = 0; n < 3; n++) {
             t.bfirst[n] = L.bfirst[n]; t.bn_rounds[n] = L.bn_rounds[n]; t.slot_base[n] = L.slot_base[n]; t.layers_in_net[n] = L.layers_in_net[n]; t.first_layer[n] = P.nets[n].first;
             for (int h = 0; h < 2; h++) { t.start_tile[n][h] = L.start_tile[n][h]; t.start_layer[n][h] = L.start_layer[n][h]; t.start_perm[n][h] = L.start_perm[n][h]; }
         }
         t.btotal_rounds = L.btotal_rounds; t.slots_per_cta = L.slots_per_cta; t.n_eval = L.n_eval; t.lg_off = (L.bwarea_bytes + 127) & ~127; t.dh_extra = mz_lr_alias_fits(c->spp.bias_floats, P.hidden_pad) ? 0 : 1;
-        t.f.f = a; t.xsave = c->d_xsave; t.dzsave = c->d_dzsave; t.dbg = getenv("MUZERO_B200_LR_STAMPS") ? c->d_stats + 4 : nullptr;
+        t.f.f = a; t.xsave = xsave; t.dzsave = dzsave; t.dbg = getenv("MUZERO_B200_LR_STAMPS") ? c->d_stats + 4 : nullptr;
         t.inv_g_sum = c->d_lossout + 7;                                    // (slot 7 of the loss scratch is free)
         { launch_scope ls(c, 3); mz_k_inv_g_sum<<<1, 1024, 0, c->stream>>>(B, c->batch.gscale, (P.per && c->batch.weights) ? c->batch.weights : nullptr, c->d_lossout + 7); }
         { launch_scope ls(c, 3); mz_k_learn_bptt_tc<<<tiles, MZ_SP_THREADS, c->smem_bytes_lr, c->stream>>>(P, t); }
-        mz_dw_args d{}; d.xsave = c->d_xsave; d.dzsave = c->d_dzsave; d.gpart = c->d_gpart_tc; d.tiles = tiles; d.chunks = chunks; d.slots_per_cta = L.slots_per_cta; d.n_eval = L.n_eval;
+        mz_dw_args d{}; d.xsave = xsave; d.dzsave = dzsave; d.gpart = gpart; d.tiles = tiles; d.chunks = chunks; d.slots_per_cta = L.slots_per_cta; d.n_eval = L.n_eval;
         for (int n = 0; n < 3; n++) { d.slot_base[n] = L.slot_base[n]; d.layers_in_net[n] = L.layers_in_net[n]; d.first_layer[n] = P.nets[n].first; }
         { launch_scope ls(c, 3); mz_k_learn_dw<<<dim3((unsigned)P.n_layers, (unsigned)chunks), 128, MZ_DW_STAGES * 2 * MZ_SP_TILE_BYTES + 1024, c->stream>>>(P, d); }
         // (use_batch_norm: the images these kernels read are the folded layers (mz_k_pack_images), so the sums are dW', db': same chain rule as below)
-        if (c->cfg.use_batch_norm) { launch_scope ls(c, 4); mz_k_grad_reduce_bn<<<dim3((unsigned)P.n_layers, 16), 256, 0, c->stream>>>(P, chunks, c->d_gpart_tc, c->d_w, grad_out(c)); }
-        else { launch_scope ls(c, 4); mz_k_grad_reduce<<<(P.total_floats + 255) / 256, 256, 0, c->stream>>>(P.total_floats, chunks, c->d_gpart_tc, c->d_w, grad_out(c)); }
+        if (c->cfg.use_batch_norm) { launch_scope ls(c, 4); mz_k_grad_reduce_bn<<<dim3((unsigned)P.n_layers, 16), 256, 0, c->stream>>>(P, chunks, gpart, c->d_w, grad_out(c)); }
+        else { launch_scope ls(c, 4); mz_k_grad_reduce<<<(P.total_floats + 255) / 256, 256, 0, c->stream>>>(P.total_floats, chunks, gpart, c->d_w, grad_out(c)); }
     } else if (grad_mode == MZ_GRAD_BPTT) {   // forward + backward through the unroll in one kernel; per-tile partial gradients
         if (!c->smem_bytes_bptt) return fail(c, MZ_E_UNSUPPORTED, "MZ_GRAD_BPTT is not built for this network: it needs every layer output and every layer input other than the observation stack to be at most 64 wide, and its buffers to fit one CTA's shared memory");
-        if (tiles > c->bptt_tiles_cap) {
-            if (c->d_act) cudaFree(c->d_act);
-            if (c->d_gpart) cudaFree(c->d_gpart);
-            c->d_act = nullptr; c->d_gpart = nullptr; c->bptt_tiles_cap = 0;
-            MZ_CUDA(c, dmalloc(&c->d_act, (size_t)tiles * c->bptt.plan.tile_floats));
-            MZ_CUDA(c, dmalloc(&c->d_gpart, (size_t)tiles * P.total_floats));
-            c->bptt_tiles_cap = tiles;
-        }
-        mz_bptt_args b{}; b.f = a; b.act = c->d_act; b.gpart = c->d_gpart; b.stages[0] = c->d_bstages[0]; b.stages[1] = c->d_bstages[1];
+        float *act, *gpart;
+        MZ_TRY(h2d<float>(c, c->bptt_act, nullptr, (size_t)tiles * c->bptt.plan.tile_floats, &act));
+        MZ_TRY(h2d<float>(c, c->bptt_gpart, nullptr, (size_t)tiles * P.total_floats, &gpart));
+        mz_bptt_args b{}; b.f = a; b.act = act; b.gpart = gpart; b.stages[0] = c->d_bstages[0]; b.stages[1] = c->d_bstages[1];
         b.dim_wide = c->bptt_dims[0]; b.dim_narrow = c->bptt_dims[1]; b.wfloats[0] = c->bptt_dims[2]; b.wfloats[1] = c->bptt_dims[3];
         if (c->cfg.use_batch_norm) {   // BatchNorm in test mode = a Dense layer with folded weights: the kernel runs on the folded copy, the reduce applies the chain rule
             if (!c->d_w_fold) MZ_CUDA(c, dmalloc(&c->d_w_fold, (size_t)P.total_floats));
@@ -414,23 +424,18 @@ int launch_learn_forward(mz_ctx *c, int B, int grad_mode = MZ_GRAD_REFERENCE_L2)
             b.f.wglob = c->d_w_fold;
         }
         { launch_scope ls(c, 3); mz_k_learn_bptt<<<tiles, MZ_THREADS, c->smem_bytes_bptt, c->stream>>>(P, c->bptt.plan, b); }
-        if (c->cfg.use_batch_norm) { launch_scope ls(c, 4); mz_k_grad_reduce_bn<<<dim3((unsigned)P.n_layers, 16), 256, 0, c->stream>>>(P, tiles, c->d_gpart, c->d_w, grad_out(c)); }
-        else { launch_scope ls(c, 4); mz_k_grad_reduce<<<(P.total_floats + 255) / 256, 256, 0, c->stream>>>(P.total_floats, tiles, c->d_gpart, c->d_w, grad_out(c)); }
-    } else if (grad_mode == MZ_GRAD_REFERENCE_L2 && c->cfg.nn_mode == MZ_NN_SPLIT_MMA) {   // the unroll on the tensor cores (mz_kernels_sp.cuh)
+        if (c->cfg.use_batch_norm) { launch_scope ls(c, 4); mz_k_grad_reduce_bn<<<dim3((unsigned)P.n_layers, 16), 256, 0, c->stream>>>(P, tiles, gpart, c->d_w, grad_out(c)); }
+        else { launch_scope ls(c, 4); mz_k_grad_reduce<<<(P.total_floats + 255) / 256, 256, 0, c->stream>>>(P.total_floats, tiles, gpart, c->d_w, grad_out(c)); }
+    } else if (path == 1) {   // the unroll on the tensor cores (mz_kernels_sp.cuh)
         MZ_TRY(ensure_images(c));
         mz_learn_sp_args t{}; t.sp = c->spa; t.B = B; t.batch = c->batch; t.pred_values = c->d_pv; t.pred_rewards = c->d_pr; t.pred_policies = c->d_pp;
         launch_scope ls(c, 3); mz_k_learn_forward_sp<<<tiles, MZ_SP_THREADS, c->smem_bytes_sp, c->stream>>>(P, t);
-    } else if (grad_mode == MZ_GRAD_REFERENCE_L2) {
+    } else {
         launch_scope ls(c, 3);
         if (c->cfg.use_batch_norm) mz_k_learn_forward<true><<<tiles, MZ_THREADS, c->smem_bytes, c->stream>>>(P, a);
         else mz_k_learn_forward<false><<<tiles, MZ_THREADS, c->smem_bytes, c->stream>>>(P, a);
-    } else return fail(c, MZ_E_ARG, "unknown grad_mode %d", grad_mode);
-    { launch_scope ls(c, 3); const int ry = P.K + 1 < MZ_LOSS_RY ? P.K + 1 : MZ_LOSS_RY;
-      mz_k_loss_rows<<<(B + 31) / 32, dim3(32, (unsigned)ry), 0, c->stream>>>(P, B, c->batch, c->d_pv, c->d_pr, c->d_pp, c->d_rowv, c->d_rowr, c->d_rowp, c->d_rowinvg); }
-    if (c->d_fc_mask) {   // use_batch_norm: sum(theta^2) over Flux.params leaves out the BatchNorm statistics
-        { launch_scope ls(c, 3); mz_k_loss_reduce<<<4, 1024, 0, c->stream>>>(P, B, c->d_rowv, c->d_rowr, c->d_rowp, c->d_rowinvg, c->d_w, c->d_lossout, 4); }
-        { launch_scope ls(c, 3); mz_k_rn_sqnorm<<<3, 1024, 0, c->stream>>>(c->fc_net_bounds[0], c->fc_net_bounds[1], c->fc_net_bounds[2], c->fc_net_bounds[3], c->d_w, c->d_fc_mask, c->d_lossout); }
-    } else { launch_scope ls(c, 3); mz_k_loss_reduce<<<7, 1024, 0, c->stream>>>(P, B, c->d_rowv, c->d_rowr, c->d_rowp, c->d_rowinvg, c->d_w, c->d_lossout); }
+    }
+    launch_loss(c, B);
     MZ_CUDA(c, cudaGetLastError());
     return MZ_OK;
 }
@@ -447,50 +452,31 @@ int finish_losses(mz_ctx *c, int B, float *losses) {
     for (int n = 0; n < 3; n++) losses[n] = data + (float)o[4 + n];
     return MZ_OK;
 }
+// one learning! update of the parameter store.  The BatchNorm statistics (d_mask = 0) have zero gradient and stay put.
 int launch_update(mz_ctx *c, int64_t t, int grad_mode) {
-    if (c->cfg.net_type == MZ_NET_RESNET) {   // ADAM on 2 * theta over Flux.params; the BatchNorm statistics have zero gradient and stay put
-        const int n = c->M.P.n_params;
-        if (t == 1 && c->adam_t > 1) { MZ_CUDA(c, cudaMemsetAsync(c->d_rn_m, 0, (size_t)n * 4, c->stream)); MZ_CUDA(c, cudaMemsetAsync(c->d_rn_v, 0, (size_t)n * 4, c->stream)); }
-        if (t == 1 || c->adam_t == 0) { c->bp1 = 0.9; c->bp2 = 0.999; c->adam_t = 1; }
-        { launch_scope ls(c, 4); mz_k_grad_l2_masked<<<(n + 255) / 256, 256, 0, c->stream>>>(n, c->d_rn_theta, c->d_rn_mask, c->d_rn_grad); }
-        float scale = 1.0f;
-        if (c->comm) {
-            ncclResult_t r = g_nccl.AllReduce(c->d_rn_grad, c->d_rn_grad, (size_t)n, ncclFloat, ncclSum, c->comm, c->stream);
-            if (r != ncclSuccess) return fail(c, MZ_E_NCCL, "ncclAllReduce: %s", g_nccl.GetErrorString(r));
-            scale = 1.0f / (float)c->nranks;
-        }
-        { launch_scope ls(c, 4); mz_k_adam<<<(n + 255) / 256, 256, 0, c->stream>>>(n, c->d_rn_theta, c->d_rn_m, c->d_rn_v, c->d_rn_grad, mzh::cos_schedule(t), c->bp1, c->bp2, scale); }
-        MZ_CUDA(c, cudaGetLastError());
-        c->bp1 *= 0.9; c->bp2 *= 0.999; c->adam_t++;
-        c->rn_dirty = true;
-        return MZ_OK;
+    const int n = c->store_floats;
+    if (t == 1) {   // learning! builds a fresh optimiser (Learning.jl:318): restarting at step 1 clears the moments too
+        if (c->adam_t > 1) { MZ_CUDA(c, cudaMemsetAsync(c->d_m, 0, (size_t)n * 4, c->stream)); MZ_CUDA(c, cudaMemsetAsync(c->d_v, 0, (size_t)n * 4, c->stream)); }
+        adam_seek(c, 0);
     }
-    const int n = c->M.P.total_floats;
-    if (t == 1 && c->adam_t > 1) {   // learning! builds a fresh optimiser (Learning.jl:318): restarting at step 1 clears the moments too
-        MZ_CUDA(c, cudaMemsetAsync(c->d_m, 0, (size_t)n * 4, c->stream)); MZ_CUDA(c, cudaMemsetAsync(c->d_v, 0, (size_t)n * 4, c->stream));
-    }
-    if (t == 1 || c->adam_t == 0) { c->bp1 = 0.9; c->bp2 = 0.999; c->adam_t = 1; }
     // MZ_GRAD_BPTT: d_grad was produced by launch_learn_forward (mz_k_learn_bptt + mz_k_grad_reduce)
     if (grad_mode == MZ_GRAD_REFERENCE_L2 && !c->p2p && !c->comm) {   // one GPU: gradient (2 * theta) and update in one launch
-        { launch_scope ls(c, 4); mz_k_adam_l2<<<(n + 255) / 256, 256, 0, c->stream>>>(n, c->d_w, c->d_m, c->d_v, c->d_grad, c->d_fc_mask, mzh::cos_schedule(t), c->bp1, c->bp2); }
-        MZ_CUDA(c, cudaGetLastError());
-        c->bp1 *= 0.9; c->bp2 *= 0.999; c->adam_t++;
-        c->w_version++;
-        return MZ_OK;
-    }
-    if (grad_mode == MZ_GRAD_REFERENCE_L2) { launch_scope ls(c, 4); if (c->d_fc_mask) mz_k_grad_l2_masked<<<(n + 255) / 256, 256, 0, c->stream>>>(n, c->d_w, c->d_fc_mask, grad_out(c)); else mz_k_grad_l2<<<(n + 255) / 256, 256, 0, c->stream>>>(n, c->d_w, grad_out(c)); }
-    float scale = 1.0f;
-    if (c->p2p) {    // data-parallel over peer memory: ONE kernel waits for the peers' gradients, sums them in rank order over NVLink and applies ADAM
-        mz_dp_args d{}; d.rank = c->rank; d.nranks = c->nranks; d.step = ++c->dp_step; d.n = n; d.flags_local = c->d_xflags;
-        for (int r = 0; r < c->nranks; r++) { d.peer_grad[r] = c->peer_grad[r] + (size_t)(d.step & 1u) * (size_t)n; d.peer_flags[r] = c->peer_flags[r]; }
-        launch_scope ls(c, 4); mz_k_dp_adam<<<(n + 255) / 256, 256, 0, c->stream>>>(c->d_w, c->d_m, c->d_v, d, mzh::cos_schedule(t), c->bp1, c->bp2, 1.0f / (float)c->nranks);
+        launch_scope ls(c, 4); mz_k_adam_l2<<<(n + 255) / 256, 256, 0, c->stream>>>(n, c->d_w, c->d_m, c->d_v, c->d_grad, c->d_mask, mzh::cos_schedule(t), c->bp1, c->bp2);
     } else {
-        if (c->comm) {   // data-parallel through NCCL: sum gradients over ranks, average in the update
-            ncclResult_t r = g_nccl.AllReduce(c->d_grad, c->d_grad, (size_t)n, ncclFloat, ncclSum, c->comm, c->stream);
-            if (r != ncclSuccess) return fail(c, MZ_E_NCCL, "ncclAllReduce: %s", g_nccl.GetErrorString(r));
-            scale = 1.0f / (float)c->nranks;
+        if (grad_mode == MZ_GRAD_REFERENCE_L2) { launch_scope ls(c, 4); mz_k_l2_grad<<<(n + 255) / 256, 256, 0, c->stream>>>(n, c->d_w, c->d_mask, grad_out(c)); }
+        if (c->p2p) {    // data-parallel over peer memory: ONE kernel waits for the peers' gradients, sums them in rank order over NVLink and applies ADAM
+            mz_dp_args d{}; d.rank = c->rank; d.nranks = c->nranks; d.step = ++c->dp_step; d.n = n; d.flags_local = c->d_xflags;
+            for (int r = 0; r < c->nranks; r++) { d.peer_grad[r] = c->peer_grad[r] + (size_t)(d.step & 1u) * (size_t)n; d.peer_flags[r] = c->peer_flags[r]; }
+            launch_scope ls(c, 4); mz_k_dp_adam<<<(n + 255) / 256, 256, 0, c->stream>>>(c->d_w, c->d_m, c->d_v, d, mzh::cos_schedule(t), c->bp1, c->bp2, 1.0f / (float)c->nranks);
+        } else {
+            float scale = 1.0f;
+            if (c->comm) {   // data-parallel through NCCL: sum gradients over ranks, average in the update
+                ncclResult_t r = g_nccl.AllReduce(c->d_grad, c->d_grad, (size_t)n, ncclFloat, ncclSum, c->comm, c->stream);
+                if (r != ncclSuccess) return fail(c, MZ_E_NCCL, "ncclAllReduce: %s", g_nccl.GetErrorString(r));
+                scale = 1.0f / (float)c->nranks;
+            }
+            launch_scope ls(c, 4); mz_k_adam<<<(n + 255) / 256, 256, 0, c->stream>>>(n, c->d_w, c->d_m, c->d_v, c->d_grad, mzh::cos_schedule(t), c->bp1, c->bp2, scale);
         }
-        launch_scope ls(c, 4); mz_k_adam<<<(n + 255) / 256, 256, 0, c->stream>>>(n, c->d_w, c->d_m, c->d_v, c->d_grad, mzh::cos_schedule(t), c->bp1, c->bp2, scale);
     }
     MZ_CUDA(c, cudaGetLastError());
     c->bp1 *= 0.9; c->bp2 *= 0.999; c->adam_t++;
@@ -585,16 +571,6 @@ int mz_create(const mz_config *cfg, int device, mz_ctx **out) {
         MZ_CREATE(cudaMalloc((void **)&c->d_rn_image, (size_t)c->rn.image_bytes + 4096));
         MZ_CREATE(dmalloc(&c->d_rn_steps, c->rn.steps.size() + 1));
         MZ_CREATE(cudaMemcpy(c->d_rn_steps, c->rn.steps.data(), c->rn.steps.size() * sizeof(mz_rn_step), cudaMemcpyHostToDevice));
-        c->rn_blob.assign((size_t)c->M.P.n_params, 0.0f);
-        {   // learner state: fp32 parameters (blob order), ADAM moments, gradient, the mask of Flux.params (everything but the BatchNorm statistics)
-            const size_t np = (size_t)c->M.P.n_params;
-            MZ_CREATE(dmalloc(&c->d_rn_theta, np)); MZ_CREATE(dmalloc(&c->d_rn_m, np)); MZ_CREATE(dmalloc(&c->d_rn_v, np)); MZ_CREATE(dmalloc(&c->d_rn_grad, np));
-            MZ_CREATE(cudaMalloc((void **)&c->d_rn_mask, np + 16));
-            MZ_CREATE(cudaMemset(c->d_rn_theta, 0, np * 4)); MZ_CREATE(cudaMemset(c->d_rn_m, 0, np * 4)); MZ_CREATE(cudaMemset(c->d_rn_v, 0, np * 4));
-            std::vector<unsigned char> mask(np, 1);
-            for (int n = 0; n < 3; n++) for (const mzh::rn_unit &u : c->rn.units[n]) if (u.kind == 0) for (int i = 0; i < u.cout; i++) { mask[(size_t)u.mu_off + i] = 0; mask[(size_t)u.var_off + i] = 0; }
-            MZ_CREATE(cudaMemcpy(c->d_rn_mask, mask.data(), np, cudaMemcpyHostToDevice));
-        }
     }
     const mz_params &P = c->M.P;
     c->smem_bytes = resnet ? 0 : mz_smem_bytes(c->M.max_dim, c->M.max_layer_floats, P.hidden_pad, P.S);
@@ -711,15 +687,21 @@ int mz_create(const mz_config *cfg, int device, mz_ctx **out) {
     MZ_CREATE(cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking)); c->own_stream = true;
     MZ_CREATE(cudaStreamCreateWithFlags(&c->stream2, cudaStreamNonBlocking));
     for (int i = 0; i < 2; i++) MZ_CREATE(cudaEventCreateWithFlags(&c->ev_search[i], cudaEventDisableTiming));
-    const size_t nf = (size_t)P.total_floats;
+    c->packed = !resnet;
+    c->store_floats = resnet ? P.n_params : P.total_floats;
+    const size_t nf = (size_t)c->store_floats;
     MZ_CREATE(dmalloc(&c->d_w, nf)); MZ_CREATE(dmalloc(&c->d_m, nf)); MZ_CREATE(dmalloc(&c->d_v, nf)); MZ_CREATE(dmalloc(&c->d_grad, nf));
     MZ_CREATE(cudaMemset(c->d_w, 0, nf * 4)); MZ_CREATE(cudaMemset(c->d_m, 0, nf * 4)); MZ_CREATE(cudaMemset(c->d_v, 0, nf * 4));
-    if (!resnet && cfg->use_batch_norm) {   // Flux.params of a BatchNorm are beta and gamma: the running statistics take no part in sum(abs2, theta), its gradient or ADAM
+    if (resnet || cfg->use_batch_norm) {   // Flux.params of a BatchNorm are beta and gamma: the running statistics take no part in sum(abs2, theta), its gradient or ADAM
         std::vector<unsigned char> mask(nf + 16, 1);
-        for (int i = 0; i < P.n_layers; i++) if (P.layers[i].bn) for (int o = 0; o < 2 * P.layers[i].out_pad; o++) mask[(size_t)P.layers[i].b_off + 3 * P.layers[i].out_pad + o] = 0;
-        MZ_CREATE(cudaMalloc((void **)&c->d_fc_mask, nf + 16)); MZ_CREATE(cudaMemcpy(c->d_fc_mask, mask.data(), nf + 16, cudaMemcpyHostToDevice));
-        for (int n = 0; n < 3; n++) c->fc_net_bounds[n] = P.layers[P.nets[n].first].w_off;
-        c->fc_net_bounds[3] = (int)nf;
+        if (resnet) {
+            for (int n = 0; n < 3; n++) for (const mzh::rn_unit &u : c->rn.units[n]) if (u.kind == 0) for (int i = 0; i < u.cout; i++) { mask[(size_t)u.mu_off + i] = 0; mask[(size_t)u.var_off + i] = 0; }
+        } else {
+            for (int i = 0; i < P.n_layers; i++) if (P.layers[i].bn) for (int o = 0; o < 2 * P.layers[i].out_pad; o++) mask[(size_t)P.layers[i].b_off + 3 * P.layers[i].out_pad + o] = 0;
+        }
+        MZ_CREATE(cudaMalloc((void **)&c->d_mask, nf + 16)); MZ_CREATE(cudaMemcpy(c->d_mask, mask.data(), nf + 16, cudaMemcpyHostToDevice));
+        for (int n = 0; n < 3; n++) c->net_bounds[n] = resnet ? c->rn.base[n] : P.layers[P.nets[n].first].w_off;
+        c->net_bounds[3] = (int)nf;
     }
     MZ_CREATE(dmalloc(&c->d_pbc0, c->M.pbc0.size())); MZ_CREATE(dmalloc(&c->d_sqrtN, c->M.sqrtN.size()));
     MZ_CREATE(cudaMemcpy(c->d_pbc0, c->M.pbc0.data(), c->M.pbc0.size() * 8, cudaMemcpyHostToDevice));
@@ -734,15 +716,7 @@ int mz_create(const mz_config *cfg, int device, mz_ctx **out) {
     MZ_CREATE(dmalloc(&s.h_reward, G * Tm)); MZ_CREATE(dmalloc(&s.h_to_play, G * Tm)); MZ_CREATE(dmalloc(&s.h_cv, G * Tm * P.A)); MZ_CREATE(dmalloc(&s.h_rv, G * Tm));
     MZ_CREATE(cudaMemset(s.status, 0, G * sizeof(int32_t)));
     MZ_CREATE(cudaMemset(s.h_p1, 0, G * Tm * sizeof(uint64_t))); MZ_CREATE(cudaMemset(s.h_p2, 0, G * Tm * sizeof(uint64_t)));   // the board before move 0 is empty
-    mz_ring &r = c->ring; r.capacity = (int64_t)R;
-    MZ_CREATE(dmalloc(&r.game_id, R)); MZ_CREATE(dmalloc(&r.T, R));
-    MZ_CREATE(dmalloc(&r.h_p1, R * Tm)); MZ_CREATE(dmalloc(&r.h_p2, R * Tm)); MZ_CREATE(dmalloc(&r.h_action, R * Tm));
-    MZ_CREATE(dmalloc(&r.h_reward, R * Tm)); MZ_CREATE(dmalloc(&r.h_to_play, R * Tm)); MZ_CREATE(dmalloc(&r.h_cv, R * Tm * P.A)); MZ_CREATE(dmalloc(&r.h_rv, R * Tm));
-    MZ_CREATE(dmalloc(&r.q_pos, R * Tm)); MZ_CREATE(dmalloc(&r.q_game, R)); MZ_CREATE(dmalloc(&r.prefix, R)); MZ_CREATE(dmalloc(&r.upd, R * Tm));
-    MZ_CREATE(cudaMemset(r.q_pos, 0, R * Tm * 4)); MZ_CREATE(cudaMemset(r.q_game, 0, R * 4)); MZ_CREATE(cudaMemset(r.upd, 0, R * Tm * 8));
-    MZ_CREATE(dmalloc(&r.h_rrv, R * Tm)); MZ_CREATE(dmalloc(&r.reanalysed, R)); MZ_CREATE(cudaMemset(r.reanalysed, 0, R)); MZ_CREATE(cudaMemset(r.h_rrv, 0, R * Tm * sizeof(float)));
-    MZ_CREATE(dmalloc(&r.counters, 8)); MZ_CREATE(cudaMemset(r.counters, 0, 8 * sizeof(int64_t)));
-    MZ_CREATE(cudaMemset(r.T, 0, R * sizeof(int32_t)));
+    if (const int rr = alloc_ring(c, c->ring, R)) { mz_destroy(c); return rr; }
     MZ_CREATE(dmalloc(&c->d_stats, 64)); MZ_CREATE(cudaMemset(c->d_stats, 0, 64 * sizeof(unsigned long long)));
     MZ_CREATE(dmalloc(&c->d_lossout, 8));
     MZ_CREATE(cudaMallocHost((void **)&c->h_counters, 8 * sizeof(int64_t)));
@@ -763,14 +737,16 @@ int mz_destroy(mz_ctx *c) {
     if (c->stream) cudaStreamSynchronize(c->stream);
     collect_timings(c);
     if (c->comm && g_nccl.CommDestroy) { p2p_teardown(c); g_nccl.CommDestroy(c->comm); }
-    void *ptrs[] = {c->d_fc_mask, c->d_w_fold, c->d_w_lat, c->d_rn_theta, c->d_rn_m, c->d_rn_v, c->d_rn_grad, c->d_rn_h, c->d_rn_nh, c->d_rn_sa, c->d_rn_o1, c->d_rn_o2, c->d_rn_r, c->d_rn_mask, c->d_rn_pool, c->d_brounds, c->d_xsave, c->d_dzsave, c->d_gpart_tc, c->d_w_sp, c->d_bias_sp, c->d_rounds_sp, c->d_rn_image, c->d_rn_steps, c->d_bstages[0], c->d_bstages[1], c->d_act, c->d_gpart, c->d_w_tc, c->d_bias_tc, c->d_w, c->d_m, c->d_v, c->d_grad, c->d_pbc0, c->d_sqrtN, c->d_trees, c->slots.p1, c->slots.p2, c->slots.player, c->slots.T,
+    void *ptrs[] = {c->d_mask, c->d_w_fold, c->d_w_lat, c->d_brounds, c->d_w_sp, c->d_bias_sp, c->d_rounds_sp, c->d_rn_image, c->d_rn_steps, c->d_bstages[0], c->d_bstages[1], c->d_w_tc, c->d_bias_tc, c->d_w, c->d_m, c->d_v, c->d_grad, c->d_pbc0, c->d_sqrtN, c->d_trees, c->slots.p1, c->slots.p2, c->slots.player, c->slots.T,
                     c->slots.status, c->slots.game_id, c->slots.fin_list, c->slots.h_p1, c->slots.h_p2, c->slots.h_action, c->slots.h_reward, c->slots.h_to_play,
-                    c->slots.h_cv, c->slots.h_rv, c->ring.game_id, c->ring.T, c->ring.h_p1, c->ring.h_p2, c->ring.h_action, c->ring.h_reward,
-                    c->ring.h_to_play, c->ring.h_cv, c->ring.h_rv, c->ring.h_rrv, c->ring.reanalysed, c->ring.q_pos, c->ring.q_game, c->ring.prefix, c->ring.upd, c->ring.counters, c->d_stats, c->d_lossout, c->batch.index, c->batch.obs,
+                    c->slots.h_cv, c->slots.h_rv, c->d_stats, c->d_lossout, c->batch.index, c->batch.obs,
                     c->batch.actions, c->batch.values, c->batch.rewards, c->batch.policies, c->batch.gscale, c->batch.weights, c->d_pv, c->d_pr, c->d_pp,
                     c->d_rowv, c->d_rowp, c->d_rowinvg, c->d_rowr};
     for (void *p : ptrs) if (p) cudaFree(p);
     for (auto &b : c->scratch) b.release();
+    for (auto &b : c->rn_buf) b.release();
+    for (dev_buf *b : {&c->bptt_act, &c->bptt_gpart, &c->lr_xsave, &c->lr_dzsave, &c->lr_gpart}) b->release();
+    free_ring(c->ring);
     free_ring(c->play_ring);
     if (c->h_lat_stage) cudaFreeHost(c->h_lat_stage);
     if (c->d_lat_stage) cudaFree(c->d_lat_stage);
@@ -1530,20 +1506,10 @@ int mz_learn_gradients_w(mz_ctx *c, int grad_mode, int B, const float *obs_batch
     MZ_TRY(upload_batch(c, B, obs_batch, action_batch, value_batch, reward_batch, policy_batch, gscale));
     if (weight_batch) MZ_CUDA(c, cudaMemcpyAsync(c->batch.weights, weight_batch, (size_t)B * 4, cudaMemcpyHostToDevice, c->stream));
     MZ_TRY(launch_learn_forward(c, B, grad_mode));
-    if (c->cfg.net_type == MZ_NET_RESNET) {   // parameters, and therefore the gradient, are in blob order already
-        const int np = c->M.P.n_params;
-        { launch_scope ls(c, 4); mz_k_grad_l2_masked<<<(np + 255) / 256, 256, 0, c->stream>>>(np, c->d_rn_theta, c->d_rn_mask, c->d_rn_grad); }
-        MZ_CUDA(c, cudaMemcpyAsync(grad, c->d_rn_grad, (size_t)np * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
-        return finish_losses(c, B, losses);
-    }
-    const int n = c->M.P.total_floats;
-    if (grad_mode == MZ_GRAD_REFERENCE_L2) { launch_scope ls(c, 4); if (c->d_fc_mask) mz_k_grad_l2_masked<<<(n + 255) / 256, 256, 0, c->stream>>>(n, c->d_w, c->d_fc_mask, grad_out(c)); else mz_k_grad_l2<<<(n + 255) / 256, 256, 0, c->stream>>>(n, c->d_w, grad_out(c)); }
-    std::vector<float> dev((size_t)n), src((size_t)c->M.P.n_params);
-    MZ_CUDA(c, cudaMemcpyAsync(dev.data(), grad_out(c), dev.size() * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
-    MZ_TRY(finish_losses(c, B, losses));
-    mzh::unpack_weights(c->M.P, dev.data(), src.data());
-    memcpy(grad, src.data(), src.size() * sizeof(float));
-    return MZ_OK;
+    const int n = c->store_floats;
+    if (grad_mode == MZ_GRAD_REFERENCE_L2) { launch_scope ls(c, 4); mz_k_l2_grad<<<(n + 255) / 256, 256, 0, c->stream>>>(n, c->d_w, c->d_mask, grad_out(c)); }
+    MZ_TRY(store_to_host(c, grad_out(c), grad));
+    return finish_losses(c, B, losses);
 }
 int mz_learn_step(mz_ctx *c, int64_t t, int grad_mode, float *losses) {
     MZ_CHECK_CTX(c);
@@ -1577,53 +1543,24 @@ int mz_learn_steps(mz_ctx *c, int64_t t0, int n, int grad_mode, float *losses) {
 int mz_get_optimizer_state(mz_ctx *c, float *m, float *v, int64_t n, int64_t *steps_done) {
     MZ_CHECK_CTX(c);
     if (!m || !v || !steps_done || n != c->M.P.n_params) return fail(c, MZ_E_ARG, "bad arguments (need %d floats per moment)", c->M.P.n_params);
-    if (c->cfg.net_type == MZ_NET_RESNET) {   // the ResNet learner keeps its state in blob order
-        MZ_CUDA(c, cudaMemcpyAsync(m, c->d_rn_m, (size_t)n * 4, cudaMemcpyDeviceToHost, c->stream)); MZ_CUDA(c, cudaMemcpyAsync(v, c->d_rn_v, (size_t)n * 4, cudaMemcpyDeviceToHost, c->stream));
-        MZ_CUDA(c, cudaStreamSynchronize(c->stream));
-        *steps_done = c->adam_t > 0 ? c->adam_t - 1 : 0;
-        return MZ_OK;
-    }
-    std::vector<float> dev((size_t)c->M.P.total_floats);
-    for (int which = 0; which < 2; which++) {
-        MZ_CUDA(c, cudaMemcpyAsync(dev.data(), which ? c->d_v : c->d_m, dev.size() * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
-        MZ_CUDA(c, cudaStreamSynchronize(c->stream));
-        mzh::unpack_weights(c->M.P, dev.data(), which ? v : m);
-    }
-    *steps_done = c->adam_t > 0 ? c->adam_t - 1 : 0;
+    MZ_TRY(store_to_host(c, c->d_m, m));
+    MZ_TRY(store_to_host(c, c->d_v, v));
+    *steps_done = c->adam_t - 1;
     return MZ_OK;
 }
 int mz_set_optimizer_state(mz_ctx *c, const float *m, const float *v, int64_t n, int64_t steps_done) {
     MZ_CHECK_CTX(c);
     if (!m || !v || steps_done < 0 || n != c->M.P.n_params) return fail(c, MZ_E_ARG, "bad arguments (need %d floats per moment)", c->M.P.n_params);
-    if (c->cfg.net_type == MZ_NET_RESNET) {
-        MZ_CUDA(c, cudaMemcpyAsync(c->d_rn_m, m, (size_t)n * 4, cudaMemcpyHostToDevice, c->stream)); MZ_CUDA(c, cudaMemcpyAsync(c->d_rn_v, v, (size_t)n * 4, cudaMemcpyHostToDevice, c->stream));
-        MZ_CUDA(c, cudaStreamSynchronize(c->stream));
-        c->adam_t = steps_done + 1; c->bp1 = 0.9; c->bp2 = 0.999;
-        for (int64_t i = 0; i < steps_done; i++) { c->bp1 *= 0.9; c->bp2 *= 0.999; }
-        if (steps_done == 0) c->adam_t = 0;
-        return MZ_OK;
-    }
-    std::vector<float> dev((size_t)c->M.P.total_floats);
-    for (int which = 0; which < 2; which++) {
-        mzh::pack_weights(c->M.P, which ? v : m, dev.data());
-        MZ_CUDA(c, cudaMemcpyAsync(which ? c->d_v : c->d_m, dev.data(), dev.size() * sizeof(float), cudaMemcpyHostToDevice, c->stream));
-        MZ_CUDA(c, cudaStreamSynchronize(c->stream));
-    }
-    c->adam_t = steps_done + 1; c->bp1 = 0.9; c->bp2 = 0.999;           // beta^t by repeated product, as the running state builds it
-    for (int64_t i = 0; i < steps_done; i++) { c->bp1 *= 0.9; c->bp2 *= 0.999; }
-    if (steps_done == 0) c->adam_t = 0;
+    MZ_TRY(store_from_host(c, c->d_m, m));
+    MZ_TRY(store_from_host(c, c->d_v, v));
+    adam_seek(c, steps_done);
     return MZ_OK;
 }
 int mz_optimizer_reset(mz_ctx *c) {
     MZ_CHECK_CTX(c);
-    if (c->cfg.net_type == MZ_NET_RESNET) {
-        MZ_CUDA(c, cudaMemsetAsync(c->d_rn_m, 0, (size_t)c->M.P.n_params * 4, c->stream)); MZ_CUDA(c, cudaMemsetAsync(c->d_rn_v, 0, (size_t)c->M.P.n_params * 4, c->stream));
-        c->adam_t = 0; c->bp1 = 0.9; c->bp2 = 0.999;
-        return MZ_OK;
-    }
-    MZ_CUDA(c, cudaMemsetAsync(c->d_m, 0, (size_t)c->M.P.total_floats * 4, c->stream));
-    MZ_CUDA(c, cudaMemsetAsync(c->d_v, 0, (size_t)c->M.P.total_floats * 4, c->stream));
-    c->adam_t = 0; c->bp1 = 0.9; c->bp2 = 0.999;
+    MZ_CUDA(c, cudaMemsetAsync(c->d_m, 0, (size_t)c->store_floats * 4, c->stream));
+    MZ_CUDA(c, cudaMemsetAsync(c->d_v, 0, (size_t)c->store_floats * 4, c->stream));
+    adam_seek(c, 0);
     return MZ_OK;
 }
 
@@ -1714,15 +1651,7 @@ int mz_comm_destroy(mz_ctx *c) {
     c->rank = 0; c->nranks = 1;
     return MZ_OK;
 }
-// which kernels a learner step of `grad_mode` runs on in this context: 0 = fp32 SIMT (mz_k_learn_forward / mz_k_learn_bptt), 1 = the unroll forward
-// on the tensor cores (mz_k_learn_forward_sp), 2 = forward and backward on the tensor cores (mz_k_learn_bptt_tc + mz_k_learn_dw), 3 = ResNet: unroll
-// through the bf16 inference kernel (mz_k_rn_forward), -1 = not available (ResNet with MZ_GRAD_BPTT)
-int mz_learner_path(mz_ctx *c, int grad_mode) {
-    if (c && c->cfg.net_type == MZ_NET_RESNET) return grad_mode == MZ_GRAD_REFERENCE_L2 ? 3 : -1;
-    if (!c || c->cfg.net_type != MZ_NET_FEEDFORWARD || c->cfg.nn_mode != MZ_NN_SPLIT_MMA) return 0;
-    if (grad_mode == MZ_GRAD_BPTT) return (c->lrp.ok && !getenv("MUZERO_B200_BPTT_SIMT")) ? 2 : 0;
-    return 1;
-}
+int mz_learner_path(mz_ctx *c, int grad_mode) { return c ? learner_path(c, grad_mode) : 0; }
 // 0 = no communicator, 1 = ncclAllReduce + mz_k_adam, 2 = mz_k_dp_adam over peer memory (NVLink loads, fused with the update)
 int mz_comm_mode(mz_ctx *c) { if (!c) return 0; return c->p2p ? 2 : c->comm ? 1 : 0; }
 

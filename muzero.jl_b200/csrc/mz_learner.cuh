@@ -183,7 +183,7 @@ __global__ void __launch_bounds__(1024) mz_k_loss_reduce(const __grid_constant__
     __shared__ double red[1024];
     const int tid = threadIdx.x;
     // one CTA per quantity (grid = 7): the seven reductions are independent; each keeps its own fixed summation tree
-    for (int what = blockIdx.x; what < nwhat; what += gridDim.x) {   // nwhat = 4: the data terms only (ResNet: mz_k_rn_sqnorm adds the rest)
+    for (int what = blockIdx.x; what < nwhat; what += gridDim.x) {   // nwhat = 4: the data terms only (mz_k_sqnorm_masked adds the rest)
         double acc = 0.0;
         if (what < 4) {
             for (int i = tid; i < B; i += 1024) acc += what == 0 ? (double)row_v[i] : what == 1 ? (double)row_p[i] : what == 2 ? (double)row_invg[i] : row_r[i];
@@ -201,10 +201,21 @@ __global__ void __launch_bounds__(1024) mz_k_loss_reduce(const __grid_constant__
 }
 
 // Gradients.  MZ_GRAD_REFERENCE_L2: the reference computes its predictions outside Zygote.pullback
-// (Learning.jl:347-374 vs 385-393), so the gradient of every parameter array is that of sum(abs2, theta): 2*theta (Q20).
-__global__ void mz_k_grad_l2(int n, const float *theta, float *grad) {
-    int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < n) grad[i] = theta[i] + theta[i];
+// (Learning.jl:347-374 vs 385-393), so the gradient of every parameter array is that of sum(abs2, theta): 2*theta (Q20) over Flux.params
+// (dense / conv weights and biases, BatchNorm beta / gamma), 0 for the BatchNorm running statistics.  mask: 1 = Flux parameter (NULL = all).
+__global__ void mz_k_l2_grad(int n, const float *theta, const unsigned char *mask, float *grad) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n) grad[i] = (!mask || mask[i]) ? theta[i] + theta[i] : 0.0f;
+}
+// out[4 + net] = sum of theta^2 over the Flux parameters of each network, net = [b_net, b_net+1) (one CTA per network, double accumulation)
+__global__ void __launch_bounds__(1024) mz_k_sqnorm_masked(int b0, int b1, int b2, int b3, const float *theta, const unsigned char *mask, double *out) {
+    __shared__ double red[1024];
+    const int tid = threadIdx.x, lo = blockIdx.x == 0 ? b0 : blockIdx.x == 1 ? b1 : b2, hi = blockIdx.x == 0 ? b1 : blockIdx.x == 1 ? b2 : b3;
+    double acc = 0.0;
+    for (int i = lo + tid; i < hi; i += 1024) if (mask[i]) { const double t = (double)theta[i]; acc += t * t; }
+    red[tid] = acc; __syncthreads();
+    for (int s = 512; s > 0; s >>= 1) { if (tid < s) red[tid] += red[tid + s]; __syncthreads(); }
+    if (tid == 0) out[4 + blockIdx.x] = red[0];
 }
 // Flux.ADAM apply! + update! (Q22): Float32 state, Float64 arithmetic inside the broadcast, beta powers beta^t.
 __global__ void mz_k_adam(int n, float *theta, float *m, float *v, const float *grad, double eta, double bp1, double bp2, float grad_scale) {
@@ -219,8 +230,8 @@ __global__ void mz_k_adam(int n, float *theta, float *m, float *v, const float *
     theta[i] = theta[i] - delta;
 }
 
-// MZ_GRAD_REFERENCE_L2 on one GPU: the gradient is 2 * theta over Flux.params (Q20), so mz_k_grad_l2 + mz_k_adam are one kernel (a B = 32 step is
-// bound by its launches).  Same arithmetic, same bits; the gradient is still written out.  mask: use_batch_norm (NULL = all ones).
+// MZ_GRAD_REFERENCE_L2 on one GPU: the gradient is 2 * theta over Flux.params (Q20), so mz_k_l2_grad + mz_k_adam are one kernel (a B = 32 step is
+// bound by its launches).  Same arithmetic, same bits; the gradient is still written out.  mask: as in mz_k_l2_grad.
 __global__ void mz_k_adam_l2(int n, float *theta, float *m, float *v, float *grad, const unsigned char *mask, double eta, double bp1, double bp2) {
     int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
@@ -295,19 +306,4 @@ __global__ void mz_k_rn_scatter(int B, int A, int K1, int row, int row2, const f
     }
     if (r) pr[(size_t)b * K1 + row] = r[b];
     if (rzero) pr[(size_t)b * K1] = 0.0f;
-}
-// gradient of sum(abs2, theta) over Flux.params: 2 * theta for conv / dense weights and biases and BatchNorm beta / gamma, 0 for the running statistics
-__global__ void mz_k_grad_l2_masked(int n, const float *theta, const unsigned char *mask, float *grad) {
-    const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < n) grad[i] = mask[i] ? theta[i] + theta[i] : 0.0f;
-}
-// out[4 + net] = sum of theta^2 over the trainable entries of each network (one CTA per network, double accumulation)
-__global__ void __launch_bounds__(1024) mz_k_rn_sqnorm(int b0, int b1, int b2, int b3, const float *theta, const unsigned char *mask, double *out) {
-    __shared__ double red[1024];
-    const int tid = threadIdx.x, lo = blockIdx.x == 0 ? b0 : blockIdx.x == 1 ? b1 : b2, hi = blockIdx.x == 0 ? b1 : blockIdx.x == 1 ? b2 : b3;
-    double acc = 0.0;
-    for (int i = lo + tid; i < hi; i += 1024) if (mask[i]) { const double t = (double)theta[i]; acc += t * t; }
-    red[tid] = acc; __syncthreads();
-    for (int s = 512; s > 0; s >>= 1) { if (tid < s) red[tid] += red[tid + s]; __syncthreads(); }
-    if (tid == 0) out[4 + blockIdx.x] = red[0];
 }
