@@ -32,8 +32,10 @@ enum { MZ_OK = 0, MZ_E_ARG = -1, MZ_E_CUDA = -2, MZ_E_STATE = -3, MZ_E_NCCL = -4
 enum { MZ_GAME_TICTACTOE = 0, MZ_GAME_CONNECT = 1 };
 enum { MZ_TIE_PHILOX = 0, MZ_TIE_FIRST = 1 };
 enum { MZ_GRAD_REFERENCE_L2 = 0, MZ_GRAD_BPTT = 1 };
-/* conf.opponent (src/Constructors.jl:27; select_opponent_action, src/SelfPlay.jl:311-325) */
-enum { MZ_OPP_SELF = 0, MZ_OPP_RANDOM = 1, MZ_OPP_EXPERT = 2 };
+/* conf.opponent (src/Constructors.jl:27; select_opponent_action, src/SelfPlay.jl:311-325).  MZ_OPP_NETWORK (mz_arena, mz_play_games):
+ * the other side is a second MuZero that searches its plies with the context's opponent networks (mz_set_opponent_weights,
+ * mz_snapshot_opponent) */
+enum { MZ_OPP_SELF = 0, MZ_OPP_RANDOM = 1, MZ_OPP_EXPERT = 2, MZ_OPP_NETWORK = 3 };
 /* network arithmetic of self-play / run_mcts / the network callables:
  *   MZ_NN_FP32_EXACT  fp32 SIMT, sequential-k fmaf: bit-identical to the oracle's arithmetic contract
  *   MZ_NN_BF16_TC     bf16 operands on tcgen05.mma, fp32 accumulation in TMEM
@@ -117,6 +119,13 @@ int     mz_num_params(const mz_config *cfg, int net);
 int     mz_init_weights(mz_ctx *ctx, uint64_t seed);         /* Flux.glorot_uniform, Philox-keyed */
 int     mz_set_weights(mz_ctx *ctx, int net, const float *blob, int64_t n);
 int     mz_get_weights(mz_ctx *ctx, int net, float *blob, int64_t n);
+/* the opponent networks of MZ_OPP_NETWORK: a second weight store, allocated by the first of these calls (a context that never calls them
+ * allocates nothing for it).  mz_set_opponent_weights takes the blob, net ids and lengths of mz_set_weights; net < MZ_NET_ALL replaces one
+ * network and needs a full opponent set first (MZ_E_STATE otherwise).  mz_snapshot_opponent makes the opponent a copy of the context's
+ * current weights, one device-to-device copy in stream order: snapshot, train, then mz_arena(MZ_OPP_NETWORK) measures what training
+ * changed.  Neither the learner nor mz_set_weights touches the opponent networks. */
+int     mz_set_opponent_weights(mz_ctx *ctx, int net, const float *blob, int64_t n);
+int     mz_snapshot_opponent(mz_ctx *ctx);
 /* batched callables, host buffers: repr(x (W,H,planes,B)) -> (hidden,B); pred(h) -> (value(1,B), policy(A,B));
  * dyn(sa (W,H,C+1,B)) -> (state(hidden,B), reward(1,B)) */
 int mz_representation(mz_ctx *ctx, int B, const float *stacked_obs, float *hidden);
@@ -153,7 +162,7 @@ int mz_self_play(mz_ctx *ctx, uint64_t first_game, int64_t n_games, float temper
 /* play_game(env, temperature, render, opponent, muzero_player, NNs)::GameHistory (src/SelfPlay.jl:330-382) for n_games games at once:
  * the histories come back to the caller (layout of mz_history_export; order = the order the games finished, game_id[] names them) and are
  * NOT saved -- the reference's self_play! passes them to save_game itself (:414), here mz_history_import.  opponent MZ_OPP_SELF: every
- * ply is searched; otherwise `opponent` moves for the side that is not muzero_player. */
+ * ply is searched; otherwise `opponent` moves for the side that is not muzero_player (MZ_OPP_NETWORK: as in mz_arena). */
 int mz_play_games(mz_ctx *ctx, uint64_t first_game, int n_games, float temperature, int opponent, int muzero_player, int64_t *game_id,
                   int32_t *T, float *obs, int32_t *actions, float *rewards, int32_t *to_play, float *child_visits, float *root_values,
                   int64_t *simulations /* may be NULL */);
@@ -162,7 +171,11 @@ int mz_play_games(mz_ctx *ctx, uint64_t first_game, int n_games, float temperatu
  * moving for the side that is not muzero_player (1 or 2).  The reference passes temperature 0 and, through play_game, still searches
  * with exploration noise (:359).  Finished games go to the replay ring like self-play games (opponent plies repeat the statistics of
  * the previous search, :374; zeros before the first one), so use a context of its own for evaluation.  wins / draws / losses count
- * games for MuZero: the side that completes a line first wins (TicTacToe runs one ply past a win, SURVEY Q14). */
+ * games for MuZero: the side that completes a line first wins (TicTacToe runs one ply past a win, SURVEY Q14).
+ * MZ_OPP_NETWORK: the other side's plies are searched exactly like MuZero's (run_mcts with exploration noise, Philox keys (game id, move
+ * index), select_action at `temperature`, that ply's own statistics stored) but with the opponent networks; *simulations counts both
+ * sides.  With opponent networks equal to the context's, the games are those of MZ_OPP_SELF bit for bit.  MZ_E_STATE before any opponent
+ * weights are set. */
 int mz_arena(mz_ctx *ctx, uint64_t first_game, int64_t n_games, int opponent, int muzero_player, float temperature,
              int64_t *wins, int64_t *draws, int64_t *losses, int64_t *simulations);
 /* select_opponent_action for n boards (bit masks as in mz_env_step); action[n] 1-based */

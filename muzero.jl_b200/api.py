@@ -177,6 +177,14 @@ class Engine:
     def close(self):
         self.ctx.close()
 
+    def set_opponent_networks(self, blob, net=capi.NET_ALL):
+        """The networks competitive_play(..., opponent="network") plays against (blob layout of init_networks / set_weights)."""
+        self.ctx.set_opponent_weights(blob, net)
+
+    def snapshot_opponent(self):
+        """The opponent networks become a copy of the current networks: snapshot, train, then competitive_play(opponent="network")."""
+        self.ctx.snapshot_opponent()
+
 
 class TicTacToe:
     """games/tictactoe/game.jl: the RLBase verbs the hot path calls (SelfPlay.jl:349,351,359,366-368), one board,
@@ -326,20 +334,22 @@ def play_game(engine: Engine, temperature, render=False, opponent="self", muzero
     return ReplayBuffer(engine)[info["first_key"] + info["n_games"] - 1]
 
 
-_OPPONENTS = {"self": capi.OPP_SELF, "random": capi.OPP_RANDOM, "expert": capi.OPP_EXPERT}
+_OPPONENTS = {"self": capi.OPP_SELF, "random": capi.OPP_RANDOM, "expert": capi.OPP_EXPERT, "network": capi.OPP_NETWORK}
 
 
 def competitive_play(engine: Engine, n_games: int = 1, opponent: Optional[str] = None, muzero_player: Optional[int] = None, temperature=0.0):
     """competitive_play!(; NNs) (SelfPlay.jl:421-435), batched: n_games games of play_game(env, 0.0, ..., conf.opponent, conf.muzero_player, NNs).
     The reference renders the game and returns nothing; this returns dict(wins, draws, losses, simulations) for MuZero.  The games are
-    saved to the engine's replay buffer like self-play games: evaluate on an Engine of its own (`Engine(conf, hyper)` + `set_weights`)."""
+    saved to the engine's replay buffer like self-play games: evaluate on an Engine of its own (`Engine(conf, hyper)` + `set_weights`).
+    opponent="network": the other side is a second MuZero searching with the engine's opponent networks (Engine.set_opponent_networks,
+    Engine.snapshot_opponent)."""
     conf = engine.conf
     opponent = (conf.opponent if len(conf.players) > 1 else "self") if opponent is None else opponent     # :428
     muzero_player = conf.muzero_player if muzero_player is None else muzero_player
     if opponent == "human":
         raise NotImplementedError("a human opponent has no batched meaning; use the reference's own loop (SelfPlay.jl:312-316)")
     if opponent not in _OPPONENTS:
-        raise ValueError("Wrong argument: opponent argument should be self, human, expert or random")     # :323
+        raise ValueError("Wrong argument: opponent argument should be self, human, expert, random or network")     # :323
     r = engine.ctx.arena(engine.next_game, n_games, _OPPONENTS[opponent], muzero_player, temperature)
     engine.next_game += n_games
     return r

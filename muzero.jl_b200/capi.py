@@ -18,7 +18,7 @@ GAME_TICTACTOE, GAME_CONNECT = 0, 1
 TIE_PHILOX, TIE_FIRST = 0, 1
 GRAD_REFERENCE_L2, GRAD_BPTT = 0, 1
 NET_FEEDFORWARD, NET_RESNET = 0, 1
-OPP_SELF, OPP_RANDOM, OPP_EXPERT = 0, 1, 2
+OPP_SELF, OPP_RANDOM, OPP_EXPERT, OPP_NETWORK = 0, 1, 2, 3
 NN_FP32_EXACT, NN_BF16_TC, NN_SPLIT_MMA = 0, 1, 2
 NET_REPRESENTATION, NET_PREDICTION, NET_DYNAMICS, NET_ALL = 0, 1, 2, 3
 KERNEL_FAMILIES = ("selfplay_move", "save_refill", "replay_gather", "learn_forward_loss", "adam", "nn_batch", "env")
@@ -90,6 +90,8 @@ def lib():
         "mz_init_weights": ([ctx, C.c_uint64], C.c_int),
         "mz_set_weights": ([ctx, C.c_int, f32p, C.c_int64], C.c_int),
         "mz_get_weights": ([ctx, C.c_int, f32p, C.c_int64], C.c_int),
+        "mz_set_opponent_weights": ([ctx, C.c_int, f32p, C.c_int64], C.c_int),
+        "mz_snapshot_opponent": ([ctx], C.c_int),
         "mz_representation": ([ctx, C.c_int, f32p, f32p], C.c_int),
         "mz_prediction": ([ctx, C.c_int, f32p, f32p, f32p], C.c_int),
         "mz_dynamics": ([ctx, C.c_int, f32p, f32p, f32p], C.c_int),
@@ -252,6 +254,15 @@ class Context:
         blob = np.zeros(self.num_params(net), np.float32)
         self._ck(self.L.mz_get_weights(self._h, net, _p(blob, C.c_float), blob.size))
         return blob
+
+    def set_opponent_weights(self, blob, net=NET_ALL):
+        """The opponent networks of OPP_NETWORK (same blob layout as set_weights; one network needs a full set first)."""
+        blob = _f32(blob)
+        self._ck(self.L.mz_set_opponent_weights(self._h, net, _p(blob, C.c_float), blob.size))
+
+    def snapshot_opponent(self):
+        """The opponent networks become a copy of the current weights (on the device, in stream order)."""
+        self._ck(self.L.mz_snapshot_opponent(self._h))
 
     # ---- networks ----
     def representation(self, stacked):

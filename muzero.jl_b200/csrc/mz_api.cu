@@ -63,6 +63,18 @@ struct nccl_api {
 
 extern "C" { static void p2p_teardown(mz_ctx *c); }
 
+// One set of network weights (store_floats floats in the parameter store's layout) and the images the search kernels read, each rebuilt
+// from w before its next use when version has moved past the image's (ensure_images, ensure_lat_image).  mz_ctx::own holds the context's
+// networks; mz_ctx::opp the opponent networks of MZ_OPP_NETWORK, allocated on the first mz_set_opponent_weights / mz_snapshot_opponent with
+// the images of the context's path only.
+struct mz_wstore {
+    float *w = nullptr; uint64_t version = 1, img_version = 0, lat_version = 0;
+    unsigned char *tc = nullptr; float *tc_bias = nullptr;   // MZ_NN_BF16_TC: bf16 image and bias
+    unsigned char *sp = nullptr; float *sp_bias = nullptr;   // MZ_NN_SPLIT_MMA: bf16 hi + lo image and bias
+    float *lat = nullptr;                                    // mz_k_search_lat: fp32, rows = outputs
+    unsigned char *rn = nullptr;                             // ResNet: bf16 image, BatchNorm folded
+};
+
 struct mz_ctx {
     mz_config cfg; mzh::model M; int device = 0;
     cudaStream_t stream = nullptr; bool own_stream = false;
@@ -72,9 +84,11 @@ struct mz_ctx {
     // the learner's parameter store: fp32 parameters, ADAM moments and gradient, store_floats each; packed: in the padded device layout of the
     // FeedForwardHP kernels (mzh::pack_weights), else (ResNet) in blob order.  d_mask (use_batch_norm, ResNet): 1 = Flux parameter, 0 = BatchNorm
     // running statistic; net_bounds: where each network starts in the store, and its end
-    float *d_w = nullptr, *d_m = nullptr, *d_v = nullptr, *d_grad = nullptr; int store_floats = 0; bool packed = true;
+    mz_wstore own;   // the context's networks: own.w is the store's parameter array
+    mz_wstore opp; bool opp_full = false;   // MZ_OPP_NETWORK's opponent networks (opp.w == NULL until first set); opp_full: a whole set is loaded
+    float *d_m = nullptr, *d_v = nullptr, *d_grad = nullptr; int store_floats = 0; bool packed = true;
     unsigned char *d_mask = nullptr; int net_bounds[4] = {0, 0, 0, 0};
-    unsigned char *d_w_tc = nullptr; float *d_bias_tc = nullptr; size_t smem_bytes_tc = 0;   // tensor-core weight image
+    size_t smem_bytes_tc = 0;   // tensor-core path (image: own.tc)
     // data-parallel learner over peer memory (mz_k_dp_adam): gradient exchange buffers (double-buffered) and arrival flags of every rank
     float *d_xgrad = nullptr; uint32_t *d_xflags = nullptr; float *peer_grad[MZ_DP_MAX_RANKS] = {}; uint32_t *peer_flags[MZ_DP_MAX_RANKS] = {};
     bool p2p = false; uint32_t dp_step = 0;
@@ -84,14 +98,13 @@ struct mz_ctx {
     // MZ_GRAD_BPTT on the tensor cores (mz_learner_tc.cuh): backward rounds
     mz_lr_plan lrp{}; mz_lr_bround *d_brounds = nullptr; size_t smem_bytes_lr = 0;
     // mz_k_search_lat (one tree per 2-CTA cluster, networks and tree resident in shared memory): calls with at most lat_max_roots roots
-    float *d_w_lat = nullptr; uint64_t lat_version = 0; int lat_image_floats = 0;
+    int lat_image_floats = 0;
     unsigned char *h_lat_stage = nullptr, *d_lat_stage = nullptr; size_t lat_stage_cap = 0;   // one pinned / device block for all inputs and outputs of a small run_mcts call
     bool lat_ok = false; int lat_w_floats = 0, lat_pbc_smem = 0, lat_max_roots = 0, lat_max_slots = 0; size_t smem_bytes_lat = 0;
     bool persist_ok = true;     // MUZERO_B200_PERSIST=0: one search launch per move also for single-wave self-play on the split-precision path
     bool slots_dirty = false;   // a wave is in progress or ended with an error: the slots are reset before the next one
     int refill_wave_sync = 1;   // 1: mz_k_save_refill starts new games only when every slot is free (default; MUZERO_B200_REFILL=immediate refills at once)
-    uint64_t w_version = 1, img_version = 0;   // device weights vs the tensor-core or ResNet image built from them (ensure_images)
-    mz_sp_plan spp{}; mz_sp_args spa{}; unsigned char *d_w_sp = nullptr; float *d_bias_sp = nullptr; mz_sp_round *d_rounds_sp = nullptr; size_t smem_bytes_sp = 0;   // split-precision tensor-core path
+    mz_sp_plan spp{}; mz_sp_args spa{}; mz_sp_round *d_rounds_sp = nullptr; size_t smem_bytes_sp = 0;   // split-precision tensor-core path
     double *d_pbc0 = nullptr, *d_sqrtN = nullptr;
     void *d_trees = nullptr;
     mz_slots slots{}; mz_ring ring{};
@@ -106,7 +119,7 @@ struct mz_ctx {
     int64_t adam_t = 1; double bp1 = 0.9, bp2 = 0.999;   // Flux.ADAM: the next update's step number and beta powers (adam_seek)
     ncclComm_t comm = nullptr; int rank = 0, nranks = 1;
     // net_type = MZ_NET_RESNET
-    mzh::rn_model rn; unsigned char *d_rn_image = nullptr; mz_rn_step *d_rn_steps = nullptr; size_t smem_bytes_rn = 0;
+    mzh::rn_model rn; mz_rn_step *d_rn_steps = nullptr; size_t smem_bytes_rn = 0;
     // grad_mode = MZ_GRAD_BPTT
     mzh::bptt_program bptt; mz_bstage *d_bstages[2] = {nullptr, nullptr}; size_t smem_bytes_bptt = 0;
     float *d_w_fold = nullptr;   // use_batch_norm + MZ_GRAD_BPTT: the weights with every BatchNorm folded into its Dense layer
@@ -214,13 +227,13 @@ int store_from_host(mz_ctx *c, float *d, const float *blob) {
     return MZ_OK;
 }
 int upload_weights(mz_ctx *c, const std::vector<float> &src) {
-    const int r = store_from_host(c, c->d_w, src.data());
-    c->w_version++;                                      // the images are rebuilt before their next use (ensure_images)
+    const int r = store_from_host(c, c->own.w, src.data());
+    c->own.version++;                                      // the images are rebuilt before their next use (ensure_images)
     return r;
 }
 int download_weights(mz_ctx *c, std::vector<float> &src) {
     src.resize((size_t)c->M.P.n_params);
-    return store_to_host(c, c->d_w, src.data());
+    return store_to_host(c, c->own.w, src.data());
 }
 
 int read_counters(mz_ctx *c) {
@@ -285,47 +298,48 @@ float *grad_out(mz_ctx *c) { return c->p2p ? c->d_xgrad + (size_t)((c->dp_step +
 
 // ResNet: fetch the parameters, fold BatchNorm and pack the bf16 B-operand images on the host (rn_pack, one block per program step), upload
 // the image.  (A device-side packer would save the round trip; the ResNet learner is a functional path, not a tuned one.)
-int rn_sync_image(mz_ctx *c) {
+int rn_sync_image(mz_ctx *c, mz_wstore &s) {
     std::unique_ptr<float[]> blob(new float[(size_t)c->store_floats]);   // not zero-filled: the copy overwrites all of it
-    MZ_TRY(store_to_host(c, c->d_w, blob.get()));
+    MZ_TRY(store_to_host(c, s.w, blob.get()));
     std::vector<unsigned char> image;
     mzh::rn_pack(c->rn, blob.get(), image);
-    MZ_CUDA(c, cudaMemcpyAsync(c->d_rn_image, image.data(), (size_t)c->rn.image_bytes, cudaMemcpyHostToDevice, c->stream));
+    MZ_CUDA(c, cudaMemcpyAsync(s.rn, image.data(), (size_t)c->rn.image_bytes, cudaMemcpyHostToDevice, c->stream));
     MZ_CUDA(c, cudaStreamSynchronize(c->stream));
-    c->img_version = c->w_version;
+    s.img_version = s.version;
     return MZ_OK;
 }
 
-// The tensor-core and ResNet paths read bf16 images of the weights; whenever d_w has changed (set_weights, an ADAM step) the image of the
-// context's networks is rebuilt before the next kernel that reads it (FeedForwardHP: on the device).
-int ensure_images(mz_ctx *c) {
-    if (c->img_version == c->w_version) return MZ_OK;
-    if (c->cfg.net_type == MZ_NET_RESNET) return rn_sync_image(c);
+// The tensor-core and ResNet paths read bf16 images of the weights; whenever a store's weights have changed (set_weights, an ADAM step,
+// mz_set_opponent_weights, mz_snapshot_opponent) its image is rebuilt before the next kernel that reads it (FeedForwardHP: on the device).
+int ensure_images(mz_ctx *c, mz_wstore &s) {
+    if (s.img_version == s.version) return MZ_OK;
+    if (c->cfg.net_type == MZ_NET_RESNET) return rn_sync_image(c, s);
     const mz_params &P = c->M.P;
-    mz_pack_args a{}; a.w = c->d_w;
-    if (c->cfg.nn_mode == MZ_NN_SPLIT_MMA && c->d_w_sp) {
-        a.mode = 2; a.image = c->d_w_sp; a.bias = c->d_bias_sp;
+    mz_pack_args a{}; a.w = s.w;
+    if (c->cfg.nn_mode == MZ_NN_SPLIT_MMA && s.sp) {
+        a.mode = 2; a.image = s.sp; a.bias = s.sp_bias;
         for (int i = 0; i < P.n_layers; i++) { a.off[i] = c->spp.w_off[i]; a.bytes[i] = c->spp.w_bytes[i]; a.bias_off[i] = i * 64; }
-    } else if (c->cfg.nn_mode == MZ_NN_BF16_TC && c->d_w_tc) {
-        a.mode = 1; a.image = c->d_w_tc; a.bias = c->d_bias_tc;
+    } else if (c->cfg.nn_mode == MZ_NN_BF16_TC && s.tc) {
+        a.mode = 1; a.image = s.tc; a.bias = s.tc_bias;
         for (int i = 0; i < P.n_layers; i++) { a.off[i] = P.tc_a_off[i]; a.bytes[i] = 0; a.bias_off[i] = P.tc_bias_off[i]; }
-    } else { c->img_version = c->w_version; return MZ_OK; }
+    } else { s.img_version = s.version; return MZ_OK; }
     { launch_scope ls(c, 5); mz_k_pack_images<<<dim3((unsigned)P.n_layers, 4), 256, 0, c->stream>>>(P, a); }
     MZ_CUDA(c, cudaGetLastError());
-    c->img_version = c->w_version;
+    s.img_version = s.version;
     return MZ_OK;
 }
+int ensure_images(mz_ctx *c) { return ensure_images(c, c->own); }
 
-// the weight image of mz_k_search_lat (rows = outputs), rebuilt from the device weights when they have changed since it was last used
-int ensure_lat_image(mz_ctx *c) {
-    if (c->lat_version == c->w_version) return MZ_OK;
+// the weight image of mz_k_search_lat (rows = outputs), rebuilt from the store's weights when they have changed since it was last used
+int ensure_lat_image(mz_ctx *c, mz_wstore &s) {
+    if (s.lat_version == s.version) return MZ_OK;
     const mz_params &P = c->M.P;
-    mz_pack_lat_args a{}; a.w = c->d_w; a.image = c->d_w_lat;
+    mz_pack_lat_args a{}; a.w = s.w; a.image = s.lat;
     int off = 0;
     for (int n = 0; n < 3; n++) for (int l = P.nets[n].first; l < P.nets[n].first + P.nets[n].n_trunk + P.nets[n].n_h1 + P.nets[n].n_h2; l++) { a.off[l] = off; off += mz_lat_layer_floats(P.layers[l].in, P.layers[l].out); }
     { launch_scope ls(c, 5); mz_k_pack_lat<<<dim3((unsigned)P.n_layers, 4), 256, 0, c->stream>>>(P, a); }
     MZ_CUDA(c, cudaGetLastError());
-    c->lat_version = c->w_version;
+    s.lat_version = s.version;
     return MZ_OK;
 }
 
@@ -334,7 +348,7 @@ int ensure_lat_image(mz_ctx *c) {
 // arithmetic, BatchNorm with its stored statistics: the reference computes the predictions outside the pullback, i.e. in test mode), then
 // the loss tail; the update is ADAM on 2 * theta over Flux.params (launch_update), after which the bf16 image is rebuilt (ensure_images).
 int rn_forward_dev(mz_ctx *c, int net, int B, const float *d_in, float *d_o1, float *d_o2, unsigned char *pool) {
-    mz_search_rn_args t{}; t.image = c->d_rn_image; t.steps = c->d_rn_steps; t.net = net; t.B = B; t.in = d_in; t.out1 = d_o1; t.out2 = d_o2; t.scratch_pool = pool;
+    mz_search_rn_args t{}; t.image = c->own.rn; t.steps = c->d_rn_steps; t.net = net; t.B = B; t.in = d_in; t.out1 = d_o1; t.out2 = d_o2; t.scratch_pool = pool;
     const int nt = c->rn.R.ntrees;
     launch_scope ls(c, 3); mz_k_rn_forward<<<(B + nt - 1) / nt, MZ_RN_THREADS, c->smem_bytes_rn, c->stream>>>(c->M.P, c->rn.R, t);
     return MZ_OK;
@@ -372,9 +386,9 @@ void launch_loss(mz_ctx *c, int B) {
     { launch_scope ls(c, 3); const int ry = P.K + 1 < MZ_LOSS_RY ? P.K + 1 : MZ_LOSS_RY;
       mz_k_loss_rows<<<(B + 31) / 32, dim3(32, (unsigned)ry), 0, c->stream>>>(P, B, c->batch, c->d_pv, c->d_pr, c->d_pp, c->d_rowv, c->d_rowr, c->d_rowp, c->d_rowinvg); }
     if (c->d_mask) {
-        { launch_scope ls(c, 3); mz_k_loss_reduce<<<4, 1024, 0, c->stream>>>(P, B, c->d_rowv, c->d_rowr, c->d_rowp, c->d_rowinvg, c->d_w, c->d_lossout, 4); }
-        { launch_scope ls(c, 3); mz_k_sqnorm_masked<<<3, 1024, 0, c->stream>>>(c->net_bounds[0], c->net_bounds[1], c->net_bounds[2], c->net_bounds[3], c->d_w, c->d_mask, c->d_lossout); }
-    } else { launch_scope ls(c, 3); mz_k_loss_reduce<<<7, 1024, 0, c->stream>>>(P, B, c->d_rowv, c->d_rowr, c->d_rowp, c->d_rowinvg, c->d_w, c->d_lossout); }
+        { launch_scope ls(c, 3); mz_k_loss_reduce<<<4, 1024, 0, c->stream>>>(P, B, c->d_rowv, c->d_rowr, c->d_rowp, c->d_rowinvg, c->own.w, c->d_lossout, 4); }
+        { launch_scope ls(c, 3); mz_k_sqnorm_masked<<<3, 1024, 0, c->stream>>>(c->net_bounds[0], c->net_bounds[1], c->net_bounds[2], c->net_bounds[3], c->own.w, c->d_mask, c->d_lossout); }
+    } else { launch_scope ls(c, 3); mz_k_loss_reduce<<<7, 1024, 0, c->stream>>>(P, B, c->d_rowv, c->d_rowr, c->d_rowp, c->d_rowinvg, c->own.w, c->d_lossout); }
 }
 
 int launch_learn_forward(mz_ctx *c, int B, int grad_mode = MZ_GRAD_REFERENCE_L2) {
@@ -382,7 +396,7 @@ int launch_learn_forward(mz_ctx *c, int B, int grad_mode = MZ_GRAD_REFERENCE_L2)
     const int path = learner_path(c, grad_mode);
     if (path == -1) return fail(c, MZ_E_UNSUPPORTED, "the ResNet learner implements MZ_GRAD_REFERENCE_L2 (the reference's update); the backward pass through the convolution towers is not built");
     if (path != 3 && grad_mode != MZ_GRAD_REFERENCE_L2 && grad_mode != MZ_GRAD_BPTT) return fail(c, MZ_E_ARG, "unknown grad_mode %d", grad_mode);
-    mz_learn_args a{}; a.wglob = c->d_w; a.B = B; a.max_dim = c->M.max_dim; a.max_layer_floats = c->M.max_layer_floats; a.batch = c->batch;
+    mz_learn_args a{}; a.wglob = c->own.w; a.B = B; a.max_dim = c->M.max_dim; a.max_layer_floats = c->M.max_layer_floats; a.batch = c->batch;
     a.pred_values = c->d_pv; a.pred_rewards = c->d_pr; a.pred_policies = c->d_pp;
     const int tiles = (B + MZ_ROWS - 1) / MZ_ROWS;
     if (path == 3) MZ_TRY(rn_learn_forward(c, B));
@@ -409,8 +423,8 @@ int launch_learn_forward(mz_ctx *c, int B, int grad_mode = MZ_GRAD_REFERENCE_L2)
         for (int n = 0; n < 3; n++) { d.slot_base[n] = L.slot_base[n]; d.layers_in_net[n] = L.layers_in_net[n]; d.first_layer[n] = P.nets[n].first; }
         { launch_scope ls(c, 3); mz_k_learn_dw<<<dim3((unsigned)P.n_layers, (unsigned)chunks), 128, MZ_DW_STAGES * 2 * MZ_SP_TILE_BYTES + 1024, c->stream>>>(P, d); }
         // (use_batch_norm: the images these kernels read are the folded layers (mz_k_pack_images), so the sums are dW', db': same chain rule as below)
-        if (c->cfg.use_batch_norm) { launch_scope ls(c, 4); mz_k_grad_reduce_bn<<<dim3((unsigned)P.n_layers, 16), 256, 0, c->stream>>>(P, chunks, gpart, c->d_w, grad_out(c)); }
-        else { launch_scope ls(c, 4); mz_k_grad_reduce<<<(P.total_floats + 255) / 256, 256, 0, c->stream>>>(P.total_floats, chunks, gpart, c->d_w, grad_out(c)); }
+        if (c->cfg.use_batch_norm) { launch_scope ls(c, 4); mz_k_grad_reduce_bn<<<dim3((unsigned)P.n_layers, 16), 256, 0, c->stream>>>(P, chunks, gpart, c->own.w, grad_out(c)); }
+        else { launch_scope ls(c, 4); mz_k_grad_reduce<<<(P.total_floats + 255) / 256, 256, 0, c->stream>>>(P.total_floats, chunks, gpart, c->own.w, grad_out(c)); }
     } else if (grad_mode == MZ_GRAD_BPTT) {   // forward + backward through the unroll in one kernel; per-tile partial gradients
         if (!c->smem_bytes_bptt) return fail(c, MZ_E_UNSUPPORTED, "MZ_GRAD_BPTT is not built for this network: it needs every layer output and every layer input other than the observation stack to be at most 64 wide, and its buffers to fit one CTA's shared memory");
         float *act, *gpart;
@@ -420,12 +434,12 @@ int launch_learn_forward(mz_ctx *c, int B, int grad_mode = MZ_GRAD_REFERENCE_L2)
         b.dim_wide = c->bptt_dims[0]; b.dim_narrow = c->bptt_dims[1]; b.wfloats[0] = c->bptt_dims[2]; b.wfloats[1] = c->bptt_dims[3];
         if (c->cfg.use_batch_norm) {   // BatchNorm in test mode = a Dense layer with folded weights: the kernel runs on the folded copy, the reduce applies the chain rule
             if (!c->d_w_fold) MZ_CUDA(c, dmalloc(&c->d_w_fold, (size_t)P.total_floats));
-            { launch_scope ls(c, 5); mz_k_bn_fold<<<dim3((unsigned)P.n_layers, 4), 256, 0, c->stream>>>(P, c->d_w, c->d_w_fold); }
+            { launch_scope ls(c, 5); mz_k_bn_fold<<<dim3((unsigned)P.n_layers, 4), 256, 0, c->stream>>>(P, c->own.w, c->d_w_fold); }
             b.f.wglob = c->d_w_fold;
         }
         { launch_scope ls(c, 3); mz_k_learn_bptt<<<tiles, MZ_THREADS, c->smem_bytes_bptt, c->stream>>>(P, c->bptt.plan, b); }
-        if (c->cfg.use_batch_norm) { launch_scope ls(c, 4); mz_k_grad_reduce_bn<<<dim3((unsigned)P.n_layers, 16), 256, 0, c->stream>>>(P, tiles, gpart, c->d_w, grad_out(c)); }
-        else { launch_scope ls(c, 4); mz_k_grad_reduce<<<(P.total_floats + 255) / 256, 256, 0, c->stream>>>(P.total_floats, tiles, gpart, c->d_w, grad_out(c)); }
+        if (c->cfg.use_batch_norm) { launch_scope ls(c, 4); mz_k_grad_reduce_bn<<<dim3((unsigned)P.n_layers, 16), 256, 0, c->stream>>>(P, tiles, gpart, c->own.w, grad_out(c)); }
+        else { launch_scope ls(c, 4); mz_k_grad_reduce<<<(P.total_floats + 255) / 256, 256, 0, c->stream>>>(P.total_floats, tiles, gpart, c->own.w, grad_out(c)); }
     } else if (path == 1) {   // the unroll on the tensor cores (mz_kernels_sp.cuh)
         MZ_TRY(ensure_images(c));
         mz_learn_sp_args t{}; t.sp = c->spa; t.B = B; t.batch = c->batch; t.pred_values = c->d_pv; t.pred_rewards = c->d_pr; t.pred_policies = c->d_pp;
@@ -461,13 +475,13 @@ int launch_update(mz_ctx *c, int64_t t, int grad_mode) {
     }
     // MZ_GRAD_BPTT: d_grad was produced by launch_learn_forward (mz_k_learn_bptt + mz_k_grad_reduce)
     if (grad_mode == MZ_GRAD_REFERENCE_L2 && !c->p2p && !c->comm) {   // one GPU: gradient (2 * theta) and update in one launch
-        launch_scope ls(c, 4); mz_k_adam_l2<<<(n + 255) / 256, 256, 0, c->stream>>>(n, c->d_w, c->d_m, c->d_v, c->d_grad, c->d_mask, mzh::cos_schedule(t), c->bp1, c->bp2);
+        launch_scope ls(c, 4); mz_k_adam_l2<<<(n + 255) / 256, 256, 0, c->stream>>>(n, c->own.w, c->d_m, c->d_v, c->d_grad, c->d_mask, mzh::cos_schedule(t), c->bp1, c->bp2);
     } else {
-        if (grad_mode == MZ_GRAD_REFERENCE_L2) { launch_scope ls(c, 4); mz_k_l2_grad<<<(n + 255) / 256, 256, 0, c->stream>>>(n, c->d_w, c->d_mask, grad_out(c)); }
+        if (grad_mode == MZ_GRAD_REFERENCE_L2) { launch_scope ls(c, 4); mz_k_l2_grad<<<(n + 255) / 256, 256, 0, c->stream>>>(n, c->own.w, c->d_mask, grad_out(c)); }
         if (c->p2p) {    // data-parallel over peer memory: ONE kernel waits for the peers' gradients, sums them in rank order over NVLink and applies ADAM
             mz_dp_args d{}; d.rank = c->rank; d.nranks = c->nranks; d.step = ++c->dp_step; d.n = n; d.flags_local = c->d_xflags;
             for (int r = 0; r < c->nranks; r++) { d.peer_grad[r] = c->peer_grad[r] + (size_t)(d.step & 1u) * (size_t)n; d.peer_flags[r] = c->peer_flags[r]; }
-            launch_scope ls(c, 4); mz_k_dp_adam<<<(n + 255) / 256, 256, 0, c->stream>>>(c->d_w, c->d_m, c->d_v, d, mzh::cos_schedule(t), c->bp1, c->bp2, 1.0f / (float)c->nranks);
+            launch_scope ls(c, 4); mz_k_dp_adam<<<(n + 255) / 256, 256, 0, c->stream>>>(c->own.w, c->d_m, c->d_v, d, mzh::cos_schedule(t), c->bp1, c->bp2, 1.0f / (float)c->nranks);
         } else {
             float scale = 1.0f;
             if (c->comm) {   // data-parallel through NCCL: sum gradients over ranks, average in the update
@@ -475,45 +489,47 @@ int launch_update(mz_ctx *c, int64_t t, int grad_mode) {
                 if (r != ncclSuccess) return fail(c, MZ_E_NCCL, "ncclAllReduce: %s", g_nccl.GetErrorString(r));
                 scale = 1.0f / (float)c->nranks;
             }
-            launch_scope ls(c, 4); mz_k_adam<<<(n + 255) / 256, 256, 0, c->stream>>>(n, c->d_w, c->d_m, c->d_v, c->d_grad, mzh::cos_schedule(t), c->bp1, c->bp2, scale);
+            launch_scope ls(c, 4); mz_k_adam<<<(n + 255) / 256, 256, 0, c->stream>>>(n, c->own.w, c->d_m, c->d_v, c->d_grad, mzh::cos_schedule(t), c->bp1, c->bp2, scale);
         }
     }
     MZ_CUDA(c, cudaGetLastError());
     c->bp1 *= 0.9; c->bp2 *= 0.999; c->adam_t++;
-    c->w_version++;
+    c->own.version++;
     return MZ_OK;
 }
 
 // the fields of a search launch that do not depend on where its roots come from
 static mz_search_args search_args(const mz_ctx *c, int n, int exploration) {
-    mz_search_args a{}; a.wglob = c->d_w; a.pbc0 = c->d_pbc0; a.sqrtN = c->d_sqrtN; a.tree_pool = c->d_trees; a.n = n; a.max_dim = c->M.max_dim;
+    mz_search_args a{}; a.pbc0 = c->d_pbc0; a.sqrtN = c->d_sqrtN; a.tree_pool = c->d_trees; a.n = n; a.max_dim = c->M.max_dim;
     a.max_layer_floats = c->M.max_layer_floats; a.exploration = exploration;
     return a;
 }
 // One search over the roots of `a` (MODE_API: the caller's a.n roots; MODE_SLOTS: the a.n game slots; MODE_REPLAY: a.n stored positions)
-// in ONE launch of kernel family 0 (run_wave_body relabels the last one of an idle iteration).  lat > 0: the low-latency kernel
-// (mz_kernels_lat.cuh) on roots [0, lat), one 2-CTA cluster each; otherwise the batched kernel of the context's networks.  MODE_REPLAY
-// always takes the batched kernel: the latency kernel has no instantiation for it.
+// in ONE launch of kernel family 0 (run_wave_body relabels those of an idle iteration), with the weights and images of store `ws` (NULL:
+// the context's own networks).  lat > 0: the low-latency kernel (mz_kernels_lat.cuh) on roots [0, lat), one 2-CTA cluster each; otherwise
+// the batched kernel of the context's networks.  MODE_REPLAY always takes the batched kernel: the latency kernel has no instantiation for it.
 template <int MODE>
-static void launch_search(mz_ctx *c, const mz_params &P, const mz_search_args &a, int lat) {
+static void launch_search(mz_ctx *c, const mz_params &P, const mz_search_args &args, int lat, const mz_wstore *ws = nullptr) {
+    const mz_wstore &s = ws ? *ws : c->own;
+    mz_search_args a = args; a.wglob = s.w;
     const unsigned ctas = (unsigned)((a.n + MZ_ROWS - 1) / MZ_ROWS);
     launch_scope ls(c, 0);
     if constexpr (MODE != MZ_MODE_REPLAY) {
         if (lat > 0) {
-            mz_lat_args t{}; t.base = a; t.image = c->d_w_lat; t.w_floats = c->lat_w_floats; t.pbc_smem = c->lat_pbc_smem;
+            mz_lat_args t{}; t.base = a; t.image = s.lat; t.w_floats = c->lat_w_floats; t.pbc_smem = c->lat_pbc_smem;
             mz_k_search_lat<MODE><<<2 * lat, MZ_LAT_THREADS, c->smem_bytes_lat, c->stream>>>(P, t);
             return;
         }
     }
     if (c->cfg.net_type == MZ_NET_RESNET) {
-        mz_search_rn_args t{}; t.base = a; t.image = c->d_rn_image; t.steps = c->d_rn_steps;
+        mz_search_rn_args t{}; t.base = a; t.image = s.rn; t.steps = c->d_rn_steps;
         const int nt = c->rn.R.ntrees;
         mz_k_search_rn<MODE><<<(a.n + nt - 1) / nt, MZ_RN_THREADS, c->smem_bytes_rn, c->stream>>>(P, c->rn.R, t);
     } else if (c->cfg.nn_mode == MZ_NN_SPLIT_MMA) {
-        mz_search_sp_args t{}; t.base = a; t.sp = c->spa;
+        mz_search_sp_args t{}; t.base = a; t.sp = c->spa; t.sp.image = s.sp; t.sp.bias = s.sp_bias;
         mz_k_search_sp<MODE><<<ctas, MZ_SP_SEARCH_THREADS, c->smem_bytes_sp, c->stream>>>(P, t);
     } else if (c->cfg.nn_mode == MZ_NN_BF16_TC) {
-        mz_search_tc_args t{}; t.base = a; t.w_image = c->d_w_tc; t.bias = c->d_bias_tc;
+        mz_search_tc_args t{}; t.base = a; t.w_image = s.tc; t.bias = s.tc_bias;
         mz_k_search_tc<MODE><<<ctas, MZ_THREADS, c->smem_bytes_tc, c->stream>>>(P, t);
     } else if (c->cfg.use_batch_norm) mz_k_search<MODE, true><<<ctas, MZ_THREADS, c->smem_bytes, c->stream>>>(P, a);
     else mz_k_search<MODE><<<ctas, MZ_THREADS, c->smem_bytes, c->stream>>>(P, a);
@@ -568,7 +584,7 @@ int mz_create(const mz_config *cfg, int device, mz_ctx **out) {
         if (c->smem_bytes_rn + 1024 > (size_t)prop.sharedMemPerBlockOptin) { int r = fail(nullptr, MZ_E_UNSUPPORTED, "the ResNet search kernel needs %zu B of shared memory per CTA, device allows %zu", c->smem_bytes_rn, (size_t)prop.sharedMemPerBlockOptin); mz_destroy(c); return r; }
         MZ_CREATE(allow_max_smem(mz_k_search_rn<MZ_MODE_API>, prop)); MZ_CREATE(allow_max_smem(mz_k_search_rn<MZ_MODE_SLOTS>, prop)); MZ_CREATE(allow_max_smem(mz_k_rn_forward, prop));
         MZ_CREATE(allow_max_smem(mz_k_search_rn<MZ_MODE_REPLAY>, prop));
-        MZ_CREATE(cudaMalloc((void **)&c->d_rn_image, (size_t)c->rn.image_bytes + 4096));
+        MZ_CREATE(cudaMalloc((void **)&c->own.rn, (size_t)c->rn.image_bytes + 4096));
         MZ_CREATE(dmalloc(&c->d_rn_steps, c->rn.steps.size() + 1));
         MZ_CREATE(cudaMemcpy(c->d_rn_steps, c->rn.steps.data(), c->rn.steps.size() * sizeof(mz_rn_step), cudaMemcpyHostToDevice));
     }
@@ -603,7 +619,7 @@ int mz_create(const mz_config *cfg, int device, mz_ctx **out) {
         c->lat_max_roots = cfg->nn_mode == MZ_NN_FP32_EXACT ? c->sm_count : c->sm_count / 2;
         c->lat_max_slots = 16;                                           // self-play: contexts built for one or a few games at a time (play_game)
         if (const char *el = getenv("MUZERO_B200_LAT")) c->lat_max_roots = c->lat_max_slots = atoi(el);   // measurement / test switch; 0 = off
-        if (c->lat_ok) { MZ_CREATE(allow_max_smem(mz_k_search_lat<MZ_MODE_API>, prop)); MZ_CREATE(allow_max_smem(mz_k_search_lat<MZ_MODE_SLOTS>, prop)); MZ_CREATE(dmalloc(&c->d_w_lat, (size_t)c->lat_image_floats + 64)); }
+        if (c->lat_ok) { MZ_CREATE(allow_max_smem(mz_k_search_lat<MZ_MODE_API>, prop)); MZ_CREATE(allow_max_smem(mz_k_search_lat<MZ_MODE_SLOTS>, prop)); MZ_CREATE(dmalloc(&c->own.lat, (size_t)c->lat_image_floats + 64)); }
     }
     if (!resnet) { if (const char *eb = mzh::build_bptt(P, c->bptt)) { int r = fail(nullptr, MZ_E_ARG, "%s", eb); mz_destroy(c); return r; } }
     bool bptt_fits = !resnet;
@@ -640,9 +656,9 @@ int mz_create(const mz_config *cfg, int device, mz_ctx **out) {
             MZ_CREATE(allow_max_smem(mz_k_search_tc<MZ_MODE_SLOTS>, prop));
             MZ_CREATE(allow_max_smem(mz_k_search_tc<MZ_MODE_REPLAY>, prop));
             MZ_CREATE(allow_max_smem(mz_k_nn_forward_tc, prop));
-            MZ_CREATE(cudaMalloc((void **)&c->d_w_tc, (size_t)P.tc_net_off[3] + 8192));
-            MZ_CREATE(cudaMemset(c->d_w_tc, 0, (size_t)P.tc_net_off[3] + 8192));
-            MZ_CREATE(dmalloc(&c->d_bias_tc, (size_t)P.tc_bias_floats));
+            MZ_CREATE(cudaMalloc((void **)&c->own.tc, (size_t)P.tc_net_off[3] + 8192));
+            MZ_CREATE(cudaMemset(c->own.tc, 0, (size_t)P.tc_net_off[3] + 8192));
+            MZ_CREATE(dmalloc(&c->own.tc_bias, (size_t)P.tc_bias_floats));
         } else if (cfg->nn_mode == MZ_NN_BF16_TC) {
             int r = fail(nullptr, MZ_E_UNSUPPORTED, "MZ_NN_BF16_TC needs %zu B of shared memory per CTA, device allows %zu", c->smem_bytes_tc, (size_t)prop.sharedMemPerBlockOptin);
             mz_destroy(c); return r;
@@ -659,13 +675,13 @@ int mz_create(const mz_config *cfg, int device, mz_ctx **out) {
             MZ_CREATE(allow_max_smem(mz_k_search_sp<MZ_MODE_REPLAY>, prop));
             MZ_CREATE(allow_max_smem(mz_k_nn_forward_sp, prop));
             MZ_CREATE(allow_max_smem(mz_k_learn_forward_sp, prop));
-            MZ_CREATE(cudaMalloc((void **)&c->d_w_sp, (size_t)S.image_bytes + 256));
-            MZ_CREATE(cudaMemset(c->d_w_sp, 0, (size_t)S.image_bytes + 256));
-            MZ_CREATE(dmalloc(&c->d_bias_sp, (size_t)S.bias_floats));
+            MZ_CREATE(cudaMalloc((void **)&c->own.sp, (size_t)S.image_bytes + 256));
+            MZ_CREATE(cudaMemset(c->own.sp, 0, (size_t)S.image_bytes + 256));
+            MZ_CREATE(dmalloc(&c->own.sp_bias, (size_t)S.bias_floats));
             MZ_CREATE(cudaMalloc((void **)&c->d_rounds_sp, sizeof(mz_sp_round) * MZ_SP_MAX_ROUNDS));
             MZ_CREATE(cudaMemcpy(c->d_rounds_sp, S.round, sizeof(mz_sp_round) * MZ_SP_MAX_ROUNDS, cudaMemcpyHostToDevice));
             mz_sp_args &A = c->spa;
-            A.image = c->d_w_sp; A.bias = c->d_bias_sp; A.rounds = c->d_rounds_sp;
+            A.image = c->own.sp; A.bias = c->own.sp_bias; A.rounds = c->d_rounds_sp;
             for (int n = 0; n < 3; n++) { A.first[n] = S.first[n]; A.n_rounds[n] = S.n_rounds[n]; A.set_first[n] = S.set_first[n]; A.n_sets[n] = S.n_sets[n]; }
             A.total_rounds = S.total_rounds; A.total_sets = S.total_sets; A.warea_bytes = S.warea_bytes; A.bias_floats = S.bias_floats; A.pbc_smem = S.pbc_smem; A.tail = S.tail;
             // the learner's backward rounds on the same machinery
@@ -690,8 +706,8 @@ int mz_create(const mz_config *cfg, int device, mz_ctx **out) {
     c->packed = !resnet;
     c->store_floats = resnet ? P.n_params : P.total_floats;
     const size_t nf = (size_t)c->store_floats;
-    MZ_CREATE(dmalloc(&c->d_w, nf)); MZ_CREATE(dmalloc(&c->d_m, nf)); MZ_CREATE(dmalloc(&c->d_v, nf)); MZ_CREATE(dmalloc(&c->d_grad, nf));
-    MZ_CREATE(cudaMemset(c->d_w, 0, nf * 4)); MZ_CREATE(cudaMemset(c->d_m, 0, nf * 4)); MZ_CREATE(cudaMemset(c->d_v, 0, nf * 4));
+    MZ_CREATE(dmalloc(&c->own.w, nf)); MZ_CREATE(dmalloc(&c->d_m, nf)); MZ_CREATE(dmalloc(&c->d_v, nf)); MZ_CREATE(dmalloc(&c->d_grad, nf));
+    MZ_CREATE(cudaMemset(c->own.w, 0, nf * 4)); MZ_CREATE(cudaMemset(c->d_m, 0, nf * 4)); MZ_CREATE(cudaMemset(c->d_v, 0, nf * 4));
     if (resnet || cfg->use_batch_norm) {   // Flux.params of a BatchNorm are beta and gamma: the running statistics take no part in sum(abs2, theta), its gradient or ADAM
         std::vector<unsigned char> mask(nf + 16, 1);
         if (resnet) {
@@ -737,7 +753,7 @@ int mz_destroy(mz_ctx *c) {
     if (c->stream) cudaStreamSynchronize(c->stream);
     collect_timings(c);
     if (c->comm && g_nccl.CommDestroy) { p2p_teardown(c); g_nccl.CommDestroy(c->comm); }
-    void *ptrs[] = {c->d_mask, c->d_w_fold, c->d_w_lat, c->d_brounds, c->d_w_sp, c->d_bias_sp, c->d_rounds_sp, c->d_rn_image, c->d_rn_steps, c->d_bstages[0], c->d_bstages[1], c->d_w_tc, c->d_bias_tc, c->d_w, c->d_m, c->d_v, c->d_grad, c->d_pbc0, c->d_sqrtN, c->d_trees, c->slots.p1, c->slots.p2, c->slots.player, c->slots.T,
+    void *ptrs[] = {c->opp.w, c->opp.tc, c->opp.tc_bias, c->opp.sp, c->opp.sp_bias, c->opp.lat, c->opp.rn, c->d_mask, c->d_w_fold, c->own.lat, c->d_brounds, c->own.sp, c->own.sp_bias, c->d_rounds_sp, c->own.rn, c->d_rn_steps, c->d_bstages[0], c->d_bstages[1], c->own.tc, c->own.tc_bias, c->own.w, c->d_m, c->d_v, c->d_grad, c->d_pbc0, c->d_sqrtN, c->d_trees, c->slots.p1, c->slots.p2, c->slots.player, c->slots.T,
                     c->slots.status, c->slots.game_id, c->slots.fin_list, c->slots.h_p1, c->slots.h_p2, c->slots.h_action, c->slots.h_reward, c->slots.h_to_play,
                     c->slots.h_cv, c->slots.h_rv, c->d_stats, c->d_lossout, c->batch.index, c->batch.obs,
                     c->batch.actions, c->batch.values, c->batch.rewards, c->batch.policies, c->batch.gscale, c->batch.weights, c->d_pv, c->d_pr, c->d_pp,
@@ -798,6 +814,54 @@ int mz_set_weights(mz_ctx *c, int net, const float *blob, int64_t n) {
     else { MZ_TRY(download_weights(c, src)); memcpy(src.data() + ctx_net_offset(c, net), blob, (size_t)n * sizeof(float)); }
     return upload_weights(c, src);
 }
+// the opponent store, with the images of the context's path only; on failure nothing is left half-allocated
+static int alloc_opponent(mz_ctx *c) {
+    if (c->opp.w) return MZ_OK;
+    const mz_params &P = c->M.P;
+    mz_wstore s;
+    cudaError_t e = dmalloc(&s.w, (size_t)c->store_floats);
+    if (e == cudaSuccess && c->cfg.nn_mode == MZ_NN_SPLIT_MMA && c->own.sp) {
+        e = cudaMalloc((void **)&s.sp, (size_t)c->spp.image_bytes + 256);
+        if (e == cudaSuccess) e = cudaMemsetAsync(s.sp, 0, (size_t)c->spp.image_bytes + 256, c->stream);
+        if (e == cudaSuccess) e = dmalloc(&s.sp_bias, (size_t)c->spp.bias_floats);
+    }
+    if (e == cudaSuccess && c->cfg.nn_mode == MZ_NN_BF16_TC && c->own.tc) {
+        e = cudaMalloc((void **)&s.tc, (size_t)P.tc_net_off[3] + 8192);
+        if (e == cudaSuccess) e = cudaMemsetAsync(s.tc, 0, (size_t)P.tc_net_off[3] + 8192, c->stream);
+        if (e == cudaSuccess) e = dmalloc(&s.tc_bias, (size_t)P.tc_bias_floats);
+    }
+    if (e == cudaSuccess && c->own.lat) e = dmalloc(&s.lat, (size_t)c->lat_image_floats + 64);
+    if (e == cudaSuccess && c->own.rn) e = cudaMalloc((void **)&s.rn, (size_t)c->rn.image_bytes + 4096);
+    if (e != cudaSuccess) {
+        for (void *p : {(void *)s.w, (void *)s.sp, (void *)s.sp_bias, (void *)s.tc, (void *)s.tc_bias, (void *)s.lat, (void *)s.rn}) if (p) cudaFree(p);
+        return fail(c, MZ_E_CUDA, "allocating the opponent networks: %s", cudaGetErrorString(e));
+    }
+    c->opp = s;
+    return MZ_OK;
+}
+int mz_set_opponent_weights(mz_ctx *c, int net, const float *blob, int64_t n) {
+    MZ_CHECK_CTX(c);
+    if (net < 0 || net > 3 || !blob) return fail(c, MZ_E_ARG, "bad net id or NULL blob");
+    if (n != ctx_net_params(c, net)) return fail(c, MZ_E_ARG, "weight blob has %lld floats, net %d needs %d", (long long)n, net, ctx_net_params(c, net));
+    if (net != MZ_NET_ALL && !c->opp_full)
+        return fail(c, MZ_E_STATE, "replacing one opponent network needs a full opponent set first (mz_set_opponent_weights with MZ_NET_ALL, or mz_snapshot_opponent)");
+    MZ_TRY(alloc_opponent(c));
+    std::vector<float> src((size_t)c->M.P.n_params);
+    if (net == MZ_NET_ALL) memcpy(src.data(), blob, (size_t)n * sizeof(float));
+    else { MZ_TRY(store_to_host(c, c->opp.w, src.data())); memcpy(src.data() + ctx_net_offset(c, net), blob, (size_t)n * sizeof(float)); }
+    MZ_TRY(store_from_host(c, c->opp.w, src.data()));
+    c->opp.version++;
+    c->opp_full = true;
+    return MZ_OK;
+}
+int mz_snapshot_opponent(mz_ctx *c) {
+    MZ_CHECK_CTX(c);
+    MZ_TRY(alloc_opponent(c));
+    MZ_CUDA(c, cudaMemcpyAsync(c->opp.w, c->own.w, (size_t)c->store_floats * sizeof(float), cudaMemcpyDeviceToDevice, c->stream));
+    c->opp.version++;
+    c->opp_full = true;
+    return MZ_OK;
+}
 int mz_get_weights(mz_ctx *c, int net, float *blob, int64_t n) {
     MZ_CHECK_CTX(c);
     if (net < 0 || net > 3 || !blob) return fail(c, MZ_E_ARG, "bad net id or NULL blob");
@@ -821,18 +885,18 @@ static int nn_forward(mz_ctx *c, int net, int B, const float *in, float *out1, s
     MZ_TRY(h2d(c, c->scratch[0], in, (size_t)B * in_dim, &d_in));
     MZ_TRY(h2d<float>(c, c->scratch[1], nullptr, (size_t)B * n1, &d_o1));
     MZ_TRY(h2d<float>(c, c->scratch[2], nullptr, (size_t)B * (n2 ? n2 : 1), &d_o2));
-    mz_nn_args a{}; a.wglob = c->d_w; a.B = B; a.max_dim = c->M.max_dim; a.max_layer_floats = c->M.max_layer_floats; a.net = net; a.in = d_in; a.out1 = d_o1; a.out2 = d_o2;
+    mz_nn_args a{}; a.wglob = c->own.w; a.B = B; a.max_dim = c->M.max_dim; a.max_layer_floats = c->M.max_layer_floats; a.net = net; a.in = d_in; a.out1 = d_o1; a.out2 = d_o2;
     if (resnet) {
         unsigned char *d_pool;
         MZ_TRY(h2d<unsigned char>(c, c->scratch[3], nullptr, (size_t)B * c->rn.R.node_bytes, &d_pool));
-        mz_search_rn_args t{}; t.image = c->d_rn_image; t.steps = c->d_rn_steps; t.net = net; t.B = B; t.in = d_in; t.out1 = d_o1; t.out2 = d_o2; t.scratch_pool = d_pool;
+        mz_search_rn_args t{}; t.image = c->own.rn; t.steps = c->d_rn_steps; t.net = net; t.B = B; t.in = d_in; t.out1 = d_o1; t.out2 = d_o2; t.scratch_pool = d_pool;
         const int nt = c->rn.R.ntrees;
         launch_scope ls(c, 5); mz_k_rn_forward<<<(B + nt - 1) / nt, MZ_RN_THREADS, c->smem_bytes_rn, c->stream>>>(P, c->rn.R, t);
     } else if (c->cfg.nn_mode == MZ_NN_SPLIT_MMA) {
         mz_nn_sp_args t{}; t.sp = c->spa; t.B = B; t.net = net; t.in = d_in; t.out1 = d_o1; t.out2 = d_o2;
         launch_scope ls(c, 5); mz_k_nn_forward_sp<<<(B + MZ_ROWS - 1) / MZ_ROWS, MZ_SP_THREADS, c->smem_bytes_sp, c->stream>>>(P, t);
     } else if (c->cfg.nn_mode == MZ_NN_BF16_TC) {
-        mz_nn_tc_args t{}; t.w_image = c->d_w_tc; t.bias = c->d_bias_tc; t.B = B; t.net = net; t.in = d_in; t.out1 = d_o1; t.out2 = d_o2;
+        mz_nn_tc_args t{}; t.w_image = c->own.tc; t.bias = c->own.tc_bias; t.B = B; t.net = net; t.in = d_in; t.out1 = d_o1; t.out2 = d_o2;
         launch_scope ls(c, 5); mz_k_nn_forward_tc<<<(B + MZ_ROWS - 1) / MZ_ROWS, MZ_THREADS, c->smem_bytes_tc, c->stream>>>(P, t);
     } else if (c->cfg.use_batch_norm) { launch_scope ls(c, 5); mz_k_nn_forward<true><<<(B + MZ_ROWS - 1) / MZ_ROWS, MZ_THREADS, c->smem_bytes, c->stream>>>(P, a); }
     else { launch_scope ls(c, 5); mz_k_nn_forward<false><<<(B + MZ_ROWS - 1) / MZ_ROWS, MZ_THREADS, c->smem_bytes, c->stream>>>(P, a); }
@@ -920,7 +984,7 @@ int mz_run_mcts(mz_ctx *c, int n, const float *stacked_obs, const uint32_t *lega
         // few roots: one tree per cluster in exact fp32 (mz_kernels_lat.cuh); every input in ONE pinned block and one copy each way -- at
         // this size the call's latency is what the caller sees (the reference calls run_mcts with one root at a time).  No game can be in
         // flight here: a wave ends with every slot idle or resets the slots.
-        MZ_TRY(ensure_lat_image(c));
+        MZ_TRY(ensure_lat_image(c, c->own));
         auto al = [](size_t x) { return (x + 15) & ~(size_t)15; };
         const size_t o_st = 0, o_legal = al(o_st + (size_t)n * P.stack_size * 4), o_gid = al(o_legal + (size_t)n * 4), o_mv = al(o_gid + (size_t)n * 8),
                      o_vc = al(o_mv + (size_t)n * 4), o_rv = al(o_vc + (size_t)n * P.A * 4), o_pri = al(o_rv + (size_t)n * 4), total = al(o_pri + (size_t)n * P.A * 4);
@@ -1015,14 +1079,16 @@ static int run_wave(mz_ctx *c, uint64_t first_game, int64_t n_games, float tempe
         // wave-synchronous refill hands out games num_slots at a time, in slot order: a call for more games than slots is a sequence of
         // single-wave calls, each of which the headline path plays in one launch (the other feed-forward paths: one launch per move with the
         // save / refill beside the next search)
-        unsigned long long acc[4] = {0, 0, 0, 0};
+        unsigned long long acc[4] = {0, 0, 0, 0}, tally[3] = {0, 0, 0};   // search statistics; wins / draws / losses of mz_arena(MZ_OPP_SELF)
         for (int64_t off = 0; off < n_games && rc == MZ_OK; off += G) {
             rc = run_wave_body(c, first_game + (uint64_t)off, n_games - off < G ? n_games - off : G, temperature, arena_player, arena_opponent, tally_player, nullptr, nullptr,
                                false /* a short last wave stays on this path's arithmetic: one call, one kernel family */);
             for (int i = 0; i < 4; i++) acc[i] += c->h_stats[i];
+            for (int i = 0; i < 3; i++) tally[i] += c->h_stats[61 + i];
         }
         if (rc == MZ_OK) {
             for (int i = 0; i < 4; i++) c->h_stats[i] = acc[i];
+            for (int i = 0; i < 3; i++) c->h_stats[61 + i] = tally[i];
             if (simulations) *simulations = (int64_t)acc[1];
             if (moves) *moves = (int64_t)acc[3];
             c->last_mean_depth = acc[1] ? (double)acc[0] / (double)acc[1] : 0.0;
@@ -1051,14 +1117,18 @@ static int run_wave_body(mz_ctx *c, uint64_t first_game, int64_t n_games, float 
     c->h_counters[3] = (int64_t)first_game; c->h_counters[4] = (int64_t)first_game + n_games; c->h_counters[5] = 0;
     MZ_CUDA(c, cudaMemcpyAsync(c->ring.counters + 3, c->h_counters + 3, 3 * sizeof(int64_t), cudaMemcpyHostToDevice, c->stream));
     MZ_CUDA(c, cudaMemsetAsync(c->d_stats, 0, 64 * sizeof(unsigned long long), c->stream));
+    // MZ_OPP_NETWORK: the other side's plies are searched like MuZero's, by the same kernels reading the opponent store
+    const bool vs_net = arena_player != 0 && arena_opponent == MZ_OPP_NETWORK;
     MZ_TRY(ensure_images(c));
+    if (vs_net) MZ_TRY(ensure_images(c, c->opp));
     mz_search_args a = search_args(c, G, 1 /* play_game hard-codes exploration=true, SelfPlay.jl:359 */);
     a.slots = c->slots; a.temperature = temperature; a.stats = c->d_stats;
     // A wave starts with every slot idle and games are handed out in slot order, so a call for n_games <= num_slots games only ever uses the
     // slots [0, n_games): few games go to the low-latency kernel whatever the context's size (the bf16 mode keeps its own arithmetic)
     const int G_lat = (int64_t)G < n_games ? G : (int)n_games;
     const bool use_lat = allow_lat && c->lat_ok && G_lat >= 1 && G_lat <= c->lat_max_slots && c->cfg.nn_mode != MZ_NN_BF16_TC;
-    if (use_lat) MZ_TRY(ensure_lat_image(c));
+    if (use_lat) MZ_TRY(ensure_lat_image(c, c->own));
+    if (use_lat && vs_net) MZ_TRY(ensure_lat_image(c, c->opp));
     int64_t total_moves = 0; int last_snap = 0;
     // The host runs one iteration behind the device: iteration k (opponent plies, search, save/refill, counter snapshot) is queued before
     // the snapshot of iteration k - 1 is read, so the GPU never waits for a launch.  When that snapshot says no game is active any more,
@@ -1098,7 +1168,11 @@ static int run_wave_body(mz_ctx *c, uint64_t first_game, int64_t n_games, float 
     for (int64_t k = 0;; k++) {
         if (k > n_games * (int64_t)(P.max_moves + 2) + 8) return fail(c, MZ_E_STATE, "self-play did not terminate");
         P.fin_tag = (int32_t)(k & 1);
-        if (arena_player != 0) { launch_scope ls(c, 6); mz_k_opponent_move<<<(G + 127) / 128, 128, 0, c->stream>>>(P, c->slots, G); }
+        const size_t iter_entry = c->timed.size();
+        if (vs_net) {   // the opponent's plies: slots whose side to move is the other one, then MuZero's below (a game may make both)
+            mz_params Po = P; Po.arena_player = 3 - arena_player;
+            launch_search<MZ_MODE_SLOTS>(c, Po, a, use_lat ? G_lat : 0, &c->opp);
+        } else if (arena_player != 0) { launch_scope ls(c, 6); mz_k_opponent_move<<<(G + 127) / 128, 128, 0, c->stream>>>(P, c->slots, G); }
         launch_search<MZ_MODE_SLOTS>(c, P, a, use_lat ? G_lat : 0);   // few games (play_game one game at a time): one tree per cluster, exact fp32
         const size_t search_entry = c->timed.size();                       // (timing builds) index just past this iteration's search launch
         if (overlap) { MZ_CUDA(c, cudaEventRecord(c->ev_search[k & 1], c->stream)); MZ_CUDA(c, cudaStreamWaitEvent(sB, c->ev_search[k & 1], 0)); }
@@ -1109,8 +1183,8 @@ static int run_wave_body(mz_ctx *c, uint64_t first_game, int64_t n_games, float 
         MZ_CUDA(c, cudaEventSynchronize(c->ev_wave[k & 1]));
         const int64_t active = c->h_wave[8 * (k & 1) + 5];                 // games active when iteration k started
         if (active == 0) {
-            // the iteration just queued is the idle one: keep it out of the per-family kernel statistics (family 7 = idle)
-            for (size_t i = search_entry; i-- > 0;) if (c->timed[i].family == 0) { c->timed[i].family = 7; break; }
+            // the iteration just queued is the idle one: keep its searches out of the per-family kernel statistics (family 7 = idle)
+            for (size_t i = iter_entry; i < search_entry; i++) if (c->timed[i].family == 0) c->timed[i].family = 7;
             if (c->timed.size() > search_entry) c->timed[search_entry].family = 7;
             break;
         }
@@ -1131,14 +1205,20 @@ int mz_self_play(mz_ctx *c, uint64_t first_game, int64_t n_games, float temperat
     MZ_CHECK_CTX(c);
     return run_wave(c, first_game, n_games, temperature, 0, MZ_OPP_SELF, 0, simulations, moves);
 }
+static int check_opponent_set(mz_ctx *c, int opponent) {
+    if (opponent == MZ_OPP_NETWORK && !c->opp_full)
+        return fail(c, MZ_E_STATE, "MZ_OPP_NETWORK needs opponent networks: set them with mz_set_opponent_weights or mz_snapshot_opponent");
+    return MZ_OK;
+}
 // competitive_play! (src/SelfPlay.jl:421-435) for n_games games at once
 int mz_arena(mz_ctx *c, uint64_t first_game, int64_t n_games, int opponent, int muzero_player, float temperature, int64_t *wins, int64_t *draws,
              int64_t *losses, int64_t *simulations) {
     MZ_CHECK_CTX(c);
-    if (opponent != MZ_OPP_SELF && opponent != MZ_OPP_RANDOM && opponent != MZ_OPP_EXPERT)
-        return fail(c, MZ_E_ARG, "opponent must be MZ_OPP_SELF, MZ_OPP_RANDOM or MZ_OPP_EXPERT (\"human\" has no batched meaning)");
+    if (opponent != MZ_OPP_SELF && opponent != MZ_OPP_RANDOM && opponent != MZ_OPP_EXPERT && opponent != MZ_OPP_NETWORK)
+        return fail(c, MZ_E_ARG, "opponent must be MZ_OPP_SELF, MZ_OPP_RANDOM, MZ_OPP_EXPERT or MZ_OPP_NETWORK (\"human\" has no batched meaning)");
     if (c->M.P.P != 2 && opponent != MZ_OPP_SELF) return fail(c, MZ_E_ARG, "an opponent needs a two-player game");
     if (muzero_player < 1 || muzero_player > c->M.P.P) return fail(c, MZ_E_ARG, "muzero_player %d out of range 1..%d", muzero_player, c->M.P.P);
+    MZ_TRY(check_opponent_set(c, opponent));
     // length(conf.players) == 1 ? "self" : conf.opponent (:428); "self": every ply is searched, outcomes still tallied for muzero_player
     MZ_TRY(run_wave(c, first_game, n_games, temperature, opponent == MZ_OPP_SELF ? 0 : muzero_player, opponent, muzero_player, simulations, nullptr));
     if (wins) *wins = (int64_t)c->h_stats[61];
@@ -1170,9 +1250,10 @@ int mz_play_games(mz_ctx *c, uint64_t first_game, int n_games, float temperature
                   int32_t *actions, float *rewards, int32_t *to_play, float *child_visits, float *root_values, int64_t *simulations) {
     MZ_CHECK_CTX(c);
     if (n_games < 0) return fail(c, MZ_E_ARG, "n_games < 0");
-    if (opponent != MZ_OPP_SELF && opponent != MZ_OPP_RANDOM && opponent != MZ_OPP_EXPERT)
-        return fail(c, MZ_E_ARG, "opponent must be MZ_OPP_SELF, MZ_OPP_RANDOM or MZ_OPP_EXPERT (\"human\" has no batched meaning)");
+    if (opponent != MZ_OPP_SELF && opponent != MZ_OPP_RANDOM && opponent != MZ_OPP_EXPERT && opponent != MZ_OPP_NETWORK)
+        return fail(c, MZ_E_ARG, "opponent must be MZ_OPP_SELF, MZ_OPP_RANDOM, MZ_OPP_EXPERT or MZ_OPP_NETWORK (\"human\" has no batched meaning)");
     if (opponent != MZ_OPP_SELF && (c->M.P.P != 2 || muzero_player < 1 || muzero_player > 2)) return fail(c, MZ_E_ARG, "an opponent needs a two-player game and muzero_player in 1..2");
+    MZ_TRY(check_opponent_set(c, opponent));
     if (simulations) *simulations = 0;
     if (n_games == 0) return MZ_OK;
     MZ_TRY(read_counters(c));
@@ -1273,7 +1354,7 @@ int mz_reanalyse(mz_ctx *c, int64_t key0, int n) {
     int64_t played = c->h_counters[0], have = played < c->ring.capacity ? played : c->ring.capacity, first = played - have + 1;
     if (key0 < first || key0 + n - 1 > played) return fail(c, MZ_E_ARG, "keys %lld..%lld not in the buffer (holds %lld..%lld)", (long long)key0, (long long)(key0 + n - 1), (long long)first, (long long)played);
     const mz_params &P = c->M.P;
-    mz_reanalyse_args a{}; a.wglob = c->d_w; a.max_dim = c->M.max_dim; a.max_layer_floats = c->M.max_layer_floats; a.n = n; a.key0 = key0; a.ring = c->ring;
+    mz_reanalyse_args a{}; a.wglob = c->own.w; a.max_dim = c->M.max_dim; a.max_layer_floats = c->M.max_layer_floats; a.n = n; a.key0 = key0; a.ring = c->ring;
     const int64_t total = (int64_t)n * P.Tmax;
     { launch_scope ls(c, 5);
       if (c->cfg.use_batch_norm) mz_k_reanalyse<true><<<(unsigned)((total + MZ_ROWS - 1) / MZ_ROWS), MZ_THREADS, c->smem_bytes, c->stream>>>(P, a);
@@ -1507,7 +1588,7 @@ int mz_learn_gradients_w(mz_ctx *c, int grad_mode, int B, const float *obs_batch
     if (weight_batch) MZ_CUDA(c, cudaMemcpyAsync(c->batch.weights, weight_batch, (size_t)B * 4, cudaMemcpyHostToDevice, c->stream));
     MZ_TRY(launch_learn_forward(c, B, grad_mode));
     const int n = c->store_floats;
-    if (grad_mode == MZ_GRAD_REFERENCE_L2) { launch_scope ls(c, 4); mz_k_l2_grad<<<(n + 255) / 256, 256, 0, c->stream>>>(n, c->d_w, c->d_mask, grad_out(c)); }
+    if (grad_mode == MZ_GRAD_REFERENCE_L2) { launch_scope ls(c, 4); mz_k_l2_grad<<<(n + 255) / 256, 256, 0, c->stream>>>(n, c->own.w, c->d_mask, grad_out(c)); }
     MZ_TRY(store_to_host(c, grad_out(c), grad));
     return finish_losses(c, B, losses);
 }

@@ -203,15 +203,21 @@ function self_play!(e::Engine, n_games::Integer; temperature=visit_softmax_tempe
     return sims[], moves[]
 end
 # ---- competitive_play! (src/SelfPlay.jl:421-435), batched ------------------------------------------------------
-const OPPONENTS = Dict("self" => 0, "random" => 1, "expert" => 2)
+const OPPONENTS = Dict("self" => 0, "random" => 1, "expert" => 2, "network" => 3)
+"The networks `competitive_play!(e; opponent=\"network\")` plays against: one network (`net` 0..2, after a full set) or all of them (3)."
+set_opponent_networks!(e::Engine, blob::Vector{Float32}, net::Integer=3) =
+    check(e, ccall((:mz_set_opponent_weights, LIB), Cint, (Ptr{Cvoid}, Cint, Ptr{Float32}, Int64), e.ctx, net, blob, length(blob)))
+"The opponent networks become a copy of the engine's current networks (on the device): snapshot, train, then evaluate against it."
+snapshot_opponent!(e::Engine) = check(e, ccall((:mz_snapshot_opponent, LIB), Cint, (Ptr{Cvoid},), e.ctx))
 """
 `n_games` games of `play_game(env, 0.0f0, render, conf.opponent, conf.muzero_player, NNs)` at once. The reference renders one game and
 returns nothing; this returns `(wins, draws, losses, simulations)` for MuZero. "expert" is a one-ply lookahead (the reference's
 `expert_agent()` is undefined); "human" stays with the reference's own loop. The games are saved to the engine's replay buffer like
-self-play games: evaluate on an `Engine` of its own.
+self-play games: evaluate on an `Engine` of its own. "network": the other side is a second MuZero searching with the opponent networks
+(`set_opponent_networks!`, `snapshot_opponent!`).
 """
 function competitive_play!(e::Engine, n_games::Integer=1; opponent::String="random", muzero_player::Integer=1, temperature=0.0f0)
-    haskey(OPPONENTS, opponent) || error("Wrong argument: opponent argument should be self, human, expert or random")
+    haskey(OPPONENTS, opponent) || error("Wrong argument: opponent argument should be self, human, expert, random or network")
     w = Ref{Int64}(0); d = Ref{Int64}(0); l = Ref{Int64}(0); sims = Ref{Int64}(0)
     check(e, ccall((:mz_arena, LIB), Cint, (Ptr{Cvoid}, UInt64, Int64, Cint, Cint, Cfloat, Ref{Int64}, Ref{Int64}, Ref{Int64}, Ref{Int64}),
                    e.ctx, e.next_game, n_games, OPPONENTS[opponent], muzero_player, temperature, w, d, l, sims))
@@ -317,7 +323,7 @@ select_action(node::Node, temperature) = (e = engine(); select_action(e, node, F
 
 "n games of play_game through mz_play_games: GameHistory objects in game-id order; nothing is saved."
 function play_games(e::Engine, n::Integer, temperature, opponent::String, muzero_player::Integer)
-    haskey(OPPONENTS, opponent) || error("Wrong argument: opponent argument should be self, human, expert or random")   # SelfPlay.jl:323
+    haskey(OPPONENTS, opponent) || error("Wrong argument: opponent argument should be self, human, expert, random or network")   # SelfPlay.jl:323
     Tm = Int(e.cfg.max_moves) + 1; A = Int(e.cfg.A); W, H, C = Int(e.cfg.W), Int(e.cfg.H), Int(e.cfg.C)
     gid = zeros(Int64, n); T = zeros(Int32, n); obs = zeros(Float32, W, H, C, Tm, n); act = zeros(Int32, Tm, n); rew = zeros(Float32, Tm, n)
     tp = zeros(Int32, Tm, n); cv = zeros(Float32, A, Tm, n); rv = zeros(Float32, Tm, n); sims = Ref{Int64}(0)
