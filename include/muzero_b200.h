@@ -237,6 +237,13 @@ int mz_learn_forward(mz_ctx *ctx, int B, const float *obs_batch, const float *ac
 int mz_learn_step(mz_ctx *ctx, int64_t t, int grad_mode, float *losses /* [3] */);
 /* n consecutive iterations t0 .. t0+n-1 queued back to back (no host round trip in between); losses of the last one */
 int mz_learn_steps(mz_ctx *ctx, int64_t t0, int n, int grad_mode, float *losses /* [3] */);
+/* n learning! iterations t0 .. t0+n-1 with fresh targets (MuZero Reanalyze on the batch): before step t's loss, every distinct game of
+ * get_batch(step = t) is reanalysed whole (exactly mz_reanalyse_search on that key, with the weights as they are after step t-1), then
+ * the batch is gathered from the refreshed ring and the step proceeds as mz_learn_step(t).  Queued on the device without a host round
+ * trip per step (the ResNet path has one: its weight image is packed on the host).  *simulations (may be NULL) = total simulations run.
+ * MZ_E_ARG: t0 < 1, n < 1, losses NULL; MZ_E_STATE: empty buffer or self-play in progress; grad_mode errors as mz_learn_step.  Nothing
+ * changes on an error. */
+int mz_learn_steps_reanalysed(mz_ctx *ctx, int64_t t0, int n, int grad_mode, int exploration, float *losses /* [3] */, int64_t *simulations);
 /* gradients of one caller-supplied batch without an update (parity entry point): grad[n_params] in the reference blob
  * order.  MZ_GRAD_REFERENCE_L2: what the reference's three Zygote pullbacks actually return, 2*theta (Learning.jl:385-393
  * differentiate a closure whose predictions were computed outside of it).  MZ_GRAD_BPTT: the gradient of the same loss

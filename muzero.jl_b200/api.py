@@ -403,8 +403,10 @@ def reanalyse_search(engine: Engine, key0=None, n=None, exploration=False):
     return engine.ctx.reanalyse_search(key0, n, exploration)
 
 
-def learning(engine: Engine, steps: int, grad_mode=capi.GRAD_REFERENCE_L2, log_every=0):
+def learning(engine: Engine, steps: int, grad_mode=capi.GRAD_REFERENCE_L2, log_every=0, reanalyse=False, exploration=False):
     """learning! (Learning.jl:306-438): `steps` iterations of get_batch -> unroll -> loss -> gradients -> ADAM(Cos schedule).
+    reanalyse=True: MuZero Reanalyze on every batch -- before each step, the games the batch samples are searched again with the
+    current networks (`exploration` as in reanalyse_search), so every target the step trains on is fresh.
     Returns the three losses (representation, prediction, dynamics) of the last step."""
     if len(ReplayBuffer(engine)) < 1:
         raise RuntimeError("replay buffer is empty (learning! waits for num_played_games >= 1, Learning.jl:311)")
@@ -413,7 +415,10 @@ def learning(engine: Engine, steps: int, grad_mode=capi.GRAD_REFERENCE_L2, log_e
     done = 0
     while done < steps:
         n = min(chunk, steps - done)
-        losses = engine.ctx.learn_steps(engine.training_step + 1, n, grad_mode)
+        if reanalyse:
+            losses, _ = engine.ctx.learn_steps_reanalysed(engine.training_step + 1, n, grad_mode, exploration)
+        else:
+            losses = engine.ctx.learn_steps(engine.training_step + 1, n, grad_mode)
         engine.training_step += n; done += n
         if log_every:
             print("Training Progress", engine.training_step, losses)

@@ -123,6 +123,7 @@ def lib():
         "mz_learn_forward": ([ctx, C.c_int] + [f32p] * 10, C.c_int),
         "mz_learn_step": ([ctx, C.c_int64, C.c_int, f32p], C.c_int),
         "mz_learn_steps": ([ctx, C.c_int64, C.c_int, C.c_int, f32p], C.c_int),
+        "mz_learn_steps_reanalysed": ([ctx, C.c_int64, C.c_int, C.c_int, C.c_int, f32p, i64p], C.c_int),
         "mz_learn_step_batch": ([ctx, C.c_int64, C.c_int, C.c_int] + [f32p] * 7, C.c_int),
         "mz_learn_gradients": ([ctx, C.c_int, C.c_int] + [f32p] * 8, C.c_int),
         "mz_optimizer_reset": ([ctx], C.c_int),
@@ -495,6 +496,14 @@ class Context:
         losses = np.zeros(3, np.float32)
         self._ck(self.L.mz_learn_steps(self._h, t0, n, grad_mode, _p(losses, C.c_float)))
         return losses
+
+    def learn_steps_reanalysed(self, t0, n, grad_mode=GRAD_REFERENCE_L2, exploration=False):
+        """learn_steps with fresh targets: before each step t, every distinct game of get_batch(t) is reanalysed whole with the current
+        networks (reanalyse_search on its key), then the step trains on the refreshed batch.  Returns (losses of the last step,
+        simulations run)."""
+        losses = np.zeros(3, np.float32); sims = C.c_int64()
+        self._ck(self.L.mz_learn_steps_reanalysed(self._h, t0, n, grad_mode, int(exploration), _p(losses, C.c_float), C.byref(sims)))
+        return losses, sims.value
 
     def checkpoint(self):
         """Everything needed to resume: weights, ADAM moments + step count, and the replay buffer's histories."""

@@ -116,6 +116,7 @@ struct mz_ctx {
     int64_t *h_counters = nullptr; double *h_lossout = nullptr; unsigned long long *h_stats = nullptr;   // pinned
     int64_t *h_wave = nullptr, *d_wave = nullptr; cudaEvent_t ev_wave[2] = {nullptr, nullptr};   // pinned: two snapshots of the counters, self-play runs one iteration ahead of the host
     dev_buf scratch[12];
+    dev_buf ra_roots, ra_counts;   // mz_learn_steps_reanalysed: the device-built root list, per-launch root counts + the simulation tally
     int64_t adam_t = 1; double bp1 = 0.9, bp2 = 0.999;   // Flux.ADAM: the next update's step number and beta powers (adam_seek)
     ncclComm_t comm = nullptr; int rank = 0, nranks = 1;
     // net_type = MZ_NET_RESNET
@@ -391,11 +392,19 @@ void launch_loss(mz_ctx *c, int B) {
     } else { launch_scope ls(c, 3); mz_k_loss_reduce<<<7, 1024, 0, c->stream>>>(P, B, c->d_rowv, c->d_rowr, c->d_rowp, c->d_rowinvg, c->own.w, c->d_lossout); }
 }
 
-int launch_learn_forward(mz_ctx *c, int B, int grad_mode = MZ_GRAD_REFERENCE_L2) {
-    const mz_params &P = c->M.P;
+// whether this context can take a learner step of `grad_mode` (the errors of launch_learn_forward, before it launches anything)
+int check_grad_mode(mz_ctx *c, int grad_mode) {
     const int path = learner_path(c, grad_mode);
     if (path == -1) return fail(c, MZ_E_UNSUPPORTED, "the ResNet learner implements MZ_GRAD_REFERENCE_L2 (the reference's update); the backward pass through the convolution towers is not built");
     if (path != 3 && grad_mode != MZ_GRAD_REFERENCE_L2 && grad_mode != MZ_GRAD_BPTT) return fail(c, MZ_E_ARG, "unknown grad_mode %d", grad_mode);
+    if (path == 0 && grad_mode == MZ_GRAD_BPTT && !c->smem_bytes_bptt) return fail(c, MZ_E_UNSUPPORTED, "MZ_GRAD_BPTT is not built for this network: it needs every layer output and every layer input other than the observation stack to be at most 64 wide, and its buffers to fit one CTA's shared memory");
+    return MZ_OK;
+}
+
+int launch_learn_forward(mz_ctx *c, int B, int grad_mode = MZ_GRAD_REFERENCE_L2) {
+    const mz_params &P = c->M.P;
+    MZ_TRY(check_grad_mode(c, grad_mode));
+    const int path = learner_path(c, grad_mode);
     mz_learn_args a{}; a.wglob = c->own.w; a.B = B; a.max_dim = c->M.max_dim; a.max_layer_floats = c->M.max_layer_floats; a.batch = c->batch;
     a.pred_values = c->d_pv; a.pred_rewards = c->d_pr; a.pred_policies = c->d_pp;
     const int tiles = (B + MZ_ROWS - 1) / MZ_ROWS;
@@ -426,7 +435,6 @@ int launch_learn_forward(mz_ctx *c, int B, int grad_mode = MZ_GRAD_REFERENCE_L2)
         if (c->cfg.use_batch_norm) { launch_scope ls(c, 4); mz_k_grad_reduce_bn<<<dim3((unsigned)P.n_layers, 16), 256, 0, c->stream>>>(P, chunks, gpart, c->own.w, grad_out(c)); }
         else { launch_scope ls(c, 4); mz_k_grad_reduce<<<(P.total_floats + 255) / 256, 256, 0, c->stream>>>(P.total_floats, chunks, gpart, c->own.w, grad_out(c)); }
     } else if (grad_mode == MZ_GRAD_BPTT) {   // forward + backward through the unroll in one kernel; per-tile partial gradients
-        if (!c->smem_bytes_bptt) return fail(c, MZ_E_UNSUPPORTED, "MZ_GRAD_BPTT is not built for this network: it needs every layer output and every layer input other than the observation stack to be at most 64 wide, and its buffers to fit one CTA's shared memory");
         float *act, *gpart;
         MZ_TRY(h2d<float>(c, c->bptt_act, nullptr, (size_t)tiles * c->bptt.plan.tile_floats, &act));
         MZ_TRY(h2d<float>(c, c->bptt_gpart, nullptr, (size_t)tiles * P.total_floats, &gpart));
@@ -761,7 +769,7 @@ int mz_destroy(mz_ctx *c) {
     for (void *p : ptrs) if (p) cudaFree(p);
     for (auto &b : c->scratch) b.release();
     for (auto &b : c->rn_buf) b.release();
-    for (dev_buf *b : {&c->bptt_act, &c->bptt_gpart, &c->lr_xsave, &c->lr_dzsave, &c->lr_gpart}) b->release();
+    for (dev_buf *b : {&c->bptt_act, &c->bptt_gpart, &c->lr_xsave, &c->lr_dzsave, &c->lr_gpart, &c->ra_roots, &c->ra_counts}) b->release();
     free_ring(c->ring);
     free_ring(c->play_ring);
     if (c->h_lat_stage) cudaFreeHost(c->h_lat_stage);
@@ -1618,6 +1626,63 @@ int mz_learn_steps(mz_ctx *c, int64_t t0, int n, int grad_mode, float *losses) {
         MZ_TRY(launch_per_update(c, B));
     }
     return finish_losses(c, B, losses);
+}
+// n learning! iterations t0 .. t0+n-1 with fresh targets (MuZero Reanalyze on the batch): before step t's loss, every distinct game of
+// get_batch(step = t) is reanalysed whole with the weights as step t-1 left them, then the batch is gathered again from the refreshed ring
+// and the step proceeds as mz_learn_step(t).  Bit for bit the composition get_batch(t) -> mz_reanalyse_search(k, 1) for each distinct key
+// k -> mz_learn_step(t), without its host round trips: the root list is built on the device (mz_k_batch_roots) and the replay searches
+// are launched for the upper bound min(B, stored games) x Tmax roots, in chunks of num_slots (the tree pool's capacity), each reading its
+// real root count from the device (mz_search_args::replay_n; the CTAs past it idle).  The second gather draws the same indices as the
+// first: sampling depends on the step, the ring counters and the priorities, and reanalysis changes none of them.  The ResNet path
+// packs its weight image on the host after every update (rn_sync_image): one round trip per step there.
+int mz_learn_steps_reanalysed(mz_ctx *c, int64_t t0, int n, int grad_mode, int exploration, float *losses, int64_t *simulations) {
+    MZ_CHECK_CTX(c);
+    if (simulations) *simulations = 0;
+    if (!losses || t0 < 1 || n < 1) return fail(c, MZ_E_ARG, "bad arguments");
+    const int B = c->cfg.batch_size;
+    MZ_TRY(read_counters(c));
+    if (c->h_counters[0] < 1) return fail(c, MZ_E_STATE, "replay buffer is empty (learning! waits for num_played_games >= 1, Learning.jl:311)");
+    if (c->h_counters[5] != 0) return fail(c, MZ_E_STATE, "self-play in progress");
+    MZ_TRY(check_grad_mode(c, grad_mode));
+    const mz_params &P = c->M.P;
+    const int64_t played = c->h_counters[0], have = played < c->ring.capacity ? played : c->ring.capacity;
+    const int64_t bound = (B < have ? B : have) * (int64_t)P.Tmax, chunk = c->cfg.num_slots, n_chunks = (bound + chunk - 1) / chunk;
+    int Bp = 1;
+    while (Bp < B) Bp <<= 1;
+    const size_t smem = 2 * (size_t)Bp * sizeof(int32_t);
+    int smem_max = 0;
+    MZ_CUDA(c, cudaDeviceGetAttribute(&smem_max, cudaDevAttrMaxSharedMemoryPerBlockOptin, c->device));
+    if (smem > (size_t)smem_max) return fail(c, MZ_E_UNSUPPORTED, "batch_size %d: the batch's root list is built in %zu B of shared memory, the device allows %d", B, smem, smem_max);
+    MZ_CUDA(c, cudaFuncSetAttribute(mz_k_batch_roots, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    MZ_TRY(alloc_batch(c, B));
+    int64_t *roots; int32_t *counts;
+    MZ_TRY(h2d<int64_t>(c, c->ra_roots, nullptr, (size_t)bound, &roots));
+    MZ_TRY(h2d<int32_t>(c, c->ra_counts, nullptr, (size_t)n_chunks + 4, &counts));
+    unsigned long long *tally = (unsigned long long *)(counts + ((n_chunks + 1) & ~(int64_t)1));   // 8-byte aligned, after the counts
+    MZ_CUDA(c, cudaMemsetAsync(tally, 0, sizeof(unsigned long long), c->stream));
+    for (int i = 0; i < n; i++) {
+        const int64_t t = t0 + i;
+        MZ_TRY(launch_gather(c, (uint64_t)t, B));
+        MZ_TRY(ensure_images(c));   // stale after step t-1's update (ResNet: packed on the host)
+        { launch_scope ls(c, 5); mz_k_batch_roots<<<1, 1024, smem, c->stream>>>(P, c->ring, c->batch.index, B, Bp, (int)chunk, (int)n_chunks, roots, counts, tally); }
+        MZ_CUDA(c, cudaGetLastError());
+        for (int64_t k = 0; k < n_chunks; k++) {
+            const int64_t off = k * chunk;
+            mz_search_args a = search_args(c, (int)(bound - off < chunk ? bound - off : chunk), exploration);
+            a.ring = c->ring; a.replay = roots + off; a.replay_n = counts + k;
+            launch_search<MZ_MODE_REPLAY>(c, P, a, 0);
+            MZ_CUDA(c, cudaGetLastError());
+        }
+        MZ_TRY(launch_gather(c, (uint64_t)t, B));   // the same indices, the refreshed targets (and for PER the same importance weights)
+        MZ_TRY(launch_learn_forward(c, B, grad_mode));
+        MZ_TRY(launch_update(c, t, grad_mode));
+        MZ_TRY(launch_per_update(c, B));
+    }
+    unsigned long long roots_run = 0;
+    MZ_CUDA(c, cudaMemcpyAsync(&roots_run, tally, sizeof(roots_run), cudaMemcpyDeviceToHost, c->stream));
+    MZ_TRY(finish_losses(c, B, losses));   // synchronises the stream
+    if (simulations) *simulations = (int64_t)roots_run * P.S;
+    return MZ_OK;
 }
 // ---- checkpoint / resume of the optimiser (weights: mz_get_weights / mz_set_weights; histories: mz_history_export / import) ----
 // Flux.ADAM keeps (mt, vt, beta powers) per parameter array (Learning.jl:318, 395-397); m and v cross the ABI in the blob order.

@@ -68,6 +68,9 @@ struct mz_search_args {
     // MODE_REPLAY: root i is position t of the game at ring position pos, replay[i] = pos * Tmax + t (the index of its [R][Tmax] entries).
     // Last, so that the fields the other modes read keep their offsets.
     mz_ring ring; const int64_t *replay;
+    // MODE_REPLAY: the number of roots of this launch when only the device knows it (mz_k_batch_roots writes it); roots *replay_n .. n-1
+    // are inactive and a CTA holding none of its roots idles.  NULL: all n roots are real.
+    const int32_t *replay_n;
 };
 
 // ---- lane-parallel tree operations: MZ_LANES (8) lanes of a warp cooperate on one tree.  They are the GPU-only
@@ -229,7 +232,7 @@ struct mz_root { bool active; uint32_t legal, game, move, posmask; };
 // root g: MODE_API from the caller's arrays, MODE_SLOTS from the slot's board (SelfPlay.jl:351,359); in competitive play a slot is searched
 // only on MuZero's plies.  MODE_REPLAY: stored position t of a ring game, with the root self-play searched there (board before move t,
 // its side to move, game id, move index t + 1).  valid = false (no root g for this thread: g >= a.n, or not a tree lane) gives an inactive
-// root with no legal action.
+// root with no legal action, as does a replay root past the launch's device-held count.
 template <int MODE>
 __device__ __forceinline__ mz_root mz_root_begin(const mz_params &P, const mz_search_args &a, int64_t g, bool valid) {
     mz_root R; R.active = false; R.legal = 0; R.game = 0; R.move = 0; R.posmask = 0;
@@ -237,7 +240,7 @@ __device__ __forceinline__ mz_root mz_root_begin(const mz_params &P, const mz_se
         if (valid) { R.legal = a.legal[g]; R.game = (uint32_t)a.game_id[g]; R.move = (uint32_t)a.move_idx[g]; }
         R.active = R.legal != 0;   // run_mcts asserts !isempty(legal_actions) (SelfPlay.jl:243)
     } else if (MODE == MZ_MODE_REPLAY) {
-        if (valid) {
+        if (valid && (!a.replay_n || g < *a.replay_n)) {
             const int64_t e = a.replay[g], pos = e / P.Tmax;
             mz_board b; b.p1 = a.ring.h_p1[e]; b.p2 = a.ring.h_p2[e]; b.player = a.ring.h_to_play[e];
             R.legal = mz_env_legal_b(P, b); R.game = (uint32_t)a.ring.game_id[pos]; R.move = (uint32_t)(e - pos * P.Tmax) + 1u;
@@ -261,6 +264,7 @@ __device__ __forceinline__ float mz_root_obs(const mz_params &P, const mz_search
     if (gg >= a.n) return 0.0f;
     if (MODE == MZ_MODE_API) return a.stacked[gg * P.stack_size + k];
     if (MODE == MZ_MODE_REPLAY) {
+        if (a.replay_n && gg >= *a.replay_n) return 0.0f;
         const int64_t e = a.replay[gg], pos = e / P.Tmax, row = pos * P.Tmax;
         return mz_stacked_value(P, a.ring.h_p1 + row, a.ring.h_p2 + row, a.ring.h_action + row, (int)(e - row) + 1, k);
     }
@@ -310,9 +314,11 @@ __device__ __forceinline__ void mz_root_finish(const mz_params &P, const mz_sear
 
 // Self-play launches run one iteration ahead of the host (run_wave, mz_api.cu): a CTA none of whose slots has a ply to search -- every
 // CTA of the iteration queued past the end of a wave -- returns at its first instruction, before any barrier, TMA or TMEM state exists.
-// MODE_API and MODE_REPLAY launches cover exactly their roots (the replay root list is dense): no CTA is idle.
+// MODE_API launches cover exactly their roots, and so do MODE_REPLAY launches with a host-known count (the replay root list is dense).
+// A MODE_REPLAY launch sized for an upper bound (a.replay_n set: mz_learn_steps_reanalysed) idles the CTAs past the device-held count.
 template <int MODE>
 __device__ __forceinline__ bool mz_cta_idle(const mz_params &P, const mz_search_args &a, int rows_per_cta) {
+    if (MODE == MZ_MODE_REPLAY) return a.replay_n && (int64_t)blockIdx.x * rows_per_cta >= *a.replay_n;
     if (MODE != MZ_MODE_SLOTS) return false;
     int any = 0;
     const int64_t g = (int64_t)blockIdx.x * rows_per_cta + threadIdx.x;

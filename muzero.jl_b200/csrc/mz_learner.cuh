@@ -84,6 +84,91 @@ __global__ void __launch_bounds__(1024) mz_k_per_normalise(int B, float *w) {
     for (int i = tid; i < B; i += 1024) w[i] = w[i] / mx;
 }
 
+// exclusive prefix sum of v over the 1024 threads of the CTA; *total = the sum of all.  buf: 32 ints of shared memory.
+__device__ __forceinline__ int mz_block_exscan(int v, int *buf, int *total) {
+    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+    int x = v;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) { const int y = __shfl_up_sync(0xffffffffu, x, o); if (lane >= o) x += y; }
+    if (lane == 31) buf[w] = x;
+    __syncthreads();
+    if (w == 0) {
+        int s = buf[lane];
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) { const int y = __shfl_up_sync(0xffffffffu, s, o); if (lane >= o) s += y; }
+        buf[lane] = s;
+    }
+    __syncthreads();
+    const int excl = x - v + (w ? buf[w - 1] : 0);
+    *total = buf[31];
+    __syncthreads();   // buf is reused by the next call
+    return excl;
+}
+
+// mz_learn_steps_reanalysed: the replay root list of the batch just gathered (out.index), built on the device so that the step's search
+// needs no host round trip.  Every distinct game of the batch is reanalysed whole, as mz_reanalyse_search(key, 1) does it:
+//  1. the batch's keys are sorted (bitonic, in shared memory: keys[Bp], Bp = B rounded up to a power of 2) and de-duplicated;
+//  2. each distinct game gets mz_k_reanalyse_mark's writes (reanalysed values of positions t >= T are 0, the "is set" flag raised);
+//  3. the dense root list (pos * Tmax + t, t < T) is written ordered by move t, then by key -- mz_reanalyse_search's order, which keeps
+//     the trees of a CTA at one ply: per t, a prefix count over the distinct games with T > t;
+//  4. counts[k] = the number of roots of search launch k (launches of `chunk` roots, n_chunks of them, sized for an upper bound), and
+//     *total accumulates the roots of the call (its simulations / S).
+// One CTA of 1024 threads; dynamic shared memory 2 * Bp ints.
+__global__ void __launch_bounds__(1024) mz_k_batch_roots(const __grid_constant__ mz_params P, mz_ring r, const int32_t *index, int B, int Bp,
+                                                          int chunk, int n_chunks, int64_t *roots, int32_t *counts, unsigned long long *total) {
+    extern __shared__ int32_t mz_smem_br[];
+    int32_t *keys = mz_smem_br, *uniq = mz_smem_br + Bp;
+    __shared__ int buf[32];
+    const int tid = threadIdx.x;
+    const int64_t played = r.counters[0], n_games = played < r.capacity ? played : r.capacity, first = played - n_games + 1;
+    for (int i = tid; i < Bp; i += 1024) keys[i] = i < B ? (int32_t)(index[2 * i] - first) : 0x7fffffff;   // key - first_key, padding last
+    __syncthreads();
+    for (int k = 2; k <= Bp; k <<= 1)
+        for (int j = k >> 1; j > 0; j >>= 1) {
+            for (int i = tid; i < Bp; i += 1024) {
+                const int l = i ^ j;
+                if (l > i) {
+                    const int32_t x = keys[i], y = keys[l];
+                    if ((x > y) == ((i & k) == 0)) { keys[i] = y; keys[l] = x; }
+                }
+            }
+            __syncthreads();
+        }
+    // de-duplicate: thread tid owns the contiguous items [i0, i1) of the sorted keys
+    const int per = (Bp + 1023) / 1024, i0 = tid * per < B ? tid * per : B, i1 = i0 + per < B ? i0 + per : B;
+    int c = 0;
+    for (int i = i0; i < i1; i++) c += (i == 0 || keys[i] != keys[i - 1]) ? 1 : 0;
+    int D;
+    int o = mz_block_exscan(c, buf, &D);
+    for (int i = i0; i < i1; i++) if (i == 0 || keys[i] != keys[i - 1]) uniq[o++] = keys[i];
+    __syncthreads();
+    for (int j = tid; j < D; j += 1024) {   // keys[] now holds the games' lengths; step 2
+        const int64_t pos = (first + uniq[j] - 1) % r.capacity;
+        const int T = r.T[pos];
+        keys[j] = T;
+        for (int t = T; t < P.Tmax; t++) r.h_rrv[pos * P.Tmax + t] = 0.0f;
+        r.reanalysed[pos] = 1;
+    }
+    __syncthreads();
+    const int perD = (D + 1023) / 1024, j0 = tid * perD < D ? tid * perD : D, j1 = j0 + perD < D ? j0 + perD : D;
+    int base = 0;
+    for (int t = 0; t < P.Tmax; t++) {   // step 3
+        int n = 0;
+        for (int j = j0; j < j1; j++) n += keys[j] > t ? 1 : 0;
+        int level;
+        int at = base + mz_block_exscan(n, buf, &level);
+        if (level == 0) break;           // lengths are at most Tmax: no game reaches a later move either
+        for (int j = j0; j < j1; j++)
+            if (keys[j] > t) roots[at++] = ((first + uniq[j] - 1) % r.capacity) * P.Tmax + t;
+        base += level;
+    }
+    for (int k = tid; k < n_chunks; k += 1024) {   // step 4
+        const int64_t left = (int64_t)base - (int64_t)k * chunk;
+        counts[k] = (int32_t)(left < 0 ? 0 : left < chunk ? left : chunk);
+    }
+    if (tid == 0) *total += (unsigned long long)base;
+}
+
 // K-step unroll forward for 32 samples per CTA (src/Learning.jl:347-370, Q19): row 0 = prediction(h0); for
 // i = 1..K: row i = prediction(h_{i-1}) evaluated BEFORE the dynamics step; rewards row 0 = 0.
 struct mz_learn_args { const float *wglob; int32_t B, max_dim, max_layer_floats, pad_; mz_batch batch; float *pred_values, *pred_rewards, *pred_policies; };

@@ -269,10 +269,18 @@ function reanalyse_search!(e::Engine, key0::Integer, n::Integer; exploration::Bo
     return sims[]
 end
 
-"`steps` iterations of get_batch -> unroll -> loss -> gradients -> ADAM(Cos schedule); returns the last three losses."
-function learning!(e::Engine, steps::Integer; grad_mode::Integer=0)
+"""`steps` iterations of get_batch -> unroll -> loss -> gradients -> ADAM(Cos schedule); returns the last three losses.
+`reanalyse=true`: before each step the games its batch samples are searched again with the current networks (MuZero Reanalyze,
+`exploration` as in `reanalyse_search!`), so the step trains on fresh targets."""
+function learning!(e::Engine, steps::Integer; grad_mode::Integer=0, reanalyse::Bool=false, exploration::Bool=false)
     losses = zeros(Float32, 3)
-    check(e, ccall((:mz_learn_steps, LIB), Cint, (Ptr{Cvoid}, Int64, Cint, Cint, Ptr{Float32}), e.ctx, e.training_step + 1, steps, grad_mode, losses))
+    if reanalyse
+        sims = Ref{Int64}(0)
+        check(e, ccall((:mz_learn_steps_reanalysed, LIB), Cint, (Ptr{Cvoid}, Int64, Cint, Cint, Cint, Ptr{Float32}, Ptr{Int64}),
+                       e.ctx, e.training_step + 1, steps, grad_mode, exploration ? 1 : 0, losses, sims))
+    else
+        check(e, ccall((:mz_learn_steps, LIB), Cint, (Ptr{Cvoid}, Int64, Cint, Cint, Ptr{Float32}), e.ctx, e.training_step + 1, steps, grad_mode, losses))
+    end
     e.training_step += steps
     return (l_representation=losses[1], l_prediction=losses[2], l_dynamics=losses[3])
 end
