@@ -63,10 +63,9 @@ struct nccl_api {
 
 extern "C" { static void p2p_teardown(mz_ctx *c); }
 
-// One set of network weights (store_floats floats in the parameter store's layout) and the images the search kernels read, each rebuilt
-// from w before its next use when version has moved past the image's (ensure_images, ensure_lat_image).  mz_ctx::own holds the context's
-// networks; mz_ctx::opp the opponent networks of MZ_OPP_NETWORK, allocated on the first mz_set_opponent_weights / mz_snapshot_opponent with
-// the images of the context's path only.
+// One set of network weights (store_floats floats in the parameter store's layout) and the images the search kernels read (wstore_alloc),
+// each rebuilt from w before its next use when version has moved past the image's (ensure_images, ensure_lat_image).  mz_ctx::own holds
+// the context's networks; mz_ctx::opp the opponent networks of MZ_OPP_NETWORK, allocated on first use.
 struct mz_wstore {
     float *w = nullptr; uint64_t version = 1, img_version = 0, lat_version = 0;
     unsigned char *tc = nullptr; float *tc_bias = nullptr;   // MZ_NN_BF16_TC: bf16 image and bias
@@ -227,14 +226,28 @@ int store_from_host(mz_ctx *c, float *d, const float *blob) {
     MZ_CUDA(c, cudaStreamSynchronize(c->stream));
     return MZ_OK;
 }
-int upload_weights(mz_ctx *c, const std::vector<float> &src) {
-    const int r = store_from_host(c, c->own.w, src.data());
-    c->own.version++;                                      // the images are rebuilt before their next use (ensure_images)
-    return r;
+// a weight store for this context: w, zeroed, and the images of the kernels this context can launch (mz_k_search_lat's wherever mz_run_mcts
+// and run_wave_body may take it).  On an error the store may be partly allocated: wstore_free releases it.
+cudaError_t wstore_alloc(const mz_ctx *c, mz_wstore &s) {
+#define MZ_WS(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) return e_; } while (0)
+    const mz_params &P = c->M.P; const int mode = c->cfg.nn_mode; const bool resnet = c->cfg.net_type == MZ_NET_RESNET;
+    MZ_WS(dmalloc(&s.w, (size_t)c->store_floats)); MZ_WS(cudaMemsetAsync(s.w, 0, (size_t)c->store_floats * sizeof(float), c->stream));
+    if (!resnet && mode == MZ_NN_BF16_TC) {
+        const size_t bytes = (size_t)P.tc_net_off[3] + 8192;
+        MZ_WS(cudaMalloc((void **)&s.tc, bytes)); MZ_WS(cudaMemsetAsync(s.tc, 0, bytes, c->stream)); MZ_WS(dmalloc(&s.tc_bias, (size_t)P.tc_bias_floats));
+    }
+    if (mode == MZ_NN_SPLIT_MMA) {
+        const size_t bytes = (size_t)c->spp.image_bytes + 256;
+        MZ_WS(cudaMalloc((void **)&s.sp, bytes)); MZ_WS(cudaMemsetAsync(s.sp, 0, bytes, c->stream)); MZ_WS(dmalloc(&s.sp_bias, (size_t)c->spp.bias_floats));
+    }
+    if (c->lat_ok && mode != MZ_NN_BF16_TC) MZ_WS(dmalloc(&s.lat, (size_t)c->lat_image_floats + 64));
+    if (resnet) MZ_WS(cudaMalloc((void **)&s.rn, (size_t)c->rn.image_bytes + 4096));
+#undef MZ_WS
+    return cudaSuccess;
 }
-int download_weights(mz_ctx *c, std::vector<float> &src) {
-    src.resize((size_t)c->M.P.n_params);
-    return store_to_host(c, c->own.w, src.data());
+void wstore_free(mz_wstore &s) {
+    for (void *p : {(void *)s.w, (void *)s.tc, (void *)s.tc_bias, (void *)s.sp, (void *)s.sp_bias, (void *)s.lat, (void *)s.rn}) if (p) cudaFree(p);
+    s = mz_wstore{};
 }
 
 int read_counters(mz_ctx *c) {
@@ -272,6 +285,27 @@ template <typename T> int alloc_zeroed(mz_ctx *c, dev_buf &b, size_t n, T **out)
     const size_t cap = b.cap;
     MZ_TRY(h2d<T>(c, b, nullptr, n, out));
     if (b.cap != cap) MZ_CUDA(c, cudaMemsetAsync(b.p, 0, b.cap, c->stream));
+    return MZ_OK;
+}
+// the arguments of every weight-blob call: net (MZ_NET_ALL or one network) and a blob of exactly that network's length
+int check_blob(mz_ctx *c, int net, const float *blob, int64_t n) {
+    if (net < 0 || net > 3 || !blob) return fail(c, MZ_E_ARG, "bad net id or NULL blob");
+    if (n != ctx_net_params(c, net)) return fail(c, MZ_E_ARG, "weight blob has %lld floats, net %d needs %d", (long long)n, net, ctx_net_params(c, net));
+    return MZ_OK;
+}
+// network `net` of store s from / to the caller's blob (arguments as check_blob accepts them); one network is merged into the rest of s
+int wstore_set(mz_ctx *c, mz_wstore &s, int net, const float *blob, int64_t n) {
+    std::vector<float> src((size_t)c->M.P.n_params);
+    if (net != MZ_NET_ALL) MZ_TRY(store_to_host(c, s.w, src.data()));
+    memcpy(src.data() + ctx_net_offset(c, net), blob, (size_t)n * sizeof(float));
+    const int r = store_from_host(c, s.w, src.data());
+    s.version++;                                           // the images are rebuilt before their next use (ensure_images)
+    return r;
+}
+int wstore_get(mz_ctx *c, const mz_wstore &s, int net, float *blob, int64_t n) {
+    std::vector<float> src((size_t)c->M.P.n_params);
+    MZ_TRY(store_to_host(c, s.w, src.data()));
+    memcpy(blob, src.data() + ctx_net_offset(c, net), (size_t)n * sizeof(float));
     return MZ_OK;
 }
 
@@ -330,6 +364,8 @@ int ensure_images(mz_ctx *c, mz_wstore &s) {
     return MZ_OK;
 }
 int ensure_images(mz_ctx *c) { return ensure_images(c, c->own); }
+// the split-precision kernels' arguments, reading the images of store s
+mz_sp_args sp_args(const mz_ctx *c, const mz_wstore &s) { mz_sp_args a = c->spa; a.image = s.sp; a.bias = s.sp_bias; return a; }
 
 // the weight image of mz_k_search_lat (rows = outputs), rebuilt from the store's weights when they have changed since it was last used
 int ensure_lat_image(mz_ctx *c, mz_wstore &s) {
@@ -348,11 +384,11 @@ int ensure_lat_image(mz_ctx *c, mz_wstore &s) {
 // The K-step unroll (Learning.jl:347-370) as a sequence of the batched network kernel mz_k_rn_forward on device buffers (bf16 inference
 // arithmetic, BatchNorm with its stored statistics: the reference computes the predictions outside the pullback, i.e. in test mode), then
 // the loss tail; the update is ADAM on 2 * theta over Flux.params (launch_update), after which the bf16 image is rebuilt (ensure_images).
-int rn_forward_dev(mz_ctx *c, int net, int B, const float *d_in, float *d_o1, float *d_o2, unsigned char *pool) {
-    mz_search_rn_args t{}; t.image = c->own.rn; t.steps = c->d_rn_steps; t.net = net; t.B = B; t.in = d_in; t.out1 = d_o1; t.out2 = d_o2; t.scratch_pool = pool;
+// rn_forward: one batched ResNet network on device buffers with the image of store s, a launch of kernel family `family`
+void rn_forward(mz_ctx *c, const mz_wstore &s, int family, int net, int B, const float *d_in, float *d_o1, float *d_o2, unsigned char *pool) {
+    mz_search_rn_args t{}; t.image = s.rn; t.steps = c->d_rn_steps; t.net = net; t.B = B; t.in = d_in; t.out1 = d_o1; t.out2 = d_o2; t.scratch_pool = pool;
     const int nt = c->rn.R.ntrees;
-    launch_scope ls(c, 3); mz_k_rn_forward<<<(B + nt - 1) / nt, MZ_RN_THREADS, c->smem_bytes_rn, c->stream>>>(c->M.P, c->rn.R, t);
-    return MZ_OK;
+    launch_scope ls(c, family); mz_k_rn_forward<<<(B + nt - 1) / nt, MZ_RN_THREADS, c->smem_bytes_rn, c->stream>>>(c->M.P, c->rn.R, t);
 }
 int rn_learn_forward(mz_ctx *c, int B) {
     const mz_params &P = c->M.P;
@@ -363,16 +399,16 @@ int rn_learn_forward(mz_ctx *c, int B) {
     MZ_TRY(h2d<float>(c, c->rn_buf[4], nullptr, (size_t)B * P.A, &o2)); MZ_TRY(h2d<float>(c, c->rn_buf[5], nullptr, (size_t)B, &r));
     MZ_TRY(h2d<unsigned char>(c, c->rn_buf[6], nullptr, (size_t)B * c->rn.R.node_bytes + 256, &pool));
     const int K1 = P.K + 1, tb = (B + 127) / 128;
-    MZ_TRY(rn_forward_dev(c, 0, B, c->batch.obs, h, nullptr, pool));                                      // :347
-    MZ_TRY(rn_forward_dev(c, 1, B, h, o1, o2, pool));                                                      // :351 (= row 1's prediction, Q19)
+    rn_forward(c, c->own, 3, 0, B, c->batch.obs, h, nullptr, pool);                                        // :347
+    rn_forward(c, c->own, 3, 1, B, h, o1, o2, pool);                                                       // :351 (= row 1's prediction, Q19)
     { launch_scope ls(c, 3); mz_k_rn_scatter<<<tb, 128, 0, c->stream>>>(B, P.A, K1, 0, P.K > 0 ? 1 : -1, o1, o2, nullptr, 1, c->d_pv, c->d_pp, c->d_pr); }
     for (int i = 1; i <= P.K; i++) {                                                                       // :355-370
         if (i > 1) {
-            MZ_TRY(rn_forward_dev(c, 1, B, h, o1, o2, pool));
+            rn_forward(c, c->own, 3, 1, B, h, o1, o2, pool);
             launch_scope ls(c, 3); mz_k_rn_scatter<<<tb, 128, 0, c->stream>>>(B, P.A, K1, i, -1, o1, o2, nullptr, 0, c->d_pv, c->d_pp, c->d_pr);
         }
         { launch_scope ls(c, 3); mz_k_rn_make_sa<<<(B * P.sa_size + 255) / 256, 256, 0, c->stream>>>(B, P.hidden, P.cells, P.A, K1, i - 1, h, c->batch.actions, sa); }
-        MZ_TRY(rn_forward_dev(c, 2, B, sa, nh, r, pool));
+        rn_forward(c, c->own, 3, 2, B, sa, nh, r, pool);
         { launch_scope ls(c, 3); mz_k_rn_scatter<<<tb, 128, 0, c->stream>>>(B, P.A, K1, i, -1, nullptr, nullptr, r, 0, c->d_pv, c->d_pp, c->d_pr); }
         float *t = h; h = nh; nh = t;
     }
@@ -418,7 +454,7 @@ int launch_learn_forward(mz_ctx *c, int B, int grad_mode = MZ_GRAD_REFERENCE_L2)
         unsigned char *xsave, *dzsave; float *gpart;
         MZ_TRY(alloc_zeroed(c, c->lr_xsave, bytes, &xsave)); MZ_TRY(alloc_zeroed(c, c->lr_dzsave, bytes, &dzsave));
         MZ_TRY(alloc_zeroed(c, c->lr_gpart, (size_t)chunks * P.total_floats, &gpart));
-        mz_lr_args t{}; t.sp = c->spa; t.sp.pbc_smem = 0; t.brounds = c->d_brounds;
+        mz_lr_args t{}; t.sp = sp_args(c, c->own); t.sp.pbc_smem = 0; t.brounds = c->d_brounds;
         for (int n = 0; n < 3; n++) {
             t.bfirst[n] = L.bfirst[n]; t.bn_rounds[n] = L.bn_rounds[n]; t.slot_base[n] = L.slot_base[n]; t.layers_in_net[n] = L.layers_in_net[n]; t.first_layer[n] = P.nets[n].first;
             for (int h = 0; h < 2; h++) { t.start_tile[n][h] = L.start_tile[n][h]; t.start_layer[n][h] = L.start_layer[n][h]; t.start_perm[n][h] = L.start_perm[n][h]; }
@@ -450,7 +486,7 @@ int launch_learn_forward(mz_ctx *c, int B, int grad_mode = MZ_GRAD_REFERENCE_L2)
         else { launch_scope ls(c, 4); mz_k_grad_reduce<<<(P.total_floats + 255) / 256, 256, 0, c->stream>>>(P.total_floats, tiles, gpart, c->own.w, grad_out(c)); }
     } else if (path == 1) {   // the unroll on the tensor cores (mz_kernels_sp.cuh)
         MZ_TRY(ensure_images(c));
-        mz_learn_sp_args t{}; t.sp = c->spa; t.B = B; t.batch = c->batch; t.pred_values = c->d_pv; t.pred_rewards = c->d_pr; t.pred_policies = c->d_pp;
+        mz_learn_sp_args t{}; t.sp = sp_args(c, c->own); t.B = B; t.batch = c->batch; t.pred_values = c->d_pv; t.pred_rewards = c->d_pr; t.pred_policies = c->d_pp;
         launch_scope ls(c, 3); mz_k_learn_forward_sp<<<tiles, MZ_SP_THREADS, c->smem_bytes_sp, c->stream>>>(P, t);
     } else {
         launch_scope ls(c, 3);
@@ -513,12 +549,11 @@ static mz_search_args search_args(const mz_ctx *c, int n, int exploration) {
     return a;
 }
 // One search over the roots of `a` (MODE_API: the caller's a.n roots; MODE_SLOTS: the a.n game slots; MODE_REPLAY: a.n stored positions)
-// in ONE launch of kernel family 0 (run_wave_body relabels those of an idle iteration), with the weights and images of store `ws` (NULL:
-// the context's own networks).  lat > 0: the low-latency kernel (mz_kernels_lat.cuh) on roots [0, lat), one 2-CTA cluster each; otherwise
-// the batched kernel of the context's networks.  MODE_REPLAY always takes the batched kernel: the latency kernel has no instantiation for it.
+// in ONE launch of kernel family 0 (run_wave_body relabels those of an idle iteration), with the weights and images of store s.  lat > 0:
+// the low-latency kernel (mz_kernels_lat.cuh) on roots [0, lat), one 2-CTA cluster each; otherwise the batched kernel of the context's
+// networks.  MODE_REPLAY always takes the batched kernel: the latency kernel has no instantiation for it.
 template <int MODE>
-static void launch_search(mz_ctx *c, const mz_params &P, const mz_search_args &args, int lat, const mz_wstore *ws = nullptr) {
-    const mz_wstore &s = ws ? *ws : c->own;
+static void launch_search(mz_ctx *c, const mz_params &P, const mz_search_args &args, int lat, const mz_wstore &s) {
     mz_search_args a = args; a.wglob = s.w;
     const unsigned ctas = (unsigned)((a.n + MZ_ROWS - 1) / MZ_ROWS);
     launch_scope ls(c, 0);
@@ -534,7 +569,7 @@ static void launch_search(mz_ctx *c, const mz_params &P, const mz_search_args &a
         const int nt = c->rn.R.ntrees;
         mz_k_search_rn<MODE><<<(a.n + nt - 1) / nt, MZ_RN_THREADS, c->smem_bytes_rn, c->stream>>>(P, c->rn.R, t);
     } else if (c->cfg.nn_mode == MZ_NN_SPLIT_MMA) {
-        mz_search_sp_args t{}; t.base = a; t.sp = c->spa; t.sp.image = s.sp; t.sp.bias = s.sp_bias;
+        mz_search_sp_args t{}; t.base = a; t.sp = sp_args(c, s);
         mz_k_search_sp<MODE><<<ctas, MZ_SP_SEARCH_THREADS, c->smem_bytes_sp, c->stream>>>(P, t);
     } else if (c->cfg.nn_mode == MZ_NN_BF16_TC) {
         mz_search_tc_args t{}; t.base = a; t.w_image = s.tc; t.bias = s.tc_bias;
@@ -592,7 +627,6 @@ int mz_create(const mz_config *cfg, int device, mz_ctx **out) {
         if (c->smem_bytes_rn + 1024 > (size_t)prop.sharedMemPerBlockOptin) { int r = fail(nullptr, MZ_E_UNSUPPORTED, "the ResNet search kernel needs %zu B of shared memory per CTA, device allows %zu", c->smem_bytes_rn, (size_t)prop.sharedMemPerBlockOptin); mz_destroy(c); return r; }
         MZ_CREATE(allow_max_smem(mz_k_search_rn<MZ_MODE_API>, prop)); MZ_CREATE(allow_max_smem(mz_k_search_rn<MZ_MODE_SLOTS>, prop)); MZ_CREATE(allow_max_smem(mz_k_rn_forward, prop));
         MZ_CREATE(allow_max_smem(mz_k_search_rn<MZ_MODE_REPLAY>, prop));
-        MZ_CREATE(cudaMalloc((void **)&c->own.rn, (size_t)c->rn.image_bytes + 4096));
         MZ_CREATE(dmalloc(&c->d_rn_steps, c->rn.steps.size() + 1));
         MZ_CREATE(cudaMemcpy(c->d_rn_steps, c->rn.steps.data(), c->rn.steps.size() * sizeof(mz_rn_step), cudaMemcpyHostToDevice));
     }
@@ -627,7 +661,7 @@ int mz_create(const mz_config *cfg, int device, mz_ctx **out) {
         c->lat_max_roots = cfg->nn_mode == MZ_NN_FP32_EXACT ? c->sm_count : c->sm_count / 2;
         c->lat_max_slots = 16;                                           // self-play: contexts built for one or a few games at a time (play_game)
         if (const char *el = getenv("MUZERO_B200_LAT")) c->lat_max_roots = c->lat_max_slots = atoi(el);   // measurement / test switch; 0 = off
-        if (c->lat_ok) { MZ_CREATE(allow_max_smem(mz_k_search_lat<MZ_MODE_API>, prop)); MZ_CREATE(allow_max_smem(mz_k_search_lat<MZ_MODE_SLOTS>, prop)); MZ_CREATE(dmalloc(&c->own.lat, (size_t)c->lat_image_floats + 64)); }
+        if (c->lat_ok) { MZ_CREATE(allow_max_smem(mz_k_search_lat<MZ_MODE_API>, prop)); MZ_CREATE(allow_max_smem(mz_k_search_lat<MZ_MODE_SLOTS>, prop)); }
     }
     if (!resnet) { if (const char *eb = mzh::build_bptt(P, c->bptt)) { int r = fail(nullptr, MZ_E_ARG, "%s", eb); mz_destroy(c); return r; } }
     bool bptt_fits = !resnet;
@@ -664,9 +698,6 @@ int mz_create(const mz_config *cfg, int device, mz_ctx **out) {
             MZ_CREATE(allow_max_smem(mz_k_search_tc<MZ_MODE_SLOTS>, prop));
             MZ_CREATE(allow_max_smem(mz_k_search_tc<MZ_MODE_REPLAY>, prop));
             MZ_CREATE(allow_max_smem(mz_k_nn_forward_tc, prop));
-            MZ_CREATE(cudaMalloc((void **)&c->own.tc, (size_t)P.tc_net_off[3] + 8192));
-            MZ_CREATE(cudaMemset(c->own.tc, 0, (size_t)P.tc_net_off[3] + 8192));
-            MZ_CREATE(dmalloc(&c->own.tc_bias, (size_t)P.tc_bias_floats));
         } else if (cfg->nn_mode == MZ_NN_BF16_TC) {
             int r = fail(nullptr, MZ_E_UNSUPPORTED, "MZ_NN_BF16_TC needs %zu B of shared memory per CTA, device allows %zu", c->smem_bytes_tc, (size_t)prop.sharedMemPerBlockOptin);
             mz_destroy(c); return r;
@@ -683,13 +714,10 @@ int mz_create(const mz_config *cfg, int device, mz_ctx **out) {
             MZ_CREATE(allow_max_smem(mz_k_search_sp<MZ_MODE_REPLAY>, prop));
             MZ_CREATE(allow_max_smem(mz_k_nn_forward_sp, prop));
             MZ_CREATE(allow_max_smem(mz_k_learn_forward_sp, prop));
-            MZ_CREATE(cudaMalloc((void **)&c->own.sp, (size_t)S.image_bytes + 256));
-            MZ_CREATE(cudaMemset(c->own.sp, 0, (size_t)S.image_bytes + 256));
-            MZ_CREATE(dmalloc(&c->own.sp_bias, (size_t)S.bias_floats));
             MZ_CREATE(cudaMalloc((void **)&c->d_rounds_sp, sizeof(mz_sp_round) * MZ_SP_MAX_ROUNDS));
             MZ_CREATE(cudaMemcpy(c->d_rounds_sp, S.round, sizeof(mz_sp_round) * MZ_SP_MAX_ROUNDS, cudaMemcpyHostToDevice));
-            mz_sp_args &A = c->spa;
-            A.image = c->own.sp; A.bias = c->own.sp_bias; A.rounds = c->d_rounds_sp;
+            mz_sp_args &A = c->spa;   // image and bias: sp_args, from a store
+            A.rounds = c->d_rounds_sp;
             for (int n = 0; n < 3; n++) { A.first[n] = S.first[n]; A.n_rounds[n] = S.n_rounds[n]; A.set_first[n] = S.set_first[n]; A.n_sets[n] = S.n_sets[n]; }
             A.total_rounds = S.total_rounds; A.total_sets = S.total_sets; A.warea_bytes = S.warea_bytes; A.bias_floats = S.bias_floats; A.pbc_smem = S.pbc_smem; A.tail = S.tail;
             // the learner's backward rounds on the same machinery
@@ -714,8 +742,9 @@ int mz_create(const mz_config *cfg, int device, mz_ctx **out) {
     c->packed = !resnet;
     c->store_floats = resnet ? P.n_params : P.total_floats;
     const size_t nf = (size_t)c->store_floats;
-    MZ_CREATE(dmalloc(&c->own.w, nf)); MZ_CREATE(dmalloc(&c->d_m, nf)); MZ_CREATE(dmalloc(&c->d_v, nf)); MZ_CREATE(dmalloc(&c->d_grad, nf));
-    MZ_CREATE(cudaMemset(c->own.w, 0, nf * 4)); MZ_CREATE(cudaMemset(c->d_m, 0, nf * 4)); MZ_CREATE(cudaMemset(c->d_v, 0, nf * 4));
+    MZ_CREATE(wstore_alloc(c, c->own));
+    MZ_CREATE(dmalloc(&c->d_m, nf)); MZ_CREATE(dmalloc(&c->d_v, nf)); MZ_CREATE(dmalloc(&c->d_grad, nf));
+    MZ_CREATE(cudaMemset(c->d_m, 0, nf * 4)); MZ_CREATE(cudaMemset(c->d_v, 0, nf * 4));
     if (resnet || cfg->use_batch_norm) {   // Flux.params of a BatchNorm are beta and gamma: the running statistics take no part in sum(abs2, theta), its gradient or ADAM
         std::vector<unsigned char> mask(nf + 16, 1);
         if (resnet) {
@@ -761,7 +790,8 @@ int mz_destroy(mz_ctx *c) {
     if (c->stream) cudaStreamSynchronize(c->stream);
     collect_timings(c);
     if (c->comm && g_nccl.CommDestroy) { p2p_teardown(c); g_nccl.CommDestroy(c->comm); }
-    void *ptrs[] = {c->opp.w, c->opp.tc, c->opp.tc_bias, c->opp.sp, c->opp.sp_bias, c->opp.lat, c->opp.rn, c->d_mask, c->d_w_fold, c->own.lat, c->d_brounds, c->own.sp, c->own.sp_bias, c->d_rounds_sp, c->own.rn, c->d_rn_steps, c->d_bstages[0], c->d_bstages[1], c->own.tc, c->own.tc_bias, c->own.w, c->d_m, c->d_v, c->d_grad, c->d_pbc0, c->d_sqrtN, c->d_trees, c->slots.p1, c->slots.p2, c->slots.player, c->slots.T,
+    wstore_free(c->own); wstore_free(c->opp);
+    void *ptrs[] = {c->d_mask, c->d_w_fold, c->d_brounds, c->d_rounds_sp, c->d_rn_steps, c->d_bstages[0], c->d_bstages[1], c->d_m, c->d_v, c->d_grad, c->d_pbc0, c->d_sqrtN, c->d_trees, c->slots.p1, c->slots.p2, c->slots.player, c->slots.T,
                     c->slots.status, c->slots.game_id, c->slots.fin_list, c->slots.h_p1, c->slots.h_p2, c->slots.h_action, c->slots.h_reward, c->slots.h_to_play,
                     c->slots.h_cv, c->slots.h_rv, c->d_stats, c->d_lossout, c->batch.index, c->batch.obs,
                     c->batch.actions, c->batch.values, c->batch.rewards, c->batch.policies, c->batch.gscale, c->batch.weights, c->d_pv, c->d_pr, c->d_pp,
@@ -811,54 +841,28 @@ int mz_init_weights(mz_ctx *c, uint64_t seed) {
     std::vector<float> src((size_t)c->M.P.n_params);
     if (c->cfg.net_type == MZ_NET_RESNET) mzh::rn_init_weights(c->rn, seed, src.data());
     else mzh::init_weights(c->M.P, seed, src.data());
-    return upload_weights(c, src);
+    return wstore_set(c, c->own, MZ_NET_ALL, src.data(), (int64_t)src.size());
 }
 int mz_set_weights(mz_ctx *c, int net, const float *blob, int64_t n) {
     MZ_CHECK_CTX(c);
-    if (net < 0 || net > 3 || !blob) return fail(c, MZ_E_ARG, "bad net id or NULL blob");
-    if (n != ctx_net_params(c, net)) return fail(c, MZ_E_ARG, "weight blob has %lld floats, net %d needs %d", (long long)n, net, ctx_net_params(c, net));
-    std::vector<float> src;
-    if (net == MZ_NET_ALL) src.assign(blob, blob + n);                    // whole model: nothing to merge with
-    else { MZ_TRY(download_weights(c, src)); memcpy(src.data() + ctx_net_offset(c, net), blob, (size_t)n * sizeof(float)); }
-    return upload_weights(c, src);
+    MZ_TRY(check_blob(c, net, blob, n));
+    return wstore_set(c, c->own, net, blob, n);
 }
-// the opponent store, with the images of the context's path only; on failure nothing is left half-allocated
+// the opponent store, allocated on first use; on failure nothing is left half-allocated
 static int alloc_opponent(mz_ctx *c) {
     if (c->opp.w) return MZ_OK;
-    const mz_params &P = c->M.P;
-    mz_wstore s;
-    cudaError_t e = dmalloc(&s.w, (size_t)c->store_floats);
-    if (e == cudaSuccess && c->cfg.nn_mode == MZ_NN_SPLIT_MMA && c->own.sp) {
-        e = cudaMalloc((void **)&s.sp, (size_t)c->spp.image_bytes + 256);
-        if (e == cudaSuccess) e = cudaMemsetAsync(s.sp, 0, (size_t)c->spp.image_bytes + 256, c->stream);
-        if (e == cudaSuccess) e = dmalloc(&s.sp_bias, (size_t)c->spp.bias_floats);
-    }
-    if (e == cudaSuccess && c->cfg.nn_mode == MZ_NN_BF16_TC && c->own.tc) {
-        e = cudaMalloc((void **)&s.tc, (size_t)P.tc_net_off[3] + 8192);
-        if (e == cudaSuccess) e = cudaMemsetAsync(s.tc, 0, (size_t)P.tc_net_off[3] + 8192, c->stream);
-        if (e == cudaSuccess) e = dmalloc(&s.tc_bias, (size_t)P.tc_bias_floats);
-    }
-    if (e == cudaSuccess && c->own.lat) e = dmalloc(&s.lat, (size_t)c->lat_image_floats + 64);
-    if (e == cudaSuccess && c->own.rn) e = cudaMalloc((void **)&s.rn, (size_t)c->rn.image_bytes + 4096);
-    if (e != cudaSuccess) {
-        for (void *p : {(void *)s.w, (void *)s.sp, (void *)s.sp_bias, (void *)s.tc, (void *)s.tc_bias, (void *)s.lat, (void *)s.rn}) if (p) cudaFree(p);
-        return fail(c, MZ_E_CUDA, "allocating the opponent networks: %s", cudaGetErrorString(e));
-    }
-    c->opp = s;
-    return MZ_OK;
+    const cudaError_t e = wstore_alloc(c, c->opp);
+    if (e == cudaSuccess) return MZ_OK;
+    wstore_free(c->opp);
+    return fail(c, MZ_E_CUDA, "allocating the opponent networks: %s", cudaGetErrorString(e));
 }
 int mz_set_opponent_weights(mz_ctx *c, int net, const float *blob, int64_t n) {
     MZ_CHECK_CTX(c);
-    if (net < 0 || net > 3 || !blob) return fail(c, MZ_E_ARG, "bad net id or NULL blob");
-    if (n != ctx_net_params(c, net)) return fail(c, MZ_E_ARG, "weight blob has %lld floats, net %d needs %d", (long long)n, net, ctx_net_params(c, net));
+    MZ_TRY(check_blob(c, net, blob, n));
     if (net != MZ_NET_ALL && !c->opp_full)
         return fail(c, MZ_E_STATE, "replacing one opponent network needs a full opponent set first (mz_set_opponent_weights with MZ_NET_ALL, or mz_snapshot_opponent)");
     MZ_TRY(alloc_opponent(c));
-    std::vector<float> src((size_t)c->M.P.n_params);
-    if (net == MZ_NET_ALL) memcpy(src.data(), blob, (size_t)n * sizeof(float));
-    else { MZ_TRY(store_to_host(c, c->opp.w, src.data())); memcpy(src.data() + ctx_net_offset(c, net), blob, (size_t)n * sizeof(float)); }
-    MZ_TRY(store_from_host(c, c->opp.w, src.data()));
-    c->opp.version++;
+    MZ_TRY(wstore_set(c, c->opp, net, blob, n));
     c->opp_full = true;
     return MZ_OK;
 }
@@ -872,12 +876,8 @@ int mz_snapshot_opponent(mz_ctx *c) {
 }
 int mz_get_weights(mz_ctx *c, int net, float *blob, int64_t n) {
     MZ_CHECK_CTX(c);
-    if (net < 0 || net > 3 || !blob) return fail(c, MZ_E_ARG, "bad net id or NULL blob");
-    if (n != ctx_net_params(c, net)) return fail(c, MZ_E_ARG, "weight blob has %lld floats, net %d needs %d", (long long)n, net, ctx_net_params(c, net));
-    std::vector<float> src;
-    MZ_TRY(download_weights(c, src));
-    memcpy(blob, src.data() + ctx_net_offset(c, net), (size_t)n * sizeof(float));
-    return MZ_OK;
+    MZ_TRY(check_blob(c, net, blob, n));
+    return wstore_get(c, c->own, net, blob, n);
 }
 
 // ---- batched network callables -------------------------------------------------------------------------
@@ -885,6 +885,7 @@ static int nn_forward(mz_ctx *c, int net, int B, const float *in, float *out1, s
     MZ_CHECK_CTX(c);
     if (B < 0 || (B > 0 && (!in || !out1))) return fail(c, MZ_E_ARG, "NULL buffer");
     if (B == 0) return MZ_OK;
+    const mz_wstore &s = c->own;   // the callables evaluate the context's networks
     MZ_TRY(ensure_images(c));
     const mz_params &P = c->M.P;
     const bool resnet = c->cfg.net_type == MZ_NET_RESNET;
@@ -893,18 +894,16 @@ static int nn_forward(mz_ctx *c, int net, int B, const float *in, float *out1, s
     MZ_TRY(h2d(c, c->scratch[0], in, (size_t)B * in_dim, &d_in));
     MZ_TRY(h2d<float>(c, c->scratch[1], nullptr, (size_t)B * n1, &d_o1));
     MZ_TRY(h2d<float>(c, c->scratch[2], nullptr, (size_t)B * (n2 ? n2 : 1), &d_o2));
-    mz_nn_args a{}; a.wglob = c->own.w; a.B = B; a.max_dim = c->M.max_dim; a.max_layer_floats = c->M.max_layer_floats; a.net = net; a.in = d_in; a.out1 = d_o1; a.out2 = d_o2;
+    mz_nn_args a{}; a.wglob = s.w; a.B = B; a.max_dim = c->M.max_dim; a.max_layer_floats = c->M.max_layer_floats; a.net = net; a.in = d_in; a.out1 = d_o1; a.out2 = d_o2;
     if (resnet) {
         unsigned char *d_pool;
         MZ_TRY(h2d<unsigned char>(c, c->scratch[3], nullptr, (size_t)B * c->rn.R.node_bytes, &d_pool));
-        mz_search_rn_args t{}; t.image = c->own.rn; t.steps = c->d_rn_steps; t.net = net; t.B = B; t.in = d_in; t.out1 = d_o1; t.out2 = d_o2; t.scratch_pool = d_pool;
-        const int nt = c->rn.R.ntrees;
-        launch_scope ls(c, 5); mz_k_rn_forward<<<(B + nt - 1) / nt, MZ_RN_THREADS, c->smem_bytes_rn, c->stream>>>(P, c->rn.R, t);
+        rn_forward(c, s, 5, net, B, d_in, d_o1, d_o2, d_pool);
     } else if (c->cfg.nn_mode == MZ_NN_SPLIT_MMA) {
-        mz_nn_sp_args t{}; t.sp = c->spa; t.B = B; t.net = net; t.in = d_in; t.out1 = d_o1; t.out2 = d_o2;
+        mz_nn_sp_args t{}; t.sp = sp_args(c, s); t.B = B; t.net = net; t.in = d_in; t.out1 = d_o1; t.out2 = d_o2;
         launch_scope ls(c, 5); mz_k_nn_forward_sp<<<(B + MZ_ROWS - 1) / MZ_ROWS, MZ_SP_THREADS, c->smem_bytes_sp, c->stream>>>(P, t);
     } else if (c->cfg.nn_mode == MZ_NN_BF16_TC) {
-        mz_nn_tc_args t{}; t.w_image = c->own.tc; t.bias = c->own.tc_bias; t.B = B; t.net = net; t.in = d_in; t.out1 = d_o1; t.out2 = d_o2;
+        mz_nn_tc_args t{}; t.w_image = s.tc; t.bias = s.tc_bias; t.B = B; t.net = net; t.in = d_in; t.out1 = d_o1; t.out2 = d_o2;
         launch_scope ls(c, 5); mz_k_nn_forward_tc<<<(B + MZ_ROWS - 1) / MZ_ROWS, MZ_THREADS, c->smem_bytes_tc, c->stream>>>(P, t);
     } else if (c->cfg.use_batch_norm) { launch_scope ls(c, 5); mz_k_nn_forward<true><<<(B + MZ_ROWS - 1) / MZ_ROWS, MZ_THREADS, c->smem_bytes, c->stream>>>(P, a); }
     else { launch_scope ls(c, 5); mz_k_nn_forward<false><<<(B + MZ_ROWS - 1) / MZ_ROWS, MZ_THREADS, c->smem_bytes, c->stream>>>(P, a); }
@@ -1011,7 +1010,7 @@ int mz_run_mcts(mz_ctx *c, int n, const float *stacked_obs, const uint32_t *lega
         mz_search_args a = search_args(c, n, exploration);
         a.stacked = (const float *)(d + o_st); a.legal = (const uint32_t *)(d + o_legal); a.game_id = (const uint64_t *)(d + o_gid); a.move_idx = (const int32_t *)(d + o_mv);
         a.visit_counts = (int32_t *)(d + o_vc); a.root_value = (float *)(d + o_rv); a.root_priors = (float *)(d + o_pri);
-        launch_search<MZ_MODE_API>(c, P, a, n);
+        launch_search<MZ_MODE_API>(c, P, a, n, c->own);
         MZ_CUDA(c, cudaGetLastError());
         MZ_CUDA(c, cudaMemcpyAsync(h + o_vc, d + o_vc, total - o_vc, cudaMemcpyDeviceToHost, c->stream));
         MZ_CUDA(c, cudaStreamSynchronize(c->stream));
@@ -1033,7 +1032,7 @@ int mz_run_mcts(mz_ctx *c, int n, const float *stacked_obs, const uint32_t *lega
         MZ_TRY(h2d<float>(c, c->scratch[7], nullptr, (size_t)m * P.A, &d_pri));
         mz_search_args a = search_args(c, m, exploration);
         a.stacked = d_st; a.legal = d_legal; a.game_id = d_gid; a.move_idx = d_mv; a.visit_counts = d_vc; a.root_value = d_rv; a.root_priors = d_pri;
-        launch_search<MZ_MODE_API>(c, P, a, 0);
+        launch_search<MZ_MODE_API>(c, P, a, 0, c->own);
         MZ_CUDA(c, cudaGetLastError());
         MZ_TRY(d2h(c, visit_counts + (size_t)off * P.A, d_vc, (size_t)m * P.A)); MZ_TRY(d2h(c, root_value + off, d_rv, (size_t)m));
         if (root_priors) MZ_TRY(d2h(c, root_priors + (size_t)off * P.A, d_pri, (size_t)m * P.A));
@@ -1160,7 +1159,7 @@ static int run_wave_body(mz_ctx *c, uint64_t first_game, int64_t n_games, float 
     // the end, in slot order (= game id order).  MUZERO_B200_PERSIST=0 keeps one launch per move.
     if (overlap && !use_lat && arena_player == 0 && c->cfg.net_type == MZ_NET_FEEDFORWARD && c->cfg.nn_mode == MZ_NN_SPLIT_MMA && c->persist_ok) {
         mz_search_args ap = a; ap.persist = 1;
-        launch_search<MZ_MODE_SLOTS>(c, P, ap, 0);
+        launch_search<MZ_MODE_SLOTS>(c, P, ap, 0, c->own);
         MZ_TRY(launch_save_refill(c, P, G, tally, c->d_wave + 8));
         MZ_CUDA(c, cudaGetLastError());
         MZ_CUDA(c, cudaMemcpyAsync(c->h_stats, c->d_stats, 64 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, c->stream));
@@ -1179,9 +1178,9 @@ static int run_wave_body(mz_ctx *c, uint64_t first_game, int64_t n_games, float 
         const size_t iter_entry = c->timed.size();
         if (vs_net) {   // the opponent's plies: slots whose side to move is the other one, then MuZero's below (a game may make both)
             mz_params Po = P; Po.arena_player = 3 - arena_player;
-            launch_search<MZ_MODE_SLOTS>(c, Po, a, use_lat ? G_lat : 0, &c->opp);
+            launch_search<MZ_MODE_SLOTS>(c, Po, a, use_lat ? G_lat : 0, c->opp);
         } else if (arena_player != 0) { launch_scope ls(c, 6); mz_k_opponent_move<<<(G + 127) / 128, 128, 0, c->stream>>>(P, c->slots, G); }
-        launch_search<MZ_MODE_SLOTS>(c, P, a, use_lat ? G_lat : 0);   // few games (play_game one game at a time): one tree per cluster, exact fp32
+        launch_search<MZ_MODE_SLOTS>(c, P, a, use_lat ? G_lat : 0, c->own);   // few games (play_game one game at a time): one tree per cluster, exact fp32
         const size_t search_entry = c->timed.size();                       // (timing builds) index just past this iteration's search launch
         if (overlap) { MZ_CUDA(c, cudaEventRecord(c->ev_search[k & 1], c->stream)); MZ_CUDA(c, cudaStreamWaitEvent(sB, c->ev_search[k & 1], 0)); }
         MZ_TRY(launch_save_refill(c, P, G, tally, c->d_wave + 8 * ((k + 1) & 1), sB));
@@ -1403,7 +1402,7 @@ int mz_reanalyse_search(mz_ctx *c, int64_t key0, int n, int exploration, int64_t
     for (int64_t off = 0; off < total; off += chunk) {
         mz_search_args a = search_args(c, (int)(total - off < chunk ? total - off : chunk), exploration);
         a.ring = c->ring; a.replay = d_roots + off;   // a.stats stays NULL: mz_search_stats describes self-play
-        launch_search<MZ_MODE_REPLAY>(c, P, a, 0);
+        launch_search<MZ_MODE_REPLAY>(c, P, a, 0, c->own);
         MZ_CUDA(c, cudaGetLastError());
     }
     MZ_CUDA(c, cudaStreamSynchronize(c->stream));
@@ -1670,7 +1669,7 @@ int mz_learn_steps_reanalysed(mz_ctx *c, int64_t t0, int n, int grad_mode, int e
             const int64_t off = k * chunk;
             mz_search_args a = search_args(c, (int)(bound - off < chunk ? bound - off : chunk), exploration);
             a.ring = c->ring; a.replay = roots + off; a.replay_n = counts + k;
-            launch_search<MZ_MODE_REPLAY>(c, P, a, 0);
+            launch_search<MZ_MODE_REPLAY>(c, P, a, 0, c->own);
             MZ_CUDA(c, cudaGetLastError());
         }
         MZ_TRY(launch_gather(c, (uint64_t)t, B));   // the same indices, the refreshed targets (and for PER the same importance weights)
