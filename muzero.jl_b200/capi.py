@@ -362,6 +362,14 @@ class Context:
         self._ck(self.L.mz_replay_info(self._h, C.byref(n), C.byref(k), C.byref(t)))
         return dict(n_games=n.value, first_key=k.value, total_samples=t.value)
 
+    def _stored_keys(self, key0, n):
+        """(key0, n) of a key range, the missing ones from the replay buffer: key0 its first stored key, n up to its last."""
+        if key0 is None or n is None:
+            info = self.replay_info()
+            key0 = info["first_key"] if key0 is None else key0
+            n = info["n_games"] - (key0 - info["first_key"]) if n is None else n
+        return key0, n
+
     def replay_clear(self):
         self._ck(self.L.mz_replay_clear(self._h))
 
@@ -386,10 +394,7 @@ class Context:
         return {k: np.zeros(shp, dt) for k, (shp, dt) in shapes.items()}
 
     def history_export(self, key0=None, n=None, out=None):
-        if key0 is None or n is None:
-            info = self.replay_info()
-            key0 = info["first_key"] if key0 is None else key0
-            n = info["n_games"] - (key0 - info["first_key"]) if n is None else n
+        key0, n = self._stored_keys(key0, n)
         if out is None:
             out = self.history_buffers(n)
         self._ck(self.L.mz_history_export(self._h, key0, n, _p(out["game_id"], C.c_int64), _p(out["T"], C.c_int32), _p(out["obs"], C.c_float),
@@ -428,34 +433,26 @@ class Context:
         return out
 
     def replay_priorities(self, key0=None, n=None):
-        info = self.replay_info()
-        key0 = info["first_key"] if key0 is None else key0
-        n = info["n_games"] - (key0 - info["first_key"]) if n is None else n
+        key0, n = self._stored_keys(key0, n)
         q_pos = np.zeros((n, self.s["Tmax"]), np.uint32); q_game = np.zeros(n, np.uint32)
         self._ck(self.L.mz_replay_priorities(self._h, key0, n, _p(q_pos, C.c_uint32), _p(q_game, C.c_uint32)))
         return q_pos, q_game
 
     def reanalyse(self, key0=None, n=None):
         """reanalysed_predicted_root_values of games key0 .. key0+n-1 (default: the whole buffer) from the current networks."""
-        info = self.replay_info()
-        key0 = info["first_key"] if key0 is None else key0
-        n = info["n_games"] - (key0 - info["first_key"]) if n is None else n
+        key0, n = self._stored_keys(key0, n)
         self._ck(self.L.mz_reanalyse(self._h, key0, n))
 
     def reanalyse_search(self, key0=None, n=None, exploration=False):
         """MuZero Reanalyze for games key0 .. key0+n-1 (default: the whole buffer): the search again at every stored position with the
         current networks; refreshes child_visits and the reanalysed root values.  Returns the number of simulations run."""
-        info = self.replay_info()
-        key0 = info["first_key"] if key0 is None else key0
-        n = info["n_games"] - (key0 - info["first_key"]) if n is None else n
+        key0, n = self._stored_keys(key0, n)
         sims = C.c_int64()
         self._ck(self.L.mz_reanalyse_search(self._h, key0, n, int(exploration), C.byref(sims)))
         return sims.value
 
     def reanalysed_export(self, key0=None, n=None):
-        info = self.replay_info()
-        key0 = info["first_key"] if key0 is None else key0
-        n = info["n_games"] - (key0 - info["first_key"]) if n is None else n
+        key0, n = self._stored_keys(key0, n)
         values = np.zeros((n, self.s["Tmax"]), np.float32); flags = np.zeros(n, np.int32)
         self._ck(self.L.mz_reanalysed_export(self._h, key0, n, _p(values, C.c_float), _p(flags, C.c_int32)))
         return values, flags

@@ -250,14 +250,36 @@ void wstore_free(mz_wstore &s) {
     s = mz_wstore{};
 }
 
-int read_counters(mz_ctx *c) {
-    MZ_CUDA(c, cudaMemcpyAsync(c->h_counters, c->ring.counters, 8 * sizeof(int64_t), cudaMemcpyDeviceToHost, c->stream));
+// What read_counters checks after the read, in this order: NEED_GAMES and NEED_IDLE fail with MZ_E_STATE, the keys with MZ_E_ARG.
+enum { NEED_GAMES = 1 /* at least one game is stored */, NEED_IDLE = 2 /* no self-play wave is in progress */ };
+// Reads the ring counters into h_counters (one copy, one synchronise) and checks them as `need` asks; n > 0: keys key0 .. key0+n-1 are
+// stored.
+int read_counters(mz_ctx *c, int need = 0, int64_t key0 = 0, int n = 0) {
+    MZ_CUDA(c, cudaMemcpyAsync(c->h_counters, c->ring.counters, MZ_RC_COUNT * sizeof(int64_t), cudaMemcpyDeviceToHost, c->stream));
     MZ_CUDA(c, cudaStreamSynchronize(c->stream));
+    const int64_t played = c->h_counters[MZ_RC_PLAYED_GAMES];
+    if ((need & NEED_GAMES) && played < 1) return fail(c, MZ_E_STATE, "replay buffer is empty (learning! waits for num_played_games >= 1, Learning.jl:311)");
+    if ((need & NEED_IDLE) && c->h_counters[MZ_RC_ACTIVE] != 0) return fail(c, MZ_E_STATE, "self-play in progress");
+    const int64_t first = mz_ring_span(played, c->ring.capacity).first;
+    if (n > 0 && (key0 < first || key0 + n - 1 > played))
+        return fail(c, MZ_E_ARG, "keys %lld..%lld not in the buffer (holds %lld..%lld)", (long long)key0, (long long)(key0 + n - 1), (long long)first, (long long)played);
     return MZ_OK;
 }
 int write_counters(mz_ctx *c) {
-    MZ_CUDA(c, cudaMemcpyAsync(c->ring.counters, c->h_counters, 8 * sizeof(int64_t), cudaMemcpyHostToDevice, c->stream));
+    MZ_CUDA(c, cudaMemcpyAsync(c->ring.counters, c->h_counters, MZ_RC_COUNT * sizeof(int64_t), cudaMemcpyHostToDevice, c->stream));
     MZ_CUDA(c, cudaStreamSynchronize(c->stream));
+    return MZ_OK;
+}
+// Copies the rows of keys key0 .. key0+n-1 between host [n][row] (read when kind is cudaMemcpyHostToDevice, written otherwise) and a ring
+// array [capacity][row] indexed by position: at most two copies, split where the range wraps (n <= capacity).  Queued on the stream.
+template <typename T> int ring_rows(mz_ctx *c, cudaMemcpyKind kind, T *ring, const T *host, int64_t key0, int n, size_t row) {
+    const int64_t cap = c->ring.capacity;
+    int64_t pos = mz_ring_pos(key0, cap);
+    for (int64_t j = 0, m; j < n; j += m, pos = 0) {
+        m = n - j < cap - pos ? n - j : cap - pos;
+        T *r = ring + (size_t)pos * row, *h = const_cast<T *>(host) + (size_t)j * row;
+        MZ_CUDA(c, cudaMemcpyAsync(kind == cudaMemcpyHostToDevice ? r : h, kind == cudaMemcpyHostToDevice ? h : r, (size_t)m * row * sizeof(T), kind, c->stream));
+    }
     return MZ_OK;
 }
 
@@ -1018,8 +1040,7 @@ int mz_run_mcts(mz_ctx *c, int n, const float *stacked_obs, const uint32_t *lega
         if (root_priors) memcpy(root_priors, h + o_pri, (size_t)n * P.A * 4);
         return MZ_OK;
     }
-    read_counters(c);
-    if (c->h_counters[5] != 0) return fail(c, MZ_E_STATE, "self-play in progress");
+    MZ_TRY(read_counters(c, NEED_IDLE));
     const int cap = c->cfg.num_slots;
     MZ_TRY(ensure_images(c));
     for (int off = 0; off < n; off += cap) {
@@ -1073,11 +1094,19 @@ static int slots_reset(mz_ctx *c) {
     if (c->stream2) cudaStreamSynchronize(c->stream2);
     c->slots_dirty = false;
     MZ_CUDA(c, cudaMemsetAsync(c->slots.status, 0, (size_t)c->cfg.num_slots * sizeof(int32_t), c->stream));
-    MZ_CUDA(c, cudaMemsetAsync(c->ring.counters + 5, 0, sizeof(int64_t), c->stream));
+    MZ_CUDA(c, cudaMemsetAsync(c->ring.counters + MZ_RC_ACTIVE, 0, sizeof(int64_t), c->stream));
     MZ_CUDA(c, cudaStreamSynchronize(c->stream));
     return MZ_OK;
 }
 static int run_wave_body(mz_ctx *c, uint64_t first_game, int64_t n_games, float temperature, int arena_player, int arena_opponent, int tally_player, int64_t *simulations, int64_t *moves, bool allow_lat = true);
+// the end of a wave, from its statistics in h_stats: the caller's simulations and moves (counted by the caller), mz_search_stats' means
+static void wave_results(mz_ctx *c, int64_t moves, int64_t *simulations, int64_t *moves_out) {
+    const unsigned long long *s = c->h_stats;
+    if (simulations) *simulations = (int64_t)s[MZ_ST_SIMULATIONS];
+    if (moves_out) *moves_out = moves;
+    c->last_mean_depth = s[MZ_ST_SIMULATIONS] ? (double)s[MZ_ST_DEPTH_SUM] / (double)s[MZ_ST_SIMULATIONS] : 0.0;
+    c->last_mean_legal = s[MZ_ST_MOVES] ? (double)s[MZ_ST_LEGAL_SUM] / (double)s[MZ_ST_MOVES] : 0.0;
+}
 static int run_wave(mz_ctx *c, uint64_t first_game, int64_t n_games, float temperature, int arena_player, int arena_opponent, int tally_player, int64_t *simulations, int64_t *moves) {
     int rc = MZ_OK;
     const int64_t G = c->cfg.num_slots;
@@ -1090,16 +1119,13 @@ static int run_wave(mz_ctx *c, uint64_t first_game, int64_t n_games, float tempe
         for (int64_t off = 0; off < n_games && rc == MZ_OK; off += G) {
             rc = run_wave_body(c, first_game + (uint64_t)off, n_games - off < G ? n_games - off : G, temperature, arena_player, arena_opponent, tally_player, nullptr, nullptr,
                                false /* a short last wave stays on this path's arithmetic: one call, one kernel family */);
-            for (int i = 0; i < 4; i++) acc[i] += c->h_stats[i];
-            for (int i = 0; i < 3; i++) tally[i] += c->h_stats[61 + i];
+            for (int i = 0; i < 4; i++) acc[i] += c->h_stats[MZ_ST_DEPTH_SUM + i];
+            for (int i = 0; i < 3; i++) tally[i] += c->h_stats[MZ_ST_TALLY + i];
         }
         if (rc == MZ_OK) {
-            for (int i = 0; i < 4; i++) c->h_stats[i] = acc[i];
-            for (int i = 0; i < 3; i++) c->h_stats[61 + i] = tally[i];
-            if (simulations) *simulations = (int64_t)acc[1];
-            if (moves) *moves = (int64_t)acc[3];
-            c->last_mean_depth = acc[1] ? (double)acc[0] / (double)acc[1] : 0.0;
-            c->last_mean_legal = acc[3] ? (double)acc[2] / (double)acc[3] : 0.0;
+            for (int i = 0; i < 4; i++) c->h_stats[MZ_ST_DEPTH_SUM + i] = acc[i];
+            for (int i = 0; i < 3; i++) c->h_stats[MZ_ST_TALLY + i] = tally[i];
+            wave_results(c, (int64_t)acc[MZ_ST_MOVES], simulations, moves);
         }
     } else rc = run_wave_body(c, first_game, n_games, temperature, arena_player, arena_opponent, tally_player, simulations, moves);
     if (rc != MZ_OK && rc != MZ_E_ARG) {   // a wave that failed half-way must not leave games in flight: later calls would answer MZ_E_STATE for ever
@@ -1114,16 +1140,16 @@ static int run_wave_body(mz_ctx *c, uint64_t first_game, int64_t n_games, float 
     if (first_game + (uint64_t)n_games > 0xffffffffull) return fail(c, MZ_E_ARG, "game ids must fit in 32 bits (Philox counter)");
     mz_params P = c->M.P;
     P.arena_player = arena_player; P.arena_opponent = arena_opponent; P.arena_tally = tally_player;
-    unsigned long long *tally = c->d_stats + 61;   // wins, draws, losses (the last three of the 64 counters)
+    unsigned long long *tally = c->d_stats + MZ_ST_TALLY;   // wins, draws, losses
     const int G = c->cfg.num_slots;
     // A wave starts from idle slots: a successful wave ends with every slot idle, a failed one is followed by slots_reset (run_wave), so the
     // device counters need not be read back here (two stream synchronisations per wave): only {next game id, end id, active games} go down,
     // in stream order, from pinned memory
     if (c->slots_dirty) MZ_TRY(slots_reset(c));
     c->slots_dirty = true;
-    c->h_counters[3] = (int64_t)first_game; c->h_counters[4] = (int64_t)first_game + n_games; c->h_counters[5] = 0;
-    MZ_CUDA(c, cudaMemcpyAsync(c->ring.counters + 3, c->h_counters + 3, 3 * sizeof(int64_t), cudaMemcpyHostToDevice, c->stream));
-    MZ_CUDA(c, cudaMemsetAsync(c->d_stats, 0, 64 * sizeof(unsigned long long), c->stream));
+    c->h_counters[MZ_RC_NEXT_GAME] = (int64_t)first_game; c->h_counters[MZ_RC_END_GAME] = (int64_t)first_game + n_games; c->h_counters[MZ_RC_ACTIVE] = 0;
+    MZ_CUDA(c, cudaMemcpyAsync(c->ring.counters + MZ_RC_NEXT_GAME, c->h_counters + MZ_RC_NEXT_GAME, 3 * sizeof(int64_t), cudaMemcpyHostToDevice, c->stream));
+    MZ_CUDA(c, cudaMemsetAsync(c->d_stats, 0, MZ_ST_COUNT * sizeof(unsigned long long), c->stream));
     // MZ_OPP_NETWORK: the other side's plies are searched like MuZero's, by the same kernels reading the opponent store
     const bool vs_net = arena_player != 0 && arena_opponent == MZ_OPP_NETWORK;
     MZ_TRY(ensure_images(c));
@@ -1160,16 +1186,13 @@ static int run_wave_body(mz_ctx *c, uint64_t first_game, int64_t n_games, float 
     if (overlap && !use_lat && arena_player == 0 && c->cfg.net_type == MZ_NET_FEEDFORWARD && c->cfg.nn_mode == MZ_NN_SPLIT_MMA && c->persist_ok) {
         mz_search_args ap = a; ap.persist = 1;
         launch_search<MZ_MODE_SLOTS>(c, P, ap, 0, c->own);
-        MZ_TRY(launch_save_refill(c, P, G, tally, c->d_wave + 8));
+        MZ_TRY(launch_save_refill(c, P, G, tally, c->d_wave + MZ_RC_COUNT));
         MZ_CUDA(c, cudaGetLastError());
-        MZ_CUDA(c, cudaMemcpyAsync(c->h_stats, c->d_stats, 64 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, c->stream));
+        MZ_CUDA(c, cudaMemcpyAsync(c->h_stats, c->d_stats, MZ_ST_COUNT * sizeof(unsigned long long), cudaMemcpyDeviceToHost, c->stream));
         MZ_CUDA(c, cudaStreamSynchronize(c->stream));
-        if (c->h_wave[8 + 5] != 0) return fail(c, MZ_E_STATE, "self-play did not terminate");
+        if (c->h_wave[MZ_RC_COUNT + MZ_RC_ACTIVE] != 0) return fail(c, MZ_E_STATE, "self-play did not terminate");
         c->slots_dirty = false;
-        if (simulations) *simulations = (int64_t)c->h_stats[1];
-        if (moves) *moves = (int64_t)c->h_stats[3];
-        c->last_mean_depth = c->h_stats[1] ? (double)c->h_stats[0] / (double)c->h_stats[1] : 0.0;
-        c->last_mean_legal = c->h_stats[3] ? (double)c->h_stats[2] / (double)c->h_stats[3] : 0.0;
+        wave_results(c, (int64_t)c->h_stats[MZ_ST_MOVES], simulations, moves);
         return MZ_OK;
     }
     for (int64_t k = 0;; k++) {
@@ -1183,12 +1206,12 @@ static int run_wave_body(mz_ctx *c, uint64_t first_game, int64_t n_games, float 
         launch_search<MZ_MODE_SLOTS>(c, P, a, use_lat ? G_lat : 0, c->own);   // few games (play_game one game at a time): one tree per cluster, exact fp32
         const size_t search_entry = c->timed.size();                       // (timing builds) index just past this iteration's search launch
         if (overlap) { MZ_CUDA(c, cudaEventRecord(c->ev_search[k & 1], c->stream)); MZ_CUDA(c, cudaStreamWaitEvent(sB, c->ev_search[k & 1], 0)); }
-        MZ_TRY(launch_save_refill(c, P, G, tally, c->d_wave + 8 * ((k + 1) & 1), sB));
+        MZ_TRY(launch_save_refill(c, P, G, tally, c->d_wave + MZ_RC_COUNT * ((k + 1) & 1), sB));
         MZ_TRY(snapshot((int)((k + 1) & 1)));
         last_snap = (int)((k + 1) & 1);
         MZ_CUDA(c, cudaGetLastError());
         MZ_CUDA(c, cudaEventSynchronize(c->ev_wave[k & 1]));
-        const int64_t active = c->h_wave[8 * (k & 1) + 5];                 // games active when iteration k started
+        const int64_t active = c->h_wave[MZ_RC_COUNT * (k & 1) + MZ_RC_ACTIVE];   // games active when iteration k started
         if (active == 0) {
             // the iteration just queued is the idle one: keep its searches out of the per-family kernel statistics (family 7 = idle)
             for (size_t i = iter_entry; i < search_entry; i++) if (c->timed[i].family == 0) c->timed[i].family = 7;
@@ -1198,13 +1221,10 @@ static int run_wave_body(mz_ctx *c, uint64_t first_game, int64_t n_games, float 
         total_moves += active;
     }
     if (overlap) MZ_CUDA(c, cudaStreamWaitEvent(c->stream, c->ev_wave[last_snap], 0));   // the last save / refill (tallies, counters) before anything else runs on the main stream
-    MZ_CUDA(c, cudaMemcpyAsync(c->h_stats, c->d_stats, 64 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, c->stream));
+    MZ_CUDA(c, cudaMemcpyAsync(c->h_stats, c->d_stats, MZ_ST_COUNT * sizeof(unsigned long long), cudaMemcpyDeviceToHost, c->stream));
     MZ_CUDA(c, cudaStreamSynchronize(c->stream));
     c->slots_dirty = false;
-    if (simulations) *simulations = (int64_t)c->h_stats[1];
-    if (moves) *moves = total_moves;
-    c->last_mean_depth = c->h_stats[1] ? (double)c->h_stats[0] / (double)c->h_stats[1] : 0.0;
-    c->last_mean_legal = c->h_stats[3] ? (double)c->h_stats[2] / (double)c->h_stats[3] : 0.0;
+    wave_results(c, total_moves, simulations, moves);
     return MZ_OK;
 }
 
@@ -1228,9 +1248,9 @@ int mz_arena(mz_ctx *c, uint64_t first_game, int64_t n_games, int opponent, int 
     MZ_TRY(check_opponent_set(c, opponent));
     // length(conf.players) == 1 ? "self" : conf.opponent (:428); "self": every ply is searched, outcomes still tallied for muzero_player
     MZ_TRY(run_wave(c, first_game, n_games, temperature, opponent == MZ_OPP_SELF ? 0 : muzero_player, opponent, muzero_player, simulations, nullptr));
-    if (wins) *wins = (int64_t)c->h_stats[61];
-    if (draws) *draws = (int64_t)c->h_stats[62];
-    if (losses) *losses = (int64_t)c->h_stats[63];
+    if (wins) *wins = (int64_t)c->h_stats[MZ_ST_TALLY];
+    if (draws) *draws = (int64_t)c->h_stats[MZ_ST_TALLY + 1];
+    if (losses) *losses = (int64_t)c->h_stats[MZ_ST_TALLY + 2];
     return MZ_OK;
 }
 int mz_opponent_action(mz_ctx *c, int n, const uint64_t *p1, const uint64_t *p2, const int32_t *player, int opponent, const uint64_t *game_id,
@@ -1264,9 +1284,9 @@ int mz_play_games(mz_ctx *c, uint64_t first_game, int n_games, float temperature
     if (simulations) *simulations = 0;
     if (n_games == 0) return MZ_OK;
     MZ_TRY(read_counters(c));
-    if (c->h_counters[5] != 0) MZ_TRY(slots_reset(c));
+    if (c->h_counters[MZ_RC_ACTIVE] != 0) MZ_TRY(slots_reset(c));
     if (c->play_ring.capacity < n_games) MZ_TRY(alloc_ring(c, c->play_ring, (size_t)(n_games < c->cfg.num_slots ? c->cfg.num_slots : n_games)));
-    MZ_CUDA(c, cudaMemsetAsync(c->play_ring.counters, 0, 8 * sizeof(int64_t), c->stream));
+    MZ_CUDA(c, cudaMemsetAsync(c->play_ring.counters, 0, MZ_RC_COUNT * sizeof(int64_t), c->stream));
     const int per = c->M.P.per; c->M.P.per = 0;                  // priorities belong to save_game
     std::swap(c->ring, c->play_ring);
     int rc = run_wave(c, first_game, n_games, temperature, opponent == MZ_OPP_SELF ? 0 : muzero_player, opponent, 0, simulations, nullptr);
@@ -1279,16 +1299,16 @@ int mz_play_games(mz_ctx *c, uint64_t first_game, int n_games, float temperature
 int mz_replay_info(mz_ctx *c, int64_t *n_games, int64_t *first_key, int64_t *total_samples) {
     MZ_CHECK_CTX(c);
     MZ_TRY(read_counters(c));
-    int64_t played = c->h_counters[0], n = played < c->ring.capacity ? played : c->ring.capacity;
-    if (n_games) *n_games = n;
-    if (first_key) *first_key = played - n + 1;
-    if (total_samples) *total_samples = c->h_counters[2];
+    const mz_span span = mz_ring_span(c->h_counters[MZ_RC_PLAYED_GAMES], c->ring.capacity);
+    if (n_games) *n_games = span.n;
+    if (first_key) *first_key = span.first;
+    if (total_samples) *total_samples = c->h_counters[MZ_RC_TOTAL_SAMPLES];
     return MZ_OK;
 }
 int mz_replay_clear(mz_ctx *c) {
     MZ_CHECK_CTX(c);
     MZ_TRY(slots_reset(c));
-    for (int i = 0; i < 8; i++) c->h_counters[i] = 0;
+    for (int i = 0; i < MZ_RC_COUNT; i++) c->h_counters[i] = 0;
     MZ_TRY(write_counters(c));
     MZ_CUDA(c, cudaMemsetAsync(c->ring.T, 0, (size_t)c->ring.capacity * sizeof(int32_t), c->stream));
     MZ_CUDA(c, cudaMemsetAsync(c->ring.reanalysed, 0, (size_t)c->ring.capacity, c->stream));
@@ -1300,9 +1320,7 @@ int mz_history_export(mz_ctx *c, int64_t key0, int n, int64_t *game_id, int32_t 
     MZ_CHECK_CTX(c);
     if (n < 0 || (n > 0 && (!game_id || !T || !obs || !actions || !rewards || !to_play || !child_visits || !root_values))) return fail(c, MZ_E_ARG, "NULL buffer");
     if (n == 0) return MZ_OK;
-    MZ_TRY(read_counters(c));
-    int64_t played = c->h_counters[0], have = played < c->ring.capacity ? played : c->ring.capacity, first = played - have + 1;
-    if (key0 < first || key0 + n - 1 > played) return fail(c, MZ_E_ARG, "keys %lld..%lld not in the buffer (holds %lld..%lld)", (long long)key0, (long long)(key0 + n - 1), (long long)first, (long long)played);
+    MZ_TRY(read_counters(c, 0, key0, n));
     const mz_params &P = c->M.P; const size_t Tm = (size_t)P.Tmax, N = (size_t)n;
     int64_t *d_gid; int32_t *d_T, *d_act, *d_tp; float *d_obs, *d_rew, *d_cv, *d_rv;
     MZ_TRY(h2d<int64_t>(c, c->scratch[0], nullptr, N, &d_gid)); MZ_TRY(h2d<int32_t>(c, c->scratch[1], nullptr, N, &d_T));
@@ -1326,19 +1344,17 @@ int mz_history_import(mz_ctx *c, int n, const int64_t *game_id, const int32_t *T
     if (n > c->ring.capacity) return fail(c, MZ_E_ARG, "more histories than replay_buffer_size");
     const mz_params &P = c->M.P; const size_t Tm = (size_t)P.Tmax, N = (size_t)n;
     for (int i = 0; i < n; i++) if (T[i] < 1 || T[i] > P.Tmax) return fail(c, MZ_E_ARG, "history %d has length %d outside 1..%d", i, T[i], P.Tmax);
-    MZ_TRY(read_counters(c));
-    if (c->h_counters[5] != 0) return fail(c, MZ_E_STATE, "self-play in progress");
-    // save_game bookkeeping (ReplayBuffer.jl:147-160): counters + FIFO eviction accounting
-    std::vector<int32_t> oldT((size_t)c->ring.capacity);
-    MZ_CUDA(c, cudaMemcpyAsync(oldT.data(), c->ring.T, oldT.size() * sizeof(int32_t), cudaMemcpyDeviceToHost, c->stream));
+    MZ_TRY(read_counters(c, NEED_IDLE));
+    // save_game bookkeeping (ReplayBuffer.jl:147-160): counters + FIFO eviction accounting (the lengths of the games overwritten)
+    const int64_t played = c->h_counters[MZ_RC_PLAYED_GAMES], key0 = played + 1;
+    std::vector<int32_t> oldT(N);
+    MZ_TRY(ring_rows(c, cudaMemcpyDeviceToHost, c->ring.T, oldT.data(), key0, n, 1));
     MZ_CUDA(c, cudaStreamSynchronize(c->stream));
-    int64_t played = c->h_counters[0], key0 = played + 1;
     for (int i = 0; i < n; i++) {
-        int64_t key = key0 + i, pos = (key - 1) % c->ring.capacity;
-        c->h_counters[1] += T[i]; c->h_counters[2] += T[i];
-        if (key > c->ring.capacity) c->h_counters[2] -= oldT[(size_t)pos];
+        c->h_counters[MZ_RC_PLAYED_STEPS] += T[i]; c->h_counters[MZ_RC_TOTAL_SAMPLES] += T[i];
+        if (key0 + i > c->ring.capacity) c->h_counters[MZ_RC_TOTAL_SAMPLES] -= oldT[(size_t)i];
     }
-    c->h_counters[0] = played + n;
+    c->h_counters[MZ_RC_PLAYED_GAMES] = played + n;
     int64_t *d_gid; int32_t *d_T, *d_act, *d_tp; float *d_obs, *d_rew, *d_cv, *d_rv;
     MZ_TRY(h2d(c, c->scratch[0], game_id, N, &d_gid)); MZ_TRY(h2d(c, c->scratch[1], T, N, &d_T));
     MZ_TRY(h2d(c, c->scratch[2], obs, N * Tm * P.obs_size, &d_obs)); MZ_TRY(h2d(c, c->scratch[3], actions, N * Tm, &d_act));
@@ -1356,10 +1372,7 @@ int mz_reanalyse(mz_ctx *c, int64_t key0, int n) {
     if (c->cfg.net_type != MZ_NET_FEEDFORWARD) return fail(c, MZ_E_UNSUPPORTED, "reanalyse runs the exact feed-forward networks");
     if (n < 0) return fail(c, MZ_E_ARG, "n < 0");
     if (n == 0) return MZ_OK;
-    MZ_TRY(read_counters(c));
-    if (c->h_counters[5] != 0) return fail(c, MZ_E_STATE, "self-play in progress");
-    int64_t played = c->h_counters[0], have = played < c->ring.capacity ? played : c->ring.capacity, first = played - have + 1;
-    if (key0 < first || key0 + n - 1 > played) return fail(c, MZ_E_ARG, "keys %lld..%lld not in the buffer (holds %lld..%lld)", (long long)key0, (long long)(key0 + n - 1), (long long)first, (long long)played);
+    MZ_TRY(read_counters(c, NEED_IDLE, key0, n));
     const mz_params &P = c->M.P;
     mz_reanalyse_args a{}; a.wglob = c->own.w; a.max_dim = c->M.max_dim; a.max_layer_floats = c->M.max_layer_floats; a.n = n; a.key0 = key0; a.ring = c->ring;
     const int64_t total = (int64_t)n * P.Tmax;
@@ -1380,19 +1393,15 @@ int mz_reanalyse_search(mz_ctx *c, int64_t key0, int n, int exploration, int64_t
     if (simulations) *simulations = 0;
     if (n < 0) return fail(c, MZ_E_ARG, "n < 0");
     if (n == 0) return MZ_OK;
-    MZ_TRY(read_counters(c));
-    if (c->h_counters[5] != 0) return fail(c, MZ_E_STATE, "self-play in progress");
-    int64_t played = c->h_counters[0], have = played < c->ring.capacity ? played : c->ring.capacity, first = played - have + 1;
-    if (key0 < first || key0 + n - 1 > played) return fail(c, MZ_E_ARG, "keys %lld..%lld not in the buffer (holds %lld..%lld)", (long long)key0, (long long)(key0 + n - 1), (long long)first, (long long)played);
+    MZ_TRY(read_counters(c, NEED_IDLE, key0, n));
     const mz_params &P = c->M.P;
-    const int64_t cap = c->ring.capacity, Tm = P.Tmax, pos0 = (key0 - 1) % cap, n1 = n < cap - pos0 ? n : cap - pos0;   // the range wraps after n1 games
+    const int64_t Tm = P.Tmax;
     std::vector<int32_t> T((size_t)n);
-    MZ_CUDA(c, cudaMemcpyAsync(T.data(), c->ring.T + pos0, (size_t)n1 * sizeof(int32_t), cudaMemcpyDeviceToHost, c->stream));
-    if (n1 < n) MZ_CUDA(c, cudaMemcpyAsync(T.data() + n1, c->ring.T, (size_t)(n - n1) * sizeof(int32_t), cudaMemcpyDeviceToHost, c->stream));
+    MZ_TRY(ring_rows(c, cudaMemcpyDeviceToHost, c->ring.T, T.data(), key0, n, 1));
     MZ_CUDA(c, cudaStreamSynchronize(c->stream));
     std::vector<int64_t> roots;
     for (int t = 0; t < Tm; t++)
-        for (int j = 0; j < n; j++) if (t < T[(size_t)j]) roots.push_back(((key0 + j - 1) % cap) * Tm + t);
+        for (int j = 0; j < n; j++) if (t < T[(size_t)j]) roots.push_back(mz_ring_pos(key0 + j, c->ring.capacity) * Tm + t);
     MZ_TRY(ensure_images(c));
     int64_t *d_roots;
     MZ_TRY(h2d(c, c->scratch[0], roots.data(), roots.size(), &d_roots));
@@ -1413,18 +1422,12 @@ int mz_reanalysed_export(mz_ctx *c, int64_t key0, int n, float *values, int32_t 
     MZ_CHECK_CTX(c);
     if (n < 0 || (n > 0 && (!values || !flags))) return fail(c, MZ_E_ARG, "NULL buffer");
     if (n == 0) return MZ_OK;
-    MZ_TRY(read_counters(c));
-    int64_t played = c->h_counters[0], have = played < c->ring.capacity ? played : c->ring.capacity, first = played - have + 1;
-    if (key0 < first || key0 + n - 1 > played) return fail(c, MZ_E_ARG, "keys not in the buffer");
-    const size_t Tm = (size_t)c->M.P.Tmax;
-    std::vector<uint8_t> fl((size_t)c->ring.capacity);
-    MZ_CUDA(c, cudaMemcpyAsync(fl.data(), c->ring.reanalysed, fl.size(), cudaMemcpyDeviceToHost, c->stream));
-    for (int j = 0; j < n; j++) {
-        const int64_t pos = (key0 + j - 1) % c->ring.capacity;
-        MZ_CUDA(c, cudaMemcpyAsync(values + (size_t)j * Tm, c->ring.h_rrv + (size_t)pos * Tm, Tm * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
-    }
+    MZ_TRY(read_counters(c, 0, key0, n));
+    std::vector<uint8_t> fl((size_t)n);
+    MZ_TRY(ring_rows(c, cudaMemcpyDeviceToHost, c->ring.h_rrv, values, key0, n, (size_t)c->M.P.Tmax));
+    MZ_TRY(ring_rows(c, cudaMemcpyDeviceToHost, c->ring.reanalysed, fl.data(), key0, n, 1));
     MZ_CUDA(c, cudaStreamSynchronize(c->stream));
-    for (int j = 0; j < n; j++) flags[j] = fl[(size_t)((key0 + j - 1) % c->ring.capacity)];
+    for (int j = 0; j < n; j++) flags[j] = fl[(size_t)j];
     return MZ_OK;
 }
 
@@ -1433,34 +1436,24 @@ int mz_replay_counters(mz_ctx *c, int64_t out[3]) {
     MZ_CHECK_CTX(c);
     if (!out) return fail(c, MZ_E_ARG, "NULL buffer");
     MZ_TRY(read_counters(c));
-    for (int i = 0; i < 3; i++) out[i] = c->h_counters[i];
+    out[0] = c->h_counters[MZ_RC_PLAYED_GAMES]; out[1] = c->h_counters[MZ_RC_PLAYED_STEPS]; out[2] = c->h_counters[MZ_RC_TOTAL_SAMPLES];
     return MZ_OK;
 }
 int mz_replay_set_counters(mz_ctx *c, int64_t num_played_games, int64_t num_played_steps, int64_t total_samples) {
     MZ_CHECK_CTX(c);
     if (num_played_games < 0 || num_played_steps < 0 || total_samples < 0) return fail(c, MZ_E_ARG, "counters must be >= 0");
-    MZ_TRY(read_counters(c));
-    if (c->h_counters[5] != 0) return fail(c, MZ_E_STATE, "self-play in progress");
-    c->h_counters[0] = num_played_games; c->h_counters[1] = num_played_steps; c->h_counters[2] = total_samples;
+    MZ_TRY(read_counters(c, NEED_IDLE));
+    c->h_counters[MZ_RC_PLAYED_GAMES] = num_played_games; c->h_counters[MZ_RC_PLAYED_STEPS] = num_played_steps;
+    c->h_counters[MZ_RC_TOTAL_SAMPLES] = total_samples;
     return write_counters(c);
-}
-static int keys_in_buffer(mz_ctx *c, int64_t key0, int n) {
-    MZ_TRY(read_counters(c));
-    const int64_t played = c->h_counters[0], have = played < c->ring.capacity ? played : c->ring.capacity, first = played - have + 1;
-    if (key0 < first || key0 + n - 1 > played) return fail(c, MZ_E_ARG, "keys %lld..%lld not in the buffer (holds %lld..%lld)", (long long)key0, (long long)(key0 + n - 1), (long long)first, (long long)played);
-    return MZ_OK;
 }
 int mz_replay_set_priorities(mz_ctx *c, int64_t key0, int n, const uint32_t *q_pos, const uint32_t *q_game) {
     MZ_CHECK_CTX(c);
     if (n < 0 || (n > 0 && (!q_pos || !q_game))) return fail(c, MZ_E_ARG, "NULL buffer");
     if (n == 0) return MZ_OK;
-    MZ_TRY(keys_in_buffer(c, key0, n));
-    const size_t Tm = (size_t)c->M.P.Tmax;
-    for (int j = 0; j < n; j++) {
-        const int64_t pos = (key0 + j - 1) % c->ring.capacity;
-        MZ_CUDA(c, cudaMemcpyAsync(c->ring.q_pos + (size_t)pos * Tm, q_pos + (size_t)j * Tm, Tm * 4, cudaMemcpyHostToDevice, c->stream));
-        MZ_CUDA(c, cudaMemcpyAsync(c->ring.q_game + pos, q_game + j, 4, cudaMemcpyHostToDevice, c->stream));
-    }
+    MZ_TRY(read_counters(c, 0, key0, n));
+    MZ_TRY(ring_rows(c, cudaMemcpyHostToDevice, c->ring.q_pos, q_pos, key0, n, (size_t)c->M.P.Tmax));
+    MZ_TRY(ring_rows(c, cudaMemcpyHostToDevice, c->ring.q_game, q_game, key0, n, 1));
     MZ_CUDA(c, cudaStreamSynchronize(c->stream));
     return MZ_OK;
 }
@@ -1468,15 +1461,11 @@ int mz_reanalysed_import(mz_ctx *c, int64_t key0, int n, const float *values, co
     MZ_CHECK_CTX(c);
     if (n < 0 || (n > 0 && (!values || !flags))) return fail(c, MZ_E_ARG, "NULL buffer");
     if (n == 0) return MZ_OK;
-    MZ_TRY(keys_in_buffer(c, key0, n));
-    const size_t Tm = (size_t)c->M.P.Tmax;
+    MZ_TRY(read_counters(c, 0, key0, n));
     std::vector<uint8_t> fl((size_t)n);
     for (int j = 0; j < n; j++) fl[(size_t)j] = flags[j] ? 1 : 0;
-    for (int j = 0; j < n; j++) {
-        const int64_t pos = (key0 + j - 1) % c->ring.capacity;
-        MZ_CUDA(c, cudaMemcpyAsync(c->ring.h_rrv + (size_t)pos * Tm, values + (size_t)j * Tm, Tm * sizeof(float), cudaMemcpyHostToDevice, c->stream));
-        MZ_CUDA(c, cudaMemcpyAsync(c->ring.reanalysed + pos, fl.data() + j, 1, cudaMemcpyHostToDevice, c->stream));
-    }
+    MZ_TRY(ring_rows(c, cudaMemcpyHostToDevice, c->ring.h_rrv, values, key0, n, (size_t)c->M.P.Tmax));
+    MZ_TRY(ring_rows(c, cudaMemcpyHostToDevice, c->ring.reanalysed, fl.data(), key0, n, 1));
     MZ_CUDA(c, cudaStreamSynchronize(c->stream));
     return MZ_OK;
 }
@@ -1498,12 +1487,14 @@ static int launch_per_update(mz_ctx *c, int B) {
     MZ_CUDA(c, cudaGetLastError());
     return MZ_OK;
 }
+// what every replay gather needs first: the batch buffers and a stored game
+static int gather_ready(mz_ctx *c) {
+    MZ_TRY(alloc_batch(c, c->cfg.batch_size));
+    return read_counters(c, NEED_GAMES);
+}
 static int gather_batch(mz_ctx *c, uint64_t step) {
-    const int B = c->cfg.batch_size;
-    MZ_TRY(alloc_batch(c, B));
-    MZ_TRY(read_counters(c));
-    if (c->h_counters[0] < 1) return fail(c, MZ_E_STATE, "replay buffer is empty (learning! waits for num_played_games >= 1, Learning.jl:311)");
-    return launch_gather(c, step, B);
+    MZ_TRY(gather_ready(c));
+    return launch_gather(c, step, c->cfg.batch_size);
 }
 int mz_get_batch(mz_ctx *c, uint64_t step, int32_t *index_batch, float *obs_batch, float *action_batch, float *value_batch, float *reward_batch,
                  float *policy_batch, float *gscale) {
@@ -1533,15 +1524,9 @@ int mz_replay_priorities(mz_ctx *c, int64_t key0, int n, uint32_t *q_pos, uint32
     MZ_CHECK_CTX(c);
     if (n < 0 || (n > 0 && (!q_pos || !q_game))) return fail(c, MZ_E_ARG, "NULL buffer");
     if (n == 0) return MZ_OK;
-    MZ_TRY(read_counters(c));
-    int64_t played = c->h_counters[0], have = played < c->ring.capacity ? played : c->ring.capacity, first = played - have + 1;
-    if (key0 < first || key0 + n - 1 > played) return fail(c, MZ_E_ARG, "keys not in the buffer");
-    const size_t Tm = (size_t)c->M.P.Tmax;
-    for (int j = 0; j < n; j++) {
-        const int64_t pos = (key0 + j - 1) % c->ring.capacity;
-        MZ_CUDA(c, cudaMemcpyAsync(q_pos + (size_t)j * Tm, c->ring.q_pos + (size_t)pos * Tm, Tm * 4, cudaMemcpyDeviceToHost, c->stream));
-        MZ_CUDA(c, cudaMemcpyAsync(q_game + j, c->ring.q_game + pos, 4, cudaMemcpyDeviceToHost, c->stream));
-    }
+    MZ_TRY(read_counters(c, 0, key0, n));
+    MZ_TRY(ring_rows(c, cudaMemcpyDeviceToHost, c->ring.q_pos, q_pos, key0, n, (size_t)c->M.P.Tmax));
+    MZ_TRY(ring_rows(c, cudaMemcpyDeviceToHost, c->ring.q_game, q_game, key0, n, 1));
     MZ_CUDA(c, cudaStreamSynchronize(c->stream));
     return MZ_OK;
 }
@@ -1615,9 +1600,7 @@ int mz_learn_steps(mz_ctx *c, int64_t t0, int n, int grad_mode, float *losses) {
     MZ_CHECK_CTX(c);
     if (!losses || t0 < 1 || n < 1) return fail(c, MZ_E_ARG, "bad arguments");
     const int B = c->cfg.batch_size;
-    MZ_TRY(alloc_batch(c, B));
-    MZ_TRY(read_counters(c));
-    if (c->h_counters[0] < 1) return fail(c, MZ_E_STATE, "replay buffer is empty (learning! waits for num_played_games >= 1, Learning.jl:311)");
+    MZ_TRY(gather_ready(c));
     for (int i = 0; i < n; i++) {
         MZ_TRY(launch_gather(c, (uint64_t)(t0 + i), B));
         MZ_TRY(launch_learn_forward(c, B, grad_mode));
@@ -1639,12 +1622,10 @@ int mz_learn_steps_reanalysed(mz_ctx *c, int64_t t0, int n, int grad_mode, int e
     if (simulations) *simulations = 0;
     if (!losses || t0 < 1 || n < 1) return fail(c, MZ_E_ARG, "bad arguments");
     const int B = c->cfg.batch_size;
-    MZ_TRY(read_counters(c));
-    if (c->h_counters[0] < 1) return fail(c, MZ_E_STATE, "replay buffer is empty (learning! waits for num_played_games >= 1, Learning.jl:311)");
-    if (c->h_counters[5] != 0) return fail(c, MZ_E_STATE, "self-play in progress");
+    MZ_TRY(read_counters(c, NEED_GAMES | NEED_IDLE));
     MZ_TRY(check_grad_mode(c, grad_mode));
     const mz_params &P = c->M.P;
-    const int64_t played = c->h_counters[0], have = played < c->ring.capacity ? played : c->ring.capacity;
+    const int64_t have = mz_ring_span(c->h_counters[MZ_RC_PLAYED_GAMES], c->ring.capacity).n;
     const int64_t bound = (B < have ? B : have) * (int64_t)P.Tmax, chunk = c->cfg.num_slots, n_chunks = (bound + chunk - 1) / chunk;
     int Bp = 1;
     while (Bp < B) Bp <<= 1;

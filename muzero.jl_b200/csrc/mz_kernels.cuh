@@ -43,17 +43,43 @@ struct mz_slots {          // device-resident concurrent games, SoA
     float *h_cv;             // [G][Tmax][A]
     float *h_rv;             // [G][Tmax]
 };
-struct mz_ring {           // device replay buffer: key k lives at (k-1) % capacity
+struct mz_ring {           // device replay buffer: key k lives at position mz_ring_pos(k, capacity)
     int64_t capacity;
     int64_t *game_id; int32_t *T;
     uint64_t *h_p1, *h_p2; int32_t *h_action; float *h_reward; uint8_t *h_to_play; float *h_cv; float *h_rv;
     uint32_t *q_pos, *q_game;             // conf.PER: history.priorities [R][Tmax], history.game_priority [R] (fixed point)
     unsigned long long *prefix, *upd;     // inclusive prefix sums of q_game in key order [R]; update_priorities! scratch [R][Tmax]
     float *h_rrv; uint8_t *reanalysed;   // GameHistory.reanalysed_predicted_root_values (Constructors.jl:13): [R][Tmax] + "is not nothing" flag per game
-    // counters (device): [0] num_played_games, [1] num_played_steps, [2] total_samples, [3] next game id to hand out,
-    // [4] end game id (exclusive), [5] active slots after the last refill
-    int64_t *counters;
+    int64_t *counters;                    // [MZ_RC_COUNT] (device), slots MZ_RC_*
 };
+// the slots of mz_ring::counters; the host's copy and mz_k_save_refill's snapshot have the same layout
+enum {
+    MZ_RC_PLAYED_GAMES = 0,    // num_played_games: the newest stored key
+    MZ_RC_PLAYED_STEPS = 1,    // num_played_steps
+    MZ_RC_TOTAL_SAMPLES = 2,   // total_samples: the positions of the stored games
+    MZ_RC_NEXT_GAME = 3,       // next game id to hand out
+    MZ_RC_END_GAME = 4,        // end game id (exclusive)
+    MZ_RC_ACTIVE = 5,          // active slots after the last refill: self-play is in progress while it is not 0
+    MZ_RC_PER_TOTAL = 6,       // conf.PER: the sum of the game priorities (mz_k_per_scan)
+    MZ_RC_UNUSED = 7,          // stays 0 (and is copied into the snapshot)
+    MZ_RC_COUNT = 8
+};
+// the self-play statistics of mz_search_args::stats (64 counters; the slots between them hold the phase timers of MZ_PHASE_TIMERS builds)
+enum {
+    MZ_ST_DEPTH_SUM = 0,       // sum of the leaf depths
+    MZ_ST_SIMULATIONS = 1,
+    MZ_ST_LEGAL_SUM = 2,       // sum of the roots' legal actions
+    MZ_ST_MOVES = 3,           // roots searched: one per move
+    MZ_ST_TALLY = 61,          // [3] competitive play: wins, draws, losses for MuZero
+    MZ_ST_COUNT = 64
+};
+// The ring holds the newest min(played, capacity) games: keys first .. played.
+struct mz_span { int64_t n, first; };
+__host__ __device__ __forceinline__ mz_span mz_ring_span(int64_t played, int64_t capacity) {
+    const int64_t n = played < capacity ? played : capacity;
+    return {n, played - n + 1};
+}
+__host__ __device__ __forceinline__ int64_t mz_ring_pos(int64_t key, int64_t capacity) { return (key - 1) % capacity; }
 struct mz_search_args {
     const float *wglob; const double *pbc0; const double *sqrtN; void *tree_pool;
     int32_t n, max_dim, max_layer_floats, exploration;
@@ -64,7 +90,7 @@ struct mz_search_args {
     int32_t *visit_counts; float *root_value; float *root_priors;
     // MODE_SLOTS
     mz_slots slots; float temperature;
-    unsigned long long *stats;   // [0] sum depth, [1] simulations, [2] sum legal, [3] roots
+    unsigned long long *stats;   // [MZ_ST_COUNT], slots MZ_ST_*
     // MODE_REPLAY: root i is position t of the game at ring position pos, replay[i] = pos * Tmax + t (the index of its [R][Tmax] entries).
     // Last, so that the fields the other modes read keep their offsets.
     mz_ring ring; const int64_t *replay;
@@ -281,9 +307,8 @@ __device__ __forceinline__ void mz_root_init(const mz_params &P, const mz_tree &
     if (ln == 0 && exploration && P.exploration_eps != 0.0f) mz_tree_add_noise(P, t, R.legal, R.game, R.move);
     __syncwarp(segmask);
 }
-// results of root g, lane 0 of an active tree: the launch's statistics (stats[0] sum of leaf depths, [1] simulations, [2] sum of legal
-// actions, [3] roots), then visit counts, root value and priors to the caller (MODE_API), the move of the game (MODE_SLOTS), or the
-// stored position's policy target and reanalysed root value (MODE_REPLAY)
+// results of root g, lane 0 of an active tree: the launch's statistics (MZ_ST_*), then visit counts, root value and priors to the caller
+// (MODE_API), the move of the game (MODE_SLOTS), or the stored position's policy target and reanalysed root value (MODE_REPLAY)
 template <int MODE>
 __device__ __forceinline__ void mz_root_finish(const mz_params &P, const mz_search_args &a, int64_t g, const mz_tree &t, const mz_root &R,
                                                unsigned long long depth_sum) {
@@ -296,8 +321,8 @@ __device__ __forceinline__ void mz_root_finish(const mz_params &P, const mz_sear
     const int rvc = mz_nx_visit(mz_f2bits(root.x));
     const float rv = rvc == 0 ? 0.0f : root.y / (float)rvc;                                 // node_value(root)
     if (a.stats) {
-        atomicAdd(&a.stats[0], depth_sum); atomicAdd(&a.stats[1], (unsigned long long)P.S);
-        atomicAdd(&a.stats[2], (unsigned long long)nlegal); atomicAdd(&a.stats[3], 1ull);
+        atomicAdd(&a.stats[MZ_ST_DEPTH_SUM], depth_sum); atomicAdd(&a.stats[MZ_ST_SIMULATIONS], (unsigned long long)P.S);
+        atomicAdd(&a.stats[MZ_ST_LEGAL_SUM], (unsigned long long)nlegal); atomicAdd(&a.stats[MZ_ST_MOVES], 1ull);
     }
     if (MODE == MZ_MODE_API) {
         for (int i = 0; i < P.A; i++) {
@@ -435,22 +460,23 @@ __device__ __forceinline__ void mz_per_init_game(const mz_params &P, const mz_ri
 }
 __global__ void mz_k_per_init(const __grid_constant__ mz_params P, mz_ring r, int64_t key0, int n) {
     int j = blockIdx.x * blockDim.x + threadIdx.x;
-    if (j < n) mz_per_init_game(P, r, (key0 + j - 1) % r.capacity);
+    if (j < n) mz_per_init_game(P, r, mz_ring_pos(key0 + j, r.capacity));
 }
 // Inclusive prefix sums of the game priorities in ascending key order (single CTA; integer sums: exact and order independent).
-// counters[6] = their total.
+// counters[MZ_RC_PER_TOTAL] = their total.
 __global__ void __launch_bounds__(1024) mz_k_per_scan(const __grid_constant__ mz_params P, mz_ring r) {
     __shared__ unsigned long long part[1024];
     const int tid = threadIdx.x;
-    const int64_t played = r.counters[0], n = played < r.capacity ? played : r.capacity, first_key = played - n + 1;
+    const mz_span span = mz_ring_span(r.counters[MZ_RC_PLAYED_GAMES], r.capacity);
+    const int64_t n = span.n, first_key = span.first;
     const int64_t per = (n + 1023) / 1024, lo = (int64_t)tid * per, hi = lo + per < n ? lo + per : n;
     unsigned long long s = 0;
-    for (int64_t i = lo; i < hi; i++) s += r.q_game[(first_key + i - 1) % r.capacity];
+    for (int64_t i = lo; i < hi; i++) s += r.q_game[mz_ring_pos(first_key + i, r.capacity)];
     part[tid] = s; __syncthreads();
     for (int off = 1; off < 1024; off <<= 1) { unsigned long long t = tid >= off ? part[tid - off] : 0ull; __syncthreads(); part[tid] += t; __syncthreads(); }
     unsigned long long run = tid ? part[tid - 1] : 0ull;
-    for (int64_t i = lo; i < hi; i++) { run += r.q_game[(first_key + i - 1) % r.capacity]; r.prefix[i] = run; }
-    if (tid == 1023) r.counters[6] = (int64_t)part[1023];
+    for (int64_t i = lo; i < hi; i++) { run += r.q_game[mz_ring_pos(first_key + i, r.capacity)]; r.prefix[i] = run; }
+    if (tid == 1023) r.counters[MZ_RC_PER_TOTAL] = (int64_t)part[1023];
 }
 // update_priorities! (ReplayBuffer.jl:168-183, repaired bounds; Learning.jl:400-404): rows k = 0 .. min(K, T - pos) of
 // |predicted_values - target_values|^alpha go to positions pos + k.  Batch elements apply in order (the last one wins where they
@@ -460,9 +486,9 @@ __global__ void mz_k_per_update(const __grid_constant__ mz_params P, mz_ring r, 
     const int i = blockIdx.x * blockDim.x + threadIdx.x, K1 = P.K + 1;
     if (i >= B * K1) return;
     const int b = i / K1, k = i % K1;
-    const int64_t key = index[2 * b], played = r.counters[0], n = played < r.capacity ? played : r.capacity;
-    if (key < played - n + 1 || key > played) return;                       // the game has left the buffer (:172)
-    const int64_t pos = (key - 1) % r.capacity;
+    const int64_t key = index[2 * b], played = r.counters[MZ_RC_PLAYED_GAMES];
+    if (key < mz_ring_span(played, r.capacity).first || key > played) return;   // the game has left the buffer (:172)
+    const int64_t pos = mz_ring_pos(key, r.capacity);
     const int T = r.T[pos], p = index[2 * b + 1];
     if (phase == 2) {
         if (k == 0) { uint32_t mx = 0; for (int t = 0; t < T; t++) { uint32_t q = r.q_pos[(size_t)pos * P.Tmax + t]; mx = q > mx ? q : mx; } r.q_game[pos] = mx; }
@@ -516,7 +542,7 @@ __global__ void __launch_bounds__(1024) mz_k_save_refill(const __grid_constant__
     __shared__ int active_count;
     __shared__ long long add_steps, add_samples;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    const int64_t base_key = r.counters[0], next_game = r.counters[3], end_game = r.counters[4];
+    const int64_t base_key = r.counters[MZ_RC_PLAYED_GAMES], next_game = r.counters[MZ_RC_NEXT_GAME], end_game = r.counters[MZ_RC_END_GAME];
     if (tid == 0) { active_count = 0; add_steps = 0; add_samples = 0; }
     // (1) thread t owns the contiguous slots [t*K, (t+1)*K): one exclusive scan over the CTA gives every finished slot its rank in slot
     //     order (= the order game numbers are handed out in) and every free slot its rank among the free ones
@@ -545,7 +571,7 @@ __global__ void __launch_bounds__(1024) mz_k_save_refill(const __grid_constant__
     long long steps = 0, samples = 0;
     for (int j = tid; j < total_fin; j += 1024) {
         const int g = s.fin_list[j];
-        const int64_t key = base_key + j + 1, pos = (key - 1) % r.capacity;
+        const int64_t key = base_key + j + 1, pos = mz_ring_pos(key, r.capacity);
         const int T = s.T[g];
         if (key > r.capacity) samples -= (long long)r.T[pos];              // evicted history (:156-160)
         r.game_id[pos] = s.game_id[g]; r.T[pos] = T; r.reanalysed[pos] = 0;
@@ -577,14 +603,16 @@ __global__ void __launch_bounds__(1024) mz_k_save_refill(const __grid_constant__
     __syncthreads();
     if (tid == 0) {
         const int64_t handed = !hand_out ? 0 : next_game + total_free < end_game ? total_free : (end_game - next_game > 0 ? end_game - next_game : 0);
-        r.counters[0] = base_key + total_fin;
-        r.counters[1] += add_steps;
-        r.counters[2] += add_samples;
-        r.counters[3] = next_game + handed;
-        r.counters[5] = active_count;
+        r.counters[MZ_RC_PLAYED_GAMES] = base_key + total_fin;
+        r.counters[MZ_RC_PLAYED_STEPS] += add_steps;
+        r.counters[MZ_RC_TOTAL_SAMPLES] += add_samples;
+        r.counters[MZ_RC_NEXT_GAME] = next_game + handed;
+        r.counters[MZ_RC_ACTIVE] = active_count;
         if (snap) {   // instead of a device-to-host copy between the kernels of every move (a copy-engine operation in the stream costs more than the kernel)
-            snap[0] = base_key + total_fin; snap[1] = r.counters[1]; snap[2] = r.counters[2]; snap[3] = next_game + handed; snap[4] = end_game; snap[5] = active_count;
-            snap[6] = r.counters[6]; snap[7] = r.counters[7];
+            snap[MZ_RC_PLAYED_GAMES] = base_key + total_fin; snap[MZ_RC_PLAYED_STEPS] = r.counters[MZ_RC_PLAYED_STEPS];
+            snap[MZ_RC_TOTAL_SAMPLES] = r.counters[MZ_RC_TOTAL_SAMPLES]; snap[MZ_RC_NEXT_GAME] = next_game + handed; snap[MZ_RC_END_GAME] = end_game;
+            snap[MZ_RC_ACTIVE] = active_count;
+            snap[MZ_RC_PER_TOTAL] = r.counters[MZ_RC_PER_TOTAL]; snap[MZ_RC_UNUSED] = r.counters[MZ_RC_UNUSED];
             __threadfence_system();
         }
     }
@@ -600,21 +628,21 @@ __global__ void __launch_bounds__(256) mz_k_save_copy(const __grid_constant__ mz
     const int rows = total_fin * P.Tmax;
     for (int idx = t0; idx < rows; idx += nthreads) {
         const int j = idx / P.Tmax, i = idx - j * P.Tmax;
-        const size_t so = (size_t)s.fin_list[j] * P.Tmax + i, ro = (size_t)((base_key + j) % r.capacity) * P.Tmax + i;
+        const size_t so = (size_t)s.fin_list[j] * P.Tmax + i, ro = (size_t)mz_ring_pos(base_key + j + 1, r.capacity) * P.Tmax + i;
         r.h_p1[ro] = s.h_p1[so]; r.h_p2[ro] = s.h_p2[so]; r.h_action[ro] = s.h_action[so]; r.h_reward[ro] = s.h_reward[so];
         r.h_to_play[ro] = s.h_to_play[so]; r.h_rv[ro] = s.h_rv[so];
     }
     const int row_cv = P.Tmax * P.A;
     for (int idx = t0; idx < total_fin * row_cv; idx += nthreads) {
         const int j = idx / row_cv, e = idx - j * row_cv;
-        r.h_cv[(size_t)((base_key + j) % r.capacity) * row_cv + e] = s.h_cv[(size_t)s.fin_list[j] * row_cv + e];
+        r.h_cv[(size_t)mz_ring_pos(base_key + j + 1, r.capacity) * row_cv + e] = s.h_cv[(size_t)s.fin_list[j] * row_cv + e];
     }
 }
 // initial priorities of the games just saved (save_game, ReplayBuffer.jl:136-145), from the stored histories
 __global__ void mz_k_save_per(const __grid_constant__ mz_params P, mz_slots s, mz_ring r, int n_slots) {
     const int total_fin = s.fin_list[n_slots];
     const int64_t base_key = reinterpret_cast<const int64_t *>(s.fin_list + MZ_FIN_KEY(n_slots))[0];
-    for (int j = blockIdx.x * blockDim.x + threadIdx.x; j < total_fin; j += gridDim.x * blockDim.x) mz_per_init_game(P, r, (base_key + j) % r.capacity);
+    for (int j = blockIdx.x * blockDim.x + threadIdx.x; j < total_fin; j += gridDim.x * blockDim.x) mz_per_init_game(P, r, mz_ring_pos(base_key + j + 1, r.capacity));
 }
 
 // ---- batched network callables (init_*(hyper) callables, src/Learning.jl:87-142) -------------------
@@ -676,7 +704,7 @@ __global__ void __launch_bounds__(MZ_THREADS) mz_k_reanalyse(const __grid_consta
         const int64_t item = (int64_t)blockIdx.x * MZ_ROWS + rr;
         float v = 0.0f;
         if (item < total) {
-            const int64_t pos = (a.key0 + item / P.Tmax - 1) % a.ring.capacity; const int t = (int)(item % P.Tmax);
+            const int64_t pos = mz_ring_pos(a.key0 + item / P.Tmax, a.ring.capacity); const int t = (int)(item % P.Tmax);
             if (t < a.ring.T[pos]) v = mz_stacked_value(P, a.ring.h_p1 + pos * P.Tmax, a.ring.h_p2 + pos * P.Tmax, a.ring.h_action + pos * P.Tmax, t + 1, k);
         }
         sp.in0[k * MZ_ROWS + rr] = v;
@@ -689,7 +717,7 @@ __global__ void __launch_bounds__(MZ_THREADS) mz_k_reanalyse(const __grid_consta
     __syncthreads();
     const int64_t item = (int64_t)blockIdx.x * MZ_ROWS + tid;
     if (tid < MZ_ROWS && item < total) {
-        const int64_t pos = (a.key0 + item / P.Tmax - 1) % a.ring.capacity; const int t = (int)(item % P.Tmax);
+        const int64_t pos = mz_ring_pos(a.key0 + item / P.Tmax, a.ring.capacity); const int t = (int)(item % P.Tmax);
         a.ring.h_rrv[pos * P.Tmax + t] = t < a.ring.T[pos] ? sp.outV[tid] : 0.0f;
         if (t == 0) a.ring.reanalysed[pos] = 1;
     }
@@ -700,7 +728,7 @@ __global__ void __launch_bounds__(MZ_THREADS) mz_k_reanalyse(const __grid_consta
 __global__ void mz_k_reanalyse_mark(const __grid_constant__ mz_params P, mz_ring r, int64_t key0, int n) {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= (int64_t)n * P.Tmax) return;
-    const int64_t pos = (key0 + i / P.Tmax - 1) % r.capacity; const int t = (int)(i % P.Tmax);
+    const int64_t pos = mz_ring_pos(key0 + i / P.Tmax, r.capacity); const int t = (int)(i % P.Tmax);
     if (t >= r.T[pos]) r.h_rrv[pos * P.Tmax + t] = 0.0f;
     if (t == 0) r.reanalysed[pos] = 1;
 }
@@ -743,7 +771,7 @@ __global__ void mz_k_history_export(const __grid_constant__ mz_params P, mz_ring
     int64_t per = (int64_t)P.Tmax * P.obs_size;
     if (i >= (int64_t)n * per) return;
     int j = (int)(i / per); int rem = (int)(i % per); int t = rem / P.obs_size, k = rem % P.obs_size;
-    int64_t pos = (key0 + j - 1) % r.capacity;
+    int64_t pos = mz_ring_pos(key0 + j, r.capacity);
     int Tg = r.T[pos];
     size_t ro = (size_t)pos * P.Tmax + t;
     mz_board b; b.p1 = r.h_p1[ro]; b.p2 = r.h_p2[ro]; b.player = 1;
@@ -764,7 +792,7 @@ __global__ void mz_k_history_import(const __grid_constant__ mz_params P, mz_ring
     int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n * P.Tmax) return;
     int j = i / P.Tmax, t = i % P.Tmax;
-    int64_t pos = (key0 + j - 1) % r.capacity;
+    int64_t pos = mz_ring_pos(key0 + j, r.capacity);
     size_t ro = (size_t)pos * P.Tmax + t, oo = (size_t)j * P.Tmax + t;
     uint64_t b1 = 0, b2 = 0;
     const float *o = obs + oo * P.obs_size;

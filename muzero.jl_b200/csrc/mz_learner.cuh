@@ -22,27 +22,27 @@ __global__ void __launch_bounds__(64) mz_k_replay_gather(const __grid_constant__
     const int b = blockIdx.x, tid = threadIdx.x, K1 = P.K + 1;
     if (b >= B) return;
     if (tid == 0) {
-        int64_t played = r.counters[0];
-        int64_t n_games = played < r.capacity ? played : r.capacity;
-        int64_t first_key = played - n_games + 1;
+        const mz_span span = mz_ring_span(r.counters[MZ_RC_PLAYED_GAMES], r.capacity);
+        int64_t n_games = span.n;
+        int64_t first_key = span.first;
         mz_u4 q = mz_philox(P.seed, MZ_STREAM_REPLAY, (uint32_t)step, (uint32_t)b, 0, 0);
         int64_t gi; int pos, T; int64_t key, ring;
         if (P.per) {   // sample_n_games :90-100 / sample_position :75-79 by priority: inverse CDF over the exact integer prefix sums
-            const unsigned long long Q = (unsigned long long)r.counters[6];
+            const unsigned long long Q = (unsigned long long)r.counters[MZ_RC_PER_TOTAL];
             const unsigned long long t = __umul64hi(((unsigned long long)q.x << 32) | q.z, Q);
             int64_t lo = 0, hi = n_games - 1;
             while (lo < hi) { int64_t mid = (lo + hi) >> 1; if (r.prefix[mid] > t) hi = mid; else lo = mid + 1; }
-            gi = lo; key = first_key + gi; ring = (key - 1) % r.capacity; T = r.T[ring];
+            gi = lo; key = first_key + gi; ring = mz_ring_pos(key, r.capacity); T = r.T[ring];
             const uint32_t *qp = r.q_pos + (size_t)ring * P.Tmax;
             unsigned long long Qg = 0; for (int i = 0; i < T; i++) Qg += qp[i];
             const unsigned long long t2 = __umul64hi(((unsigned long long)q.y << 32) | q.w, Qg);
             unsigned long long a2 = 0;
             for (pos = 1; pos < T; pos++) { a2 += qp[pos - 1]; if (a2 > t2) break; }
             const float game_prob = (float)((double)r.q_game[ring] / (double)Q), pos_prob = (float)((double)qp[pos - 1] / (double)Qg);
-            out.weights[b] = 1.0f / (((float)r.counters[2] * game_prob) * pos_prob);      // :213 (total_samples)
+            out.weights[b] = 1.0f / (((float)r.counters[MZ_RC_TOTAL_SAMPLES] * game_prob) * pos_prob);      // :213
         } else {
             gi = (int64_t)mz_u32_below(q.x, (uint32_t)n_games);
-            key = first_key + gi; ring = (key - 1) % r.capacity; T = r.T[ring];
+            key = first_key + gi; ring = mz_ring_pos(key, r.capacity); T = r.T[ring];
             pos = 1 + (int)mz_u32_below(q.y, (uint32_t)T);
         }
         s_pos = pos; s_T = T; s_ring = ring;
@@ -120,7 +120,7 @@ __global__ void __launch_bounds__(1024) mz_k_batch_roots(const __grid_constant__
     int32_t *keys = mz_smem_br, *uniq = mz_smem_br + Bp;
     __shared__ int buf[32];
     const int tid = threadIdx.x;
-    const int64_t played = r.counters[0], n_games = played < r.capacity ? played : r.capacity, first = played - n_games + 1;
+    const int64_t first = mz_ring_span(r.counters[MZ_RC_PLAYED_GAMES], r.capacity).first;
     for (int i = tid; i < Bp; i += 1024) keys[i] = i < B ? (int32_t)(index[2 * i] - first) : 0x7fffffff;   // key - first_key, padding last
     __syncthreads();
     for (int k = 2; k <= Bp; k <<= 1)
@@ -143,7 +143,7 @@ __global__ void __launch_bounds__(1024) mz_k_batch_roots(const __grid_constant__
     for (int i = i0; i < i1; i++) if (i == 0 || keys[i] != keys[i - 1]) uniq[o++] = keys[i];
     __syncthreads();
     for (int j = tid; j < D; j += 1024) {   // keys[] now holds the games' lengths; step 2
-        const int64_t pos = (first + uniq[j] - 1) % r.capacity;
+        const int64_t pos = mz_ring_pos(first + uniq[j], r.capacity);
         const int T = r.T[pos];
         keys[j] = T;
         for (int t = T; t < P.Tmax; t++) r.h_rrv[pos * P.Tmax + t] = 0.0f;
@@ -159,7 +159,7 @@ __global__ void __launch_bounds__(1024) mz_k_batch_roots(const __grid_constant__
         int at = base + mz_block_exscan(n, buf, &level);
         if (level == 0) break;           // lengths are at most Tmax: no game reaches a later move either
         for (int j = j0; j < j1; j++)
-            if (keys[j] > t) roots[at++] = ((first + uniq[j] - 1) % r.capacity) * P.Tmax + t;
+            if (keys[j] > t) roots[at++] = mz_ring_pos(first + uniq[j], r.capacity) * P.Tmax + t;
         base += level;
     }
     for (int k = tid; k < n_chunks; k += 1024) {   // step 4
